@@ -2,6 +2,7 @@
 """bench.py -- matched image pairs / second of the Matcher hot path (coarse match -> window gather -> fine match).
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path (one JSON line)
+    python bench.py [...] --dump-outputs DIR                      # also DIR/<name>.npy: the match lists of the last timed step
     python bench.py --impl reference [...]                        # the reference's CPU path (oracle port), rank 0 only
 
 Workload (BASELINE.json configs[1]): a batch of 64 synthetic 480x640 pairs per GPU per step -- coarse features
@@ -90,7 +91,13 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the robust / in_matcher / highres / retrieval / job blocks")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what rank 0's last timed step returned as DIR/<name>.npy, so that two "
+                         "builds can be compared output for output on the same seeded inputs (bench_outputs/ is ignored by git)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def measured_peaks():
@@ -131,6 +138,33 @@ def dram_traffic_from_profiles():
     except (OSError, ValueError, IndexError):
         return None, None, None
     return (coarse or None), (fine or None), os.path.relpath(TRAFFIC_CSV, ROOT)
+
+
+DUMP_KEYS = ("b_ids", "i_ids", "j_ids", "mconf", "mkpts0_c", "mkpts1_c", "expec_f", "mkpts0_f", "mkpts1_f")
+DUMP_MAX_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, res, max_bytes=DUMP_MAX_BYTES):
+    """Writes the match lists of one hot-path step (a capacity-sized `CoarseResult`) as out_dir/<name>.npy: the rows up to the
+    live match count, ids as float64 (exact), confidences and coordinates as float32, and `counts` (matches per pair, the
+    total, the flag word) as float64.  Should the rows need more than `max_bytes` in all, a fixed seeded sample of them is
+    written, in their order, with their indices in `rows.npy`."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    m = res.total()
+    out = {k: res[k][:m].cpu().numpy() for k in DUMP_KEYS}
+    out = {k: v.astype(np.float64 if v.dtype.kind in "iu" else np.float32) for k, v in out.items()}
+    counts = res["counts"].cpu().numpy().astype(np.float64)
+    row_bytes = sum(v[:1].nbytes for v in out.values()) + 8                 # + the row's index in rows.npy
+    budget = max_bytes - counts.nbytes - 128 * (len(out) + 2)              # (an .npy header takes 128 bytes)
+    if m * row_bytes > budget:
+        rows = np.sort(np.random.default_rng(0).choice(m, size=budget // row_bytes, replace=False))
+        out = {k: v[rows] for k, v in out.items()}
+        out["rows"] = rows.astype(np.float64)
+    out["counts"] = counts
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+    return sorted(out)
 
 
 class ClockSampler:
@@ -531,13 +565,13 @@ def main():
 
     def run_job(steps):
         """`steps` device-resident steps + the job's single gather, device-timed -> (ms max over ranks, records, sizes, my
-        checksum)"""
+        checksum, the last step's result)"""
         barrier()
         t_beg, t_end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         t_beg.record()
         runner.fork()
         for _ in range(steps):
-            step_device()
+            last = step_device()
         runner.join()
         my_sum = None
         if world > 1:
@@ -552,7 +586,7 @@ def main():
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             my_sum = job.checksum(totals=int(my_total.item()))
-        return float(t.item()), recs, sizes, my_sum
+        return float(t.item()), recs, sizes, my_sum, last
 
     def verify_gather(recs, sizes, my_sum, steps, m_step):
         """rank 0 holds every rank's live records: sizes = steps x matches per step of each rank (every rank runs the same
@@ -573,8 +607,10 @@ def main():
     clk.wait_first()
     run_job(max(args.warmup, 3))                         # warm-up: same code path as the timed region, gather included
     wall0 = time.time()
-    total_ms, recs, sizes, my_sum = run_job(args.steps)
+    total_ms, recs, sizes, my_sum, last = run_job(args.steps)
     wall1 = time.time()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
     ms_per_step = total_ms / args.steps
     value = world * n * args.steps / (total_ms / 1e3)
 
@@ -590,7 +626,7 @@ def main():
     # ---- the 4096-pair job of configs[4]: sharded over the ranks, one gather at the end ------------------------------
     job_block = None
     if job_steps > 0:
-        jms, jrecs, jsizes, jsum = run_job(job_steps)
+        jms, jrecs, jsizes, jsum, _ = run_job(job_steps)
         jver = verify_gather(jrecs, jsizes, jsum, job_steps, M) if world > 1 else None
         job_block = {"workload": f"{job_steps * n * world} synthetic pairs at 480x640 sharded over {world} GPU(s) in steps of {n} "
                                  f"pairs, one gather of the match lists at the end (BASELINE configs[4])",

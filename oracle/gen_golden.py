@@ -92,7 +92,7 @@ def main():
               f"{(data['mconf'].min().item() if data['mconf'].numel() else 0):.3f},"
               f"{(data['mconf'].max().item() if data['mconf'].numel() else 0):.3f}")
 
-    # ---- fine preprocess (window unfold + gather; with and without the coarse-feature Linears) -------
+    # ---- fine preprocess (window unfold + gather, without the coarse-feature Linears: gen_golden_fine_tf.py has those) ----
     case = COARSE_CASES["coarse_small"]
     f0, f1 = coarse_inputs(case)
     g = np.load(os.path.join(GOLDEN, "coarse_small.npz"))
@@ -103,17 +103,11 @@ def main():
     cfg_nocat = copy.deepcopy(cfg)
     cfg_nocat["fine_concat_coarse_feat"] = False
     w0, w1 = FinePreprocess(cfg_nocat).eval()(ff0, ff1, f0, f1, dict(data))
-    torch.manual_seed(5)
-    fp = FinePreprocess(copy.deepcopy(cfg)).eval()
-    m0, m1 = fp(ff0, ff1, f0, f1, dict(data))
-    keep = slice(0, 48)
+    keep = slice(0, 40)          # 40 of the 64 windows in full (the fixture stays below 1 MB), the sums of all of them
     np.savez_compressed(
         os.path.join(GOLDEN, "fine_preprocess.npz"),
-        meta=json.dumps(dict(coarse_case="coarse_small", fine_seed=21, weight_seed=5, kept=48)),
+        meta=json.dumps(dict(coarse_case="coarse_small", fine_seed=21, kept=40)),
         win0=w0[keep].numpy(), win1=w1[keep].numpy(), win0_sum=w0.sum((1, 2)).numpy(), win1_sum=w1.sum((1, 2)).numpy(),
-        merged0=m0[keep].numpy(), merged1=m1[keep].numpy(),
-        down_proj_w=fp.down_proj.weight.numpy(), down_proj_b=fp.down_proj.bias.numpy(),
-        merge_w=fp.merge_feat.weight.numpy(), merge_b=fp.merge_feat.bias.numpy(),
     )
     print(f"fine_preprocess: M={w0.shape[0]}")
 

@@ -1,6 +1,6 @@
-"""TEST INFRASTRUCTURE ONLY -- tests/golden/fine_transformer.npz from the UNMODIFIED reference.
+"""TEST INFRASTRUCTURE ONLY -- tests/golden/fine_transformer.npz and fine_merge_coarse.npz from the UNMODIFIED reference.
 
-    python oracle/gen_golden_fine_tf.py        (build container: /root/reference mounted)
+    POPE_REFERENCE_ROOT=<reference checkout> python oracle/gen_golden_fine_tf.py
 
 Runs the reference's own `LocalFeatureTransformer(config['fine'])` (src/matcher/loftr_module/transformer.py:61-106,
 d_model 128, 8 heads, layers ['self', 'cross'], linear attention) and `FinePreprocess` (fine_preprocess.py:8-59) with
@@ -84,14 +84,16 @@ def main():
     with torch.no_grad():                           # fine_preprocess.py:50-57 with the reference's own modules
         c_win = fp.down_proj(torch.cat([fc0[b_ids, i_ids], fc1[b_ids, j_ids]], 0))
         merged = fp.merge_feat(torch.cat([both, c_win[:, None, :].expand(-1, 25, -1)], -1))
-    out.update({"pre.meta": json.dumps(dict(n=n, L=L, S=S)), "pre.feat_c0": bf16_bits(fc0), "pre.feat_c1": bf16_bits(fc1),
-                "pre.b_ids": b_ids.numpy(), "pre.i_ids": i_ids.numpy(), "pre.j_ids": j_ids.numpy(),
-                "pre.merged0": merged[:KEPT].numpy(), "pre.merged1": merged[M_WINDOWS:M_WINDOWS + KEPT].numpy(),
-                "pre.merged_sum": merged.sum((1, 2)).numpy()})
+    pre = {"pre.meta": json.dumps(dict(n=n, L=L, S=S)), "pre.feat_c0": bf16_bits(fc0), "pre.feat_c1": bf16_bits(fc1),
+           "pre.b_ids": b_ids.numpy(), "pre.i_ids": i_ids.numpy(), "pre.j_ids": j_ids.numpy(),
+           "pre.merged0": merged[:KEPT].numpy(), "pre.merged1": merged[M_WINDOWS:M_WINDOWS + KEPT].numpy(),
+           "pre.merged_sum": merged.sum((1, 2)).numpy()}
     for k, v in fp.state_dict().items():
-        out["pre." + k] = bf16_bits(v) if v.dim() > 1 else v.numpy()
-    np.savez_compressed(os.path.join(GOLDEN, "fine_transformer.npz"), **out)
-    print("fine_transformer.npz:", {k: getattr(v, "shape", None) for k, v in out.items() if not k.endswith("meta")})
+        pre["pre." + k] = bf16_bits(v) if v.dim() > 1 else v.numpy()
+    # two files, each below 1 MB; the Linears' fixture shares the inputs (`meta`) of the transformer's
+    for name, arrays in (("fine_transformer.npz", out), ("fine_merge_coarse.npz", pre)):
+        np.savez_compressed(os.path.join(GOLDEN, name), **arrays)
+        print(name + ":", {k: getattr(v, "shape", None) for k, v in arrays.items() if not k.endswith("meta")})
 
 
 if __name__ == "__main__":

@@ -32,10 +32,11 @@ def test_state_dict_layout_of_vit_small():
     assert m.pos_embed.shape == (1, 37 * 37 + 1, 384) and sum(p.numel() for p in m.parameters()) == 22_056_576
 
 
-@pytest.mark.skipif(not ref_shim.reference_available(), reason="/root/reference not mounted")
+@pytest.mark.skipif(not ref_shim.reference_available(),
+                    reason="needs the unmodified reference sources (POPE_REFERENCE_ROOT), which are not part of this repository")
 def test_dino_vit_equals_reference_module():
-    if "/root/reference" not in sys.path:
-        sys.path.insert(0, "/root/reference")
+    if ref_shim.REFERENCE_ROOT not in sys.path:
+        sys.path.insert(0, ref_shim.REFERENCE_ROOT)
     from dinov2.dinov2.models.vision_transformer import vit_small   # the reference's own class, unmodified
     torch.manual_seed(1)
     ref = vit_small(patch_size=14, img_size=518, init_values=1.0, block_chunks=0).eval()

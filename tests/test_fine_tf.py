@@ -1,7 +1,7 @@
 """Fine-level transformer + FinePreprocess Linears (SURVEY.md 8(f) rank 1).
 
-CPU: the oracle restatement (oracle/pope_oracle.py: fine_transformer, fine_merge_coarse) against the fixture produced by
-the UNMODIFIED reference (oracle/gen_golden_fine_tf.py).  GPU: the bf16 CUDA path (pope_fine_transformer /
+CPU: the oracle restatement (oracle/pope_oracle.py: fine_transformer, fine_merge_coarse) and the Matcher's `loftr_fine`
+module against the fixture produced by the UNMODIFIED reference (oracle/gen_golden_fine_tf.py).  GPU: the bf16 CUDA path (pope_fine_transformer /
 pope_fine_merge_coarse through the C ABI) against the same fixture and against the oracle on other shapes.
 
 Tolerance of the bf16 path: weights and inputs are bf16 on both sides, but the CUDA path also rounds every activation
@@ -18,7 +18,7 @@ import torch
 
 from oracle import pope_oracle as O
 
-GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "fine_transformer.npz")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def _bf16(bits: np.ndarray) -> torch.Tensor:
@@ -26,18 +26,20 @@ def _bf16(bits: np.ndarray) -> torch.Tensor:
 
 
 def _load():
-    g = np.load(GOLDEN)
+    g = {}
+    for name in ("fine_transformer.npz", "fine_merge_coarse.npz"):      # the transformer's fixture, the Linears' (`pre.`)
+        g.update(np.load(os.path.join(GOLDEN, name)))
     meta = json.loads(str(g["meta"]))
     layers = []
     for l in range(len(meta["layer_names"])):
         sd = {}
-        for k in g.files:
+        for k in g:
             pre = f"tf.layers.{l}."
             if k.startswith(pre):
                 sd[k[len(pre):]] = _bf16(g[k]) if g[k].dtype == np.uint16 else torch.from_numpy(g[k])
         layers.append(sd)
     pre_sd = {k[4:]: (_bf16(g[k]) if g[k].dtype == np.uint16 else torch.from_numpy(g[k]))
-              for k in g.files if k.startswith("pre.") and ("weight" in k or "bias" in k)}
+              for k in g if k.startswith("pre.") and ("weight" in k or "bias" in k)}
     return g, meta, layers, pre_sd
 
 
@@ -59,6 +61,25 @@ def test_oracle_fine_transformer_matches_reference_fixture():
     g, meta, layers, _ = _load()
     f0, f1 = _inputs(meta["input_seed"], meta["m"])
     o0, o1 = O.fine_transformer(f0, f1, layers, meta["layer_names"])
+    k = meta["kept"]
+    assert torch.allclose(o0[:k], torch.from_numpy(g["out0"]), rtol=1e-5, atol=2e-5)
+    assert torch.allclose(o1[:k], torch.from_numpy(g["out1"]), rtol=1e-5, atol=2e-5)
+    assert torch.allclose(o0.sum((1, 2)), torch.from_numpy(g["out0_sum"]), rtol=1e-4, atol=1e-2)
+    assert torch.allclose(o1.sum((1, 2)), torch.from_numpy(g["out1_sum"]), rtol=1e-4, atol=1e-2)
+
+
+def test_fine_transformer_module_matches_reference_fixture():
+    """The Matcher's own `loftr_fine` (stock PyTorch layers for fp32 input), loaded with the reference's weights through the
+    state-dict layout, reproduces the reference's outputs."""
+    import pope_b200
+    g, meta, _, _ = _load()
+    m = pope_b200.Matcher(pope_b200.make_default_cfg()).eval()
+    sd = {k[3:]: (_bf16(v) if v.dtype == np.uint16 else torch.from_numpy(v)) for k, v in g.items() if k.startswith("tf.")}
+    m.loftr_fine.load_state_dict(sd, strict=True)
+    assert m.loftr_fine.layer_names == meta["layer_names"]
+    f0, f1 = _inputs(meta["input_seed"], meta["m"])
+    with torch.no_grad():
+        o0, o1 = m.loftr_fine(f0, f1)
     k = meta["kept"]
     assert torch.allclose(o0[:k], torch.from_numpy(g["out0"]), rtol=1e-5, atol=2e-5)
     assert torch.allclose(o1[:k], torch.from_numpy(g["out1"]), rtol=1e-5, atol=2e-5)

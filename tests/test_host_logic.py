@@ -178,6 +178,36 @@ def test_bench_reads_the_committed_ncu_table(tmp_path, monkeypatch):
     assert bench.dram_traffic_from_profiles() == (None, None, None)
 
 
+def test_bench_dump_outputs_writes_the_live_rows(tmp_path):
+    """`bench.py --dump-outputs`: the rows up to the live count of a capacity-sized result, ids exact in float64, the rest
+    float32; over the byte budget, the same seeded sample of rows on every call, within the budget."""
+    import numpy as np
+    import bench
+    from pope_b200 import ops
+    cap, n, m = 1000, 3, 700
+    g = torch.Generator().manual_seed(0)
+    res = ops.CoarseResult(n_pairs=n, counts=torch.tensor([300, 0, 400, m, 0], dtype=torch.int32))
+    for k in ("b_ids", "i_ids", "j_ids"):
+        res[k] = torch.randint(0, 4800, (cap,), generator=g) + (1 << 40)
+    for k, w in (("mconf", 0), ("mkpts0_c", 2), ("mkpts1_c", 2), ("expec_f", 3), ("mkpts1_f", 2)):
+        res[k] = torch.randn((cap, w) if w else (cap,), generator=g)
+    res["mkpts0_f"] = res["mkpts0_c"]
+    names = bench.dump_outputs(str(tmp_path / "all"), res)
+    assert names == sorted(bench.DUMP_KEYS + ("counts",))
+    for k in bench.DUMP_KEYS:
+        a = np.load(tmp_path / "all" / f"{k}.npy")
+        assert a.dtype == (np.float64 if k.endswith("_ids") else np.float32) and a.shape[0] == m, k
+        assert np.array_equal(a, res[k][:m].numpy().astype(a.dtype)), k
+    assert np.load(tmp_path / "all" / "counts.npy").tolist() == [300, 0, 400, m, 0]
+    budget = 20_000
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), res, max_bytes=budget)
+    rows = np.load(tmp_path / "a" / "rows.npy")
+    assert 0 < rows.size < m and np.all(np.diff(rows) > 0) and np.array_equal(rows, np.load(tmp_path / "b" / "rows.npy"))
+    assert np.array_equal(np.load(tmp_path / "a" / "i_ids.npy"), res["i_ids"][rows.astype(np.int64)].numpy().astype(np.float64))
+    assert sum(os.path.getsize(p) for p in (tmp_path / "a").iterdir()) <= budget
+
+
 def test_union_fetch_cover_rule():
     """The host pipeline's union fetch (csrc/pipeline.cu::fetch_union_kernel) copies a fine-map pixel iff it lies in the WxW
     window (stride `stride`, zero padding W//2: fine_preprocess.py:40-43) of at least one matched coarse cell.  The kernel

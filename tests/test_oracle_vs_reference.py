@@ -1,5 +1,6 @@
-"""Live cross-checks against the UNMODIFIED reference (only where /root/reference is mounted, i.e. the build
-container; skipped on the GPU box).  CPU only."""
+"""Live cross-checks against the UNMODIFIED reference, where its sources are present (POPE_REFERENCE_ROOT); skipped
+elsewhere.  Its recorded outputs under tests/golden are checked everywhere (test_oracle_golden.py, test_fine_tf.py,
+test_coarse_masked.py, test_host_logic.py).  CPU only."""
 import contextlib
 import copy
 import io
@@ -11,7 +12,8 @@ from oracle import pope_oracle as O
 from oracle import ref_shim
 from pope_b200 import synth
 
-pytestmark = pytest.mark.skipif(not ref_shim.reference_available(), reason="/root/reference not mounted")
+pytestmark = pytest.mark.skipif(not ref_shim.reference_available(),
+                                reason="needs the unmodified reference sources (POPE_REFERENCE_ROOT), which are not part of this repository")
 
 
 @pytest.fixture(scope="module")
