@@ -206,13 +206,6 @@ int pope_match_pairs_host(const void* feat_c0, const void* feat_c1, const void* 
                           int64_t* i_ids, int64_t* j_ids, float* mconf, float* mkpts0_f, float* mkpts1_f,
                           int32_t* counts, int32_t* flags);
 
-/* Developer diagnostics (not part of the drop-in surface).  With the environment variable POPE_TC_TRACE=<0|2> the
- * tcgen05 row (0) / column (2) sweep of CTA pair 0 records clock64() stamps per tile: 8 x u64 per tile, 512 MMA-issuer
- * records (before / after the accumulator-empty wait, after the first operand wait, after the last MMA issue) followed
- * by 512 epilogue-warp records (before / after the accumulator-full wait, after the TMEM hand-back, end of tile).
- * Copies them to `out` (host); returns the number of u64 written, 0 when tracing is off.  tools/trace_sweep.py. */
-int pope_debug_trace_read(unsigned long long* out, int max_u64);
-
 /* Match-list consumer of the eval loop (eval_linemod_json.py:118-119 `np.where(confidences > 0.9)` per crop and :146
  * `np.argmax(matching_score)` per query; SURVEY.md 8(f) rank 3, selection part), without copying the lists to the host:
  *   scores[p] = #{matches of pair p with mconf > thr};  best[g] = first arg-max of scores over the `group` consecutive

@@ -9,8 +9,7 @@ from typing import Optional
 import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# POPE_B200_LIB: developer override (experiment builds of tools/build_variant.sh); the product library is the in-tree one
-LIB_PATH = os.environ.get("POPE_B200_LIB") or os.path.join(_HERE, "libpope_b200.so")
+LIB_PATH = os.path.join(_HERE, "libpope_b200.so")
 
 POPE_F32, POPE_BF16 = 0, 1
 COARSE_AUTO, COARSE_SIMT, COARSE_TCGEN05 = 0, 1, 2
@@ -57,7 +56,6 @@ SIGNATURES = {
                                       _p, _p, _p, _p, _sz, _p]),
     "pope_running_topk": (_i, [_p, _i, _i, _p, _p, _p]),
     "pope_cosine_topk": (_i, [_p, _p, _i, _i, _i, _i, _f, _p, _p, _p, _p]),
-    "pope_debug_trace_read": (_i, [_p, _i]),
     "pope_pipeline_create": (_i, [C.POINTER(_p), _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _f, _f, _f, _f, _i, _i]),
     "pope_pipeline_run": (_i, [_p, _p, _p, _p, _p, _i, _p, _p, _p, _p, _p, _p, _p]),
     "pope_pipeline_destroy": (_i, [_p]),

@@ -84,10 +84,7 @@ extern "C" int pope_coarse_match(const void* feat_c0, const void* feat_c1, int d
 
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   cudaError_t e;
-  // clear the best-candidate records, candidate counters and "count published" words (adjacent; the single-sweep
-  // tcgen05 sequence clears / writes them all itself) and the total/flag words
-  if (!use_split && (!use_tc || coarse_tc_needs_clear(p)))
-    if ((e = cudaMemsetAsync(w.rowbest, 0, w.zero_bytes, st)) != cudaSuccess) return int(e);
+  // clear the total/flag words (each launch sequence clears the scratch it needs cleared itself)
   if ((e = cudaMemsetAsync(counts + n_pairs, 0, 2 * sizeof(int32_t), st)) != cudaSuccess) return int(e);
   if (use_split) {
     // single sweep on the split planes, then the fp32-FMA kernels as a gated fallback (no-ops unless the flag was raised)

@@ -205,6 +205,8 @@ cudaError_t run_typed(const CoarseProblem& p, const CoarseScratch& w, int32_t* f
   if (gated) {
     if (!two_sweeps_possible(p)) return cudaErrorInvalidValue;     // the gated form exists for the two-sweep scheme only
     if ((e = gated_clear_run(w.rowbest, w.zero_bytes, gate, st)) != cudaSuccess) return e;
+  } else if ((e = cudaMemsetAsync(w.rowbest, 0, w.zero_bytes, st)) != cudaSuccess) {
+    return e;
   }
   rowlse_simt_kernel<T, false><<<gr, NT, 0, st>>>(f0, f1, p.L, p.S, p.C, p.scale_log2, w.lse_r, nullptr, nullptr, nullptr, nullptr,
                                                   gate);

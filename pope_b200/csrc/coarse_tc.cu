@@ -62,20 +62,9 @@ constexpr int kEpiThreads = kEpiWarps * 32;
 // per thread; the data-movement warps need a fraction of that, the epilogue is short of registers at 96)
 constexpr int kWarpProducer = kEpiWarps, kWarpMma = kEpiWarps + 1;
 constexpr int kThreads = kEpiThreads + 128;
-#ifndef POPE_VAR_LOADBOTH
-#define POPE_VAR_LOADBOTH 0        // 1: single sweep loads both chunks of a tile before any arithmetic
-#endif
-#ifndef POPE_VAR_REGS_EPI
-#define POPE_VAR_REGS_EPI 112
-#define POPE_VAR_REGS_AUX 32
-#endif
-constexpr int kRegsEpi = POPE_VAR_REGS_EPI, kRegsAux = POPE_VAR_REGS_AUX;
+constexpr int kRegsEpi = 112, kRegsAux = 32;
 static_assert(16 * 32 * kRegsEpi + 4 * 32 * kRegsAux <= 640 * 96, "setmaxnreg would wait for registers the CTA does not own");   // 16 x 32 x 112 + 4 x 32 x 32 = 61 440 = the CTA's 640 x 96 registers (the pool is per CTA)
 constexpr uint32_t kTmemCols = 512;
-constexpr bool kLoadAll = (kEpiWarps == 8);          // all chunks TMEM -> registers before any arithmetic (needs the
-                                                     // 204-register budget of the 8-warp layout; spills with 16 warps)
-constexpr bool kPolyExp = false;                     // every 4th exp2 on the FMA pipe (measured slower: +2.5 instr/element)
-constexpr int kTraceTiles = 512;                      // developer diagnostics: tiles of CTA pair 0 that get clock stamps
 constexpr uint32_t kPeerMask = 0xFEFFFFFFu;          // clears the CTA-rank bit of a shared::cluster address -> leader CTA
 
 // dynamic shared memory layout (base aligned to 1024 B for the 128B swizzle); identical in both CTAs of a pair
@@ -98,10 +87,6 @@ __device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
 __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
-// Experiment switches of the developer builds (tools/build_variant.sh); the defaults are the product configuration.
-#ifndef POPE_VAR_WAIT_HINT
-#define POPE_VAR_WAIT_HINT 0          // > 0: suspend-time hint (ns) of the epilogue's accumulator wait
-#endif
 __device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity) {
   uint32_t ok;
   asm volatile(
@@ -111,16 +96,6 @@ __device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity) {
       : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
   return ok != 0;
 }
-// the same with a suspend-time hint: the warp may sleep up to `ns` inside the instruction instead of polling
-__device__ __forceinline__ bool mbar_try_wait_hint(uint32_t bar, uint32_t parity, uint32_t ns) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok) : "r"(bar), "r"(parity), "r"(ns) : "memory");
-  return ok != 0;
-}
 __device__ __forceinline__ long long clock_now() {
   long long t;
   asm volatile("mov.u64 %0, %%clock64;" : "=l"(t)::"memory");
@@ -128,14 +103,13 @@ __device__ __forceinline__ long long clock_now() {
 }
 // Bounded wait: a protocol bug must become a launch failure, never a hung GPU.  The clock is only read every 1024 polls
 // (read on every poll, the nine instructions of the time-out test were a fifth of all instructions the sweep issued).
-template <int HINT = 0>
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  if (HINT > 0 ? mbar_try_wait_hint(bar, parity, HINT) : mbar_try_wait(bar, parity)) return;
+  if (mbar_try_wait(bar, parity)) return;
   long long t0 = 0;
   for (;;) {
 #pragma unroll 1
     for (int k = 0; k < 1024; ++k)
-      if (HINT > 0 ? mbar_try_wait_hint(bar, parity, HINT) : mbar_try_wait(bar, parity)) return;
+      if (mbar_try_wait(bar, parity)) return;
     const long long t = clock_now();
     if (t0 == 0) t0 = t;
     else if (t - t0 > 4000000000ll) __trap();     // ~2 s at 2 GHz
@@ -242,8 +216,6 @@ struct SweepParams {
   int gate;                 // != 0: the launch is a no-op unless POPE_FLAG_ROBUST_PATH is set in *flags, and then only
                             //       the pairs with pairflag[n] != 0 are swept
   int32_t* flags;
-  unsigned long long* trace;   // developer diagnostics (POPE_TC_TRACE): clock stamps of CTA pair 0, or nullptr
-  int debug;                // developer knob (env POPE_TC_DEBUG): bit0 = epilogue does no math, bit1 = no rare path, bit3 = force three sweeps, bit4 = no single sweep, bit5 = single sweep without the per-cell candidate scan, bit7 = single sweep without the shared-memory row-bound exchange, bit9 = no candidate levels 2/3 in a unit's first tile (timing only: drops its candidates), bit10 = single sweep as one launch (no head / tail split), bits 11.. = the epilogue warp POPE_TC_TRACE stamps, bit6 = no gated redo after the single sweep
 };
 
 __device__ __forceinline__ float4 lds128(uint32_t addr) {
@@ -263,21 +235,6 @@ __device__ __forceinline__ float tmem_ld1(uint32_t taddr) {
   uint32_t r;
   asm volatile("tcgen05.ld.sync.aligned.32x32b.x1.b32 {%0}, [%1];\n\ttcgen05.wait::ld.sync.aligned;" : "=r"(r) : "r"(taddr) : "memory");
   return __uint_as_float(r);
-}
-
-// 2^x for x <= 0 on the FMA/ALU pipes (Cody-Waite split + degree-4 minimax polynomial, max rel. error 2.7e-6): one
-// element in four goes this way so that the MUFU pipe (16 ex2/clk/SM, exactly the MMA rate at one exponential per
-// accumulator element) is no longer the co-bottleneck of the log-sum-exp sweeps.
-__device__ __forceinline__ float ex2_poly(float x) {
-  x = fmaxf(x, -125.f);
-  const float t = x + 12582912.f;                 // 1.5 * 2^23: the integer part of x lands in the low mantissa bits
-  const float f = x - (t - 12582912.f);           // [-0.5, 0.5]
-  float p = 0.009570101276040077f;
-  p = fmaf(p, f, 0.05591785907745361f);
-  p = fmaf(p, f, 0.240247443318367f);
-  p = fmaf(p, f, 0.6931217908859253f);
-  p = fmaf(p, f, 0.9999992847442627f);
-  return __int_as_float(__float_as_int(p) + (__float_as_int(t) << 23));
 }
 
 // online log-sum-exp update of one row with 32 more raw accumulators (vc of them valid)
@@ -304,7 +261,7 @@ __device__ __forceinline__ float lse_update(const float (&v)[32], int vc, float 
       a0 += ex2_approx(fmaf(v[j + 0], scale, neg));
       a1 += ex2_approx(fmaf(v[j + 1], scale, neg));
       a2 += ex2_approx(fmaf(v[j + 2], scale, neg));
-      a3 += kPolyExp ? ex2_poly(fmaf(v[j + 3], scale, neg)) : ex2_approx(fmaf(v[j + 3], scale, neg));
+      a3 += ex2_approx(fmaf(v[j + 3], scale, neg));
     }
   } else {
 #pragma unroll
@@ -496,8 +453,7 @@ __device__ __forceinline__ float ss_col_reduce(const float (&cp)[8], int lane) {
 //         TMEM -- 6x the MMAs of MODE 3, which hides the epilogue completely.  The a1 and a2 blocks of the unit stay
 //         resident (128 KB), a3 and the b planes stream through a 5-stage ring.  maps: map0..2 = planes of f0,
 //         map3..5 = planes of f1.
-// TRACE: developer diagnostics instantiation (clock stamps of CTA pair 0); the product launches use TRACE = false.
-template <int MODE, bool TRACE>
+template <int MODE>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
 sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant__ CUtensorMap map1,
                 const __grid_constant__ CUtensorMap map2, const __grid_constant__ CUtensorMap map3,
@@ -529,7 +485,7 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
   volatile uint32_t* tmem_ptr_smem = reinterpret_cast<volatile uint32_t*>(smem + kSmemTmemPtr);
 
   // (a kernel launched behind this one WITH programmatic stream serialisation may start while this one runs: the column
-  //  merge of the head of a split single sweep, coarse_tc_run; ordinary launches are not affected)
+  //  merge of the head of a split single sweep, single_sweep_run; ordinary launches are not affected)
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
   if (P.gate && !(uint32_t(*reinterpret_cast<const volatile int32_t*>(P.flags)) & POPE_FLAG_ROBUST_PATH)) return;
   // (volatile read: the compiler otherwise re-derives lane bits from SR_TID.X inside the epilogue loops, ~6 S2R per chunk)
@@ -634,11 +590,7 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
         };
         for (int ct = 0; ct < ntiles; ++ct, ++tile_ctr) {
           const uint32_t s = tile_ctr & 1, acc_phase = (tile_ctr >> 1) & 1;
-          const bool tr = TRACE && P.trace && pair == 0 && tile_ctr < kTraceTiles && lane == 0;
-          unsigned long long* rec = P.trace + size_t(tile_ctr) * 8;
-          if (tr) rec[0] = clock64() | ((unsigned long long)(ct == 0) << 63);   // top bit: first tile of a unit
           mbar_wait(bar_acc_empty + 8 * s, acc_phase ^ 1);
-          if (tr) rec[1] = clock64();
           tc_fence_after();
           const uint32_t d = tmem_base + s * kTileCols;
           if (MODE == 4) {
@@ -692,7 +644,6 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
           for (int kc = 0; kc < kchunks; ++kc) {
             a_wait(ct, kc);
             mbar_wait(bar_b_full + 8 * b_stage, b_phase);
-            if (tr && kc == 0) rec[2] = clock64();
             tc_fence_after();
             const uint32_t a_addr = sbase + kSmemA + kc * kBoxBytes;
             const uint32_t b_addr = sbase + kSmemB + b_stage * kBoxBytes;
@@ -703,11 +654,9 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
               umma_commit_2sm(bar_b_empty + 8 * b_stage);  // ring slot free in both CTAs once these MMAs have read it
             }
             a_done(ct, kc);
-            if (tr && kc < 4) rec[4 + kc] = clock64();    // this chunk's four MMAs and its commit are issued
             if (++b_stage == kStages) { b_stage = 0; b_phase ^= 1; }
           }
           if (elect_one()) umma_commit_2sm(bar_acc_full + 8 * s);         // accumulator stage complete (both CTAs' epilogues)
-          if (tr) rec[3] = clock64();
         }
         a_phase ^= 1;
       }
@@ -791,19 +740,11 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
         const uint32_t s = tile_ctr & 1, acc_phase = (tile_ctr >> 1) & 1;
         const int col0 = ct * kTileCols;
         const int nvalid = min(LB - col0, kTileCols) - colofs;
-        const bool active = rows_valid > 0 && nvalid > 0 && !(P.debug & 1);
-        // developer diagnostics: epilogue warp POPE_TC_TRACE_WARP (default 0) of CTA pair 0, leader CTA
-        const bool etr = TRACE && P.trace && pair == 0 && rank == 0 && warp == (P.debug >> 11) && lane == 0 && tile_ctr < kTraceTiles;
-        unsigned long long* erec = P.trace + size_t(kTraceTiles + tile_ctr) * 8;
-        if (etr) erec[0] = clock64();
-        mbar_wait<POPE_VAR_WAIT_HINT>(bar_acc_full + 8 * s, acc_phase);
-        if (etr) erec[1] = clock64();
+        const bool active = rows_valid > 0 && nvalid > 0;
+        mbar_wait(bar_acc_full + 8 * s, acc_phase);
         tc_fence_after();
         const uint32_t tbase = tb0 + s * kTileCols;
         float v[32];
-#if POPE_VAR_LOADBOTH
-        float v2[32];
-#endif
         auto process = [&](float (&v)[32], int cc) {
           const int vc = nvalid - cc * 32;
           const int colb = col0 + colofs + cc * 32;
@@ -864,20 +805,19 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
             rowacc[rho] += d[rho];
             pass |= d[rho] > fmaf(thrm, rowacc[rho], tb[rho]);
           }
-          if (__any_sync(kFullMask, pass) && !(P.debug & 2) && !((P.debug & 512) && ct == 0)) {       // (one vote per chunk on the common path)
+          if (__any_sync(kFullMask, pass)) {       // (one vote per chunk on the common path)
 #pragma unroll
             for (int rho = 0; rho < 4; ++rho) {
               if (!__any_sync(kFullMask, d[rho] > fmaf(thrm, rowacc[rho], tb[rho]))) continue;
               float rs = rowacc[rho];
               rs += __shfl_xor_sync(kFullMask, rs, 1);
               rs += __shfl_xor_sync(kFullMask, rs, 2);
-              const float other = (P.debug & 128) ? 0.f : ex2_approx(lds32(rowbnd_addr + 32 * rho) - (kBndBias + mshift));
+              const float other = ex2_approx(lds32(rowbnd_addr + 32 * rho) - (kBndBias + mshift));
               const float bound = thrm * fmaxf(rs, other);
               tb[rho] = fmaxf(tb[rho], fmaf(-thrm, rowacc[rho], bound));
-              if (p == 0 && fabsf(mshift) < 0.5f * kBndBias && !(P.debug & 128))     // (explicit shared-space reduction: through the
-                red_max_shared(rowbnd_addr + 32 * rho,                              //  generic pointer it compiled to ATOM.E...GPU)
+              if (p == 0 && fabsf(mshift) < 0.5f * kBndBias)     // (explicit shared-space reduction: through the
+                red_max_shared(rowbnd_addr + 32 * rho,          //  generic pointer it compiled to ATOM.E...GPU)
                                __float_as_int(lg2_approx(rs) + (mshift + kBndBias - 0.004f)));
-              if (P.debug & 32) continue;
               const int i0 = 16 * (rho >> 1) + 2 * (rho & 1);
               const float e0 = v[i0], e1 = v[i0 + 1], e2 = v[i0 + 4], e3 = v[i0 + 5], e4 = v[i0 + 8], e5 = v[i0 + 9],
                           e6 = v[i0 + 12], e7 = v[i0 + 13];
@@ -900,16 +840,6 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
             }
           }
         };
-#if POPE_VAR_LOADBOTH
-        // both chunks in registers first, the TMEM stage handed back before any arithmetic
-        if (active) tmem_ld_frag(tbase, v);
-        if (active && nvalid > 32) tmem_ld_frag(tbase + 32, v2);
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive_leader(bar_acc_empty + 8 * s);
-        if (active) process(v, 0);
-        if (active && nvalid > 32) process(v2, 1);
-#else
         if (active) {
           tmem_ld_frag(tbase, v);
           process(v, 0);
@@ -918,10 +848,7 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive_leader(bar_acc_empty + 8 * s);
-        if (etr) erec[2] = clock64();
         if (active && nvalid > 32) process(v, 1);
-        if (etr) erec[3] = clock64();
-#endif
         cp_ptr += kTileCols;
         cs_ptr += kTileCols / 32;
       }
@@ -1028,11 +955,7 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
           }
           asm volatile("bar.sync 1, %0;" ::"n"(kEpiThreads) : "memory");
         }
-        const bool etr = TRACE && P.trace && pair == 0 && rank == 0 && warp == 0 && lane == 0 && tile_ctr < kTraceTiles;
-        unsigned long long* erec = P.trace + size_t(kTraceTiles + tile_ctr) * 8;
-        if (etr) erec[0] = clock64();
         mbar_wait(bar_acc_full + 8 * s, acc_phase);
-        if (etr) erec[1] = clock64();
         tc_fence_after();
         const uint32_t tbase = tmem_base + lane_addr + s * kTileCols + colq * kSpan;
         const int nvalid = min(LB - col0, kTileCols) - colq * kSpan;   // valid columns from this thread's first one
@@ -1041,7 +964,7 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
 #pragma unroll 1
           for (int cc = 0; cc < kChunks; ++cc) {
             const int vc = nvalid - cc * 32;
-            if (vc <= 0 || (P.debug & 1)) break;
+            if (vc <= 0) break;
             float v[32];
             tmem_ld32(tbase + cc * 32, v);
             const uint32_t lb = sbase + kSmemLc + (s * kTileCols + colq * kSpan + cc * 32) * 4;
@@ -1051,7 +974,7 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
               const float4 l4 = lds128(lb + j4 * 4);
               any |= (v[j4 + 0] > lrp + l4.x) | (v[j4 + 1] > lrp + l4.y) | (v[j4 + 2] > lrp + l4.z) | (v[j4 + 3] > lrp + l4.w);
             }
-            if (__any_sync(kFullMask, any) && !(P.debug & 2)) {
+            if (__any_sync(kFullMask, any)) {
               uint32_t mask = 0;
 #pragma unroll
               for (int j = 0; j < 32; ++j) mask |= (v[j] > lrp + lds32(lb + j * 4)) ? (1u << j) : 0u;
@@ -1083,7 +1006,7 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
             // per-element scan runs only for the threads whose chunk maximum passes (the row's match, typically once).
             const float b = (m_run + lg2_approx(s_run) + P.log2_thr) * inv_scale;
             const float bound = isfinite(b) ? b - (1e-5f * fabsf(b) + 0.005f * inv_scale) : INFINITY;
-            if (cmax > bound && !(P.debug & 2)) {
+            if (cmax > bound) {
               const int colb = col0 + colq * kSpan + cc * 32;
 #pragma unroll
               for (int j = 0; j < 32; ++j)
@@ -1091,43 +1014,21 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
                   list_cnt = list_push<kCandSlots>(mylist, list_cnt, bound * scale, v[j] * scale, colb + j, P.flags, nullptr);
             }
           };
-          const bool skip = (P.debug & 1) != 0;
-          if (kLoadAll) {
-            // every chunk of the thread is pulled into registers first, the stage is handed back, then all arithmetic
-            float v[kChunks][32];
-#pragma unroll
-            for (int cc = 0; cc < kChunks; ++cc)
-              if (nvalid - cc * 32 > 0 && !skip) tmem_ld32(tbase + cc * 32, v[cc]);
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive_leader(bar_acc_empty + 8 * s);
-#pragma unroll
-            for (int cc = 0; cc < kChunks; ++cc) {
-              const int vc = nvalid - cc * 32;
-              if (vc > 0 && !skip) {
-                const float cmax = lse_update(v[cc], vc, scale, m_run, s_run);
-                if (listing) scan(v[cc], cc, vc, cmax);
-              }
-            }
-          } else {
-            static_assert(kLoadAll || kChunks == 2, "the chunk-by-chunk epilogue is written for two chunks per thread");
-            const int vc0 = nvalid, vc1 = nvalid - 32;
-            float v[32];
-            if (vc0 > 0 && !skip) {
-              tmem_ld32(tbase, v);
-              const float cmax = lse_update(v, vc0, scale, m_run, s_run);
-              if (listing) scan(v, 0, vc0, cmax);
-            }
-            if (vc1 > 0 && !skip) tmem_ld32(tbase + 32, v);
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive_leader(bar_acc_empty + 8 * s);
-            if (etr) erec[2] = clock64();
-            if (vc1 > 0 && !skip) {
-              const float cmax = lse_update(v, vc1, scale, m_run, s_run);
-              if (listing) scan(v, 1, vc1, cmax);
-            }
-            if (etr) erec[3] = clock64();
+          static_assert(kChunks == 2, "the chunk-by-chunk epilogue is written for two chunks per thread");
+          const int vc0 = nvalid, vc1 = nvalid - 32;
+          float v[32];
+          if (vc0 > 0) {
+            tmem_ld32(tbase, v);
+            const float cmax = lse_update(v, vc0, scale, m_run, s_run);
+            if (listing) scan(v, 0, vc0, cmax);
+          }
+          if (vc1 > 0) tmem_ld32(tbase + 32, v);
+          tc_fence_before();
+          __syncwarp();
+          if (lane == 0) mbar_arrive_leader(bar_acc_empty + 8 * s);
+          if (vc1 > 0) {
+            const float cmax = lse_update(v, vc1, scale, m_run, s_run);
+            if (listing) scan(v, 1, vc1, cmax);
           }
         }
       }
@@ -1217,22 +1118,20 @@ bool make_map(CUtensorMap* m, const void* base, int n, int rows, int C) {
              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-unsigned long long* g_trace = nullptr;     // developer diagnostics buffer (allocated on first use of POPE_TC_TRACE)
-
-unsigned long long* trace_get() { return g_trace; }
-}  // namespace
-unsigned long long* trace_buffer() { return trace_get(); }
-
-static int debug_knob() {
+// Test hooks (environment variable POPE_TC_DEBUG), the references the tests hold the product sequence to:
+//   16   = no single sweep: the two-sweep online-softmax launch runs ungated, for every pair (bf16 features);
+//   1024 = the single sweep runs as one launch, without the head / tail cut (bf16 and fp32 features).
+constexpr int kHookTwoSweeps = 16, kHookOneLaunch = 1024;
+int debug_knob() {
   const char* dbg = getenv("POPE_TC_DEBUG");
   return dbg ? atoi(dbg) : 0;
 }
 
-// Head/tail cut of the single sweep (see coarse_tc_run): the number of leading pairs whose units fill whole rounds of the
+// Head/tail cut of the single sweep (see single_sweep_run): the number of leading pairs whose units fill whole rounds of the
 // static schedule, or 0 when the sweep should stay one launch.
-static int split_head(int n, int upp, int max_pairs, int debug) {
+int split_head(int n, int upp, int max_pairs) {
   const int u0 = n * upp;
-  if ((debug & 1024) || n <= 1 || u0 <= max_pairs || u0 % max_pairs == 0) return 0;
+  if (n <= 1 || u0 <= max_pairs || u0 % max_pairs == 0) return 0;
   const int rounds = (u0 + max_pairs - 1) / max_pairs;
   const int h = ((u0 / max_pairs) * max_pairs) / upp;                          // pairs that fit the full rounds
   const int ua = h * upp, ub = u0 - ua;
@@ -1242,7 +1141,69 @@ static int split_head(int n, int upp, int max_pairs, int debug) {
   return 0;
 }
 
-bool coarse_tc_needs_clear(const CoarseProblem& p) { return !(two_sweeps_possible(p) && !(debug_knob() & (8 | 16))); }
+using SweepKernel = decltype(&sweep_tc_kernel<0>);
+
+// per-device attribute, cheap: set on every call so that any device of a multi-GPU process is covered
+cudaError_t allow_smem(SweepKernel k) { return cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemAlloc); }
+
+// CTA pairs of the persistent sweeps on the current device: one per two SMs
+cudaError_t cta_pairs(int* max_pairs) {
+  int dev = 0, sms = 0;
+  cudaError_t e;
+  if ((e = cudaGetDevice(&dev)) != cudaSuccess) return e;
+  if ((e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
+  *max_pairs = sms / 2;
+  return cudaSuccess;
+}
+
+// the parameters every sweep launch shares; the pairs, units and gate are set per launch
+SweepParams sweep_params(const CoarseProblem& p, const CoarseScratch& w, int32_t* flags) {
+  SweepParams P{};
+  P.n = p.n; P.L0 = p.L; P.L1 = p.S; P.kchunks = p.C / kBoxK;
+  P.scale_log2 = p.scale_log2; P.log2_thr = p.log2_thr;
+  P.lse_out0 = w.lse_r; P.lse_out1 = w.lse_c; P.lse_r = w.lse_r; P.lse_c = w.lse_c; P.rowbest = w.rowbest; P.colbest = w.colbest;
+  P.cand_cnt = w.cand_cnt; P.cand = w.cand; P.flags = flags; P.colpart = w.colpart; P.cshift = w.cshift; P.pairflag = w.pairflag;
+  return P;
+}
+
+// Single sweep over the rows of S (`kernel`: MODE 3 for bf16 features, MODE 4 for fp32 features as three bf16 planes) and
+// the merge of its column partial sums into the column log-sum-exp.  Clears the pair flags; the merge resets colbest and
+// the "count published" words itself, so rowbest..ready need no memset.  Raises POPE_FLAG_ROBUST_PATH when the exponentials
+// of a pair leave the safe range.  The candidate lists are evaluated by the caller, behind the fallback of its dtype.
+// The unit schedule is static: u0 units over max_pairs CTA pairs run in ceil(u0 / max_pairs) rounds, and the last round
+// is usually part empty (64 pairs at 480x640: 1 216 units = 16 rounds of 74 + 32).  When the pairs can be cut into a
+// head that fills whole rounds and a tail that fits the last round without adding one, the sweep is launched twice --
+// head, then tail -- and the column merge of the head's pairs runs on the SMs the tail leaves idle: the sweep kernel
+// announces its dependents at once (griddepcontrol.launch_dependents) and merge(head), which needs nothing from the
+// tail (the head sweep has completed before the tail started), is launched behind the tail with programmatic stream
+// serialisation: ONE merge launch over all pairs, whose blocks for the head's pairs never wait and whose blocks for the
+// tail's pairs (the last of the grid) wait for the tail sweep (griddepcontrol.wait).  Everything behind it is ordinary.
+cudaError_t single_sweep_run(SweepKernel kernel, const CUtensorMap (&m)[6], const CoarseProblem& p, const CoarseScratch& w,
+                             int32_t* flags, cudaStream_t st) {
+  int max_pairs = 0;
+  cudaError_t e;
+  if ((e = cta_pairs(&max_pairs)) != cudaSuccess) return e;
+  if ((e = allow_smem(kernel)) != cudaSuccess) return e;
+  const SweepParams P = sweep_params(p, w, flags);
+  const int upp = (p.L + kUnitRows - 1) / kUnitRows;                           // units per pair
+  if ((e = cudaMemsetAsync(w.pairflag, 0, sizeof(int) * p.n, st)) != cudaSuccess) return e;
+  const int head = (debug_knob() & kHookOneLaunch) ? 0 : split_head(p.n, upp, max_pairs);
+  auto sweep = [&](int n_base, int n_count) -> cudaError_t {
+    SweepParams Q = P;
+    Q.n_base = n_base; Q.n = n_count;
+    Q.units_dir0 = Q.total_units = n_count * upp;
+    kernel<<<2 * min(Q.total_units, max_pairs), kThreads, kSmemAlloc, st>>>(m[0], m[1], m[2], m[3], m[4], m[5], Q);
+    return cudaGetLastError();
+  };
+  if (head > 0) {
+    if ((e = sweep(0, head)) != cudaSuccess) return e;
+    if ((e = sweep(head, p.n - head)) != cudaSuccess) return e;
+    return colsum_reduce_run(p, w, flags, st, 0, p.n, head);
+  }
+  if ((e = sweep(0, p.n)) != cudaSuccess) return e;
+  return colsum_reduce_run(p, w, flags, st, 0, p.n);
+}
+}  // namespace
 
 bool coarse_tc_supported(const CoarseProblem& p) {
   return p.dtype == POPE_BF16 && p.C % kBoxK == 0 && p.C >= kBoxK && p.C <= kBoxK * kMaxKChunks;
@@ -1250,8 +1211,7 @@ bool coarse_tc_supported(const CoarseProblem& p) {
 
 // fp32 features on the tensor cores through the three-way bf16 split (single-sweep path only: thr > 0.15)
 bool coarse_tc_split_supported(const CoarseProblem& p) {
-  return p.dtype == POPE_F32 && p.C % kBoxK == 0 && p.C >= kBoxK && p.C <= kBoxK * kMaxKChunks && two_sweeps_possible(p) &&
-         !(debug_knob() & (8 | 16));
+  return p.dtype == POPE_F32 && p.C % kBoxK == 0 && p.C >= kBoxK && p.C <= kBoxK * kMaxKChunks && two_sweeps_possible(p);
 }
 
 size_t coarse_tc_split_bytes(int n, int L, int S, int C) { return 3 * 2 * (size_t(n) * L * C + size_t(n) * S * C) + 6 * 256; }
@@ -1274,137 +1234,46 @@ cudaError_t coarse_tc_split_run(const CoarseProblem& p, const CoarseScratch& w, 
   CUtensorMap m[6];
   for (int k = 0; k < 6; ++k)
     if (!make_map(&m[k], pl[k], p.n, k < 3 ? p.L : p.S, p.C)) return cudaErrorInvalidValue;
-  int dev = 0, sms = 0;
-  if ((e = cudaGetDevice(&dev)) != cudaSuccess) return e;
-  if ((e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
-  auto k4 = sweep_tc_kernel<4, false>;
-  if ((e = cudaFuncSetAttribute(k4, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemAlloc)) != cudaSuccess) return e;
-  SweepParams P{};
-  P.debug = debug_knob();
-  P.n = p.n; P.L0 = p.L; P.L1 = p.S; P.kchunks = p.C / kBoxK;
-  P.scale_log2 = p.scale_log2; P.log2_thr = p.log2_thr;
-  P.lse_out0 = w.lse_r; P.lse_out1 = w.lse_c; P.lse_r = w.lse_r; P.lse_c = w.lse_c; P.rowbest = w.rowbest; P.colbest = w.colbest;
-  P.cand_cnt = w.cand_cnt; P.cand = w.cand; P.flags = flags; P.colpart = w.colpart; P.cshift = w.cshift; P.pairflag = w.pairflag;
-  const int upp = (p.L + kUnitRows - 1) / kUnitRows, max_pairs = sms / 2;
-  if ((e = cudaMemsetAsync(w.pairflag, 0, sizeof(int) * p.n, st)) != cudaSuccess) return e;
-  // head / tail launches with the head's column merge overlapped, as in coarse_tc_run
-  const int head = split_head(p.n, upp, max_pairs, P.debug);
-  auto sweep = [&](int n_base, int n_count) -> cudaError_t {
-    SweepParams Q = P;
-    Q.n_base = n_base; Q.n = n_count;
-    Q.units_dir0 = Q.total_units = n_count * upp;
-    k4<<<2 * min(Q.total_units, max_pairs), kThreads, kSmemAlloc, st>>>(m[0], m[1], m[2], m[3], m[4], m[5], Q);
-    return cudaGetLastError();
-  };
-  if (head > 0) {
-    if ((e = sweep(0, head)) != cudaSuccess) return e;
-    if ((e = sweep(head, p.n - head)) != cudaSuccess) return e;
-    if ((e = colsum_reduce_run(p, w, flags, st, 0, p.n, head)) != cudaSuccess) return e;
-  } else {
-    if ((e = sweep(0, p.n)) != cudaSuccess) return e;
-    if ((e = colsum_reduce_run(p, w, flags, st, 0, p.n)) != cudaSuccess) return e;
-  }
+  if ((e = single_sweep_run(sweep_tc_kernel<4>, m, p, w, flags, st)) != cudaSuccess) return e;
   return cand_eval_lists_run(p, w, flags, 2, st);       // mode 2: 2^x lists; a no-op once the fallback flag is up
 }
 
 cudaError_t coarse_tc_run(const CoarseProblem& p, const CoarseScratch& w, int32_t* flags, cudaStream_t st) {
-  CUtensorMap map0, map1;
-  if (!make_map(&map0, p.f0, p.n, p.L, p.C) || !make_map(&map1, p.f1, p.n, p.S, p.C)) return cudaErrorInvalidValue;
-  int dev = 0, sms = 0;
+  CUtensorMap m[6];                                     // MODES 0-3 read the first two maps only
+  if (!make_map(&m[0], p.f0, p.n, p.L, p.C) || !make_map(&m[1], p.f1, p.n, p.S, p.C)) return cudaErrorInvalidValue;
+  m[2] = m[4] = m[0];
+  m[3] = m[5] = m[1];
+  int max_pairs = 0;
   cudaError_t e;
-  if ((e = cudaGetDevice(&dev)) != cudaSuccess) return e;
-  if ((e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
-  // per-device attribute, cheap: set on every call so that any device of a multi-GPU process is covered
-  auto k0 = sweep_tc_kernel<0, false>, k1 = sweep_tc_kernel<1, false>, k2 = sweep_tc_kernel<2, false>;
-  auto k3 = sweep_tc_kernel<3, false>;
-  const char* trace_env = getenv("POPE_TC_TRACE");         // developer diagnostics: "0" / "2" = trace that sweep mode
-  const int trace_mode = trace_env ? atoi(trace_env) : -1;
-  if (trace_mode == 0) k0 = sweep_tc_kernel<0, true>;
-  if (trace_mode == 2) k2 = sweep_tc_kernel<2, true>;
-  if (trace_mode == 3) k3 = sweep_tc_kernel<3, true>;
-  if ((e = cudaFuncSetAttribute(k3, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemAlloc)) != cudaSuccess) return e;
-  if ((e = cudaFuncSetAttribute(k0, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemAlloc)) != cudaSuccess) return e;
-  if ((e = cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemAlloc)) != cudaSuccess) return e;
-  if ((e = cudaFuncSetAttribute(k2, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemAlloc)) != cudaSuccess) return e;
-  SweepParams P{};
-  P.debug = debug_knob();
-  if (trace_mode >= 0 && !g_trace) {
-    if ((e = cudaMalloc(&g_trace, sizeof(unsigned long long) * 8 * 2 * kTraceTiles)) != cudaSuccess) return e;
-    if ((e = cudaMemset(g_trace, 0, sizeof(unsigned long long) * 8 * 2 * kTraceTiles)) != cudaSuccess) return e;
-  }
-  P.n = p.n;
-  P.L0 = p.L; P.L1 = p.S;
-  P.kchunks = p.C / kBoxK;
-  P.scale_log2 = p.scale_log2; P.log2_thr = p.log2_thr;
-  P.lse_out0 = w.lse_r; P.lse_out1 = w.lse_c;
-  P.lse_r = w.lse_r; P.lse_c = w.lse_c; P.rowbest = w.rowbest; P.colbest = w.colbest;
-  P.cand_cnt = w.cand_cnt; P.cand = w.cand; P.flags = flags; P.colpart = w.colpart; P.cshift = w.cshift; P.pairflag = w.pairflag;
+  if ((e = cta_pairs(&max_pairs)) != cudaSuccess) return e;
+  SweepParams P = sweep_params(p, w, flags);
   const int u0 = p.n * ((p.L + kUnitRows - 1) / kUnitRows), u1 = p.n * ((p.S + kUnitRows - 1) / kUnitRows);
-  const int max_pairs = sms / 2;
+  auto launch = [&](SweepKernel k, int total_units) -> cudaError_t {
+    if ((e = allow_smem(k)) != cudaSuccess) return e;
+    P.units_dir0 = u0; P.total_units = total_units;
+    k<<<2 * min(total_units, max_pairs), kThreads, kSmemAlloc, st>>>(m[0], m[1], m[2], m[3], m[4], m[5], P);
+    return cudaGetLastError();
+  };
   // A cell with conf > thr has p_row > thr, and a row has fewer than 1/thr such cells: with thr > 1/kCandSlots the
   // column sweep can list them and the third (candidate) sweep is not needed.
-  const bool two_sweeps = two_sweeps_possible(p) && !(P.debug & 8);
-  if (two_sweeps) {
-    if (!(P.debug & 16)) {
-      // single sweep over the rows of S: row sums, column partial sums and candidate lists in one pass; raises
-      // POPE_FLAG_ROBUST_PATH when the unshifted exponentials leave the safe range (debug bit4 skips it)
-      P.trace = trace_mode == 3 ? g_trace : nullptr;
-      if ((e = cudaMemsetAsync(w.pairflag, 0, sizeof(int) * p.n, st)) != cudaSuccess) return e;
-      // The unit schedule is static: u0 units over max_pairs CTA pairs run in ceil(u0 / max_pairs) rounds, and the last round
-      // is usually part empty (64 pairs at 480x640: 1 216 units = 16 rounds of 74 + 32).  When the pairs can be cut into a
-      // head that fills whole rounds and a tail that fits the last round without adding one, the sweep is launched twice --
-      // head, then tail -- and the column merge of the head's pairs runs on the SMs the tail leaves idle: the sweep kernel
-      // announces its dependents at once (griddepcontrol.launch_dependents) and merge(head), which needs nothing from the
-      // tail (the head sweep has completed before the tail started), is launched behind the tail with programmatic stream
-      // serialisation: ONE merge launch over all pairs, whose blocks for the head's pairs never wait and whose blocks for the
-      // tail's pairs (the last of the grid) wait for the tail sweep (griddepcontrol.wait).  Everything behind it is ordinary.
-      const int upp = (p.L + kUnitRows - 1) / kUnitRows;                       // units per pair
-      const int head = split_head(p.n, upp, max_pairs, P.debug);
-      auto sweep = [&](int n_base, int n_count) -> cudaError_t {
-        SweepParams Q = P;
-        Q.n_base = n_base; Q.n = n_count;
-        Q.units_dir0 = Q.total_units = n_count * upp;
-        k3<<<2 * min(Q.total_units, max_pairs), kThreads, kSmemAlloc, st>>>(map0, map1, map0, map1, map0, map1, Q);
-        return cudaGetLastError();
-      };
-      if (head > 0) {
-        if ((e = sweep(0, head)) != cudaSuccess) return e;
-        if ((e = sweep(head, p.n - head)) != cudaSuccess) return e;
-        if ((e = colsum_reduce_run(p, w, flags, st, 0, p.n, head)) != cudaSuccess) return e;
-      } else {
-        if ((e = sweep(0, p.n)) != cudaSuccess) return e;
-        if ((e = colsum_reduce_run(p, w, flags, st, 0, p.n)) != cudaSuccess) return e;
-      }
-      P.units_dir0 = u0; P.total_units = u0;
+  if (two_sweeps_possible(p)) {
+    if (debug_knob() & kHookTwoSweeps) {
+      // without the single sweep's column merge nothing resets colbest and the "count published" words
+      if ((e = cudaMemsetAsync(w.rowbest, 0, w.zero_bytes, st)) != cudaSuccess) return e;
+    } else {
+      // single sweep over the rows of S: row sums, column partial sums and candidate lists in one pass
+      if ((e = single_sweep_run(sweep_tc_kernel<3>, m, p, w, flags, st)) != cudaSuccess) return e;
       P.gate = 1;
-      if (P.debug & 64) return cand_eval_lists_run(p, w, flags, 0, st);      // developer knob: no gated redo (inspect the single sweep)
     }
     // robust two-sweep path (online softmax per row, both directions in one launch; the direction-0 units also fill the
     // per-thread candidate lists); after the single sweep it only runs if the flag was raised
-    P.units_dir0 = u0; P.total_units = u0 + u1;
-    P.trace = trace_mode == 2 ? g_trace : nullptr;
-    k2<<<2 * min(P.total_units, max_pairs), kThreads, kSmemAlloc, st>>>(map0, map1, map0, map1, map0, map1, P);
-    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+    if ((e = launch(sweep_tc_kernel<2>, u0 + u1)) != cudaSuccess) return e;
     return cand_eval_lists_run(p, w, flags, 0, st);
   }
   // three sweeps (small thresholds): both log-sum-exp directions in one launch, then the candidate sweep
-  P.units_dir0 = u0; P.total_units = u0 + u1;
-  P.trace = trace_mode == 0 ? g_trace : nullptr;
-  k0<<<2 * min(P.total_units, max_pairs), kThreads, kSmemAlloc, st>>>(map0, map1, map0, map1, map0, map1, P);
-  if ((e = cudaGetLastError()) != cudaSuccess) return e;
-  P.total_units = u0;
-  k1<<<2 * min(P.total_units, max_pairs), kThreads, kSmemAlloc, st>>>(map0, map1, map0, map1, map0, map1, P);
-  return cudaGetLastError();
+  if ((e = cudaMemsetAsync(w.rowbest, 0, w.zero_bytes, st)) != cudaSuccess) return e;
+  if ((e = launch(sweep_tc_kernel<0>, u0 + u1)) != cudaSuccess) return e;
+  return launch(sweep_tc_kernel<1>, u0);
 }
 
 }  // namespace pope
-
-// Developer diagnostics: copies the clock stamps written under POPE_TC_TRACE (8 x u64 per tile: MMA-issuer records
-// first, then epilogue-warp records) to the host; returns the number of u64 copied (0 when tracing is off).
-extern "C" int pope_debug_trace_read(unsigned long long* out, int max_u64) {
-  const int n = 8 * 2 * 512;
-  unsigned long long* src = pope::trace_buffer();
-  if (!out || max_u64 < n || !src) return 0;
-  if (cudaMemcpy(out, src, sizeof(unsigned long long) * n, cudaMemcpyDeviceToHost) != cudaSuccess) return 0;
-  return n;
-}

@@ -124,8 +124,8 @@ struct CoarseProblem {
 };
 
 // coarse_simt.cu -- fp32-FMA kernels (fp32 or bf16 inputs): the fp32 product path and the cross-check for tcgen05.
-// gated: every launch is a no-op unless POPE_FLAG_ROBUST_PATH is set in *flags (the fallback of the fp32 tensor-core path);
-// the gated sequence starts by clearing the best-candidate records and counters itself.
+// gated: every launch is a no-op unless POPE_FLAG_ROBUST_PATH is set in *flags (the fallback of the fp32 tensor-core path).
+// Both forms start by clearing the best-candidate records and counters themselves (the gated one only behind the flag).
 cudaError_t coarse_simt_run(const CoarseProblem& p, const CoarseScratch& w, int32_t* flags, cudaStream_t st, bool gated = false);
 // coarse_tc.cu -- tcgen05/TMEM/TMA kernels (bf16 inputs, C in {64,128,192,256})
 bool coarse_tc_supported(const CoarseProblem& p);
@@ -151,8 +151,6 @@ cudaError_t cand_eval_lists_run(const CoarseProblem& p, const CoarseScratch& w, 
 // (the tail of a split single sweep) still runs; only the blocks of the pairs >= wait_from wait for that kernel
 cudaError_t colsum_reduce_run(const CoarseProblem& p, const CoarseScratch& w, int32_t* flags, cudaStream_t st, int n_base, int n_count,
                               int wait_from = -1);
-// does coarse_tc_run need rowbest / colbest / cand_cnt cleared beforehand?  (not on the single-sweep launch sequence)
-bool coarse_tc_needs_clear(const CoarseProblem& p);
 // a thr large enough that a row's cells with p_row > thr fit its kCandSlots candidate slots
 inline bool two_sweeps_possible(const CoarseProblem& p) { return exp2f(p.log2_thr) * float(kCandSlots) > 1.2f; }
 // coarse_finalize.cu -- mutual test, border removal, ordered compaction

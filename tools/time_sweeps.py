@@ -1,4 +1,5 @@
-"""Times the coarse stage with CUDA events; used with POPE_TC_DEBUG experiments.
+"""Times the coarse stage with CUDA events.  Under the test hooks of csrc/coarse_tc.cu it times their reference sequences:
+POPE_TC_DEBUG=16 (two-sweep online softmax, ungated) and POPE_TC_DEBUG=1024 (the single sweep as one launch).
     python tools/time_sweeps.py                 64 pairs at 480x640 (60x80 tokens), bf16
     python tools/time_sweeps.py highres [n]     n (default 4) pairs at 960x1280 (120x160 = 19 200 tokens, BASELINE configs[3])
     python tools/time_sweeps.py f32 [simt]      64 pairs, fp32 features: tensor-core split path (default) or the fp32-FMA kernels
