@@ -313,6 +313,16 @@ size_t pope_fine_tf_workspace_bytes(int64_t m_windows, int window_tokens);
 int pope_fine_transformer(void* feat0, void* feat1, int64_t m_windows, int window_tokens, const void* weights,
                           int n_layers, const int* layer_kinds, void* workspace, size_t workspace_bytes, void* stream);
 
+/* pope_fine_transformer bounded by a live count kept on the device, so that it can follow pope_coarse_match /
+ * pope_fine_gather without a host sync (and be captured in a CUDA graph).  m_windows is the launch capacity: tensor maps,
+ * grids and the workspace are sized by it.  m_dev (may be NULL = all m_windows windows): device int32 live window count,
+ * e.g. counts + n_pairs of pope_coarse_match; windows at or past min(*m_dev, m_windows) are never written and their
+ * contents never reach a live window.  A live count of 0 is a no-op.  Same results as pope_fine_transformer on the live
+ * windows, bit for bit.  pope_fine_transformer(...) is pope_fine_transformer_ex(..., m_dev = NULL, ...). */
+int pope_fine_transformer_ex(void* feat0, void* feat1, int64_t m_windows, const int32_t* m_dev, int window_tokens,
+                             const void* weights, int n_layers, const int* layer_kinds,
+                             void* workspace, size_t workspace_bytes, void* stream);
+
 /* Bytes of device scratch pope_fine_merge_coarse needs (gathered + projected coarse rows, per-window vectors). */
 size_t pope_fine_merge_workspace_bytes(int64_t m_windows);
 
@@ -323,6 +333,15 @@ int pope_fine_merge_coarse(void* win0, void* win1, int64_t m_windows, int window
                            const void* feat_c1, int L, int S, int C, const int64_t* b_ids, const int64_t* i_ids,
                            const int64_t* j_ids, const void* weights, void* workspace, size_t workspace_bytes,
                            void* stream);
+
+/* pope_fine_merge_coarse bounded by a live count kept on the device (the convention of pope_fine_transformer_ex):
+ * m_windows is the capacity (length of the id arrays and of the windows, workspace sized by it), m_dev (may be NULL)
+ * the device int32 live count; ids, windows and scratch rows at or past min(*m_dev, m_windows) are never read or written
+ * (scratch: rows of either side).  Same results as pope_fine_merge_coarse on the live windows, bit for bit. */
+int pope_fine_merge_coarse_ex(void* win0, void* win1, int64_t m_windows, const int32_t* m_dev, int window_tokens,
+                              const void* feat_c0, const void* feat_c1, int L, int S, int C,
+                              const int64_t* b_ids, const int64_t* i_ids, const int64_t* j_ids, const void* weights,
+                              void* workspace, size_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }

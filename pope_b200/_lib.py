@@ -40,6 +40,8 @@ SIGNATURES = {
     "pope_fine_merge_workspace_bytes": (_sz, [_i64]),
     "pope_fine_transformer": (_i, [_p, _p, _i64, _i, _p, _i, C.POINTER(_i), _p, _sz, _p]),
     "pope_fine_merge_coarse": (_i, [_p, _p, _i64, _i, _p, _p, _i, _i, _i, _p, _p, _p, _p, _p, _sz, _p]),
+    "pope_fine_transformer_ex": (_i, [_p, _p, _i64, _p, _i, _p, _i, C.POINTER(_i), _p, _sz, _p]),
+    "pope_fine_merge_coarse_ex": (_i, [_p, _p, _i64, _p, _i, _p, _p, _i, _i, _i, _p, _p, _p, _p, _p, _sz, _p]),
     "pope_match_order_by_ref": (_i, [_p, _i, _i, _p, _p, _p]),
     "pope_savetxt_f32": (_i, [C.c_char_p, _p, _i64, _i]),
     "pope_savetxt_f64": (_i, [C.c_char_p, _p, _i64, _i]),

@@ -59,14 +59,39 @@ struct LinParams {
   const float* beta;
   const float* rowvec;         // EPI_ADDVEC: [T / rows_per_vec, 128]
   int rows_per_vec;
+  const int32_t* live;         // if set: device count of live items; rows >= *live * rows_per_item are not written and
+  int rows_per_item;           // tiles past them not run (T is the capacity the tensor maps and the grid are sized for)
+  __nv_bfloat16* out_rows[3];  // output blocks as plain pointers (row pitch out_pitch), for the one 32-row box that
+  int out_pitch[3];            // straddles the live bound: a TMA store of it would write rows past the bound
 };
+
+// Live part of a capacity-sized launch: cap, or min(cap, *live * per_item) when a device count is given.  Every kernel
+// reads the count once, at its start; it is written by an earlier kernel in stream order.  (None of these kernels uses
+// programmatic dependent launch; one that does must read it after griddepcontrol.wait.)
+__device__ __forceinline__ int64_t live_count(int64_t cap, const int32_t* live, int64_t per_item) {
+  return live ? min(cap, int64_t(max(*live, 0)) * per_item) : cap;
+}
 
 __device__ __forceinline__ uint32_t pack_bf16(float a, float b) {
   __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
   return *reinterpret_cast<uint32_t*>(&h);
 }
 
-// mapO[j]: output block j as a [T, 128] bf16 tensor (box 64 x 32 rows); mapR: residual [T, 128] (EPI_LN_RES)
+// A 32-row output box that straddles the live bound is not TMA-stored (the store would write the rows past the bound):
+// each lane below the bound copies its own 64-column half row out of the 128B-swizzled staging box instead.
+__device__ __forceinline__ void store_staged_half_row(uint32_t my_row, uint32_t sw, __nv_bfloat16* dst) {
+#pragma unroll
+  for (int c8 = 0; c8 < 8; ++c8) {
+    uint4 r;
+    asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w)
+                 : "r"(my_row + ((uint32_t(c8) ^ sw) << 4)));
+    reinterpret_cast<uint4*>(dst)[c8] = r;
+  }
+}
+
+// mapO[j]: output block j as a [T, 128] bf16 tensor (box 64 x 32 rows); mapR: residual [T, 128] (EPI_LN_RES).
+// kBounded: P.live is set (a separate instantiation, so that the unbounded launches keep their code and registers)
+template <bool kBounded>
 __global__ void __launch_bounds__(kLinThreads, 1)
 linear_tc_kernel(const __grid_constant__ CUtensorMap mapX0, const __grid_constant__ CUtensorMap mapX1,
                  const __grid_constant__ CUtensorMap mapW, const __grid_constant__ CUtensorMap mapO0,
@@ -81,8 +106,18 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapX0, const __grid_constan
   const uint32_t bar_acc_full = bar_x_empty + 8 * kMaxStages, bar_acc_empty = bar_acc_full + 8 * kSlots;
   const uint32_t bar_res = bar_acc_empty + 8 * kSlots;           // one per epilogue warp (residual tile landed)
   volatile uint32_t* tmem_ptr_smem = reinterpret_cast<volatile uint32_t*>(smem + kSmemTmemPtr);
+  // live rows: read into shared memory once, so the epilogue re-reads it where needed instead of holding a register
+  volatile int* live_rows_smem = reinterpret_cast<volatile int*>(smem + kSmemTmemPtr + 8);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int ntiles = (P.T + kTile - 1) / kTile;
+  int ntiles;
+  {
+    const int T = kBounded ? int(live_count(P.T, P.live, P.rows_per_item)) : P.T;
+    ntiles = (T + kTile - 1) / kTile;
+    if (kBounded) {
+      if (int(blockIdx.x) >= ntiles) return;         // capacity-sized grid, fewer live tiles: no load issued, no TMEM held
+      if (threadIdx.x == 0) *live_rows_smem = T;     // (every thread read the same count; published by the sync below)
+    }
+  }
   const uint32_t smem_x = sbase + kSmemW + P.nblk * P.kchunks * kBoxBytes;
   const int stages = P.stages;
 
@@ -245,7 +280,7 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapX0, const __grid_constan
             }
           }
         } else if (mode == EPI_ADDVEC) {
-          if (row < P.T) {
+          if (row < (kBounded ? *live_rows_smem : P.T)) {
             const float4* a4 = reinterpret_cast<const float4*>(P.rowvec + size_t(row / P.rows_per_vec) * kD);
 #pragma unroll
             for (int c = 0; c < kD; c += 4) {
@@ -255,13 +290,15 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapX0, const __grid_constan
           }
         }
         if (P.out_f32) {
-          if (row < P.T) {
+          if (row < (kBounded ? *live_rows_smem : P.T)) {
             float4* o = reinterpret_cast<float4*>(P.out_f32 + size_t(row) * kD);
 #pragma unroll
             for (int c = 0; c < kD; c += 4) o[c >> 2] = make_float4(v[c], v[c + 1], v[c + 2], v[c + 3]);
           }
         } else {
           const CUtensorMap* mo = j == 0 ? &mapO0 : (j == 1 ? &mapO1 : &mapO2);
+          const int T = kBounded ? *live_rows_smem : P.T;
+          const bool whole_box = !kBounded || row0 + 32 <= T || T == P.T;
 #pragma unroll
           for (int half = 0; half < 2; ++half) {
             if (lane == 0) tma_store_wait_read();               // the previous store out of this box has read it
@@ -276,9 +313,14 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapX0, const __grid_constan
             }
             fence_proxy_async();
             __syncwarp();
-            if (lane == 0) {
-              tma_store_2d(mo, stage_buf, half * 64, row0);     // rows past T are clipped by the tensor map
-              tma_store_commit();
+            if (whole_box) {
+              if (lane == 0) {
+                tma_store_2d(mo, stage_buf, half * 64, row0);   // rows past the capacity are clipped by the tensor map
+                tma_store_commit();
+              }
+            } else {
+              if (row < T) store_staged_half_row(my_row, sw, P.out_rows[j] + size_t(row) * P.out_pitch[j] + half * 64);
+              __syncwarp();                                     // every lane has read its row before the box is refilled
             }
           }
         }
@@ -323,10 +365,12 @@ static_assert(kFmTmemPtr + 16 <= kFmW1 && kFmEnd + 1024 <= 227 * 1024, "fused-ML
 constexpr int kFmAlloc = kFmEnd + 1024;
 }  // namespace fm
 
+template <bool kBounded>                                         // as linear_tc_kernel
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fm::kFmThreads, 1)
 mlp_fused_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constant__ CUtensorMap mapM1,
                  const __grid_constant__ CUtensorMap mapW1, const __grid_constant__ CUtensorMap mapW2,
-                 const __grid_constant__ CUtensorMap mapO, const __grid_constant__ CUtensorMap mapR, int T,
+                 const __grid_constant__ CUtensorMap mapO, const __grid_constant__ CUtensorMap mapR, int T_cap,
+                 const int32_t* live, int rows_per_item, __nv_bfloat16* __restrict__ out,
                  const float* __restrict__ gamma, const float* __restrict__ beta) {
   using namespace fm;
   extern __shared__ uint8_t smem_raw[];
@@ -340,10 +384,19 @@ mlp_fused_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constant
   const uint32_t bar_d2_full = bar_h_full + 8, bar_d2_empty = bar_d2_full + 16;      // d2_empty: one per TMEM buffer
   const uint32_t bar_res = bar_d2_empty + 16;                    // 8: one per epilogue warp
   volatile uint32_t* tmem_ptr_smem = reinterpret_cast<volatile uint32_t*>(smem + kFmTmemPtr);
+  volatile int* live_rows_smem = reinterpret_cast<volatile int*>(smem + kFmTmemPtr + 8);   // as in linear_tc_kernel
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t rank = tc2::cluster_ctarank();
   const int pair = blockIdx.x >> 1, npairs = gridDim.x >> 1;
-  const int ntiles = (T + 2 * kTile - 1) / (2 * kTile);          // 256-row tiles
+  int ntiles;                                                    // 256-row tiles
+  {
+    const int T = kBounded ? int(live_count(T_cap, live, rows_per_item)) : T_cap;
+    ntiles = (T + 2 * kTile - 1) / (2 * kTile);
+    if (kBounded) {
+      if (pair >= ntiles) return;      // both CTAs of the pair read the same count: neither issues a load nor allocates
+      if (threadIdx.x == 0) *live_rows_smem = T;
+    }
+  }
 
   if (warp == 0 && lane == 0) {
     prefetch_tmap(&mapX); prefetch_tmap(&mapM1); prefetch_tmap(&mapW1); prefetch_tmap(&mapW2);
@@ -534,6 +587,8 @@ mlp_fused_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constant
         }
         __syncwarp();
       }
+      const int T = kBounded ? *live_rows_smem : T_cap;
+      const bool whole_box = !kBounded || row0 + 32 <= T || T == T_cap;
 #pragma unroll
       for (int half = 0; half < 2; ++half) {
         if (lane == 0) tma_store_wait_read();
@@ -548,9 +603,14 @@ mlp_fused_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constant
         }
         fence_proxy_async();
         __syncwarp();
-        if (lane == 0) {
-          tma_store_2d(&mapO, stage_buf, half * 64, row0);
-          tma_store_commit();
+        if (whole_box) {
+          if (lane == 0) {
+            tma_store_2d(&mapO, stage_buf, half * 64, row0);
+            tma_store_commit();
+          }
+        } else {
+          if (row0 + lane < T) store_staged_half_row(my_row, sw, out + size_t(row0 + lane) * kD + half * 64);
+          __syncwarp();
         }
       }
     }
@@ -575,13 +635,13 @@ constexpr int kAttnWarps = 4;
 
 __global__ void __launch_bounds__(kAttnWarps * 32)
 fine_attn_kernel(const __nv_bfloat16* __restrict__ q, const __nv_bfloat16* __restrict__ k, const __nv_bfloat16* __restrict__ v,
-                 __nv_bfloat16* __restrict__ out, int64_t m, int S, float eps) {
+                 __nv_bfloat16* __restrict__ out, int64_t m, const int32_t* live, int S, float eps) {
   __shared__ float kv_s[kAttnWarps][kHeads][kHeadDim][kHeadDim + 1];
   __shared__ float ks_s[kAttnWarps][kHeads][kHeadDim];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int h = lane >> 2, r = lane & 3;
   const int64_t w = int64_t(blockIdx.x) * kAttnWarps + warp;
-  if (w >= m) return;
+  if (w >= live_count(m, live, 1)) return;
   const size_t base = size_t(w) * S * kD;
   float kv[4][kHeadDim], ks[4];
 #pragma unroll
@@ -771,7 +831,8 @@ __device__ __forceinline__ void attn_window_core(uint32_t sq, uint32_t sk, uint3
 
 __global__ void __launch_bounds__(kMmaWarps * 32)
 fine_attn_mma_kernel(const __nv_bfloat16* __restrict__ q, const __nv_bfloat16* __restrict__ k,
-                     const __nv_bfloat16* __restrict__ v, __nv_bfloat16* __restrict__ out, int64_t m, int S, float eps) {
+                     const __nv_bfloat16* __restrict__ v, __nv_bfloat16* __restrict__ out, int64_t m, const int32_t* live,
+                     int S, float eps) {
   extern __shared__ __align__(128) uint8_t attn_smem[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int g = lane >> 2, t = lane & 3;
@@ -781,8 +842,9 @@ fine_attn_mma_kernel(const __nv_bfloat16* __restrict__ q, const __nv_bfloat16* _
     asm volatile("st.shared.v4.b32 [%0], {%1, %1, %1, %1};" ::"r"(sq + i * 16), "r"(0u) : "memory");
   __syncwarp();
   const int nchunk = S * (kD * 2 / 16);                     // 16-byte chunks of one [S, 128] tile
+  const int64_t m_live = live_count(m, live, 1);
 
-  for (int64_t w = int64_t(blockIdx.x) * kMmaWarps + warp; w < m; w += int64_t(gridDim.x) * kMmaWarps) {
+  for (int64_t w = int64_t(blockIdx.x) * kMmaWarps + warp; w < m_live; w += int64_t(gridDim.x) * kMmaWarps) {
     const size_t base = size_t(w) * S * kD;
     // ---- load: chunk c of row r lands at r * 256 + ((c ^ (r & 7)) << 4) --------------------------------------------
     for (int i = lane; i < nchunk; i += 32) {
@@ -799,18 +861,21 @@ fine_attn_mma_kernel(const __nv_bfloat16* __restrict__ q, const __nv_bfloat16* _
   }
 }
 
-// rows [0, m): f0[b, i, :], rows [m, 2m): f1[b, j, :]   (fine_preprocess.py:50-51, the cat along dim 0)
+// rows [0, m): f0[b, i, :], rows [m, 2m): f1[b, j, :]   (fine_preprocess.py:50-51, the cat along dim 0); with a live count
+// only rows [0, live) and [m, m + live) (the ids past it are never read)
 __global__ void __launch_bounds__(256) gather_coarse_rows_kernel(const __nv_bfloat16* __restrict__ f0,
                                                                 const __nv_bfloat16* __restrict__ f1,
                                                                 const int64_t* __restrict__ b_ids,
                                                                 const int64_t* __restrict__ i_ids,
-                                                                const int64_t* __restrict__ j_ids, int64_t m, int L, int S,
-                                                                int C, __nv_bfloat16* __restrict__ out) {
+                                                                const int64_t* __restrict__ j_ids, int64_t m,
+                                                                const int32_t* __restrict__ live, int L, int S, int C,
+                                                                __nv_bfloat16* __restrict__ out) {
   const int64_t row = int64_t(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (row >= 2 * m) return;
   const int lane = threadIdx.x & 31;
   const bool second = row >= m;
   const int64_t mm = second ? row - m : row;
+  if (mm >= live_count(m, live, 1)) return;
   const __nv_bfloat16* src = second ? f1 + (size_t(b_ids[mm]) * S + size_t(j_ids[mm])) * C
                                     : f0 + (size_t(b_ids[mm]) * L + size_t(i_ids[mm])) * C;
   for (int c = lane * 8; c < C; c += 256)
@@ -848,9 +913,10 @@ bool make_map2d(CUtensorMap* m, const void* base, int64_t rows, int cols, int64_
 struct Src { const void* ptr; int cols; int64_t pitch; };   // one K-part of the activations
 struct Dst { void* ptr; int64_t pitch; };                   // one 128-column block of the output (bf16, row pitch in elements)
 
-// Y[T, N] = epilogue(cat(X0, X1)[T, K] . W[N, K]^T);  out[j] receives output columns [128 j, 128 j + 128)
-cudaError_t linear_run(int64_t T, Src x0, Src x1, const void* W, int N, int K, int64_t w_pitch, const Dst (&out)[3],
-                       const __nv_bfloat16* resid, LinParams P, cudaStream_t st) {
+// Y[T, N] = epilogue(cat(X0, X1)[T, K] . W[N, K]^T);  out[j] receives output columns [128 j, 128 j + 128).
+// live (may be null): device count of live items of rows_per_item rows each; T is then the capacity.
+cudaError_t linear_run(int64_t T, const int32_t* live, int rows_per_item, Src x0, Src x1, const void* W, int N, int K,
+                       int64_t w_pitch, const Dst (&out)[3], const __nv_bfloat16* resid, LinParams P, cudaStream_t st) {
   if (T <= 0) return cudaSuccess;
   if (T > 0x7fffffff - kTile || N % 128 || K % kBoxK || (N / 128) * (K / kBoxK) > kMaxWBoxes || N / 128 > 3)
     return cudaErrorInvalidValue;
@@ -864,9 +930,13 @@ cudaError_t linear_run(int64_t T, Src x0, Src x1, const void* W, int N, int K, i
     const bool used = !P.out_f32 && j < N / 128;
     if (used && !out[j].ptr) return cudaErrorInvalidValue;
     if (!make_map2d(&mo[j], used ? out[j].ptr : any_out, T, kD, used ? out[j].pitch : kD, 32)) return cudaErrorInvalidValue;
+    P.out_rows[j] = used ? static_cast<__nv_bfloat16*>(out[j].ptr) : nullptr;
+    P.out_pitch[j] = used ? int(out[j].pitch) : 0;
   }
   if (!make_map2d(&mr, resid ? static_cast<const void*>(resid) : any_out, T, kD, kD, 32)) return cudaErrorInvalidValue;
   P.T = int(T);
+  P.live = live;
+  P.rows_per_item = rows_per_item;
   P.kchunks = K / kBoxK;
   P.kchunks0 = x0.cols / kBoxK;
   P.nblk = N / 128;
@@ -876,15 +946,16 @@ cudaError_t linear_run(int64_t T, Src x0, Src x1, const void* W, int N, int K, i
   cudaError_t e;
   if ((e = cudaGetDevice(&dev)) != cudaSuccess) return e;
   if ((e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
-  if ((e = cudaFuncSetAttribute(linear_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemAlloc)) != cudaSuccess) return e;
+  const auto kernel = live ? linear_tc_kernel<true> : linear_tc_kernel<false>;
+  if ((e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemAlloc)) != cudaSuccess) return e;
   const int ntiles = int((T + kTile - 1) / kTile);
-  linear_tc_kernel<<<min(ntiles, sms), kLinThreads, kSmemAlloc, st>>>(m0, m1, mw, mo[0], mo[1], mo[2], mr, P);
+  kernel<<<min(ntiles, sms), kLinThreads, kSmemAlloc, st>>>(m0, m1, mw, mo[0], mo[1], mo[2], mr, P);
   return cudaGetLastError();
 }
 
 // x <- x + LayerNorm(W2 . relu(W1 . cat(x, m1))) in place, one launch
-cudaError_t mlp_fused_run(__nv_bfloat16* x, const __nv_bfloat16* m1, int64_t T, const void* W1, const void* W2, const float* gamma,
-                          const float* beta, cudaStream_t st) {
+cudaError_t mlp_fused_run(__nv_bfloat16* x, const __nv_bfloat16* m1, int64_t T, const int32_t* live, int rows_per_item,
+                          const void* W1, const void* W2, const float* gamma, const float* beta, cudaStream_t st) {
   if (T <= 0) return cudaSuccess;
   if (T > 0x7fffffff - 2 * kTile) return cudaErrorInvalidValue;
   CUtensorMap mx, mm, mw1, mw2, mo, mr;
@@ -895,10 +966,11 @@ cudaError_t mlp_fused_run(__nv_bfloat16* x, const __nv_bfloat16* m1, int64_t T, 
   cudaError_t e;
   if ((e = cudaGetDevice(&dev)) != cudaSuccess) return e;
   if ((e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
-  if ((e = cudaFuncSetAttribute(mlp_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, fm::kFmAlloc)) != cudaSuccess)
-    return e;
+  const auto kernel = live ? mlp_fused_kernel<true> : mlp_fused_kernel<false>;
+  if ((e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, fm::kFmAlloc)) != cudaSuccess) return e;
   const int ntiles = int((T + 2 * kTile - 1) / (2 * kTile));
-  mlp_fused_kernel<<<2 * min(ntiles, sms / 2), fm::kFmThreads, fm::kFmAlloc, st>>>(mx, mm, mw1, mw2, mo, mr, int(T), gamma, beta);
+  kernel<<<2 * min(ntiles, sms / 2), fm::kFmThreads, fm::kFmAlloc, st>>>(mx, mm, mw1, mw2, mo, mr, int(T), live, rows_per_item, x,
+                                                                         gamma, beta);
   return cudaGetLastError();
 }
 
@@ -934,10 +1006,10 @@ TfScratch carve_tf(void* base, int64_t m, int S) {
 }
 
 cudaError_t attention_run(const __nv_bfloat16* q, const __nv_bfloat16* k, const __nv_bfloat16* v, __nv_bfloat16* out, int64_t m,
-                          int S, cudaStream_t st) {
+                          const int32_t* live, int S, cudaStream_t st) {
   const bool force_simt = getenv("POPE_ATTN_SIMT") != nullptr;             // developer knob: the fp32 SIMT kernel
   if (S > kTileRows || force_simt) {
-    fine_attn_kernel<<<unsigned((m + kAttnWarps - 1) / kAttnWarps), kAttnWarps * 32, 0, st>>>(q, k, v, out, m, S, 1e-6f);
+    fine_attn_kernel<<<unsigned((m + kAttnWarps - 1) / kAttnWarps), kAttnWarps * 32, 0, st>>>(q, k, v, out, m, live, S, 1e-6f);
     return cudaGetLastError();
   }
   int dev = 0, sms = 0;
@@ -948,13 +1020,13 @@ cudaError_t attention_run(const __nv_bfloat16* q, const __nv_bfloat16* k, const 
   if ((e = cudaFuncSetAttribute(fine_attn_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)) != cudaSuccess) return e;
   const int64_t blocks = (m + kMmaWarps - 1) / kMmaWarps;
   fine_attn_mma_kernel<<<unsigned(blocks < int64_t(sms) * 2 ? blocks : int64_t(sms) * 2), kMmaWarps * 32, smem, st>>>(q, k, v, out, m,
-                                                                                                                 S, 1e-6f);
+                                                                                                                 live, S, 1e-6f);
   return cudaGetLastError();
 }
 
 // x <- x + norm2(mlp(cat(x, norm1(merge(attention(q(x), k(src), v(src)))))))      (transformer.py:34-58), in place on x
-cudaError_t encoder_layer(__nv_bfloat16* x, const __nv_bfloat16* src, int64_t m, int S, const char* wl, const TfScratch& w,
-                          cudaStream_t st) {
+cudaError_t encoder_layer(__nv_bfloat16* x, const __nv_bfloat16* src, int64_t m, const int32_t* live, int S, const char* wl,
+                          const TfScratch& w, cudaStream_t st) {
   const int64_t T = m * S;
   const float* ln = reinterpret_cast<const float*>(wl + kOffLn);
   const Src none{nullptr, 0, 0};
@@ -963,31 +1035,31 @@ cudaError_t encoder_layer(__nv_bfloat16* x, const __nv_bfloat16* src, int64_t m,
   if (x == src) {                       // self: one pass over x produces q, k, v
     P.mode[0] = EPI_ELU1; P.mode[1] = EPI_ELU1; P.mode[2] = EPI_SCALE; P.scale = 1.f / float(S);
     const Dst o[3] = {{w.q, kD}, {w.k, kD}, {w.v, kD}};
-    if ((e = linear_run(T, {x, kD, kD}, none, wl + kOffQkv, 384, kD, kD, o, nullptr, P, st)) != cudaSuccess) return e;
+    if ((e = linear_run(T, live, S, {x, kD, kD}, none, wl + kOffQkv, 384, kD, kD, o, nullptr, P, st)) != cudaSuccess) return e;
   } else {
     P.mode[0] = EPI_ELU1;
     const Dst oq[3] = {{w.q, kD}, {nullptr, 0}, {nullptr, 0}};
-    if ((e = linear_run(T, {x, kD, kD}, none, wl + kOffQkv, 128, kD, kD, oq, nullptr, P, st)) != cudaSuccess) return e;
+    if ((e = linear_run(T, live, S, {x, kD, kD}, none, wl + kOffQkv, 128, kD, kD, oq, nullptr, P, st)) != cudaSuccess) return e;
     P.mode[0] = EPI_ELU1; P.mode[1] = EPI_SCALE; P.scale = 1.f / float(S);
     const Dst okv[3] = {{w.k, kD}, {w.v, kD}, {nullptr, 0}};
-    if ((e = linear_run(T, {src, kD, kD}, none, wl + kOffQkv + 128 * 128 * 2, 256, kD, kD, okv, nullptr, P, st)) != cudaSuccess)
+    if ((e = linear_run(T, live, S, {src, kD, kD}, none, wl + kOffQkv + 128 * 128 * 2, 256, kD, kD, okv, nullptr, P, st)) != cudaSuccess)
       return e;
   }
-  if ((e = attention_run(w.q, w.k, w.v, w.msg, m, S, st)) != cudaSuccess) return e;
+  if ((e = attention_run(w.q, w.k, w.v, w.msg, m, live, S, st)) != cudaSuccess) return e;
   P = LinParams{};
   P.mode[0] = EPI_LN; P.gamma = ln; P.beta = ln + 128;
   const Dst om[3] = {{w.m1, kD}, {nullptr, 0}, {nullptr, 0}};
-  if ((e = linear_run(T, {w.msg, kD, kD}, none, wl + kOffMerge, 128, kD, kD, om, nullptr, P, st)) != cudaSuccess) return e;
+  if ((e = linear_run(T, live, S, {w.msg, kD, kD}, none, wl + kOffMerge, 128, kD, kD, om, nullptr, P, st)) != cudaSuccess) return e;
   const bool unfused_mlp = getenv("POPE_MLP_UNFUSED") != nullptr;            // developer knob: the two separate launches
-  if (!unfused_mlp) return mlp_fused_run(x, w.m1, T, wl + kOffMlp1, wl + kOffMlp2, ln + 256, ln + 384, st);
+  if (!unfused_mlp) return mlp_fused_run(x, w.m1, T, live, S, wl + kOffMlp1, wl + kOffMlp2, ln + 256, ln + 384, st);
   P = LinParams{};
   P.mode[0] = EPI_RELU; P.mode[1] = EPI_RELU;
   const Dst oh[3] = {{w.h, 2 * kD}, {w.h + kD, 2 * kD}, {nullptr, 0}};
-  if ((e = linear_run(T, {x, kD, kD}, {w.m1, kD, kD}, wl + kOffMlp1, 256, 256, 256, oh, nullptr, P, st)) != cudaSuccess) return e;
+  if ((e = linear_run(T, live, S, {x, kD, kD}, {w.m1, kD, kD}, wl + kOffMlp1, 256, 256, 256, oh, nullptr, P, st)) != cudaSuccess) return e;
   P = LinParams{};
   P.mode[0] = EPI_LN_RES; P.gamma = ln + 256; P.beta = ln + 384;
   const Dst ox[3] = {{x, kD}, {nullptr, 0}, {nullptr, 0}};
-  return linear_run(T, {w.h, 2 * kD, 2 * kD}, none, wl + kOffMlp2, 128, 256, 256, ox, x, P, st);
+  return linear_run(T, live, S, {w.h, 2 * kD, 2 * kD}, none, wl + kOffMlp2, 128, 256, 256, ox, x, P, st);
 }
 
 }  // namespace
@@ -1000,11 +1072,13 @@ extern "C" size_t pope_fine_tf_workspace_bytes(int64_t m_windows, int window_tok
   return carve_tf(nullptr, m_windows, window_tokens).bytes;
 }
 
-extern "C" int pope_fine_transformer(void* feat0, void* feat1, int64_t m_windows, int window_tokens, const void* weights,
-                                     int n_layers, const int* layer_kinds, void* workspace, size_t workspace_bytes,
-                                     void* stream) {
+extern "C" int pope_fine_transformer_ex(void* feat0, void* feat1, int64_t m_windows, const int32_t* m_dev, int window_tokens,
+                                        const void* weights, int n_layers, const int* layer_kinds, void* workspace,
+                                        size_t workspace_bytes, void* stream) {
   if (!feat0 || !feat1 || !weights || !layer_kinds || !workspace) return POPE_ERR_INVALID_ARG;
   if (m_windows < 0 || window_tokens <= 0 || n_layers < 0) return POPE_ERR_INVALID_ARG;
+  for (int l = 0; l < n_layers; ++l)
+    if (layer_kinds[l] != 0 && layer_kinds[l] != 1) return POPE_ERR_INVALID_ARG;
   if ((reinterpret_cast<uintptr_t>(feat0) | reinterpret_cast<uintptr_t>(feat1) | reinterpret_cast<uintptr_t>(weights) |
        reinterpret_cast<uintptr_t>(workspace)) & 15u)
     return POPE_ERR_ALIGNMENT;
@@ -1018,16 +1092,21 @@ extern "C" int pope_fine_transformer(void* feat0, void* feat1, int64_t m_windows
     const char* wl = static_cast<const char*>(weights) + size_t(l) * kLayerBytes;
     cudaError_t e;
     if (layer_kinds[l] == 0) {            // 'self'  (transformer.py:96-98)
-      if ((e = encoder_layer(x0, x0, m_windows, window_tokens, wl, w, st)) != cudaSuccess) return int(e);
-      if ((e = encoder_layer(x1, x1, m_windows, window_tokens, wl, w, st)) != cudaSuccess) return int(e);
-    } else if (layer_kinds[l] == 1) {     // 'cross' (:99-101): feat1 attends to the UPDATED feat0
-      if ((e = encoder_layer(x0, x1, m_windows, window_tokens, wl, w, st)) != cudaSuccess) return int(e);
-      if ((e = encoder_layer(x1, x0, m_windows, window_tokens, wl, w, st)) != cudaSuccess) return int(e);
-    } else {
-      return POPE_ERR_INVALID_ARG;
+      if ((e = encoder_layer(x0, x0, m_windows, m_dev, window_tokens, wl, w, st)) != cudaSuccess) return int(e);
+      if ((e = encoder_layer(x1, x1, m_windows, m_dev, window_tokens, wl, w, st)) != cudaSuccess) return int(e);
+    } else {                              // 'cross' (:99-101): feat1 attends to the UPDATED feat0
+      if ((e = encoder_layer(x0, x1, m_windows, m_dev, window_tokens, wl, w, st)) != cudaSuccess) return int(e);
+      if ((e = encoder_layer(x1, x0, m_windows, m_dev, window_tokens, wl, w, st)) != cudaSuccess) return int(e);
     }
   }
   return POPE_OK;
+}
+
+extern "C" int pope_fine_transformer(void* feat0, void* feat1, int64_t m_windows, int window_tokens, const void* weights,
+                                     int n_layers, const int* layer_kinds, void* workspace, size_t workspace_bytes,
+                                     void* stream) {
+  return pope_fine_transformer_ex(feat0, feat1, m_windows, nullptr, window_tokens, weights, n_layers, layer_kinds, workspace,
+                                  workspace_bytes, stream);
 }
 
 static size_t merge_scratch_bytes(int64_t m) {
@@ -1039,10 +1118,10 @@ extern "C" size_t pope_fine_merge_workspace_bytes(int64_t m_windows) {
   return m_windows > 0 ? merge_scratch_bytes(m_windows) : 0;
 }
 
-extern "C" int pope_fine_merge_coarse(void* win0, void* win1, int64_t m_windows, int window_tokens, const void* feat_c0,
-                                      const void* feat_c1, int L, int S, int C, const int64_t* b_ids, const int64_t* i_ids,
-                                      const int64_t* j_ids, const void* weights, void* workspace, size_t workspace_bytes,
-                                      void* stream) {
+extern "C" int pope_fine_merge_coarse_ex(void* win0, void* win1, int64_t m_windows, const int32_t* m_dev, int window_tokens,
+                                         const void* feat_c0, const void* feat_c1, int L, int S, int C, const int64_t* b_ids,
+                                         const int64_t* i_ids, const int64_t* j_ids, const void* weights, void* workspace,
+                                         size_t workspace_bytes, void* stream) {
   if (!win0 || !win1 || !feat_c0 || !feat_c1 || !b_ids || !i_ids || !j_ids || !weights || !workspace)
     return POPE_ERR_INVALID_ARG;
   if (m_windows < 0 || window_tokens <= 0 || L <= 0 || S <= 0) return POPE_ERR_INVALID_ARG;
@@ -1058,28 +1137,48 @@ extern "C" int pope_fine_merge_coarse(void* win0, void* win1, int64_t m_windows,
   const char* wp = static_cast<const char*>(weights);
   const float* bias = reinterpret_cast<const float*>(wp + kOffPreBias);
   gather_coarse_rows_kernel<<<unsigned((2 * m + 7) / 8), 256, 0, st>>>(
-      static_cast<const __nv_bfloat16*>(feat_c0), static_cast<const __nv_bfloat16*>(feat_c1), b_ids, i_ids, j_ids, m, L, S, C, cg);
+      static_cast<const __nv_bfloat16*>(feat_c0), static_cast<const __nv_bfloat16*>(feat_c1), b_ids, i_ids, j_ids, m, m_dev, L, S,
+      C, cg);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return int(e);
-  // feat_c_win = down_proj(cat(c0, c1))                                                  (fine_preprocess.py:50-51)
+  // The [2m, .] arrays hold side 1 from row m (the capacity) on, so with a live count their live rows are [0, live) and
+  // [m, m + live): each side is then its own launch, bounded by the count.  Without one, both sides are a single launch.
+  const int nseg = m_dev ? 2 : 1;
+  const int64_t seg = 2 * m / nseg;
   const Src none{nullptr, 0, 0};
   LinParams P{};
-  P.mode[0] = EPI_COPY; P.bias = bias;
-  const Dst od[3] = {{cd, kD}, {nullptr, 0}, {nullptr, 0}};
-  if ((e = linear_run(2 * m, {cg, 256, 256}, none, wp + kOffDown, 128, 256, 256, od, nullptr, P, st)) != cudaSuccess) return int(e);
-  // merge_feat(cat(win, repeat(c))) = win . Wa^T + (c . Wb^T + bias): the second term once per window       (:52-55)
-  P = LinParams{};
-  P.out_f32 = cvec; P.mode[0] = EPI_COPY; P.bias = bias + 128;
-  const Dst onone[3] = {{nullptr, 0}, {nullptr, 0}, {nullptr, 0}};
-  if ((e = linear_run(2 * m, {cd, kD, kD}, none, wp + kOffMergeFeat + 128 * 2, 128, 128, 256, onone, nullptr, P, st)) != cudaSuccess)
-    return int(e);
+  for (int s = 0; s < nseg; ++s) {
+    // feat_c_win = down_proj(cat(c0, c1))                                                (fine_preprocess.py:50-51)
+    P = LinParams{};
+    P.mode[0] = EPI_COPY; P.bias = bias;
+    const Dst od[3] = {{cd + s * seg * kD, kD}, {nullptr, 0}, {nullptr, 0}};
+    if ((e = linear_run(seg, m_dev, 1, {cg + s * seg * 256, 256, 256}, none, wp + kOffDown, 128, 256, 256, od, nullptr, P, st)) !=
+        cudaSuccess)
+      return int(e);
+    // merge_feat(cat(win, repeat(c))) = win . Wa^T + (c . Wb^T + bias): the second term once per window     (:52-55)
+    P = LinParams{};
+    P.out_f32 = cvec + s * seg * kD; P.mode[0] = EPI_COPY; P.bias = bias + 128;
+    const Dst onone[3] = {{nullptr, 0}, {nullptr, 0}, {nullptr, 0}};
+    if ((e = linear_run(seg, m_dev, 1, {cd + s * seg * kD, kD, kD}, none, wp + kOffMergeFeat + 128 * 2, 128, 128, 256, onone, nullptr,
+                        P, st)) != cudaSuccess)
+      return int(e);
+  }
   for (int side = 0; side < 2; ++side) {
     void* win = side ? win1 : win0;
     P = LinParams{};
     P.mode[0] = EPI_ADDVEC; P.rowvec = cvec + size_t(side) * m * kD; P.rows_per_vec = window_tokens;
     const Dst ow[3] = {{win, kD}, {nullptr, 0}, {nullptr, 0}};
-    if ((e = linear_run(m * window_tokens, {win, kD, kD}, none, wp + kOffMergeFeat, 128, 128, 256, ow, nullptr, P, st)) != cudaSuccess)
+    if ((e = linear_run(m * window_tokens, m_dev, window_tokens, {win, kD, kD}, none, wp + kOffMergeFeat, 128, 128, 256, ow, nullptr,
+                        P, st)) != cudaSuccess)
       return int(e);
   }
   return POPE_OK;
+}
+
+extern "C" int pope_fine_merge_coarse(void* win0, void* win1, int64_t m_windows, int window_tokens, const void* feat_c0,
+                                      const void* feat_c1, int L, int S, int C, const int64_t* b_ids, const int64_t* i_ids,
+                                      const int64_t* j_ids, const void* weights, void* workspace, size_t workspace_bytes,
+                                      void* stream) {
+  return pope_fine_merge_coarse_ex(win0, win1, m_windows, nullptr, window_tokens, feat_c0, feat_c1, L, S, C, b_ids, i_ids, j_ids,
+                                   weights, workspace, workspace_bytes, stream);
 }

@@ -123,13 +123,15 @@ class DeviceBatchRunner:
     reduction, list evaluation, compaction) that need a fraction of an SM each; on alternating streams they run beside
     the next batch's sweep (B200, 64 pairs at 480x640: 0.97 -> 0.91 ms per batch).  No host synchronisation anywhere:
     results are capacity-sized `CoarseResult`s whose match count stays on the device; call `join()` before reading them
-    on another stream."""
+    on another stream.  With `submit(..., fine_level=Matcher.fine_level(device))` each batch also runs the bf16
+    FinePreprocess Linears and fine transformer (see `ops.match_pairs_device`), in a fine scratch kept per stream."""
 
     def __init__(self, device, n_streams: int = 2):
         self.device = torch.device(device)
         self.streams = ([torch.cuda.Stream(device=self.device) for _ in range(n_streams)] if n_streams > 1
                         else [torch.cuda.current_stream(self.device)])
         self.workspaces = [None] * len(self.streams)
+        self.fine_workspaces = [None] * len(self.streams)
         self._k = 0
         self._pending = []          # weak references to the results submitted since the last join()
 
@@ -152,20 +154,24 @@ class DeviceBatchRunner:
             res = ref()
             if res is not None and st != cur:
                 for key, v in res.items():
-                    if key != "workspace" and isinstance(v, torch.Tensor) and v.is_cuda:   # (the scratch stays with its stream)
+                    if key not in ("workspace", "fine_workspace") and isinstance(v, torch.Tensor) and v.is_cuda:   # (the scratch stays with its stream)
                         v.record_stream(cur)
         self._pending.clear()
 
-    def submit(self, feat_c0, feat_c1, feat_f0, feat_f1, hw0_i, hw0_c, hw1_c, after=None, **kw):
+    def submit(self, feat_c0, feat_c1, feat_f0, feat_f1, hw0_i, hw0_c, hw1_c, after=None, fine_level=None, **kw):
         """Queues one batch; returns (result, stream it was queued on).  `after(result)` runs inside the batch's stream
         context (e.g. to append the batch's records to a job buffer)."""
         from . import ops
         k = self._k % len(self.streams)
         self._k += 1
         with torch.cuda.stream(self.streams[k]):
+            if fine_level is not None:
+                kw.update(fine_level=fine_level, fine_workspace=self.fine_workspaces[k])
             res = ops.match_pairs_device(feat_c0, feat_c1, feat_f0, feat_f1, hw0_i, hw0_c, hw1_c,
                                          workspace=self.workspaces[k], **kw)
             self.workspaces[k] = res["workspace"]
+            if fine_level is not None:
+                self.fine_workspaces[k] = res["fine_workspace"]
             if after is not None:
                 after(res)
         if len(self._pending) >= 64:         # callers that never join(): forget the results that are gone

@@ -43,6 +43,17 @@ class Matcher(nn.Module):
         self.fine_preprocess.cuda_bf16 = bool(on)
         self.loftr_fine.inplace = bool(on)
 
+    def fine_level(self, device) -> dict:
+        """The packed bf16 weights of the fine level for `ops.match_pairs_device(..., fine_level=...)` (and the driver's
+        batched steps built on it): {"pre": FinePreprocess' down_proj + merge_feat (None when fine_concat_coarse_feat is
+        off), "layers": the fine transformer's layers, "layer_names": their 'self' / 'cross' schedule}.  The packed
+        tensors are the modules' own caches, repacked only when a parameter changes."""
+        if not self.loftr_fine.cuda_supported():
+            raise NotImplementedError("the CUDA fine transformer covers d_model 128 / 8 heads / linear attention")
+        dev = torch.device(device)
+        pre = self.fine_preprocess._packed_weights(dev) if self.fine_preprocess.cat_c_feat else None
+        return {"pre": pre, "layers": self.loftr_fine._packed_weights(dev), "layer_names": list(self.loftr_fine.layer_names)}
+
     def forward(self, data: dict, only_att_fea: bool = False):
         img0, img1 = data["image0"], data["image1"]
         data.update({"bs": img0.size(0), "hw0_i": img0.shape[2:], "hw1_i": img1.shape[2:]})

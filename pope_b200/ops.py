@@ -160,11 +160,19 @@ def fine_tf_workspace(m: int, ww: int, dev, workspace: Optional[torch.Tensor] = 
     return workspace
 
 
+def _check_m_dev(m_dev: Optional[torch.Tensor], dev) -> None:
+    if m_dev is not None and (m_dev.dtype != torch.int32 or m_dev.numel() < 1 or m_dev.device != dev):
+        raise _lib.PopeError("m_dev must be a device int32 tensor (the live count) on the device of the windows")
+
+
 def fine_transformer(feat0: torch.Tensor, feat1: torch.Tensor, packed_layers: torch.Tensor, layer_names,
-                     workspace: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+                     workspace: Optional[torch.Tensor] = None, m_dev: Optional[torch.Tensor] = None
+                     ) -> Tuple[torch.Tensor, torch.Tensor]:
     """LocalFeatureTransformer.forward on bf16 windows [M, WW, 128], IN PLACE (returns the same tensors).
-    `packed_layers`: concatenation of pack_fine_layer() of every layer, `layer_names`: 'self' / 'cross'."""
+    `packed_layers`: concatenation of pack_fine_layer() of every layer, `layer_names`: 'self' / 'cross'.
+    `m_dev` (device int32): live window count; M is then the capacity and windows >= *m_dev are left untouched."""
     dev = require_cuda(feat0, feat1, packed_layers)
+    _check_m_dev(m_dev, dev)
     if feat0.dtype != torch.bfloat16 or feat1.dtype != torch.bfloat16:
         raise _lib.PopeError("the CUDA fine transformer takes bfloat16 windows")
     if feat0.shape != feat1.shape or feat0.dim() != 3 or feat0.shape[2] != 128:
@@ -184,17 +192,19 @@ def fine_transformer(feat0: torch.Tensor, feat1: torch.Tensor, packed_layers: to
     workspace = fine_tf_workspace(M, WW, dev, workspace)
     arr = (_lib.C.c_int * max(len(kinds), 1))(*kinds)
     with torch.cuda.device(dev):
-        st = lib().pope_fine_transformer(ptr(feat0), ptr(feat1), M, WW, ptr(packed_layers), len(kinds), arr,
-                                         ptr(workspace), workspace.numel(), stream_ptr(dev))
+        st = lib().pope_fine_transformer_ex(ptr(feat0), ptr(feat1), M, ptr(m_dev), WW, ptr(packed_layers), len(kinds), arr,
+                                            ptr(workspace), workspace.numel(), stream_ptr(dev))
     check(st, "pope_fine_transformer")
     return feat0, feat1
 
 
 def fine_merge_coarse(win0: torch.Tensor, win1: torch.Tensor, feat_c0: torch.Tensor, feat_c1: torch.Tensor, b_ids, i_ids,
-                      j_ids, packed_pre: torch.Tensor, workspace: Optional[torch.Tensor] = None
-                      ) -> Tuple[torch.Tensor, torch.Tensor]:
-    """FinePreprocess' down_proj / merge_feat on bf16 windows [M, WW, 128], IN PLACE (returns the same tensors)."""
+                      j_ids, packed_pre: torch.Tensor, workspace: Optional[torch.Tensor] = None,
+                      m_dev: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """FinePreprocess' down_proj / merge_feat on bf16 windows [M, WW, 128], IN PLACE (returns the same tensors).
+    `m_dev` (device int32): live window count; M is then the capacity and windows / ids >= *m_dev are never touched."""
     dev = require_cuda(win0, win1, feat_c0, feat_c1, b_ids, i_ids, j_ids, packed_pre)
+    _check_m_dev(m_dev, dev)
     for t in (win0, win1, feat_c0, feat_c1):
         if t.dtype != torch.bfloat16 or not t.is_contiguous():
             raise _lib.PopeError("fine_merge_coarse takes contiguous bfloat16 tensors")
@@ -207,9 +217,9 @@ def fine_merge_coarse(win0: torch.Tensor, win1: torch.Tensor, feat_c0: torch.Ten
     if workspace is None or workspace.numel() < need or workspace.device != dev:
         workspace = torch.empty(need, dtype=torch.uint8, device=dev)
     with torch.cuda.device(dev):
-        st = lib().pope_fine_merge_coarse(ptr(win0), ptr(win1), M, WW, ptr(feat_c0), ptr(feat_c1), L, S, C_,
-                                          ptr(b_ids.contiguous()), ptr(i_ids.contiguous()), ptr(j_ids.contiguous()),
-                                          ptr(packed_pre), ptr(workspace), workspace.numel(), stream_ptr(dev))
+        st = lib().pope_fine_merge_coarse_ex(ptr(win0), ptr(win1), M, ptr(m_dev), WW, ptr(feat_c0), ptr(feat_c1), L, S, C_,
+                                             ptr(b_ids.contiguous()), ptr(i_ids.contiguous()), ptr(j_ids.contiguous()),
+                                             ptr(packed_pre), ptr(workspace), workspace.numel(), stream_ptr(dev))
     check(st, "pope_fine_merge_coarse")
     return win0, win1
 
@@ -292,11 +302,46 @@ def running_topk(scores: torch.Tensor, k: int = 3):
     return slot_s, slot_i
 
 
+def fine_level_workspace(m: int, ww: int, dev, workspace: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Scratch of the bf16 fine level for m windows of ww tokens: the FinePreprocess Linears and the fine transformer run
+    one after the other on one stream, so they share it (its size is the transformer's, 7 planes of [m * ww, 128] bf16)."""
+    need = max(lib().pope_fine_tf_workspace_bytes(int(m), int(ww)), lib().pope_fine_merge_workspace_bytes(int(m)), 16)
+    if workspace is None or workspace.numel() < need or workspace.device != dev:
+        workspace = torch.empty(need, dtype=torch.uint8, device=dev)
+    return workspace
+
+
+def _check_fine_level_inputs(feat_c0, feat_c1, feat_f0, feat_f1, W) -> None:
+    require_cuda(feat_c0, feat_c1, feat_f0, feat_f1)
+    if feat_c0.dtype != torch.bfloat16 or feat_c1.dtype != torch.bfloat16 or feat_c0.shape[-1] != 256:
+        raise _lib.PopeError("the bf16 fine level takes bfloat16 coarse features with C = 256")
+    if feat_f0.dtype != torch.bfloat16 or feat_f1.dtype != torch.bfloat16 or feat_f0.shape[1] != 128 \
+            or feat_f1.shape[1] != 128:
+        raise _lib.PopeError("the bf16 fine level takes bfloat16 fine maps with Cf = 128")
+    if W != 5:
+        raise _lib.PopeError("the bf16 fine level takes 5 x 5 windows")
+
+
 def match_pairs_device(feat_c0, feat_c1, feat_f0, feat_f1, hw0_i, hw0_c, hw1_c, thr=0.2, border_rm=2,
-                       temperature=0.1, W=5, impl=_lib.COARSE_AUTO, workspace=None, fused_fine=None) -> CoarseResult:
+                       temperature=0.1, W=5, impl=_lib.COARSE_AUTO, workspace=None, fused_fine=None, fine_level=None,
+                       fine_workspace=None) -> CoarseResult:
     """The hot path on device-resident inputs with NO host synchronisation: coarse match -> window gather ->
     fine match, the match count staying on the device (`m_dev`).  Returns the capacity-sized CoarseResult
-    extended with `expec_f`, `mkpts0_f`, `mkpts1_f` (and `win0`, `win1` on the unfused route)."""
+    extended with `expec_f`, `mkpts0_f`, `mkpts1_f` (and `win0`, `win1` on the unfused route).
+
+    `fine_level` (`Matcher.fine_level(device)`): also run what Matcher.forward runs between gather and fine matching --
+    FinePreprocess' two Linears and the fine transformer, in bf16 (csrc/fine_tf.cu) -- so that the step computes what
+    `Matcher(config, fine_cuda_bf16=True)` computes, bit for bit on the live rows, still without a host sync: every launch
+    is bounded by the device match count.  Needs bf16 coarse features (C = 256), bf16 fine maps (Cf = 128) and W = 5, and
+    takes the unfused route.  The result then also holds `fine_workspace` (pass it back in to reuse it).  Memory is sized
+    by the capacity n * L, not by the match count: at 64 pairs x 480x640 (307 200 windows) that is 3.9 GB of windows plus
+    13.8 GB of fine scratch per call, about 17.7 GB; the Matcher flow, sized by the count, needs about half of that at the
+    synthetic inputs' match rate."""
+    if fine_level is not None:
+        _check_fine_level_inputs(feat_c0, feat_c1, feat_f0, feat_f1, W)
+        if fused_fine:
+            raise _lib.PopeError("fine_level runs between window gather and fine matching: it takes the unfused route")
+        fused_fine = False
     res = coarse_match(feat_c0, feat_c1, hw0_c, hw1_c, hw0_i[0] / hw0_c[0], thr, border_rm, temperature, impl, workspace)
     n = res["n_pairs"]
     m_dev = res["counts"][n:n + 1]
@@ -304,7 +349,18 @@ def match_pairs_device(feat_c0, feat_c1, feat_f0, feat_f1, hw0_i, hw0_c, hw1_c, 
     coord_scale = (W // 2) * (hw0_i[0] / feat_f0.shape[2])
     if fused_fine is None:      # fused kernel needs channels-last maps; plain NCHW takes the two-kernel route
         fused_fine = feat_f0.stride(1) == 1 and feat_f1.stride(1) == 1 and feat_f0.shape[1] == 128 and W == 5
-    if fused_fine:
+    if fine_level is not None:
+        win0, win1 = fine_gather(feat_f0, feat_f1, res["b_ids"], res["i_ids"], res["j_ids"], hw0_c[1], hw1_c[1],
+                                 stride, W, m_dev)
+        cap = win0.shape[0]
+        fine_workspace = fine_level_workspace(cap, W * W, win0.device, fine_workspace)
+        if fine_level["pre"] is not None:
+            fine_merge_coarse(win0, win1, feat_c0.contiguous(), feat_c1.contiguous(), res["b_ids"], res["i_ids"],
+                              res["j_ids"], fine_level["pre"], fine_workspace, m_dev)
+        fine_transformer(win0, win1, fine_level["layers"], fine_level["layer_names"], fine_workspace, m_dev)
+        expec, mk1f = fine_match(win0, win1, res["mkpts1_c"], coord_scale, m_dev)
+        res.update(win0=win0, win1=win1, fine_workspace=fine_workspace)
+    elif fused_fine:
         # (match_order_by_ref + order= was measured neutral on B200: 10 us of sorting buys 13 us of gather; not used)
         expec, mk1f = fine_match_maps(feat_f0, feat_f1, res["b_ids"], res["i_ids"], res["j_ids"], res["mkpts1_c"],
                                       hw0_c[1], hw1_c[1], stride, coord_scale, W, m_dev)
