@@ -172,7 +172,9 @@ int pope_running_topk(const float* scores, int R, int k, float* slot_scores, int
  *             image 0 in place over the host link, and of image 1's map only the union of the matched cells' 5x5 windows is
  *             fetched (every needed pixel once) into the device slot (pageable maps are copied in bulk; POPE_PIPELINE_F1 =
  *             union | windows | bulk in the environment selects the form for image 1, see pope_pipeline_last_f1_mode;
- *             POPE_PIPELINE_WINDOWS_IN_PLACE=0 is the older spelling of bulk).
+ *             POPE_PIPELINE_WINDOWS_IN_PLACE=0 is the older spelling of bulk).  With a fine level attached
+ *             (pope_pipeline_set_fine_level) the fine transformer needs all 25 pixels of image 0's windows, so image 0's
+ *             map reaches the device in the same form as image 1's (a pageable image-0 buffer is copied whole).
  *   Outputs : per-pair slots of cap = min(L,S) entries: i_ids, j_ids int64[n][cap]; mconf float[n][cap];
  *             mkpts0_f, mkpts1_f float[n][cap][2]; counts int32[n]; flags (optional, may be NULL) int32[1] = OR of the
  *             POPE_FLAG_* bits of all chunks.  pope_pipeline_run returns after every copy has landed. */
@@ -187,15 +189,34 @@ int pope_pipeline_run(pope_pipeline_t* pl, const void* feat_c0, const void* feat
                       int64_t* i_ids, int64_t* j_ids, float* mconf, float* mkpts0_f, float* mkpts1_f,
                       int32_t* counts, int32_t* flags);
 int pope_pipeline_destroy(pope_pipeline_t* pl);
-/* Bytes that crossed the host link towards the device during the last pope_pipeline_run: the bulk copies plus, when
- * feat_f0 is page-locked, the centre pixels the fine kernel read directly from host memory (one Cf-vector per match;
- * the rest of image 0's fine map is never needed by this pipeline and is not transferred). */
+/* Bytes that crossed the host link towards the device during the last pope_pipeline_run: the bulk copies plus what the
+ * kernels read from page-locked fine maps.  Without a fine level that is, of image 0, the centre pixel of every matched
+ * cell (one Cf-vector per match: the rest of image 0's map is not needed and is not transferred), and of image 1 the union
+ * of the windows (union form) or every window whole (windows form).  With a fine level image 0 is counted like image 1:
+ * the pixels of its windows' union, M x 25 Cf-vectors, or the whole map. */
 int64_t pope_pipeline_last_h2d_bytes(const pope_pipeline_t* pl);
 /* How image 1's fine map reached the device in the last pope_pipeline_run: 0 = whole map copied (pageable buffer, or
- * POPE_PIPELINE_F1=bulk), 1 = the fine kernel read every match's 5x5 window in place (POPE_PIPELINE_F1=windows), 2 = the
+ * POPE_PIPELINE_F1=bulk), 1 = the kernels read every match's 5x5 window in place (POPE_PIPELINE_F1=windows), 2 = the
  * union of the matched cells' windows was fetched once per pixel into the device map (POPE_PIPELINE_F1=union); -1 for a
- * null handle.  No counterpart in the reference (its loop copies whole images, eval_linemod_json.py:103-122). */
+ * null handle.  With a fine level image 0 took the same form unless its buffer is pageable.  No counterpart in the
+ * reference (its loop copies whole images, eval_linemod_json.py:103-122). */
 int pope_pipeline_last_f1_mode(const pope_pipeline_t* pl);
+/* Attach the bf16 fine level (FinePreprocess Linears + fine transformer) to a pipeline: from now on every chunk runs
+ * coarse match -> window gather -> [merge_feat/down_proj] -> n_layers encoder layers -> fine match, which is what
+ * Matcher(config, fine_cuda_bf16=True) computes.  pre (may be NULL = fine_concat_coarse_feat off), layers: device
+ * pointers in the packed layouts of pope_fine_merge_coarse / pope_fine_transformer below, 16-byte aligned, on the
+ * pipeline's device, caller-owned and alive while the pipeline runs; layer_kinds[l] in {0 self, 1 cross}, copied.
+ * Requires a POPE_BF16 pipeline with C == 256 (Cf == 128 and W == 5 are already required by pope_pipeline_create).
+ * layers == NULL detaches the level again: the pipeline then runs exactly as one that never had it.
+ * The first attach allocates, once per pipeline and shared by its two slots (everything that touches them runs on the one
+ * compute stream), the windows win0 / win1 [chunk * min(L,S), 25, 128] bf16 and one fine scratch of
+ * max(pope_fine_tf_workspace_bytes(chunk * min(L,S), 25), pope_fine_merge_workspace_bytes(chunk * min(L,S))) bytes;
+ * pope_pipeline_destroy frees them.  At 16 pairs x 480x640 per chunk (76 800 windows) that is 0.98 GB of windows plus
+ * 3.4 GB of scratch (computed from the sizes).
+ * Returns POPE_ERR_INVALID_ARG (null handle; layers without layer_kinds or with n_layers < 1; a kind other than 0 / 1),
+ * POPE_ERR_DTYPE (fp32 pipeline), POPE_ERR_SHAPE (C != 256), POPE_ERR_ALIGNMENT, or a cudaError_t from an allocation. */
+int pope_pipeline_set_fine_level(pope_pipeline_t* pl, const void* pre, const void* layers, int n_layers,
+                                 const int* layer_kinds);
 
 /* One-shot convenience: create + run + destroy. */
 int pope_match_pairs_host(const void* feat_c0, const void* feat_c1, const void* feat_f0, const void* feat_f1,

@@ -63,6 +63,7 @@ SIGNATURES = {
     "pope_pipeline_destroy": (_i, [_p]),
     "pope_pipeline_last_h2d_bytes": (_i64, [_p]),
     "pope_pipeline_last_f1_mode": (_i, [_p]),
+    "pope_pipeline_set_fine_level": (_i, [_p, _p, _p, _i, C.POINTER(_i)]),
     "pope_match_pairs_host": (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _f, _f, _f, _f, _i, _i,
                                    _i, _i, _p, _p, _p, _p, _p, _p, _p]),
 }

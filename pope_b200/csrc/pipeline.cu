@@ -4,7 +4,9 @@
 // calls per test pair, each followed by three .cpu() syncs) by a chunked, double-buffered stream pipeline:
 //   copy stream   : host -> device copies of chunk k+1
 //   compute stream: coarse match -> fused window gather + fine match -> per-pair slotting of chunk k (no host sync:
-//                   the match count stays on the device and gates the fine kernels)
+//                   the match count stays on the device and gates the fine kernels); with a fine level attached
+//                   (pope_pipeline_set_fine_level) coarse match -> window gather -> FinePreprocess Linears -> fine
+//                   transformer -> fine match -> slotting, every launch bounded by the same device count
 //   drain stream  : device -> host copies of chunk k-1
 // One host synchronisation at the very end.
 #include <new>
@@ -40,7 +42,7 @@ __global__ void __launch_bounds__(256) slot_kernel(const int32_t* __restrict__ c
   }
 }
 
-// ---- union fetch of image 1's fine windows ---------------------------------------------------------------------------
+// ---- union fetch of the fine windows (image 1; with a fine level also image 0) ----------------------------------------
 // The 5x5 windows of neighbouring matched cells overlap (window pitch = fine_stride < 5) and reads from page-locked host memory
 // are not kept in L2, so fetching window by window moves the shared pixels once per window.  Instead the chunk's matched
 // image-1 cells are marked in a byte map, and one kernel walks the fine map's pixels: a pixel that lies in the window of at
@@ -111,11 +113,26 @@ __global__ void __launch_bounds__(256) fetch_union_kernel(const uint4* __restric
   if (threadIdx.x == 0 && s_cnt) atomicAdd(fetched, (unsigned long long)s_cnt);
 }
 
+// the union fetch of one chunk's [n, Hf, Wf, Cf] fine map whose matched cells of the hc x wc grid are marked in cellmask
+cudaError_t launch_fetch_union(const char* src, char* dst, const uint8_t* cellmask, int n, int Hf, int Wf, int hc, int wc,
+                               int stride, int half, size_t pixel_bytes, unsigned long long* fetched, cudaStream_t st) {
+  const int64_t np = int64_t(n) * Hf * Wf;
+  const int lpp = int(pixel_bytes / 16), ppw = kFetchIt * (32 / lpp);                 // pixels per warp
+  const unsigned blocks = unsigned((np + 8 * ppw - 1) / (8 * ppw));                   // 8 warps per block
+  const uint4* s = reinterpret_cast<const uint4*>(src);
+  uint4* d = reinterpret_cast<uint4*>(dst);
+  if (lpp == 16)
+    fetch_union_kernel<16><<<blocks, 256, 0, st>>>(s, d, cellmask, np, Hf, Wf, hc, wc, stride, half, fetched);
+  else
+    fetch_union_kernel<32><<<blocks, 256, 0, st>>>(s, d, cellmask, np, Hf, Wf, hc, wc, stride, half, fetched);
+  return cudaGetLastError();
+}
+
 // default of POPE_PIPELINE_F1 for page-locked fine maps
 constexpr bool kF1UnionDefault = true;
 
 struct Slot {
-  char *fc0 = nullptr, *fc1 = nullptr, *ff0 = nullptr, *ff1 = nullptr, *ws = nullptr, *win0 = nullptr, *win1 = nullptr;
+  char *fc0 = nullptr, *fc1 = nullptr, *ff0 = nullptr, *ff1 = nullptr, *ws = nullptr;
   int64_t *b_ids = nullptr, *i_ids = nullptr, *j_ids = nullptr, *o_i = nullptr, *o_j = nullptr;
   float *mconf = nullptr, *mk0 = nullptr, *mk1 = nullptr, *expec = nullptr, *mk1f = nullptr, *o_conf = nullptr,
         *o_mk0 = nullptr, *o_mk1 = nullptr;
@@ -137,9 +154,18 @@ struct pope_pipeline {
   int last_f1_mode = 0;            // how image 1's fine map reached the device in the last run: 0 bulk, 1 windows in place, 2 union fetch
   int64_t last_h2d_bytes = 0;      // bytes that crossed the host link towards the device in the last run
   cudaStream_t s_copy = nullptr, s_comp = nullptr, s_drain = nullptr;
-  unsigned long long* fetched = nullptr;     // device: pixels of image 1's fine map the union fetch has copied in this run
+  unsigned long long* fetched = nullptr;     // device: pixels of the fine maps the union fetch has copied in this run
   unsigned long long* h_fetched = nullptr;   // pinned staging for it
   Slot slot[2];
+  // the bf16 fine level (pope_pipeline_set_fine_level): caller-owned packed weights; windows, image 0's cell mask and
+  // scratch are allocated on the first attach and shared by both slots (all of it is touched on s_comp only)
+  const void* fine_pre = nullptr;
+  const void* fine_layers = nullptr;
+  int fine_n_layers = 0;
+  int* fine_kinds = nullptr;                 // host copy of layer_kinds
+  char *win0 = nullptr, *win1 = nullptr, *fine_ws = nullptr;
+  size_t fine_ws_bytes = 0;
+  uint8_t* cellmask0 = nullptr;              // [chunk, L] matched image-0 cells of the chunk (union fetch of image 0)
 };
 
 #define PL_CUDA(x)                                   \
@@ -152,7 +178,7 @@ extern "C" int pope_pipeline_destroy(pope_pipeline_t* pl) {
   if (!pl) return POPE_OK;
   cudaSetDevice(pl->device);
   for (Slot& s : pl->slot) {
-    void* bufs[] = {s.fc0, s.fc1, s.ff0, s.ff1, s.ws, s.win0, s.win1, s.b_ids, s.i_ids, s.j_ids, s.o_i, s.o_j, s.mconf,
+    void* bufs[] = {s.fc0, s.fc1, s.ff0, s.ff1, s.ws, s.b_ids, s.i_ids, s.j_ids, s.o_i, s.o_j, s.mconf,
                     s.mk0, s.mk1, s.expec, s.mk1f, s.o_conf, s.o_mk0, s.o_mk1, s.counts, s.cellmask};
     for (void* b : bufs) if (b) cudaFree(b);
     if (s.h_counts) cudaFreeHost(s.h_counts);
@@ -162,6 +188,9 @@ extern "C" int pope_pipeline_destroy(pope_pipeline_t* pl) {
   }
   if (pl->fetched) cudaFree(pl->fetched);
   if (pl->h_fetched) cudaFreeHost(pl->h_fetched);
+  void* fine_bufs[] = {pl->win0, pl->win1, pl->fine_ws, pl->cellmask0};
+  for (void* b : fine_bufs) if (b) cudaFree(b);
+  free(pl->fine_kinds);
   if (pl->s_copy) cudaStreamDestroy(pl->s_copy);
   if (pl->s_comp) cudaStreamDestroy(pl->s_comp);
   if (pl->s_drain) cudaStreamDestroy(pl->s_drain);
@@ -225,6 +254,50 @@ fail:
   return rc;
 }
 
+extern "C" int pope_pipeline_set_fine_level(pope_pipeline_t* pl, const void* pre, const void* layers, int n_layers,
+                                            const int* layer_kinds) {
+  if (!pl) return POPE_ERR_INVALID_ARG;
+  if (!layers) {                 // detach; the windows and scratch stay allocated until pope_pipeline_destroy
+    pl->fine_pre = pl->fine_layers = nullptr;
+    pl->fine_n_layers = 0;
+    return POPE_OK;
+  }
+  if (n_layers < 1 || !layer_kinds) return POPE_ERR_INVALID_ARG;
+  for (int l = 0; l < n_layers; ++l)
+    if (layer_kinds[l] != 0 && layer_kinds[l] != 1) return POPE_ERR_INVALID_ARG;
+  if (pl->dtype != POPE_BF16) return POPE_ERR_DTYPE;
+  if (pl->C != 256) return POPE_ERR_SHAPE;
+  if ((reinterpret_cast<uintptr_t>(pre) | reinterpret_cast<uintptr_t>(layers)) & 15u) return POPE_ERR_ALIGNMENT;
+  int rc = POPE_OK;
+  int* kinds = static_cast<int*>(malloc(sizeof(int) * size_t(n_layers)));
+  if (!kinds) return int(cudaErrorMemoryAllocation);
+  for (int l = 0; l < n_layers; ++l) kinds[l] = layer_kinds[l];
+  if (!pl->win0) {
+    // sized by the chunk's capacity, like every other slot buffer: the launches are bounded by the device count
+    const int64_t m = int64_t(pl->chunk) * pl->cap;
+    const size_t win_bytes = size_t(m) * pl->W * pl->W * pl->Cf * 2;
+    const size_t tf = pope_fine_tf_workspace_bytes(m, pl->W * pl->W), mg = pope_fine_merge_workspace_bytes(m);
+    PL_CUDA(cudaSetDevice(pl->device));
+    PL_CUDA(cudaMalloc(&pl->win0, win_bytes));
+    PL_CUDA(cudaMalloc(&pl->win1, win_bytes));
+    PL_CUDA(cudaMalloc(&pl->fine_ws, tf > mg ? tf : mg));
+    PL_CUDA(cudaMalloc(&pl->cellmask0, size_t(pl->chunk) * pl->L));
+    pl->fine_ws_bytes = tf > mg ? tf : mg;
+  }
+  free(pl->fine_kinds);
+  pl->fine_kinds = kinds;
+  pl->fine_pre = pre;
+  pl->fine_layers = layers;
+  pl->fine_n_layers = n_layers;
+  return POPE_OK;
+fail:
+  free(kinds);
+  cudaFree(pl->win0); cudaFree(pl->win1); cudaFree(pl->fine_ws); cudaFree(pl->cellmask0);   // (cudaFree(NULL) is a no-op)
+  pl->win0 = pl->win1 = pl->fine_ws = nullptr;
+  pl->cellmask0 = nullptr;
+  return rc;
+}
+
 extern "C" int pope_pipeline_run(pope_pipeline_t* pl, const void* feat_c0, const void* feat_c1, const void* feat_f0,
                                  const void* feat_f1, int n_pairs, int64_t* i_ids, int64_t* j_ids, float* mconf,
                                  float* mkpts0_f, float* mkpts1_f, int32_t* counts, int32_t* flags) {
@@ -240,8 +313,8 @@ extern "C" int pope_pipeline_run(pope_pipeline_t* pl, const void* feat_c0, const
   const int64_t st0[4] = {int64_t(Hf0) * Wf0 * int64_t(Cf), 1, int64_t(Wf0) * int64_t(Cf), int64_t(Cf)};
   const int64_t st1[4] = {int64_t(Hf1) * Wf1 * int64_t(Cf), 1, int64_t(Wf1) * int64_t(Cf), int64_t(Cf)};
   const float coord_scale = float(pl->W / 2) * pl->fine_scale;
-  // Of image 0's fine map the pipeline only ever reads the centre pixel of each MATCHED cell (window 0 contributes its
-  // centre row to the fine correlation, fine_matching.py:43).  When the caller's buffer is page-locked (device-
+  // Without a fine level, of image 0's fine map the pipeline only ever reads the centre pixel of each MATCHED cell (window
+  // 0 contributes its centre row to the fine correlation, fine_matching.py:43).  When the caller's buffer is page-locked (device-
   // addressable under UVA) the fused fine kernel fetches those pixels straight from host memory (M x 256 B per chunk
   // instead of copying the whole 1/2-resolution map); pageable buffers fall back to the bulk copy.
   const char* f0_dev_view = nullptr;
@@ -272,7 +345,12 @@ extern "C" int pope_pipeline_run(pope_pipeline_t* pl, const void* feat_c0, const
     if (!bulk) f1_dev_view = host_view(feat_f1);
     if (!f1_dev_view || (Cf * e != 256 && Cf * e != 512)) f1_union = false;
   }
-  const int64_t n_pix1 = int64_t(Hf1) * Wf1;          // pixels of one image-1 fine map
+  // With a fine level the transformer needs all W*W pixels of image 0's windows, not only their centres, so image 0 takes
+  // the form chosen for image 1: its windows' union is fetched into the slot's device map, the gather reads its windows in
+  // place, or (image 1 copied whole, or a pageable image-0 buffer) the whole map is copied.  (f0_union implies f1_union.)
+  const bool fine = pl->fine_layers != nullptr;
+  if (fine && !f1_dev_view) f0_dev_view = nullptr;
+  const bool f0_union = fine && f1_union && f0_dev_view;
   int64_t h2d = 0;
   int32_t flag_acc = 0;
   int n_chunks = (n_pairs + pl->chunk - 1) / pl->chunk;
@@ -305,23 +383,43 @@ extern "C" int pope_pipeline_run(pope_pipeline_t* pl, const void* feat_c0, const
     if (f1_union) {
       PL_CUDA(cudaMemsetAsync(s.cellmask, 0, size_t(n) * S, pl->s_comp));
       mark_cells_kernel<<<64, 256, 0, pl->s_comp>>>(s.counts + n, int64_t(capt), s.b_ids, s.j_ids, int(S), s.cellmask);
-      const uint4* src = reinterpret_cast<const uint4*>(f1_dev_view + p0 * ff1_pair);
-      const int64_t np = int64_t(n) * n_pix1;
-      const int lpp = int(Cf * e / 16), ppw = kFetchIt * (32 / lpp);                   // pixels per warp
-      const unsigned blocks = unsigned((np + 8 * ppw - 1) / (8 * ppw));                // 8 warps per block
-      if (lpp == 16)
-        fetch_union_kernel<16><<<blocks, 256, 0, pl->s_comp>>>(src, reinterpret_cast<uint4*>(s.ff1), s.cellmask, np, Hf1, Wf1,
-                                                             pl->h1c, pl->w1c, pl->fstride, pl->W / 2, pl->fetched);
-      else
-        fetch_union_kernel<32><<<blocks, 256, 0, pl->s_comp>>>(src, reinterpret_cast<uint4*>(s.ff1), s.cellmask, np, Hf1, Wf1,
-                                                             pl->h1c, pl->w1c, pl->fstride, pl->W / 2, pl->fetched);
-      PL_CUDA(cudaGetLastError());
+      PL_CUDA(launch_fetch_union(f1_dev_view + p0 * ff1_pair, s.ff1, s.cellmask, n, Hf1, Wf1, pl->h1c, pl->w1c, pl->fstride,
+                                 pl->W / 2, Cf * e, pl->fetched, pl->s_comp));
     }
-    rc = pope_fine_match_maps(f0_dev_view ? static_cast<const void*>(f0_dev_view + p0 * ff0_pair) : s.ff0,
-                              (f1_dev_view && !f1_union) ? static_cast<const void*>(f1_dev_view + p0 * ff1_pair) : s.ff1, pl->dtype, n, pl->Cf, Hf0, Wf0, st0, Hf1, Wf1, st1, pl->w0c, pl->w1c,
-                              pl->fstride, pl->W, s.b_ids, s.i_ids, s.j_ids, int64_t(capt), s.counts + n, nullptr, s.mk1,
-                              coord_scale, s.expec, s.mk1f, pl->s_comp);
-    if (rc) goto fail;
+    if (f0_union) {
+      PL_CUDA(cudaMemsetAsync(pl->cellmask0, 0, size_t(n) * L, pl->s_comp));
+      mark_cells_kernel<<<64, 256, 0, pl->s_comp>>>(s.counts + n, int64_t(capt), s.b_ids, s.i_ids, int(L), pl->cellmask0);
+      PL_CUDA(launch_fetch_union(f0_dev_view + p0 * ff0_pair, s.ff0, pl->cellmask0, n, Hf0, Wf0, pl->h0c, pl->w0c, pl->fstride,
+                                 pl->W / 2, Cf * e, pl->fetched, pl->s_comp));
+    }
+    if (fine) {
+      // gather -> [down_proj / merge_feat] -> encoder layers -> fine match on the windows, all bounded by the chunk's count
+      const int64_t m = int64_t(capt);
+      const int32_t* m_dev = s.counts + n;
+      const int ww = pl->W * pl->W;
+      rc = pope_fine_gather((f0_dev_view && !f0_union) ? static_cast<const void*>(f0_dev_view + p0 * ff0_pair) : s.ff0,
+                            (f1_dev_view && !f1_union) ? static_cast<const void*>(f1_dev_view + p0 * ff1_pair) : s.ff1,
+                            pl->dtype, n, pl->Cf, Hf0, Wf0, st0, Hf1, Wf1, st1, pl->w0c, pl->w1c, pl->fstride, pl->W, s.b_ids,
+                            s.i_ids, s.j_ids, m, m_dev, pl->win0, pl->win1, pl->s_comp);
+      if (rc) goto fail;
+      if (pl->fine_pre) {
+        rc = pope_fine_merge_coarse_ex(pl->win0, pl->win1, m, m_dev, ww, s.fc0, s.fc1, pl->L, pl->S, pl->C, s.b_ids, s.i_ids,
+                                       s.j_ids, pl->fine_pre, pl->fine_ws, pl->fine_ws_bytes, pl->s_comp);
+        if (rc) goto fail;
+      }
+      rc = pope_fine_transformer_ex(pl->win0, pl->win1, m, m_dev, ww, pl->fine_layers, pl->fine_n_layers, pl->fine_kinds,
+                                    pl->fine_ws, pl->fine_ws_bytes, pl->s_comp);
+      if (rc) goto fail;
+      rc = pope_fine_match(pl->win0, pl->win1, pl->dtype, m, m_dev, ww, pl->Cf, s.mk1, coord_scale, s.expec, s.mk1f,
+                           pl->s_comp);
+      if (rc) goto fail;
+    } else {
+      rc = pope_fine_match_maps(f0_dev_view ? static_cast<const void*>(f0_dev_view + p0 * ff0_pair) : s.ff0,
+                                (f1_dev_view && !f1_union) ? static_cast<const void*>(f1_dev_view + p0 * ff1_pair) : s.ff1, pl->dtype, n, pl->Cf, Hf0, Wf0, st0, Hf1, Wf1, st1, pl->w0c, pl->w1c,
+                                pl->fstride, pl->W, s.b_ids, s.i_ids, s.j_ids, int64_t(capt), s.counts + n, nullptr, s.mk1,
+                                coord_scale, s.expec, s.mk1f, pl->s_comp);
+      if (rc) goto fail;
+    }
     slot_kernel<<<n, 256, 0, pl->s_comp>>>(s.counts, n, int(cap), s.i_ids, s.j_ids, s.mconf, s.mk0, s.mk1f, s.o_i, s.o_j,
                                            s.o_conf, s.o_mk0, s.o_mk1);
     PL_CUDA(cudaGetLastError());
@@ -343,10 +441,11 @@ extern "C" int pope_pipeline_run(pope_pipeline_t* pl, const void* feat_c0, const
   if (f0_dev_view || (f1_dev_view && !f1_union)) {   // what the fine kernel read in place also crossed the host link
     int64_t m = 0;
     for (int p = 0; p < n_pairs; ++p) m += counts[p];
-    if (f0_dev_view) h2d += m * int64_t(Cf * e);                                             // image 0: the centre pixels
+    if (f0_dev_view && !fine) h2d += m * int64_t(Cf * e);                                    // image 0: the centre pixels
+    if (f0_dev_view && fine && !f0_union) h2d += m * int64_t(pl->W * pl->W) * int64_t(Cf * e);   // image 0: every window whole
     if (f1_dev_view && !f1_union) h2d += m * int64_t(pl->W * pl->W) * int64_t(Cf * e);       // image 1: every window whole
   }
-  if (f1_union) h2d += int64_t(*pl->h_fetched) * int64_t(Cf * e);            // every pixel of the windows' union exactly once
+  if (f1_union) h2d += int64_t(*pl->h_fetched) * int64_t(Cf * e);   // every pixel of the windows' union(s) exactly once
   pl->last_f1_mode = f1_union ? 2 : f1_dev_view ? 1 : 0;
   pl->last_h2d_bytes = h2d;
   return POPE_OK;

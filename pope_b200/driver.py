@@ -30,13 +30,37 @@ def _fine_to_nhwc(ff: torch.Tensor) -> torch.Tensor:
     return ff.permute(0, 2, 3, 1).contiguous()
 
 
+def _check_fine_level(fine_level: dict, dtype: torch.dtype, C_coarse: int, device: int):
+    """What `pope_pipeline_set_fine_level` needs, checked before any GPU call; returns its (pre, layers, kinds) arguments."""
+    if dtype != torch.bfloat16 or C_coarse != 256:
+        raise _lib.PopeError("the bf16 fine level needs a bfloat16 pipeline with C_coarse = 256")
+    names, layers, pre = list(fine_level["layer_names"]), fine_level["layers"], fine_level["pre"]
+    if not names or any(nm not in ("self", "cross") for nm in names) \
+            or layers.numel() != len(names) * _lib.FINE_TF_LAYER_BYTES:
+        raise _lib.PopeError("the fine level's layer names and packed layers do not agree")
+    if pre is not None and pre.numel() != _lib.FINE_PRE_BYTES:
+        raise _lib.PopeError("the fine level's packed FinePreprocess weights have the wrong size")
+    dev = torch.device("cuda", device)
+    for t in (layers, pre):
+        if t is not None and (t.device != dev or t.dtype != torch.uint8 or not t.is_contiguous()):
+            raise _lib.PopeError(f"the fine level's packed weights must be contiguous uint8 tensors on {dev} "
+                                 f"(Matcher.fine_level({dev}))")
+    return pre, layers, (C.c_int * len(names))(*[0 if nm == "self" else 1 for nm in names])
+
+
 class Pipeline:
-    """Owns one `pope_pipeline_t` (device slots + streams for one geometry)."""
+    """Owns one `pope_pipeline_t` (device slots + streams for one geometry).
+
+    `fine_level` (`Matcher.fine_level(torch.device("cuda", device))`): every chunk also runs what Matcher.forward runs between
+    window gather and fine matching -- FinePreprocess' two Linears and the fine transformer, in bf16 -- so that the results
+    equal `ops.match_pairs_device(..., fine_level=...)` and thereby `Matcher(config, fine_cuda_bf16=True)`, bit for bit.
+    Needs a bf16 pipeline with C_coarse = 256.  The pipeline keeps a reference to the dict, so the packed weights outlive
+    the handle; it allocates windows and fine scratch for one chunk (0.98 GB + 3.4 GB at 16 pairs of 480x640)."""
 
     def __init__(self, dtype: torch.dtype, chunk_pairs: int, hw0_i: Sequence[int], hw0_c: Sequence[int],
                  hw1_c: Sequence[int], C_coarse: int = 256, C_fine: int = 128, fine_stride: int = 4, W: int = 5,
                  thr: float = 0.2, border_rm: int = 2, temperature: float = 0.1, impl: int = _lib.COARSE_AUTO,
-                 device: int = 0):
+                 device: int = 0, fine_level: Optional[dict] = None):
         self.dtype, self.chunk, self.device = dtype, chunk_pairs, device
         self.hw0_c, self.hw1_c = tuple(hw0_c), tuple(hw1_c)
         self.L, self.S = hw0_c[0] * hw0_c[1], hw1_c[0] * hw1_c[1]
@@ -46,6 +70,8 @@ class Pipeline:
         code = _lib.POPE_BF16 if dtype == torch.bfloat16 else _lib.POPE_F32
         if dtype not in (torch.float32, torch.bfloat16):
             raise _lib.PopeError(f"unsupported dtype {dtype}")
+        if fine_level is not None:
+            _check_fine_level(fine_level, dtype, C_coarse, device)
         pixel_scale = hw0_i[0] / hw0_c[0]
         fine_scale = hw0_i[0] / (hw0_c[0] * fine_stride)
         st = lib().pope_pipeline_create(C.byref(self._h), device, code, chunk_pairs, C_coarse, C_fine,
@@ -53,6 +79,27 @@ class Pipeline:
                                         float(pixel_scale), float(fine_scale), float(temperature), float(thr),
                                         int(border_rm), int(impl))
         check(st, "pope_pipeline_create")
+        self.fine_level = None
+        if fine_level is not None:
+            try:
+                self.set_fine_level(fine_level)
+            except BaseException:
+                self.close()
+                raise
+
+    def set_fine_level(self, fine_level: Optional[dict]) -> None:
+        """Attach a fine level (see the class docstring) or, with None, detach it: the pipeline then returns what a pipeline
+        created without one returns."""
+        if fine_level is None:
+            check(lib().pope_pipeline_set_fine_level(self._h, None, None, 0, None), "pope_pipeline_set_fine_level")
+            self.fine_level = None
+            return
+        pre, layers, kinds = _check_fine_level(fine_level, self.dtype, self.C, self.device)
+        # the weights may have been packed just now on torch's stream, which the pipeline's own streams do not wait for
+        torch.cuda.current_stream(layers.device).synchronize()
+        check(lib().pope_pipeline_set_fine_level(self._h, None if pre is None else pre.data_ptr(), layers.data_ptr(),
+                                                 len(kinds), kinds), "pope_pipeline_set_fine_level")
+        self.fine_level = fine_level          # keeps the packed tensors alive while the handle may read them
 
     def alloc_outputs(self, n: int, pinned: bool = True) -> Dict[str, torch.Tensor]:
         kw = dict(pin_memory=pinned)
@@ -65,7 +112,9 @@ class Pipeline:
                 "flags": torch.zeros(1, dtype=torch.int32, **kw)}
 
     def run(self, feat_c0, feat_c1, feat_f0_nhwc, feat_f1_nhwc, out: Optional[Dict[str, torch.Tensor]] = None):
-        """Inputs: CPU tensors feat_c* [n,L|S,C], feat_f*_nhwc [n,Hf,Wf,Cf] (memory order), same dtype."""
+        """Inputs: CPU tensors feat_c* [n,L|S,C], feat_f*_nhwc [n,Hf,Wf,Cf] (memory order), same dtype.  Outputs: per-pair
+        slots (`flatten_slots` packs them) holding what `ops.match_pairs_device` returns on the same inputs -- with the fine
+        level attached, what it returns with `fine_level=`."""
         n = feat_c0.shape[0]
         for t in (feat_c0, feat_c1, feat_f0_nhwc, feat_f1_nhwc):
             if t.dtype != self.dtype or not t.is_contiguous() or t.device.type != "cpu":
@@ -94,11 +143,13 @@ class Pipeline:
 
 
 def match_pairs_host(feat_c0, feat_c1, feat_f0, feat_f1, hw0_i, hw0_c, hw1_c, chunk_pairs: int = 16, device: int = 0,
-                     **kw) -> Dict[str, torch.Tensor]:
-    """One-shot host-buffer entry: feat_f* are logical [N, Cf, Hf, Wf] CPU tensors (channels-last is free)."""
+                     fine_level: Optional[dict] = None, **kw) -> Dict[str, torch.Tensor]:
+    """One-shot host-buffer entry: feat_f* are logical [N, Cf, Hf, Wf] CPU tensors (channels-last is free).  With
+    `fine_level` (`Matcher.fine_level(torch.device("cuda", device))`) the results equal what
+    `Matcher(config, fine_cuda_bf16=True)` computes from these features (see `Pipeline`)."""
     n = feat_c0.shape[0]
     pl = Pipeline(feat_c0.dtype, min(chunk_pairs, n), hw0_i, hw0_c, hw1_c, feat_c0.shape[2], feat_f0.shape[1],
-                  feat_f0.shape[2] // hw0_c[0], device=device, **kw)
+                  feat_f0.shape[2] // hw0_c[0], device=device, fine_level=fine_level, **kw)
     try:
         return pl.run(_pin(feat_c0), _pin(feat_c1), _fine_to_nhwc(feat_f0), _fine_to_nhwc(feat_f1))
     finally:
