@@ -212,7 +212,7 @@ int pope_pipeline_last_f1_mode(const pope_pipeline_t* pl);
  * compute stream), the windows win0 / win1 [chunk * min(L,S), 25, 128] bf16 and one fine scratch of
  * max(pope_fine_tf_workspace_bytes(chunk * min(L,S), 25), pope_fine_merge_workspace_bytes(chunk * min(L,S))) bytes;
  * pope_pipeline_destroy frees them.  At 16 pairs x 480x640 per chunk (76 800 windows) that is 0.98 GB of windows plus
- * 3.4 GB of scratch (computed from the sizes).
+ * 2.5 GB of scratch (computed from the sizes).
  * Returns POPE_ERR_INVALID_ARG (null handle; layers without layer_kinds or with n_layers < 1; a kind other than 0 / 1),
  * POPE_ERR_DTYPE (fp32 pipeline), POPE_ERR_SHAPE (C != 256), POPE_ERR_ALIGNMENT, or a cudaError_t from an allocation. */
 int pope_pipeline_set_fine_level(pope_pipeline_t* pl, const void* pre, const void* layers, int n_layers,
@@ -325,7 +325,7 @@ int pope_write_png_batch(const char* const* paths, const unsigned char* const* i
 #define POPE_FINE_TF_LAYER_BYTES 329728
 #define POPE_FINE_PRE_BYTES 132096
 
-/* Bytes of device scratch for m_windows windows of window_tokens tokens (7 activation planes of [m*tokens, 128] bf16). */
+/* Bytes of device scratch for m_windows windows of window_tokens tokens (5 activation planes of [m*tokens, 128] bf16). */
 size_t pope_fine_tf_workspace_bytes(int64_t m_windows, int window_tokens);
 
 /* feat0, feat1: [m_windows, window_tokens, 128] bf16, updated IN PLACE by n_layers encoder layers;

@@ -7,13 +7,14 @@
 //   src/matcher/loftr_module/transformer.py:95-104     ('self' / 'cross' layer schedule)
 //   src/matcher/loftr_module/fine_preprocess.py:50-57  (down_proj of the matched coarse features, merge_feat on
 //                                                       cat(window, coarse))
-// Every Linear is one launch of linear_tc_kernel: a persistent, weight-stationary tcgen05 GEMM (the whole weight matrix
-// stays in shared memory, 128-token tiles of the activations stream through a TMA ring, accumulators in TMEM) whose
-// epilogue applies what follows the Linear in the reference (feature map, 1/S scale, ReLU, LayerNorm, residual, bias,
-// per-window vector) before the row is written back as bf16.  The attention itself (8 heads x 16 x 16 per 25-token
-// window) is a warp-per-window fp32 kernel.  Activations are bf16 in HBM, all arithmetic accumulates in fp32.
+// Every Linear outside the encoder MLP is one launch of linear_tc_kernel: a persistent, weight-stationary tcgen05 GEMM
+// (the whole weight matrix stays in shared memory, 128-token tiles of the activations stream through a TMA ring,
+// accumulators in TMEM) whose epilogue applies what follows the Linear in the reference (feature map, 1/S scale,
+// LayerNorm, bias, per-window vector) before the row is written back as bf16.  The encoder MLP (both Linears, the ReLU
+// between them, LayerNorm2 and the residual) is one launch of mlp_fused_kernel.  The attention itself (8 heads x 16 x 16
+// per window) is a warp-per-window kernel: mma.sync tensor cores for windows of at most 32 tokens, fp32 SIMT above.
+// Activations are bf16 in HBM, all arithmetic accumulates in fp32.
 #include <cuda.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "tc_ptx.cuh"
@@ -38,24 +39,24 @@ constexpr int kSmemBudget = 227 * 1024 - 1024;        // dynamic shared memory w
 // layout: [staging: 8 x 4 KB][barriers][weights: nbox x 16 KB][ring: stages x 16 KB]
 constexpr int kSmemOut = 0;
 constexpr int kSmemBar = kSmemOut + kEpiWarps * kStageOutBytes;
-constexpr int kNumBars = 1 + 2 * kMaxStages + 2 * kSlots + kEpiWarps;
+constexpr int kNumBars = 1 + 2 * kMaxStages + 2 * kSlots;
 constexpr int kSmemTmemPtr = kSmemBar + kNumBars * 8;
-constexpr int kSmemW = 34 * 1024;                     // first 1024-aligned offset past the barriers
+constexpr int kSmemW = 34 * 1024;                     // 1024-aligned, past the barriers (sets the ring depth below)
 static_assert(kSmemTmemPtr + 16 <= kSmemW, "barrier block overlaps the weights");
 constexpr int kSmemAlloc = kSmemBudget;               // > 113 KB -> one CTA per SM, so the CTA may take all 512 TMEM columns
 
-enum EpiMode : int { EPI_COPY = 0, EPI_ELU1 = 1, EPI_SCALE = 2, EPI_RELU = 3, EPI_LN = 4, EPI_LN_RES = 5, EPI_ADDVEC = 6 };
+enum EpiMode : int { EPI_COPY = 0, EPI_ELU1 = 1, EPI_SCALE = 2, EPI_LN = 3, EPI_ADDVEC = 4 };
 
 struct LinParams {
   int T;                       // token rows
-  int kchunks, kchunks0;       // K/64; the first kchunks0 chunks come from source 0, the rest from source 1 (torch.cat)
+  int kchunks;                 // K/64
   int nblk;                    // N/128
   int stages;                  // ring depth that fits beside the weights
   float* out_f32;              // if set: the (single) output block is written as fp32 rows [T, 128] with plain stores
   int mode[3];
   float scale;                 // EPI_SCALE
   const float* bias;           // [N] or nullptr, added before the mode is applied
-  const float* gamma;          // EPI_LN / EPI_LN_RES: [128]
+  const float* gamma;          // EPI_LN: [128]
   const float* beta;
   const float* rowvec;         // EPI_ADDVEC: [T / rows_per_vec, 128]
   int rows_per_vec;
@@ -89,14 +90,13 @@ __device__ __forceinline__ void store_staged_half_row(uint32_t my_row, uint32_t 
   }
 }
 
-// mapO[j]: output block j as a [T, 128] bf16 tensor (box 64 x 32 rows); mapR: residual [T, 128] (EPI_LN_RES).
+// mapX: activations [T, K]; mapO[j]: output block j as a [T, 128] bf16 tensor (box 64 x 32 rows).
 // kBounded: P.live is set (a separate instantiation, so that the unbounded launches keep their code and registers)
 template <bool kBounded>
 __global__ void __launch_bounds__(kLinThreads, 1)
-linear_tc_kernel(const __grid_constant__ CUtensorMap mapX0, const __grid_constant__ CUtensorMap mapX1,
-                 const __grid_constant__ CUtensorMap mapW, const __grid_constant__ CUtensorMap mapO0,
-                 const __grid_constant__ CUtensorMap mapO1, const __grid_constant__ CUtensorMap mapO2,
-                 const __grid_constant__ CUtensorMap mapR, const LinParams P) {
+linear_tc_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constant__ CUtensorMap mapW,
+                 const __grid_constant__ CUtensorMap mapO0, const __grid_constant__ CUtensorMap mapO1,
+                 const __grid_constant__ CUtensorMap mapO2, const LinParams P) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   const uint32_t sbase = smem_u32(smem);
@@ -104,7 +104,6 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapX0, const __grid_constan
   const uint32_t bar_w_full = bar0;
   const uint32_t bar_x_full = bar0 + 8, bar_x_empty = bar_x_full + 8 * kMaxStages;
   const uint32_t bar_acc_full = bar_x_empty + 8 * kMaxStages, bar_acc_empty = bar_acc_full + 8 * kSlots;
-  const uint32_t bar_res = bar_acc_empty + 8 * kSlots;           // one per epilogue warp (residual tile landed)
   volatile uint32_t* tmem_ptr_smem = reinterpret_cast<volatile uint32_t*>(smem + kSmemTmemPtr);
   // live rows: read into shared memory once, so the epilogue re-reads it where needed instead of holding a register
   volatile int* live_rows_smem = reinterpret_cast<volatile int*>(smem + kSmemTmemPtr + 8);
@@ -122,12 +121,11 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapX0, const __grid_constan
   const int stages = P.stages;
 
   if (warp == 0 && lane == 0) {
-    prefetch_tmap(&mapX0); prefetch_tmap(&mapX1); prefetch_tmap(&mapW);
-    prefetch_tmap(&mapO0); prefetch_tmap(&mapO1); prefetch_tmap(&mapO2); prefetch_tmap(&mapR);
+    prefetch_tmap(&mapX); prefetch_tmap(&mapW);
+    prefetch_tmap(&mapO0); prefetch_tmap(&mapO1); prefetch_tmap(&mapO2);
     mbar_init(bar_w_full, 1);
     for (int s = 0; s < kMaxStages; ++s) { mbar_init(bar_x_full + 8 * s, 1); mbar_init(bar_x_empty + 8 * s, 1); }
     for (int s = 0; s < kSlots; ++s) { mbar_init(bar_acc_full + 8 * s, 1); mbar_init(bar_acc_empty + 8 * s, 4); }
-    for (int s = 0; s < kEpiWarps; ++s) mbar_init(bar_res + 8 * s, 1);
     fence_barrier_init();
   }
   if (warp == 1) {
@@ -152,9 +150,7 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapX0, const __grid_constan
         for (int kc = 0; kc < P.kchunks; ++kc) {
           mbar_wait(bar_x_empty + 8 * stage, phase ^ 1);
           mbar_expect_tx(bar_x_full + 8 * stage, kBoxBytes);
-          const bool second = kc >= P.kchunks0;
-          tma_load_2d(smem_x + stage * kBoxBytes, second ? &mapX1 : &mapX0, bar_x_full + 8 * stage,
-                      (second ? kc - P.kchunks0 : kc) * kBoxK, t * kTile);
+          tma_load_2d(smem_x + stage * kBoxBytes, &mapX, bar_x_full + 8 * stage, kc * kBoxK, t * kTile);
           if (++stage == stages) { stage = 0; phase ^= 1; }
         }
     }
@@ -193,14 +189,15 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapX0, const __grid_constan
   } else {
     // =============================== epilogue: thread = token row, 128 channels in registers =========================
     // Rows leave through a 128B-swizzled shared-memory box and a TMA store (a thread-per-row store to global memory
-    // touches 32 different lines per instruction and was measured LSU-bound); the residual rows arrive the same way.
+    // touches 32 different lines per instruction and was measured LSU-bound).
     const int ew = warp - 2, set = ew >> 2, quad = warp & 3;
     const uint32_t lane_addr = uint32_t(quad * 32) << 16;
     const uint32_t stage_buf = sbase + kSmemOut + ew * kStageOutBytes;
     const uint32_t my_row = stage_buf + lane * 128;
     const uint32_t sw = uint32_t(lane & 7);
-    const uint32_t bar_my_res = bar_res + 8 * ew;
-    uint32_t res_phase = 0;
+    // my_row is 128-byte aligned, so chunk c8 of the row sits at my_row_sw ^ (c8 << 4): one LOP3 per store, which keeps
+    // ptxas from holding the eight chunk addresses across the item loop (at the 168-register cap it spilled them)
+    const uint32_t my_row_sw = my_row + (sw << 4);
     uint32_t item = 0;
     for (int t = blockIdx.x; t < ntiles; t += gridDim.x) {
       const int row0 = t * kTile + quad * 32, row = row0 + lane;
@@ -229,10 +226,7 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapX0, const __grid_constan
         } else if (mode == EPI_SCALE) {
 #pragma unroll
           for (int c = 0; c < kD; ++c) v[c] *= P.scale;
-        } else if (mode == EPI_RELU) {
-#pragma unroll
-          for (int c = 0; c < kD; ++c) v[c] = fmaxf(v[c], 0.f);
-        } else if (mode == EPI_LN || mode == EPI_LN_RES) {
+        } else if (mode == EPI_LN) {
           float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
 #pragma unroll
           for (int c = 0; c < kD; c += 4) { s0 += v[c]; s1 += v[c + 1]; s2 += v[c + 2]; s3 += v[c + 3]; }
@@ -251,33 +245,6 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapX0, const __grid_constan
             const float4 g = __ldg(g4 + (c >> 2)), b = __ldg(b4 + (c >> 2));
             v[c] = fmaf((v[c] - mean) * rstd, g.x, b.x); v[c + 1] = fmaf((v[c + 1] - mean) * rstd, g.y, b.y);
             v[c + 2] = fmaf((v[c + 2] - mean) * rstd, g.z, b.z); v[c + 3] = fmaf((v[c + 3] - mean) * rstd, g.w, b.w);
-          }
-          if (mode == EPI_LN_RES) {
-            // + x: the warp's 32 residual rows come through the staging box, one 64-column half at a time
-#pragma unroll
-            for (int half = 0; half < 2; ++half) {
-              if (lane == 0) {
-                tma_store_wait_read();                          // the box may still be the source of an earlier store
-                mbar_expect_tx(bar_my_res, kStageOutBytes);
-                tma_load_2d(stage_buf, &mapR, bar_my_res, half * 64, row0);
-              }
-              __syncwarp();
-              mbar_wait(bar_my_res, res_phase);
-              res_phase ^= 1;
-#pragma unroll
-              for (int c8 = 0; c8 < 8; ++c8) {
-                uint4 r;
-                asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w)
-                             : "r"(my_row + ((uint32_t(c8) ^ sw) << 4)));
-                const uint32_t w[4] = {r.x, r.y, r.z, r.w};
-#pragma unroll
-                for (int e = 0; e < 4; ++e) {
-                  v[half * 64 + c8 * 8 + 2 * e] += __uint_as_float(w[e] << 16);
-                  v[half * 64 + c8 * 8 + 2 * e + 1] += __uint_as_float(w[e] & 0xffff0000u);
-                }
-              }
-              __syncwarp();                                     // everyone has read the box before it is refilled
-            }
           }
         } else if (mode == EPI_ADDVEC) {
           if (row < (kBounded ? *live_rows_smem : P.T)) {
@@ -307,7 +274,7 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapX0, const __grid_constan
             for (int c8 = 0; c8 < 8; ++c8) {
               const int c = half * 64 + c8 * 8;
               asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};"
-                           ::"r"(my_row + ((uint32_t(c8) ^ sw) << 4)), "r"(pack_bf16(v[c], v[c + 1])),
+                           ::"r"(my_row_sw ^ (uint32_t(c8) << 4)), "r"(pack_bf16(v[c], v[c + 1])),
                              "r"(pack_bf16(v[c + 2], v[c + 3])), "r"(pack_bf16(v[c + 4], v[c + 5])),
                              "r"(pack_bf16(v[c + 6], v[c + 7])) : "memory");
             }
@@ -342,7 +309,7 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapX0, const __grid_constan
 // pair along their output dimension (W1: 2 x 128 of 256 rows, W2: 2 x 64 of 128 rows), which is what makes them fit:
 //   MMA 1   D1[256 x 256] = cat(x, m1) . W1^T     (x / m1 tiles stream through a TMA ring; K = 256)
 //   epi 1   relu(D1) -> bf16 -> the hidden tile h, written straight into shared memory in the K-major 128B-swizzled
-//           operand layout (never to HBM: saves 4 of the 8 activation planes the two separate launches move)
+//           operand layout (never to HBM: saves 4 of the 8 activation planes two separate Linear launches would move)
 //   MMA 2   D2[256 x 128] = h . W2^T
 //   epi 2   LayerNorm2, + x (residual rows by TMA), bf16, TMA store in place
 // warp 0: TMA producer, warp 1: TMEM allocator + MMA issuer (leader CTA), warps 2-5: epilogue 2 of every tile, warps 6-9:
@@ -910,22 +877,19 @@ bool make_map2d(CUtensorMap* m, const void* base, int64_t rows, int cols, int64_
              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-struct Src { const void* ptr; int cols; int64_t pitch; };   // one K-part of the activations
 struct Dst { void* ptr; int64_t pitch; };                   // one 128-column block of the output (bf16, row pitch in elements)
 
-// Y[T, N] = epilogue(cat(X0, X1)[T, K] . W[N, K]^T);  out[j] receives output columns [128 j, 128 j + 128).
+// Y[T, N] = epilogue(X[T, K] . W[N, K]^T), X contiguous bf16;  out[j] receives output columns [128 j, 128 j + 128).
 // live (may be null): device count of live items of rows_per_item rows each; T is then the capacity.
-cudaError_t linear_run(int64_t T, const int32_t* live, int rows_per_item, Src x0, Src x1, const void* W, int N, int K,
-                       int64_t w_pitch, const Dst (&out)[3], const __nv_bfloat16* resid, LinParams P, cudaStream_t st) {
+cudaError_t linear_run(int64_t T, const int32_t* live, int rows_per_item, const void* X, const void* W, int N, int K,
+                       int64_t w_pitch, const Dst (&out)[3], LinParams P, cudaStream_t st) {
   if (T <= 0) return cudaSuccess;
   if (T > 0x7fffffff - kTile || N % 128 || K % kBoxK || (N / 128) * (K / kBoxK) > kMaxWBoxes || N / 128 > 3)
     return cudaErrorInvalidValue;
-  CUtensorMap m0, m1, mw, mo[3], mr;
-  if (!make_map2d(&m0, x0.ptr, T, x0.cols, x0.pitch)) return cudaErrorInvalidValue;
-  if (!make_map2d(&m1, x1.ptr ? x1.ptr : x0.ptr, T, x1.ptr ? x1.cols : x0.cols, x1.ptr ? x1.pitch : x0.pitch))
-    return cudaErrorInvalidValue;
+  CUtensorMap mx, mw, mo[3];
+  if (!make_map2d(&mx, X, T, K, K)) return cudaErrorInvalidValue;
   if (!make_map2d(&mw, W, N, K, w_pitch)) return cudaErrorInvalidValue;
-  const void* any_out = P.out_f32 ? x0.ptr : out[0].ptr;       // unused maps still have to be valid descriptors
+  const void* any_out = P.out_f32 ? X : out[0].ptr;            // unused maps still have to be valid descriptors
   for (int j = 0; j < 3; ++j) {
     const bool used = !P.out_f32 && j < N / 128;
     if (used && !out[j].ptr) return cudaErrorInvalidValue;
@@ -933,12 +897,10 @@ cudaError_t linear_run(int64_t T, const int32_t* live, int rows_per_item, Src x0
     P.out_rows[j] = used ? static_cast<__nv_bfloat16*>(out[j].ptr) : nullptr;
     P.out_pitch[j] = used ? int(out[j].pitch) : 0;
   }
-  if (!make_map2d(&mr, resid ? static_cast<const void*>(resid) : any_out, T, kD, kD, 32)) return cudaErrorInvalidValue;
   P.T = int(T);
   P.live = live;
   P.rows_per_item = rows_per_item;
   P.kchunks = K / kBoxK;
-  P.kchunks0 = x0.cols / kBoxK;
   P.nblk = N / 128;
   P.stages = min(kMaxStages, (kSmemBudget - 1024 - kSmemW - P.nblk * P.kchunks * kBoxBytes) / kBoxBytes);
   if (P.stages < 2) return cudaErrorInvalidValue;
@@ -949,7 +911,7 @@ cudaError_t linear_run(int64_t T, const int32_t* live, int rows_per_item, Src x0
   const auto kernel = live ? linear_tc_kernel<true> : linear_tc_kernel<false>;
   if ((e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemAlloc)) != cudaSuccess) return e;
   const int ntiles = int((T + kTile - 1) / kTile);
-  kernel<<<min(ntiles, sms), kLinThreads, kSmemAlloc, st>>>(m0, m1, mw, mo[0], mo[1], mo[2], mr, P);
+  kernel<<<min(ntiles, sms), kLinThreads, kSmemAlloc, st>>>(mx, mw, mo[0], mo[1], mo[2], P);
   return cudaGetLastError();
 }
 
@@ -989,7 +951,7 @@ constexpr size_t kOffPreBias = kOffMergeFeat + 128 * 256 * 2;  // fp32: down_pro
 constexpr size_t kPreBytes = kOffPreBias + 2 * 128 * 4;
 static_assert(kPreBytes == POPE_FINE_PRE_BYTES, "include/pope_b200.h documents this layout");
 
-struct TfScratch { __nv_bfloat16 *q, *k, *v, *msg, *m1, *h; size_t bytes; };
+struct TfScratch { __nv_bfloat16 *q, *k, *v, *msg, *m1; size_t bytes; };
 TfScratch carve_tf(void* base, int64_t m, int S) {
   TfScratch w;
   char* p = static_cast<char*>(base);
@@ -1000,15 +962,13 @@ TfScratch carve_tf(void* base, int64_t m, int S) {
   w.v = reinterpret_cast<__nv_bfloat16*>(p + off); off += unit;
   w.msg = reinterpret_cast<__nv_bfloat16*>(p + off); off += unit;
   w.m1 = reinterpret_cast<__nv_bfloat16*>(p + off); off += unit;
-  w.h = reinterpret_cast<__nv_bfloat16*>(p + off); off += 2 * unit;
   w.bytes = off;
   return w;
 }
 
 cudaError_t attention_run(const __nv_bfloat16* q, const __nv_bfloat16* k, const __nv_bfloat16* v, __nv_bfloat16* out, int64_t m,
                           const int32_t* live, int S, cudaStream_t st) {
-  const bool force_simt = getenv("POPE_ATTN_SIMT") != nullptr;             // developer knob: the fp32 SIMT kernel
-  if (S > kTileRows || force_simt) {
+  if (S > kTileRows) {
     fine_attn_kernel<<<unsigned((m + kAttnWarps - 1) / kAttnWarps), kAttnWarps * 32, 0, st>>>(q, k, v, out, m, live, S, 1e-6f);
     return cudaGetLastError();
   }
@@ -1029,37 +989,26 @@ cudaError_t encoder_layer(__nv_bfloat16* x, const __nv_bfloat16* src, int64_t m,
                           const TfScratch& w, cudaStream_t st) {
   const int64_t T = m * S;
   const float* ln = reinterpret_cast<const float*>(wl + kOffLn);
-  const Src none{nullptr, 0, 0};
   cudaError_t e;
   LinParams P{};
   if (x == src) {                       // self: one pass over x produces q, k, v
     P.mode[0] = EPI_ELU1; P.mode[1] = EPI_ELU1; P.mode[2] = EPI_SCALE; P.scale = 1.f / float(S);
     const Dst o[3] = {{w.q, kD}, {w.k, kD}, {w.v, kD}};
-    if ((e = linear_run(T, live, S, {x, kD, kD}, none, wl + kOffQkv, 384, kD, kD, o, nullptr, P, st)) != cudaSuccess) return e;
+    if ((e = linear_run(T, live, S, x, wl + kOffQkv, 384, kD, kD, o, P, st)) != cudaSuccess) return e;
   } else {
     P.mode[0] = EPI_ELU1;
     const Dst oq[3] = {{w.q, kD}, {nullptr, 0}, {nullptr, 0}};
-    if ((e = linear_run(T, live, S, {x, kD, kD}, none, wl + kOffQkv, 128, kD, kD, oq, nullptr, P, st)) != cudaSuccess) return e;
+    if ((e = linear_run(T, live, S, x, wl + kOffQkv, 128, kD, kD, oq, P, st)) != cudaSuccess) return e;
     P.mode[0] = EPI_ELU1; P.mode[1] = EPI_SCALE; P.scale = 1.f / float(S);
     const Dst okv[3] = {{w.k, kD}, {w.v, kD}, {nullptr, 0}};
-    if ((e = linear_run(T, live, S, {src, kD, kD}, none, wl + kOffQkv + 128 * 128 * 2, 256, kD, kD, okv, nullptr, P, st)) != cudaSuccess)
-      return e;
+    if ((e = linear_run(T, live, S, src, wl + kOffQkv + 128 * 128 * 2, 256, kD, kD, okv, P, st)) != cudaSuccess) return e;
   }
   if ((e = attention_run(w.q, w.k, w.v, w.msg, m, live, S, st)) != cudaSuccess) return e;
   P = LinParams{};
   P.mode[0] = EPI_LN; P.gamma = ln; P.beta = ln + 128;
   const Dst om[3] = {{w.m1, kD}, {nullptr, 0}, {nullptr, 0}};
-  if ((e = linear_run(T, live, S, {w.msg, kD, kD}, none, wl + kOffMerge, 128, kD, kD, om, nullptr, P, st)) != cudaSuccess) return e;
-  const bool unfused_mlp = getenv("POPE_MLP_UNFUSED") != nullptr;            // developer knob: the two separate launches
-  if (!unfused_mlp) return mlp_fused_run(x, w.m1, T, live, S, wl + kOffMlp1, wl + kOffMlp2, ln + 256, ln + 384, st);
-  P = LinParams{};
-  P.mode[0] = EPI_RELU; P.mode[1] = EPI_RELU;
-  const Dst oh[3] = {{w.h, 2 * kD}, {w.h + kD, 2 * kD}, {nullptr, 0}};
-  if ((e = linear_run(T, live, S, {x, kD, kD}, {w.m1, kD, kD}, wl + kOffMlp1, 256, 256, 256, oh, nullptr, P, st)) != cudaSuccess) return e;
-  P = LinParams{};
-  P.mode[0] = EPI_LN_RES; P.gamma = ln + 256; P.beta = ln + 384;
-  const Dst ox[3] = {{x, kD}, {nullptr, 0}, {nullptr, 0}};
-  return linear_run(T, live, S, {w.h, 2 * kD, 2 * kD}, none, wl + kOffMlp2, 128, 256, 256, ox, x, P, st);
+  if ((e = linear_run(T, live, S, w.msg, wl + kOffMerge, 128, kD, kD, om, P, st)) != cudaSuccess) return e;
+  return mlp_fused_run(x, w.m1, T, live, S, wl + kOffMlp1, wl + kOffMlp2, ln + 256, ln + 384, st);
 }
 
 }  // namespace
@@ -1145,22 +1094,18 @@ extern "C" int pope_fine_merge_coarse_ex(void* win0, void* win1, int64_t m_windo
   // [m, m + live): each side is then its own launch, bounded by the count.  Without one, both sides are a single launch.
   const int nseg = m_dev ? 2 : 1;
   const int64_t seg = 2 * m / nseg;
-  const Src none{nullptr, 0, 0};
   LinParams P{};
   for (int s = 0; s < nseg; ++s) {
     // feat_c_win = down_proj(cat(c0, c1))                                                (fine_preprocess.py:50-51)
     P = LinParams{};
     P.mode[0] = EPI_COPY; P.bias = bias;
     const Dst od[3] = {{cd + s * seg * kD, kD}, {nullptr, 0}, {nullptr, 0}};
-    if ((e = linear_run(seg, m_dev, 1, {cg + s * seg * 256, 256, 256}, none, wp + kOffDown, 128, 256, 256, od, nullptr, P, st)) !=
-        cudaSuccess)
-      return int(e);
+    if ((e = linear_run(seg, m_dev, 1, cg + s * seg * 256, wp + kOffDown, 128, 256, 256, od, P, st)) != cudaSuccess) return int(e);
     // merge_feat(cat(win, repeat(c))) = win . Wa^T + (c . Wb^T + bias): the second term once per window     (:52-55)
     P = LinParams{};
     P.out_f32 = cvec + s * seg * kD; P.mode[0] = EPI_COPY; P.bias = bias + 128;
     const Dst onone[3] = {{nullptr, 0}, {nullptr, 0}, {nullptr, 0}};
-    if ((e = linear_run(seg, m_dev, 1, {cd + s * seg * kD, kD, kD}, none, wp + kOffMergeFeat + 128 * 2, 128, 128, 256, onone, nullptr,
-                        P, st)) != cudaSuccess)
+    if ((e = linear_run(seg, m_dev, 1, cd + s * seg * kD, wp + kOffMergeFeat + 128 * 2, 128, 128, 256, onone, P, st)) != cudaSuccess)
       return int(e);
   }
   for (int side = 0; side < 2; ++side) {
@@ -1168,8 +1113,7 @@ extern "C" int pope_fine_merge_coarse_ex(void* win0, void* win1, int64_t m_windo
     P = LinParams{};
     P.mode[0] = EPI_ADDVEC; P.rowvec = cvec + size_t(side) * m * kD; P.rows_per_vec = window_tokens;
     const Dst ow[3] = {{win, kD}, {nullptr, 0}, {nullptr, 0}};
-    if ((e = linear_run(m * window_tokens, m_dev, window_tokens, {win, kD, kD}, none, wp + kOffMergeFeat, 128, 128, 256, ow, nullptr,
-                        P, st)) != cudaSuccess)
+    if ((e = linear_run(m * window_tokens, m_dev, window_tokens, win, wp + kOffMergeFeat, 128, 128, 256, ow, P, st)) != cudaSuccess)
       return int(e);
   }
   return POPE_OK;

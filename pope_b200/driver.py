@@ -55,7 +55,7 @@ class Pipeline:
     window gather and fine matching -- FinePreprocess' two Linears and the fine transformer, in bf16 -- so that the results
     equal `ops.match_pairs_device(..., fine_level=...)` and thereby `Matcher(config, fine_cuda_bf16=True)`, bit for bit.
     Needs a bf16 pipeline with C_coarse = 256.  The pipeline keeps a reference to the dict, so the packed weights outlive
-    the handle; it allocates windows and fine scratch for one chunk (0.98 GB + 3.4 GB at 16 pairs of 480x640)."""
+    the handle; it allocates windows and fine scratch for one chunk (0.98 GB + 2.5 GB at 16 pairs of 480x640)."""
 
     def __init__(self, dtype: torch.dtype, chunk_pairs: int, hw0_i: Sequence[int], hw0_c: Sequence[int],
                  hw1_c: Sequence[int], C_coarse: int = 256, C_fine: int = 128, fine_stride: int = 4, W: int = 5,

@@ -252,5 +252,6 @@ class FineTransformerB200(LocalFeatureTransformer):
         if not self.inplace:
             feat0, feat1 = feat0.clone(), feat1.clone()
         feat0, feat1 = feat0.contiguous(), feat1.contiguous()
-        self._workspace = ops.fine_tf_workspace(feat0.shape[0], feat0.shape[1], feat0.device, self._workspace)
+        self._workspace = ops.fine_level_workspace(feat0.shape[0], feat0.shape[1], feat0.device, self._workspace,
+                                                   merge=False)
         return ops.fine_transformer(feat0, feat1, self._packed_weights(feat0.device), self.layer_names, self._workspace)

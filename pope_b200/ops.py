@@ -153,13 +153,6 @@ def pack_fine_pre(sd: Dict[str, torch.Tensor], device) -> torch.Tensor:
     return out
 
 
-def fine_tf_workspace(m: int, ww: int, dev, workspace: Optional[torch.Tensor] = None) -> torch.Tensor:
-    need = lib().pope_fine_tf_workspace_bytes(int(m), int(ww))
-    if workspace is None or workspace.numel() < need or workspace.device != dev:
-        workspace = torch.empty(max(need, 16), dtype=torch.uint8, device=dev)
-    return workspace
-
-
 def _check_m_dev(m_dev: Optional[torch.Tensor], dev) -> None:
     if m_dev is not None and (m_dev.dtype != torch.int32 or m_dev.numel() < 1 or m_dev.device != dev):
         raise _lib.PopeError("m_dev must be a device int32 tensor (the live count) on the device of the windows")
@@ -189,7 +182,7 @@ def fine_transformer(feat0: torch.Tensor, feat1: torch.Tensor, packed_layers: to
     M, WW, _ = feat0.shape
     if M == 0:
         return feat0, feat1
-    workspace = fine_tf_workspace(M, WW, dev, workspace)
+    workspace = fine_level_workspace(M, WW, dev, workspace, merge=False)
     arr = (_lib.C.c_int * max(len(kinds), 1))(*kinds)
     with torch.cuda.device(dev):
         st = lib().pope_fine_transformer_ex(ptr(feat0), ptr(feat1), M, ptr(m_dev), WW, ptr(packed_layers), len(kinds), arr,
@@ -213,9 +206,7 @@ def fine_merge_coarse(win0: torch.Tensor, win1: torch.Tensor, feat_c0: torch.Ten
         return win0, win1
     n, L, C_ = feat_c0.shape
     S = feat_c1.shape[1]
-    need = lib().pope_fine_merge_workspace_bytes(int(M))
-    if workspace is None or workspace.numel() < need or workspace.device != dev:
-        workspace = torch.empty(need, dtype=torch.uint8, device=dev)
+    workspace = fine_level_workspace(M, WW, dev, workspace, transformer=False)
     with torch.cuda.device(dev):
         st = lib().pope_fine_merge_coarse_ex(ptr(win0), ptr(win1), M, ptr(m_dev), WW, ptr(feat_c0), ptr(feat_c1), L, S, C_,
                                              ptr(b_ids.contiguous()), ptr(i_ids.contiguous()), ptr(j_ids.contiguous()),
@@ -302,10 +293,14 @@ def running_topk(scores: torch.Tensor, k: int = 3):
     return slot_s, slot_i
 
 
-def fine_level_workspace(m: int, ww: int, dev, workspace: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """Scratch of the bf16 fine level for m windows of ww tokens: the FinePreprocess Linears and the fine transformer run
-    one after the other on one stream, so they share it (its size is the transformer's, 7 planes of [m * ww, 128] bf16)."""
-    need = max(lib().pope_fine_tf_workspace_bytes(int(m), int(ww)), lib().pope_fine_merge_workspace_bytes(int(m)), 16)
+def fine_level_workspace(m: int, ww: int, dev, workspace: Optional[torch.Tensor] = None, merge: bool = True,
+                         transformer: bool = True) -> torch.Tensor:
+    """Scratch of the bf16 fine level for m windows of ww tokens, sized for the stages that will use it: the FinePreprocess
+    Linears (`merge`) and the fine transformer (`transformer`, 5 planes of [m * ww, 128] bf16).  They run one after the
+    other on one stream, so with both the scratch is shared (at 25 tokens its size is the transformer's).  A stage that
+    is handed no scratch gets one of its own size only, so a caller that does not share pays for no more than it uses."""
+    need = max(lib().pope_fine_tf_workspace_bytes(int(m), int(ww)) if transformer else 0,
+               lib().pope_fine_merge_workspace_bytes(int(m)) if merge else 0, 16)
     if workspace is None or workspace.numel() < need or workspace.device != dev:
         workspace = torch.empty(need, dtype=torch.uint8, device=dev)
     return workspace
@@ -335,7 +330,7 @@ def match_pairs_device(feat_c0, feat_c1, feat_f0, feat_f1, hw0_i, hw0_c, hw1_c, 
     is bounded by the device match count.  Needs bf16 coarse features (C = 256), bf16 fine maps (Cf = 128) and W = 5, and
     takes the unfused route.  The result then also holds `fine_workspace` (pass it back in to reuse it).  Memory is sized
     by the capacity n * L, not by the match count: at 64 pairs x 480x640 (307 200 windows) that is 3.9 GB of windows plus
-    13.8 GB of fine scratch per call, about 17.7 GB; the Matcher flow, sized by the count, needs about half of that at the
+    9.8 GB of fine scratch per call, about 13.8 GB; the Matcher flow, sized by the count, needs about half of that at the
     synthetic inputs' match rate."""
     if fine_level is not None:
         _check_fine_level_inputs(feat_c0, feat_c1, feat_f0, feat_f1, W)

@@ -84,6 +84,33 @@ def test_ex_entry_points_reject_bad_arguments_before_touching_the_gpu():
     assert h.pope_fine_merge_coarse_ex(*bad) == 0
 
 
+@pytest.mark.parametrize("m,S", [(1, 25), (3, 25), (8, 25), (1003, 25), (307200, 25), (5, 49), (77, 9)])
+def test_fine_tf_workspace_is_five_planes(m, S):
+    """The transformer's scratch is q, k, v, message and merged message: five 256-byte-aligned [m * S, 128] bf16 planes.
+    At S = 25 it also covers the merge's scratch, so the fine level's shared scratch is the transformer's size."""
+    h = _lib.lib()
+    plane = (m * S * 128 * 2 + 255) // 256 * 256
+    assert h.pope_fine_tf_workspace_bytes(m, S) == 5 * plane
+    if S == 25:
+        assert h.pope_fine_tf_workspace_bytes(m, S) >= h.pope_fine_merge_workspace_bytes(m)
+    assert h.pope_fine_tf_workspace_bytes(0, S) == 0 and h.pope_fine_tf_workspace_bytes(m, 0) == 0
+
+
+def test_fine_level_workspace_is_sized_for_the_stages_that_use_it():
+    """The Matcher flow hands the merge no scratch: it must get the merge's bytes, not the transformer's five planes.
+    A scratch that is large enough is reused, one that is too small is replaced."""
+    h, cpu = _lib.lib(), torch.device("cpu")
+    m = 1003
+    tf, mg = h.pope_fine_tf_workspace_bytes(m, 25), h.pope_fine_merge_workspace_bytes(m)
+    assert mg < tf
+    assert ops.fine_level_workspace(m, 25, cpu, transformer=False).numel() == mg
+    assert ops.fine_level_workspace(m, 25, cpu, merge=False).numel() == tf
+    shared = ops.fine_level_workspace(m, 25, cpu)
+    assert shared.numel() == tf
+    assert ops.fine_level_workspace(m, 25, cpu, shared, transformer=False) is shared
+    assert ops.fine_level_workspace(m, 25, cpu, shared[:mg - 1], transformer=False).numel() == mg
+
+
 def test_fine_level_packs_the_matcher_weights_and_rejects_what_it_cannot_run():
     m = pope_b200.Matcher(pope_b200.make_default_cfg()).eval()
     fl = m.fine_level("cpu")

@@ -43,10 +43,10 @@ def _load():
     return g, meta, layers, pre_sd
 
 
-def _inputs(seed, m):
+def _inputs(seed, m, ww=25):
     gen = torch.Generator().manual_seed(seed)
-    return (torch.randn(m, 25, 128, generator=gen).to(torch.bfloat16).float(),
-            torch.randn(m, 25, 128, generator=gen).to(torch.bfloat16).float())
+    return (torch.randn(m, ww, 128, generator=gen).to(torch.bfloat16).float(),
+            torch.randn(m, ww, 128, generator=gen).to(torch.bfloat16).float())
 
 
 def _rel_err(got: torch.Tensor, want: torch.Tensor):
@@ -245,31 +245,19 @@ def test_matcher_bf16_fine_path_vs_fp32_module_flow():
 
 
 @pytest.mark.gpu
-def test_cuda_fine_transformer_alternative_kernels_agree():
-    """The developer knobs select the kernels the default path replaced (fp32 SIMT attention instead of mma.sync, two
-    Linear launches instead of the fused CTA-pair MLP); all of them implement the same layer, so their outputs agree to
-    bf16 rounding noise and each stays within the tolerance against the oracle."""
+@pytest.mark.parametrize("m", [1, 300])
+def test_cuda_fine_transformer_7x7_windows_vs_oracle(m):
+    """7 x 7 windows (`fine_window_size` 7): 49 tokens exceed the 32-row tile of the mma.sync attention, so the fp32 SIMT
+    attention kernel runs.  49 * m rows leave a ragged 128-row tile for both counts."""
     from pope_b200 import ops
     dev = torch.device("cuda:0")
-    g, meta, layers, _ = _load()
-    f0, f1 = _inputs(321, 300)
-    packed = _cuda_layers(layers, dev)
+    _, meta, layers, _ = _load()
+    f0, f1 = _inputs(321 + m, m, 49)
+    d0, d1 = f0.to(dev, torch.bfloat16), f1.to(dev, torch.bfloat16)
+    ops.fine_transformer(d0, d1, _cuda_layers(layers, dev), meta["layer_names"])
+    torch.cuda.synchronize()
     want0, want1 = O.fine_transformer(f0, f1, layers, meta["layer_names"])
-    outs = {}
-    for knob in (None, "POPE_ATTN_SIMT", "POPE_MLP_UNFUSED"):
-        if knob:
-            os.environ[knob] = "1"
-        try:
-            d0, d1 = f0.to(dev, torch.bfloat16), f1.to(dev, torch.bfloat16)
-            ops.fine_transformer(d0, d1, packed, meta["layer_names"])
-            torch.cuda.synchronize()
-        finally:
-            if knob:
-                del os.environ[knob]
-        outs[knob] = (d0.float().cpu(), d1.float().cpu())
-        for got, want in zip(outs[knob], (want0, want1)):
-            rms, mx = _rel_err(got, want)
-            assert rms < 1.5e-2 and mx < 8e-2, (knob, rms, mx)
-    for knob in ("POPE_ATTN_SIMT", "POPE_MLP_UNFUSED"):
-        for a, b in zip(outs[None], outs[knob]):
-            assert _rel_err(a, b)[0] < 1e-2, knob
+    for got, want in ((d0.cpu(), want0), (d1.cpu(), want1)):
+        assert torch.isfinite(got.float()).all()
+        rms, mx = _rel_err(got, want)
+        assert rms < 1.5e-2 and mx < 8e-2, (m, rms, mx)

@@ -14,7 +14,7 @@ g = torch.Generator(device=dev).manual_seed(1)
 w0 = torch.randn(M, 25, 128, device=dev, generator=g).to(torch.bfloat16)
 w1 = torch.randn(M, 25, 128, device=dev, generator=g).to(torch.bfloat16)
 packed = torch.cat([ops.pack_fine_layer({k: v for k, v in l.state_dict().items()}, dev) for l in m.loftr_fine.layers])
-ws = ops.fine_tf_workspace(M, 25, dev)
+ws = ops.fine_level_workspace(M, 25, dev, merge=False)
 names = m.loftr_fine.layer_names
 
 def timed(fn, reps=3):
