@@ -40,9 +40,12 @@
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "tc_ptx.cuh"
 
 namespace pope {
 namespace {
+
+using namespace tc1;
 
 constexpr int kStages = 8;              // B ring depth
 constexpr int kBoxRows = 128;           // rows per TMA box = rows of A / of the B half held by one CTA
@@ -65,7 +68,7 @@ constexpr int kThreads = kEpiThreads + 128;
 constexpr int kRegsEpi = 112, kRegsAux = 32;
 static_assert(16 * 32 * kRegsEpi + 4 * 32 * kRegsAux <= 640 * 96, "setmaxnreg would wait for registers the CTA does not own");   // 16 x 32 x 112 + 4 x 32 x 32 = 61 440 = the CTA's 640 x 96 registers (the pool is per CTA)
 constexpr uint32_t kTmemCols = 512;
-constexpr uint32_t kPeerMask = 0xFEFFFFFFu;          // clears the CTA-rank bit of a shared::cluster address -> leader CTA
+constexpr uint32_t kIdesc = tc2::idesc_bf16_m256(kTileCols);   // every MMA: M = 256 (128 rows per CTA), N = one tile
 
 // dynamic shared memory layout (base aligned to 1024 B for the 128B swizzle); identical in both CTAs of a pair
 constexpr int kSmemA = 0;                                            // 4 k-chunks x 16 KB
@@ -74,123 +77,6 @@ constexpr int kSmemA = 0;                                            // 4 k-chun
 constexpr int kSmemAlloc = 2 * kMaxKChunks * kBoxBytes + 5 * kBoxBytes + 2 * 2 * kTileCols * 4 + 3 * 128 * 8 + 256 + 16 + 1024;
 static_assert(kSmemAlloc >= kMaxKChunks * kBoxBytes + kStages * kBoxBytes + 2 * 2 * kTileCols * 4 + 3 * 128 * 8 + 256 + 16 + 1024 &&
               kSmemAlloc <= 227 * 1024, "shared-memory allocation");
-
-// ---- PTX wrappers ---------------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
-
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-  return ok != 0;
-}
-__device__ __forceinline__ long long clock_now() {
-  long long t;
-  asm volatile("mov.u64 %0, %%clock64;" : "=l"(t)::"memory");
-  return t;
-}
-// Bounded wait: a protocol bug must become a launch failure, never a hung GPU.  The clock is only read every 1024 polls
-// (read on every poll, the nine instructions of the time-out test were a fifth of all instructions the sweep issued).
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  if (mbar_try_wait(bar, parity)) return;
-  long long t0 = 0;
-  for (;;) {
-#pragma unroll 1
-    for (int k = 0; k < 1024; ++k)
-      if (mbar_try_wait(bar, parity)) return;
-    const long long t = clock_now();
-    if (t0 == 0) t0 = t;
-    else if (t - t0 > 4000000000ll) __trap();     // ~2 s at 2 GHz
-  }
-}
-__device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-
-// 2-SM TMA load: data lands in the executing CTA's shared memory, the transaction bytes are credited to the
-// LEADER CTA's barrier (rank bit cleared)
-__device__ __forceinline__ void tma_load_3d_2sm(uint32_t dst, const CUtensorMap* map, uint32_t bar, int c0, int c1, int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-      ::"r"(dst), "l"(map), "r"(bar & kPeerMask), "r"(c0), "r"(c1), "r"(c2) : "memory");
-}
-// arrive on the leader CTA's copy of a barrier (from either CTA of the pair)
-__device__ __forceinline__ void mbar_arrive_leader(uint32_t bar) {
-  asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(bar & kPeerMask) : "memory");
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-// one lane of a converged warp (the way the tensor-core instructions are issued: ptxas keeps their operands in uniform
-// registers when the single-thread region is entered through elect.sync)
-__device__ __forceinline__ bool elect_one() {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "elect.sync _|p, 0xffffffff;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok));
-  return ok != 0;
-}
-__device__ __forceinline__ void prefetch_tmap(const CUtensorMap* map) {
-  asm volatile("prefetch.tensormap [%0];" ::"l"(map) : "memory");
-}
-
-// K-major, 128B-swizzled operand tile: rows 128 B apart, 8-row groups 1024 B apart (SBO), LBO unused (=1), version 1.
-__device__ __forceinline__ uint64_t umma_desc(uint32_t smem_addr) {
-  return uint64_t((smem_addr & 0x3ffffu) >> 4) | (uint64_t(1) << 16) | (uint64_t(1024 >> 4) << 32) | (uint64_t(1) << 46) |
-         (uint64_t(2) << 61);
-}
-// kind::f16, A = B = bf16 (K-major), D = fp32, M = 256 (128 per CTA), N = 256
-constexpr uint32_t kIdesc = (1u << 4) | (1u << 7) | (1u << 10) | (uint32_t(kTileCols >> 3) << 17) | (uint32_t(256 >> 4) << 24);
-
-__device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(kIdesc), "r"(accumulate) : "memory");
-}
-// arrives on the barrier at this offset in BOTH CTAs once all previously issued MMAs have completed
-__device__ __forceinline__ void umma_commit_2sm(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(bar), "h"(uint16_t(3)) : "memory");
-}
-// 32 lanes x 32 consecutive fp32 columns -> 32 registers per thread; the wait is part of the same statement so the
-// registers are valid when it retires.
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
-  uint32_t r[32];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-      "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];\n\t"
-      "tcgen05.wait::ld.sync.aligned;"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr) : "memory");
-#pragma unroll
-  for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
-}
 
 struct SweepParams {
   // direction d: stationary operand = feature set d (rows LA[d]), streamed operand = the other one
@@ -492,7 +378,7 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
   uint32_t lane_u;
   asm volatile("mov.u32 %0, %%laneid;" : "=r"(lane_u));
   const int warp = threadIdx.x >> 5, lane = int(lane_u);
-  const uint32_t rank = cluster_ctarank();          // 0 = leader (issues the MMAs), 1 = peer
+  const uint32_t rank = tc2::cluster_ctarank();     // 0 = leader (issues the MMAs), 1 = peer
   const int pair = blockIdx.x >> 1, npairs = gridDim.x >> 1;
 
   if (warp == kWarpProducer && lane == 0) {
@@ -511,13 +397,12 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
     fence_barrier_init();
   }
   if (warp == kWarpMma) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(sbase + kSmemTmemPtr), "r"(kTmemCols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+    tc2::tmem_alloc(sbase + kSmemTmemPtr, kTmemCols);
+    tc2::tmem_relinquish();
   }
   tc_fence_before();
   __syncthreads();
-  cluster_sync_all();                                // peer barriers are initialised before anyone signals them
+  tc2::cluster_sync_all();                           // peer barriers are initialised before anyone signals them
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr_smem;
   const int kchunks = P.kchunks;
@@ -549,9 +434,9 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
         const CUtensorMap* mapB = dir ? &map0 : &map1;
         const int arow = rb * kUnitRows + int(rank) * kBoxRows;
         auto ring_load = [&](const CUtensorMap* mp, int kc, int row) {
-          mbar_wait(bar_b_empty + 8 * b_stage, b_phase ^ 1);
+          mbar_wait_batched(bar_b_empty + 8 * b_stage, b_phase ^ 1);
           if (rank == 0) mbar_expect_tx(bar_b_full + 8 * b_stage, 2 * kBoxBytes);
-          tma_load_3d_2sm(sbase + kSmemB + b_stage * kBoxBytes, mp, bar_b_full + 8 * b_stage, kc * kBoxK, row, n);
+          tc2::tma_load_3d_2sm(sbase + kSmemB + b_stage * kBoxBytes, mp, bar_b_full + 8 * b_stage, kc * kBoxK, row, n);
           if (++b_stage == kStages) { b_stage = 0; b_phase ^= 1; }
         };
         const int ntiles = ((dir ? P.L0 : P.L1) + kTileCols - 1) / kTileCols;
@@ -583,14 +468,14 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
         // k-chunk kc of the stationary block: awaited before its first use in the unit's first tile, handed back to the
         // loader right after its last use in the unit's last tile
         auto a_wait = [&](int ct, int kc) {
-          if (ct == 0) { mbar_wait(bar_a_full + 8 * kc, a_phase); tc_fence_after(); }
+          if (ct == 0) { mbar_wait_batched(bar_a_full + 8 * kc, a_phase); tc_fence_after(); }
         };
         auto a_done = [&](int ct, int kc) {
-          if (ct == ntiles - 1 && elect_one()) umma_commit_2sm(bar_a_empty + 8 * kc);
+          if (ct == ntiles - 1 && elect_one()) tc2::umma_commit(bar_a_empty + 8 * kc);
         };
         for (int ct = 0; ct < ntiles; ++ct, ++tile_ctr) {
           const uint32_t s = tile_ctr & 1, acc_phase = (tile_ctr >> 1) & 1;
-          mbar_wait(bar_acc_empty + 8 * s, acc_phase ^ 1);
+          mbar_wait_batched(bar_acc_empty + 8 * s, acc_phase ^ 1);
           tc_fence_after();
           const uint32_t d = tmem_base + s * kTileCols;
           if (MODE == 4) {
@@ -599,18 +484,18 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
             auto mma4 = [&](uint32_t a_addr, uint32_t b_addr) {
               if (elect_one()) {
 #pragma unroll
-                for (int ks = 0; ks < kBoxK / 16; ++ks) umma_bf16(d, umma_desc(a_addr + ks * 32), umma_desc(b_addr + ks * 32), first | uint32_t(ks));
+                for (int ks = 0; ks < kBoxK / 16; ++ks) tc2::umma_bf16(d, umma_desc(a_addr + ks * 32), umma_desc(b_addr + ks * 32), kIdesc, first | uint32_t(ks));
               }
               first = 1u;
             };
             auto ring_wait = [&]() {
-              mbar_wait(bar_b_full + 8 * b_stage, b_phase);
+              mbar_wait_batched(bar_b_full + 8 * b_stage, b_phase);
               tc_fence_after();
               const uint32_t addr = sbase + kSmemB + b_stage * kBoxBytes;
               return addr;
             };
             auto ring_done = [&]() {
-              if (elect_one()) umma_commit_2sm(bar_b_empty + 8 * b_stage);
+              if (elect_one()) tc2::umma_commit(bar_b_empty + 8 * b_stage);
               if (++b_stage == kStages) { b_stage = 0; b_phase ^= 1; }
             };
             for (int kc = 0; kc < kchunks; ++kc) {
@@ -618,7 +503,7 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
               const uint32_t a3 = ring_wait();
               const uint32_t a3_stage = b_stage;
               uint32_t nxt = b_stage + 1 == kStages ? 0 : b_stage + 1;
-              mbar_wait(bar_b_full + 8 * nxt, nxt == 0 ? b_phase ^ 1 : b_phase);
+              mbar_wait_batched(bar_b_full + 8 * nxt, nxt == 0 ? b_phase ^ 1 : b_phase);
               tc_fence_after();
               const uint32_t b1 = sbase + kSmemB + nxt * kBoxBytes;
               mma4(sbase + kSmemA + kc * kBoxBytes, b1);
@@ -643,20 +528,20 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
           } else
           for (int kc = 0; kc < kchunks; ++kc) {
             a_wait(ct, kc);
-            mbar_wait(bar_b_full + 8 * b_stage, b_phase);
+            mbar_wait_batched(bar_b_full + 8 * b_stage, b_phase);
             tc_fence_after();
             const uint32_t a_addr = sbase + kSmemA + kc * kBoxBytes;
             const uint32_t b_addr = sbase + kSmemB + b_stage * kBoxBytes;
             if (elect_one()) {
 #pragma unroll
               for (int ks = 0; ks < kBoxK / 16; ++ks)
-                umma_bf16(d, umma_desc(a_addr + ks * 32), umma_desc(b_addr + ks * 32), (kc | ks) ? 1u : 0u);
-              umma_commit_2sm(bar_b_empty + 8 * b_stage);  // ring slot free in both CTAs once these MMAs have read it
+                tc2::umma_bf16(d, umma_desc(a_addr + ks * 32), umma_desc(b_addr + ks * 32), kIdesc, (kc | ks) ? 1u : 0u);
+              tc2::umma_commit(bar_b_empty + 8 * b_stage);  // ring slot free in both CTAs once these MMAs have read it
             }
             a_done(ct, kc);
             if (++b_stage == kStages) { b_stage = 0; b_phase ^= 1; }
           }
-          if (elect_one()) umma_commit_2sm(bar_acc_full + 8 * s);         // accumulator stage complete (both CTAs' epilogues)
+          if (elect_one()) tc2::umma_commit(bar_acc_full + 8 * s);         // accumulator stage complete (both CTAs' epilogues)
         }
         a_phase ^= 1;
       }
@@ -674,11 +559,11 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
         const CUtensorMap* mapA = dir ? &map1 : &map0;
         const int arow = rb * kUnitRows + int(rank) * kBoxRows;
         for (int kc = 0; kc < kchunks; ++kc) {
-          mbar_wait(bar_a_empty + 8 * kc, a_phase ^ 1);
+          mbar_wait_batched(bar_a_empty + 8 * kc, a_phase ^ 1);
           if (rank == 0) mbar_expect_tx(bar_a_full + 8 * kc, (MODE == 4 ? 4 : 2) * kBoxBytes);
-          tma_load_3d_2sm(sbase + kSmemA + kc * kBoxBytes, mapA, bar_a_full + 8 * kc, kc * kBoxK, arow, n);
+          tc2::tma_load_3d_2sm(sbase + kSmemA + kc * kBoxBytes, mapA, bar_a_full + 8 * kc, kc * kBoxK, arow, n);
           if (MODE == 4)      // a2 block behind the a1 block
-            tma_load_3d_2sm(sbase + kSmemA + (kMaxKChunks + kc) * kBoxBytes, &map1, bar_a_full + 8 * kc, kc * kBoxK, arow, n);
+            tc2::tma_load_3d_2sm(sbase + kSmemA + (kMaxKChunks + kc) * kBoxBytes, &map1, bar_a_full + 8 * kc, kc * kBoxK, arow, n);
         }
         a_phase ^= 1;
       }
@@ -741,7 +626,7 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
         const int col0 = ct * kTileCols;
         const int nvalid = min(LB - col0, kTileCols) - colofs;
         const bool active = rows_valid > 0 && nvalid > 0;
-        mbar_wait(bar_acc_full + 8 * s, acc_phase);
+        mbar_wait_batched(bar_acc_full + 8 * s, acc_phase);
         tc_fence_after();
         const uint32_t tbase = tb0 + s * kTileCols;
         float v[32];
@@ -847,7 +732,7 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
         if (active && nvalid > 32) tmem_ld_frag(tbase + 32, v);
         tc_fence_before();
         __syncwarp();
-        if (lane == 0) mbar_arrive_leader(bar_acc_empty + 8 * s);
+        if (lane == 0) tc2::mbar_arrive_leader(bar_acc_empty + 8 * s);
         if (active && nvalid > 32) process(v, 1);
         cp_ptr += kTileCols;
         cs_ptr += kTileCols / 32;
@@ -955,7 +840,7 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
           }
           asm volatile("bar.sync 1, %0;" ::"n"(kEpiThreads) : "memory");
         }
-        mbar_wait(bar_acc_full + 8 * s, acc_phase);
+        mbar_wait_batched(bar_acc_full + 8 * s, acc_phase);
         tc_fence_after();
         const uint32_t tbase = tmem_base + lane_addr + s * kTileCols + colq * kSpan;
         const int nvalid = min(LB - col0, kTileCols) - colq * kSpan;   // valid columns from this thread's first one
@@ -997,7 +882,7 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
           }
           tc_fence_before();
           __syncwarp();
-          if (lane == 0) mbar_arrive_leader(bar_acc_empty + 8 * s);
+          if (lane == 0) tc2::mbar_arrive_leader(bar_acc_empty + 8 * s);
         } else {
           // ---- log-sum-exp sweeps: the accumulator stage is handed back to the MMA issuer as soon as this warp's
           //      last TMEM load has retired; the second chunk's arithmetic and every atomic run after the hand-back ----
@@ -1025,7 +910,7 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
           if (vc1 > 0) tmem_ld32(tbase + 32, v);
           tc_fence_before();
           __syncwarp();
-          if (lane == 0) mbar_arrive_leader(bar_acc_empty + 8 * s);
+          if (lane == 0) tc2::mbar_arrive_leader(bar_acc_empty + 8 * s);
           if (vc1 > 0) {
             const float cmax = lse_update(v, vc1, scale, m_run, s_run);
             if (listing) scan(v, 1, vc1, cmax);
@@ -1059,10 +944,10 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
 
   tc_fence_before();
   __syncthreads();
-  cluster_sync_all();                                // the peer may still be signalling / reading this CTA's memory
+  tc2::cluster_sync_all();                           // the peer may still be signalling / reading this CTA's memory
   if (warp == kWarpMma) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kTmemCols) : "memory");
+    tc2::tmem_dealloc(tmem_base, kTmemCols);
   }
 }
 
@@ -1089,22 +974,6 @@ __global__ void __launch_bounds__(256) split3_kernel(const float4* __restrict__ 
 }
 
 // ---- host side ------------------------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn encode_fn() {
-  static EncodeTiledFn fn = [] {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess ||
-        q != cudaDriverEntryPointSuccess)
-      p = nullptr;
-    return reinterpret_cast<EncodeTiledFn>(p);
-  }();
-  return fn;
-}
-
 // [n, rows, C] bf16, box = 64 k x 128 rows x 1 pair, 128-byte swizzle, zero fill past the last row
 bool make_map(CUtensorMap* m, const void* base, int n, int rows, int C) {
   EncodeTiledFn enc = encode_fn();

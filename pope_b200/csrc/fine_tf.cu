@@ -129,8 +129,8 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constant
     fence_barrier_init();
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(sbase + kSmemTmemPtr), "r"(512u) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc(sbase + kSmemTmemPtr, 512u);
+    tmem_relinquish();
   }
   tc_fence_before();
   __syncthreads();
@@ -300,7 +300,7 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constant
   __syncthreads();
   if (warp == 1) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
+    tmem_dealloc(tmem_base, 512u);
   }
 }
 
@@ -378,8 +378,8 @@ mlp_fused_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constant
     fence_barrier_init();
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(sbase + kFmTmemPtr), "r"(512u) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+    tc2::tmem_alloc(sbase + kFmTmemPtr, 512u);
+    tc2::tmem_relinquish();
   }
   tc_fence_before();
   __syncthreads();
@@ -589,7 +589,7 @@ mlp_fused_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constant
   tc2::cluster_sync_all();                                       // the peer may still be signalling / reading this CTA
   if (warp == 1) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
+    tc2::tmem_dealloc(tmem_base, 512u);
   }
 }
 
@@ -850,20 +850,6 @@ __global__ void __launch_bounds__(256) gather_coarse_rows_kernel(const __nv_bflo
 }
 
 // ---- host side ---------------------------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn encode_fn() {
-  static EncodeTiledFn fn = [] {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess ||
-        q != cudaDriverEntryPointSuccess)
-      p = nullptr;
-    return reinterpret_cast<EncodeTiledFn>(p);
-  }();
-  return fn;
-}
 // [rows, cols] bf16 with a row pitch of `pitch` elements, box = 64 columns x box_rows rows, 128-byte swizzle, zero fill
 bool make_map2d(CUtensorMap* m, const void* base, int64_t rows, int cols, int64_t pitch, int box_rows = kTile) {
   EncodeTiledFn enc = encode_fn();

@@ -1,5 +1,7 @@
-// tc_ptx.cuh -- PTX wrappers for the single-CTA tcgen05 / TMEM / TMA kernels (fine_tf.cu).  sm_100a only.
-// (coarse_tc.cu keeps its own cta_group::2 variants next to the kernel that uses them.)
+// tc_ptx.cuh -- the PTX layer of the tcgen05 / TMEM / TMA kernels (coarse_tc.cu, fine_tf.cu).  sm_100a only.
+// mbarriers, TMA, the UMMA descriptors, tcgen05.mma / commit / ld, TMEM allocation and the CTA-pair (cluster) helpers live
+// here and nowhere else; tc1 holds the single-CTA (cta_group::1) forms and everything that does not depend on the CTA
+// group, tc2 the CTA-pair (cta_group::2) forms.  Host side: the cuTensorMapEncodeTiled entry point.
 #pragma once
 #include <cuda.h>
 #include <stdint.h>
@@ -27,14 +29,43 @@ __device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity) {
       : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
   return ok != 0;
 }
-// Bounded wait: a protocol bug must become a launch failure, never a hung GPU.
+// Bounded waits: a protocol bug must become a launch failure, never a hung GPU.  Two loops, both giving up after ~2 s at
+// 2 GHz, because neither is best for every kernel:
+//   mbar_wait          reads the clock once and tests a poll counter on every poll (the fine-level kernels: with the
+//                      batched loop, mlp_fused_kernel spills more);
+//   mbar_wait_batched  polls in batches of 1024 and reads the clock between batches only (the coarse sweep: there the
+//                      nine instructions of a time-out test on every poll were a fifth of all instructions it issued).
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
   if (mbar_try_wait(bar, parity)) return;
   const long long t0 = clock64();
   uint32_t spins = 0;
   while (!mbar_try_wait(bar, parity)) {
-    if ((++spins & 255u) == 0 && clock64() - t0 > 4000000000ll) __trap();     // ~2 s at 2 GHz
+    if ((++spins & 255u) == 0 && clock64() - t0 > 4000000000ll) __trap();
   }
+}
+__device__ __forceinline__ void mbar_wait_batched(uint32_t bar, uint32_t parity) {
+  if (mbar_try_wait(bar, parity)) return;
+  long long t0 = 0;
+  for (;;) {
+#pragma unroll 1
+    for (int k = 0; k < 1024; ++k)
+      if (mbar_try_wait(bar, parity)) return;
+    long long t;
+    asm volatile("mov.u64 %0, %%clock64;" : "=l"(t)::"memory");
+    if (t0 == 0) t0 = t;
+    else if (t - t0 > 4000000000ll) __trap();
+  }
+}
+// one lane of a converged warp (the way the tensor-core instructions are issued: ptxas keeps their operands in uniform
+// registers when the single-thread region is entered through elect.sync)
+__device__ __forceinline__ bool elect_one() {
+  uint32_t ok;
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "elect.sync _|p, 0xffffffff;\n\t"
+      "selp.u32 %0, 1, 0, p;\n\t}"
+      : "=r"(ok));
+  return ok != 0;
 }
 __device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
@@ -76,7 +107,18 @@ __device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t a_desc, uint
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
 }
-// 32 lanes x 32 consecutive fp32 columns -> 32 registers per thread (lane = TMEM lane = accumulator row)
+// TMEM allocation (one whole warp): the base address of ncols columns is written to shared memory at dst
+__device__ __forceinline__ void tmem_alloc(uint32_t dst, uint32_t ncols) {
+  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst), "r"(ncols) : "memory");
+}
+__device__ __forceinline__ void tmem_relinquish() {
+  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+}
+__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
+  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
+}
+// 32 lanes x 32 consecutive fp32 columns -> 32 registers per thread (lane = TMEM lane = accumulator row); the wait is part
+// of the same statement so the registers are valid when it retires
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, float* v) {
   uint32_t r[32];
   asm volatile(
@@ -127,6 +169,11 @@ __device__ __forceinline__ void tma_load_2d_2sm(uint32_t dst, const CUtensorMap*
       "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
       ::"r"(dst), "l"(map), "r"(bar & kPeerMask), "r"(c0), "r"(c1) : "memory");
 }
+__device__ __forceinline__ void tma_load_3d_2sm(uint32_t dst, const CUtensorMap* map, uint32_t bar, int c0, int c1, int c2) {
+  asm volatile(
+      "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
+      ::"r"(dst), "l"(map), "r"(bar & kPeerMask), "r"(c0), "r"(c1), "r"(c2) : "memory");
+}
 // arrive on the leader CTA's copy of a barrier (from either CTA of the pair)
 __device__ __forceinline__ void mbar_arrive_leader(uint32_t bar) {
   asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(bar & kPeerMask) : "memory");
@@ -152,5 +199,31 @@ __device__ __forceinline__ void umma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
                ::"r"(bar), "h"(uint16_t(3)) : "memory");
 }
+// TMEM allocation for the pair: one warp of each CTA of the pair runs these together
+__device__ __forceinline__ void tmem_alloc(uint32_t dst, uint32_t ncols) {
+  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst), "r"(ncols) : "memory");
+}
+__device__ __forceinline__ void tmem_relinquish() {
+  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+}
+__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
+  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
+}
 }  // namespace tc2
+
+// ---- host side: the driver's tensor-map encoder, looked up once through the runtime (no link against libcuda) ------------
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
+                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+inline EncodeTiledFn encode_fn() {
+  static EncodeTiledFn fn = [] {
+    void* p = nullptr;
+    cudaDriverEntryPointQueryResult q;
+    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess ||
+        q != cudaDriverEntryPointSuccess)
+      p = nullptr;
+    return reinterpret_cast<EncodeTiledFn>(p);
+  }();
+  return fn;
+}
 }  // namespace pope
