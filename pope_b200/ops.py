@@ -377,7 +377,7 @@ def scratch_views(workspace: torch.Tensor, n: int, L: int, S: int) -> Dict[str, 
     G, B = (L + 31) // 32, (S + 31) // 32
     off, out = 0, {}
     for name, nbytes, dt, shape in (("rowbest", 8 * n * L, torch.int64, (n, L)), ("colbest", 8 * n * S, torch.int64, (n, S)),
-                                    ("cand_cnt", 8 * n * L, torch.int16, (n, L, 4)), ("ready", 4 * n, torch.int32, (n,)),
+                                    ("cand_cnt", 8 * n * L, torch.int16, (n, L, 4)), ("ready", 4 * (n + 1), torch.int32, (n + 1,)),
                                     ("lse_r", 4 * n * L, torch.float32, (n, L)), ("lse_c", 4 * n * S, torch.float32, (n, S)),
                                     ("cand", 8 * n * L * 4 * 24, torch.int64, (n, L, 16, 6)),
                                     ("cbound", 4 * n * G * 32, torch.float32, (n, G * 32)), ("cminb", 4 * n * G, torch.float32, (n, G)),
