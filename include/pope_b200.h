@@ -364,6 +364,39 @@ int pope_fine_merge_coarse_ex(void* win0, void* win1, int64_t m_windows, const i
                               const int64_t* b_ids, const int64_t* i_ids, const int64_t* j_ids, const void* weights,
                               void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- coarse-level transformer (bf16) ----------------------------------------------------------------------------------
+ * Replace src/matcher/matcher.py:57-58 (pos_encoding + rearrange to token-major) and transformer.py:34-58,95-104 +
+ * linear_attention.py:21-47 for LocalFeatureTransformer(config['coarse']): d_model 256, 8 heads, 'linear' attention,
+ * no masks.  The attention is global over each pair's source tokens.
+ *
+ * Packed weights of ONE d_model-256 LoFTREncoderLayer, POPE_COARSE_TF_LAYER_BYTES bytes, matrices bf16 row-major
+ * [out, in] exactly like nn.Linear.weight, LayerNorm parameters fp32:
+ *   +0        q_proj.weight | k_proj.weight | v_proj.weight   [768, 256]
+ *   +393216   merge.weight                                    [256, 256]
+ *   +524288   mlp.0.weight                                    [512, 512]
+ *   +1048576  mlp.2.weight                                    [256, 512]
+ *   +1310720  norm1.weight, norm1.bias, norm2.weight, norm2.bias   4 x [256] fp32                                       */
+#define POPE_COARSE_TF_LAYER_BYTES 1314816
+
+/* Bytes of device scratch for n_pairs pairs of L and S tokens (5 activation planes of [n_pairs * max(L, S), 256] bf16,
+ * the attention's per-chunk partial sums and its reduced KV); 0 for a non-positive or too large shape. */
+size_t pope_coarse_tf_workspace_bytes(int64_t n_pairs, int L, int S);
+
+/* feat0: [n_pairs, L, 256], feat1: [n_pairs, S, 256] bf16, contiguous, updated IN PLACE by n_layers encoder layers;
+ * layer_kinds[l] = 0 ('self') or 1 ('cross': feat0 attends to feat1, then feat1 to the new feat0), weights = n_layers
+ * consecutive packed layers.  Pointers 16-byte aligned (POPE_ERR_ALIGNMENT).  n_pairs * max(L, S) must stay below 2^31
+ * - 256 and n_pairs <= 65535 (POPE_ERR_SHAPE).  Argument errors return before any CUDA call; never synchronises,
+ * allocates nothing; n_pairs == 0 is a no-op.  Each pair's output depends on that pair's inputs only, bit for bit. */
+int pope_coarse_transformer(void* feat0, void* feat1, int64_t n_pairs, int L, int S, const void* weights, int n_layers,
+                            const int* layer_kinds, void* workspace, size_t workspace_bytes, void* stream);
+
+/* PositionEncodingSine + flatten(2).transpose(1, 2) + .to(bfloat16):
+ *   out[b, y * W + x, c] = bf16(feat[b, c, y, x] + pe[c, y, x])      (fp32 sum, one round to nearest even)
+ * feat: [n, C, H, W] fp32 contiguous (4-byte aligned), pe: the encoding's [C, pe_h, pe_w] fp32 buffer, out: [n, H * W, C]
+ * bf16 (16-byte aligned).  C must be 256 and H <= pe_h, W <= pe_w (POPE_ERR_SHAPE); n == 0 is a no-op. */
+int pope_coarse_pos_encode(const void* feat, const void* pe, int64_t n, int C, int H, int W, int pe_h, int pe_w, void* out,
+                           void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -19,6 +19,7 @@ FLAG_ROBUST_PATH = 4
 FLAG_CAPACITY = 8
 FINE_TF_LAYER_BYTES = 329728      # include/pope_b200.h: packed weights of one LoFTREncoderLayer (d_model 128)
 FINE_PRE_BYTES = 132096           # ... of FinePreprocess' down_proj + merge_feat
+COARSE_TF_LAYER_BYTES = 1314816   # ... of one d_model-256 LoFTREncoderLayer (the coarse transformer)
 
 _p, _i, _i64, _f, _sz = C.c_void_p, C.c_int, C.c_int64, C.c_float, C.c_size_t
 
@@ -42,6 +43,9 @@ SIGNATURES = {
     "pope_fine_merge_coarse": (_i, [_p, _p, _i64, _i, _p, _p, _i, _i, _i, _p, _p, _p, _p, _p, _sz, _p]),
     "pope_fine_transformer_ex": (_i, [_p, _p, _i64, _p, _i, _p, _i, C.POINTER(_i), _p, _sz, _p]),
     "pope_fine_merge_coarse_ex": (_i, [_p, _p, _i64, _p, _i, _p, _p, _i, _i, _i, _p, _p, _p, _p, _p, _sz, _p]),
+    "pope_coarse_tf_workspace_bytes": (_sz, [_i64, _i, _i]),
+    "pope_coarse_transformer": (_i, [_p, _p, _i64, _i, _i, _p, _i, C.POINTER(_i), _p, _sz, _p]),
+    "pope_coarse_pos_encode": (_i, [_p, _p, _i64, _i, _i, _i, _i, _i, _p, _p]),
     "pope_match_order_by_ref": (_i, [_p, _i, _i, _p, _p, _p]),
     "pope_savetxt_f32": (_i, [C.c_char_p, _p, _i64, _i]),
     "pope_savetxt_f64": (_i, [C.c_char_p, _p, _i64, _i]),

@@ -73,11 +73,6 @@ __device__ __forceinline__ int64_t live_count(int64_t cap, const int32_t* live, 
   return live ? min(cap, int64_t(max(*live, 0)) * per_item) : cap;
 }
 
-__device__ __forceinline__ uint32_t pack_bf16(float a, float b) {
-  __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
-  return *reinterpret_cast<uint32_t*>(&h);
-}
-
 // A 32-row output box that straddles the live bound is not TMA-stored (the store would write the rows past the bound):
 // each lane below the bound copies its own 64-column half row out of the 128B-swizzled staging box instead.
 __device__ __forceinline__ void store_staged_half_row(uint32_t my_row, uint32_t sw, __nv_bfloat16* dst) {
@@ -850,19 +845,6 @@ __global__ void __launch_bounds__(256) gather_coarse_rows_kernel(const __nv_bflo
 }
 
 // ---- host side ---------------------------------------------------------------------------------------------------------
-// [rows, cols] bf16 with a row pitch of `pitch` elements, box = 64 columns x box_rows rows, 128-byte swizzle, zero fill
-bool make_map2d(CUtensorMap* m, const void* base, int64_t rows, int cols, int64_t pitch, int box_rows = kTile) {
-  EncodeTiledFn enc = encode_fn();
-  if (!enc) return false;
-  cuuint64_t dims[2] = {cuuint64_t(cols), cuuint64_t(rows)};
-  cuuint64_t strides[1] = {cuuint64_t(pitch) * 2};
-  cuuint32_t box[2] = {kBoxK, cuuint32_t(box_rows)};
-  cuuint32_t estr[2] = {1, 1};
-  return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
-             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
 struct Dst { void* ptr; int64_t pitch; };                   // one 128-column block of the output (bf16, row pitch in elements)
 
 // Y[T, N] = epilogue(X[T, K] . W[N, K]^T), X contiguous bf16;  out[j] receives output columns [128 j, 128 j + 128).

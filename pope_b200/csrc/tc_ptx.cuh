@@ -4,6 +4,7 @@
 // group, tc2 the CTA-pair (cta_group::2) forms.  Host side: the cuTensorMapEncodeTiled entry point.
 #pragma once
 #include <cuda.h>
+#include <cuda_bf16.h>
 #include <stdint.h>
 
 namespace pope {
@@ -87,6 +88,10 @@ __device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk
 __device__ __forceinline__ void tma_store_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 __device__ __forceinline__ void tma_store_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
+__device__ __forceinline__ uint32_t pack_bf16(float a, float b) {
+  __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
+  return *reinterpret_cast<uint32_t*>(&h);
+}
 // K-major, 128B-swizzled operand tile: rows 128 B apart, 8-row groups 1024 B apart (SBO), LBO unused (=1), version 1.
 __device__ __forceinline__ uint64_t umma_desc(uint32_t smem_addr) {
   return uint64_t((smem_addr & 0x3ffffu) >> 4) | (uint64_t(1) << 16) | (uint64_t(1024 >> 4) << 32) | (uint64_t(1) << 46) |
@@ -225,5 +230,17 @@ inline EncodeTiledFn encode_fn() {
     return reinterpret_cast<EncodeTiledFn>(p);
   }();
   return fn;
+}
+// [rows, cols] bf16 with a row pitch of `pitch` elements, box = 64 columns x box_rows rows, 128-byte swizzle, zero fill
+inline bool make_map2d(CUtensorMap* m, const void* base, int64_t rows, int cols, int64_t pitch, int box_rows = 128) {
+  EncodeTiledFn enc = encode_fn();
+  if (!enc) return false;
+  cuuint64_t dims[2] = {cuuint64_t(cols), cuuint64_t(rows)};
+  cuuint64_t strides[1] = {cuuint64_t(pitch) * 2};
+  cuuint32_t box[2] = {64, cuuint32_t(box_rows)};
+  cuuint32_t estr[2] = {1, 1};
+  return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
+             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 }  // namespace pope

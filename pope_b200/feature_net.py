@@ -255,3 +255,45 @@ class FineTransformerB200(LocalFeatureTransformer):
         self._workspace = ops.fine_level_workspace(feat0.shape[0], feat0.shape[1], feat0.device, self._workspace,
                                                    merge=False)
         return ops.fine_transformer(feat0, feat1, self._packed_weights(feat0.device), self.layer_names, self._workspace)
+
+
+class CoarseTransformerB200(LocalFeatureTransformer):
+    """`loftr_coarse` with the encoder layers running in libpope_b200.so (csrc/coarse_tf.cu: tcgen05 Linears with fused
+    feature-map / LayerNorm / ReLU / residual epilogues + global linear attention reduced in a fixed order) when it is
+    handed CUDA bfloat16 features [N, L, 256] / [N, S, 256]; same parameters, same state-dict keys as
+    LocalFeatureTransformer (transformer.py:61-106).  fp32 features keep the stock PyTorch layers (the reference's
+    precision); masks (padded batches) are not supported by the CUDA path.
+
+    `inplace`: update the given feature tensors (the Matcher owns them) instead of working on copies."""
+
+    def __init__(self, config: dict, d_model: Optional[int] = None, LAYER_NAMES: Optional[List[str]] = None):
+        super().__init__(config, d_model, LAYER_NAMES)
+        self.inplace = False
+        self._packed = None
+        self._packed_key = None
+        self._workspace = None
+
+    def cuda_supported(self) -> bool:
+        return self.d_model == 256 and self.nhead == 8 and self.config["attention"] == "linear"
+
+    def _packed_weights(self, dev):
+        from . import ops
+        key = (str(dev),) + tuple((p.data_ptr(), p._version) for p in self.parameters())
+        if self._packed is None or self._packed_key != key:
+            self._packed = torch.cat([ops.pack_coarse_layer(layer.state_dict(), dev) for layer in self.layers])
+            self._packed_key = key
+        return self._packed
+
+    def forward(self, feat0, feat1, mask0=None, mask1=None):
+        if not (feat0.is_cuda and feat0.dtype == torch.bfloat16 and feat1.dtype == torch.bfloat16):
+            return super().forward(feat0, feat1, mask0, mask1)
+        if mask0 is not None or mask1 is not None or not self.cuda_supported():
+            raise NotImplementedError("the CUDA coarse transformer covers d_model 256 / 8 heads / linear attention without masks")
+        from . import ops
+        assert self.d_model == feat0.size(2), "the feature number of src and transformer must be equal"
+        if not self.inplace:
+            feat0, feat1 = feat0.clone(), feat1.clone()
+        feat0, feat1 = feat0.contiguous(), feat1.contiguous()
+        self._workspace = ops.coarse_tf_workspace(feat0.shape[0], feat0.shape[1], feat1.shape[1], feat0.device,
+                                                  self._workspace)
+        return ops.coarse_transformer(feat0, feat1, self._packed_weights(feat0.device), self.layer_names, self._workspace)

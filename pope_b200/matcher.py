@@ -6,7 +6,8 @@ mkpts0_c, mkpts1_c, mconf, W, expec_f, mkpts0_f, mkpts1_f), same sub-module name
 state-dict keys, and the same `load_state_dict` that strips a leading 'matcher.' (:81-85).
 
 Steps 3-5 of the forward (coarse match, fine-window gather, fine match; matcher.py:71-79) run in
-libpope_b200.so; the backbone and the two transformers are stock PyTorch modules (feature_net.py).
+libpope_b200.so; the backbone and the two transformers are stock PyTorch modules (feature_net.py) unless the bf16
+CUDA paths are switched on (`fine_cuda_bf16`, `coarse_cuda_bf16`).
 """
 from __future__ import annotations
 
@@ -14,27 +15,31 @@ import torch
 import torch.nn as nn
 
 from .coarse_matching import CoarseMatching
-from .feature_net import FineTransformerB200, LocalFeatureTransformer, PositionEncodingSine, build_backbone
+from .feature_net import CoarseTransformerB200, FineTransformerB200, PositionEncodingSine, build_backbone
 from .fine_matching import FineMatching
 from .fine_preprocess import FinePreprocess
 
 
 class Matcher(nn.Module):
-    def __init__(self, config: dict, fine_cuda_bf16: bool = False):
+    def __init__(self, config: dict, fine_cuda_bf16: bool = False, coarse_cuda_bf16: bool = False):
         """`fine_cuda_bf16` (not in the reference): run the fine level -- window gather, FinePreprocess Linears, fine
         transformer, fine matching -- in bfloat16 inside libpope_b200.so instead of fp32 torch modules between the CUDA
-        stages.  Parameters and state-dict keys are unchanged either way."""
+        stages.  `coarse_cuda_bf16` (not in the reference): add the position encoding, lay the coarse maps out token-major
+        and run the coarse transformer in bfloat16 inside libpope_b200.so; the coarse matcher then takes the bf16
+        features, and `forward(data, only_att_fea=True)` returns them as bfloat16.  Parameters and state-dict keys are
+        unchanged either way."""
         super().__init__()
         self.config = config
         self.backbone = build_backbone(config)
         self.pos_encoding = PositionEncodingSine(config["coarse"]["d_model"],
                                                  temp_bug_fix=config["coarse"]["temp_bug_fix"])
-        self.loftr_coarse = LocalFeatureTransformer(config["coarse"])
+        self.loftr_coarse = CoarseTransformerB200(config["coarse"])
         self.coarse_matching = CoarseMatching(config["match_coarse"])
         self.fine_preprocess = FinePreprocess(config)
         self.loftr_fine = FineTransformerB200(config["fine"])
         self.fine_matching = FineMatching()
         self.set_fine_cuda_bf16(fine_cuda_bf16)
+        self.set_coarse_cuda_bf16(coarse_cuda_bf16)
 
     def set_fine_cuda_bf16(self, on: bool) -> None:
         if on and not self.loftr_fine.cuda_supported():
@@ -42,6 +47,12 @@ class Matcher(nn.Module):
         self.fine_cuda_bf16 = bool(on)
         self.fine_preprocess.cuda_bf16 = bool(on)
         self.loftr_fine.inplace = bool(on)
+
+    def set_coarse_cuda_bf16(self, on: bool) -> None:
+        if on and not self.loftr_coarse.cuda_supported():
+            raise NotImplementedError("the CUDA coarse transformer covers d_model 256 / 8 heads / linear attention")
+        self.coarse_cuda_bf16 = bool(on)
+        self.loftr_coarse.inplace = bool(on)
 
     def fine_level(self, device) -> dict:
         """The packed bf16 weights of the fine level for `ops.match_pairs_device(..., fine_level=...)` (and the driver's
@@ -65,17 +76,24 @@ class Matcher(nn.Module):
         data.update({"hw0_c": feat_c0.shape[2:], "hw1_c": feat_c1.shape[2:],
                      "hw0_f": feat_f0.shape[2:], "hw1_f": feat_f1.shape[2:]})
 
-        # [N, C, H, W] -> [N, HW, C] after adding the position encoding
-        feat_c0 = self.pos_encoding(feat_c0).flatten(2).transpose(1, 2)
-        feat_c1 = self.pos_encoding(feat_c1).flatten(2).transpose(1, 2)
         mask_c0 = mask_c1 = None
         if "mask0" in data:
             mask_c0, mask_c1 = data["mask0"].flatten(-2), data["mask1"].flatten(-2)
+        # [N, C, H, W] -> [N, HW, C] after adding the position encoding
+        if self.coarse_cuda_bf16 and feat_c0.is_cuda:      # (with masks, loftr_coarse raises NotImplementedError)
+            from . import ops
+            feat_c0 = ops.coarse_pos_encode(feat_c0, self.pos_encoding.pe)
+            feat_c1 = ops.coarse_pos_encode(feat_c1, self.pos_encoding.pe)
+        else:
+            feat_c0 = self.pos_encoding(feat_c0).flatten(2).transpose(1, 2)
+            feat_c1 = self.pos_encoding(feat_c1).flatten(2).transpose(1, 2)
         feat_c0, feat_c1 = self.loftr_coarse(feat_c0, feat_c1, mask_c0, mask_c1)
         if only_att_fea:
             return feat_c0, feat_c1
 
         self.coarse_matching(feat_c0, feat_c1, data, mask_c0=mask_c0, mask_c1=mask_c1)
+        if feat_c0.dtype != feat_f0.dtype and not self.fine_cuda_bf16:     # the stock fine level runs in the maps' dtype
+            feat_c0, feat_c1 = feat_c0.to(feat_f0.dtype), feat_c1.to(feat_f0.dtype)
         win0, win1 = self.fine_preprocess(feat_f0, feat_f1, feat_c0, feat_c1, data)
         if win0.size(0) != 0:
             win0, win1 = self.loftr_fine(win0, win1)

@@ -191,6 +191,86 @@ def fine_transformer(feat0: torch.Tensor, feat1: torch.Tensor, packed_layers: to
     return feat0, feat1
 
 
+def pack_coarse_layer(sd: Dict[str, torch.Tensor], device) -> torch.Tensor:
+    """One LoFTREncoderLayer state dict (d_model 256) -> the packed byte layout of include/pope_b200.h
+    (POPE_COARSE_TF_LAYER_BYTES)."""
+    mats = [sd["q_proj.weight"], sd["k_proj.weight"], sd["v_proj.weight"], sd["merge.weight"], sd["mlp.0.weight"],
+            sd["mlp.2.weight"]]
+    shapes = [(256, 256)] * 4 + [(512, 512), (256, 512)]
+    for t, shp in zip(mats, shapes):
+        if tuple(t.shape) != shp:
+            raise _lib.PopeError(f"coarse transformer weight of shape {tuple(t.shape)}, expected {shp} (d_model 256, 8 heads)")
+    for k in ("norm1.weight", "norm1.bias", "norm2.weight", "norm2.bias"):
+        if tuple(sd[k].shape) != (256,):
+            raise _lib.PopeError(f"coarse transformer {k} of shape {tuple(sd[k].shape)}, expected (256,)")
+    w = torch.cat([t.detach().to(device=device, dtype=torch.bfloat16).reshape(-1) for t in mats]).view(torch.uint8)
+    ln = torch.cat([sd[k].detach().to(device=device, dtype=torch.float32).reshape(-1)
+                    for k in ("norm1.weight", "norm1.bias", "norm2.weight", "norm2.bias")]).view(torch.uint8)
+    out = torch.cat([w, ln])
+    assert out.numel() == _lib.COARSE_TF_LAYER_BYTES
+    return out
+
+
+def coarse_transformer(feat0: torch.Tensor, feat1: torch.Tensor, packed_layers: torch.Tensor, layer_names,
+                       workspace: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """LocalFeatureTransformer.forward (d_model 256, 8 heads, linear attention, no masks) on bf16 token-major features
+    feat0 [N, L, 256] and feat1 [N, S, 256], IN PLACE (returns the same tensors).  `packed_layers`: concatenation of
+    pack_coarse_layer() of every layer, `layer_names`: 'self' / 'cross'.  `workspace`: reused when large enough."""
+    dev = require_cuda(feat0, feat1, packed_layers)
+    if feat0.dtype != torch.bfloat16 or feat1.dtype != torch.bfloat16:
+        raise _lib.PopeError("the CUDA coarse transformer takes bfloat16 features")
+    if feat0.dim() != 3 or feat1.dim() != 3 or feat0.shape[0] != feat1.shape[0] or feat0.shape[2] != 256 \
+            or feat1.shape[2] != 256:
+        raise _lib.PopeError("feat0 / feat1 must be [N, L, 256] / [N, S, 256]")
+    if not (feat0.is_contiguous() and feat1.is_contiguous()):
+        raise _lib.PopeError("the CUDA coarse transformer updates its inputs in place: pass contiguous tensors")
+    kinds = []
+    for name in layer_names:
+        if name not in ("self", "cross"):
+            raise KeyError(name)
+        kinds.append(0 if name == "self" else 1)
+    if packed_layers.numel() != len(kinds) * _lib.COARSE_TF_LAYER_BYTES:
+        raise _lib.PopeError("packed_layers does not hold one packed layer per layer name")
+    n, L, S = feat0.shape[0], feat0.shape[1], feat1.shape[1]
+    if n == 0 or L == 0 or S == 0:
+        return feat0, feat1
+    workspace = coarse_tf_workspace(n, L, S, dev, workspace)
+    arr = (_lib.C.c_int * max(len(kinds), 1))(*kinds)
+    with torch.cuda.device(dev):
+        st = lib().pope_coarse_transformer(ptr(feat0), ptr(feat1), n, L, S, ptr(packed_layers), len(kinds), arr,
+                                           ptr(workspace), workspace.numel(), stream_ptr(dev))
+    check(st, "pope_coarse_transformer")
+    return feat0, feat1
+
+
+def coarse_tf_workspace(n: int, L: int, S: int, dev, workspace: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Scratch of the CUDA coarse transformer for n pairs of L and S tokens; `workspace` is returned when large enough."""
+    need = lib().pope_coarse_tf_workspace_bytes(int(n), int(L), int(S))
+    if need == 0:
+        raise _lib.PopeError(f"coarse transformer shape n={n}, L={L}, S={S} is outside what the kernels index")
+    if workspace is None or workspace.numel() < need or workspace.device != dev:
+        workspace = torch.empty(need, dtype=torch.uint8, device=dev)
+    return workspace
+
+
+def coarse_pos_encode(feat: torch.Tensor, pe: torch.Tensor) -> torch.Tensor:
+    """PositionEncodingSine + flatten(2).transpose(1, 2) + .to(torch.bfloat16) in one kernel: feat [N, 256, H, W] fp32 ->
+    [N, H*W, 256] bf16, bit-identical to `(feat + pe[..., :H, :W]).flatten(2).transpose(1, 2).to(torch.bfloat16)`.
+    `pe`: the encoding's `pe` buffer [1, 256, Hmax, Wmax] fp32."""
+    dev = require_cuda(feat, pe)
+    if feat.dtype != torch.float32 or pe.dtype != torch.float32 or feat.dim() != 4 or pe.dim() != 4 or pe.shape[0] != 1:
+        raise _lib.PopeError("coarse_pos_encode takes an fp32 [N, C, H, W] map and the fp32 [1, C, Hmax, Wmax] encoding")
+    if pe.shape[1] != feat.shape[1]:
+        raise _lib.PopeError("the encoding and the map differ in channels")
+    feat, pe = feat.contiguous(), pe.contiguous()
+    n, c, h, w = feat.shape
+    out = torch.empty(n, h * w, c, dtype=torch.bfloat16, device=dev)
+    with torch.cuda.device(dev):
+        st = lib().pope_coarse_pos_encode(ptr(feat), ptr(pe), n, c, h, w, pe.shape[2], pe.shape[3], ptr(out), stream_ptr(dev))
+    check(st, "pope_coarse_pos_encode")
+    return out
+
+
 def fine_merge_coarse(win0: torch.Tensor, win1: torch.Tensor, feat_c0: torch.Tensor, feat_c1: torch.Tensor, b_ids, i_ids,
                       j_ids, packed_pre: torch.Tensor, workspace: Optional[torch.Tensor] = None,
                       m_dev: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
