@@ -390,6 +390,30 @@ size_t pope_coarse_tf_workspace_bytes(int64_t n_pairs, int L, int S);
 int pope_coarse_transformer(void* feat0, void* feat1, int64_t n_pairs, int L, int S, const void* weights, int n_layers,
                             const int* layer_kinds, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- coarse-level transformer at fp32 accuracy ------------------------------------------------------------------------
+ * The same layers on fp32 features, computed on the bf16 tensor cores with every GEMM operand split into three bf16 terms
+ * w = w1 + w2 + w3 (24 mantissa bits) and the six significant products accumulated in fp32; activations, the attention,
+ * the LayerNorms and the residuals are fp32.  Results agree with the fp32 modules up to rounding.
+ *
+ * Packed weights of ONE layer, POPE_COARSE_TF_F32_LAYER_BYTES bytes: every matrix as three consecutive bf16 planes
+ * [plane][out][in] (w1 = bf16(w), w2 = bf16(w - w1), w3 = bf16(w - w1 - w2), each residual exact in fp32), LayerNorm
+ * parameters fp32:
+ *   +0        q_proj | k_proj | v_proj   3 planes of [768, 256]  (planes 393216 bytes apart)
+ *   +1179648  merge.weight               3 planes of [256, 256]  (131072 bytes apart)
+ *   +1572864  mlp.0.weight               3 planes of [512, 512]  (524288 bytes apart)
+ *   +3145728  mlp.2.weight               3 planes of [256, 512]  (262144 bytes apart)
+ *   +3932160  norm1.weight, norm1.bias, norm2.weight, norm2.bias   4 x [256] fp32                                       */
+#define POPE_COARSE_TF_F32_LAYER_BYTES 3936256
+
+/* Bytes of device scratch of pope_coarse_transformer_f32 (5 fp32 activation planes and 9 bf16 split planes of
+ * [n_pairs * max(L, S), 256], the attention's partial sums and reduced KV); 0 for a non-positive or too large shape. */
+size_t pope_coarse_tf_f32_workspace_bytes(int64_t n_pairs, int L, int S);
+
+/* pope_coarse_transformer on fp32 features [n_pairs, L, 256] / [n_pairs, S, 256] (contiguous, updated IN PLACE) with
+ * weights packed as above.  Same argument checks, limits and guarantees as pope_coarse_transformer. */
+int pope_coarse_transformer_f32(void* feat0, void* feat1, int64_t n_pairs, int L, int S, const void* weights, int n_layers,
+                                const int* layer_kinds, void* workspace, size_t workspace_bytes, void* stream);
+
 /* PositionEncodingSine + flatten(2).transpose(1, 2) + .to(bfloat16):
  *   out[b, y * W + x, c] = bf16(feat[b, c, y, x] + pe[c, y, x])      (fp32 sum, one round to nearest even)
  * feat: [n, C, H, W] fp32 contiguous (4-byte aligned), pe: the encoding's [C, pe_h, pe_w] fp32 buffer, out: [n, H * W, C]

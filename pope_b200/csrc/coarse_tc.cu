@@ -40,6 +40,7 @@
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "split3.cuh"
 #include "tc_ptx.cuh"
 
 namespace pope {
@@ -948,28 +949,6 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap map0, const __grid_constant_
   if (warp == kWarpMma) {
     tc_fence_after();
     tc2::tmem_dealloc(tmem_base, kTmemCols);
-  }
-}
-
-// fp32 -> three bf16 planes with a = a1 + a2 + a3 (each residual is exact in fp32): 8 + 8 + 8 mantissa bits
-__global__ void __launch_bounds__(256) split3_kernel(const float4* __restrict__ in, uint2* __restrict__ p1, uint2* __restrict__ p2,
-                                                    uint2* __restrict__ p3, size_t n4) {
-  for (size_t i = size_t(blockIdx.x) * blockDim.x + threadIdx.x; i < n4; i += size_t(gridDim.x) * blockDim.x) {
-    const float4 a = __ldcs(in + i);
-    const float v[4] = {a.x, a.y, a.z, a.w};
-    uint32_t h1[4], h2[4], h3[4];
-#pragma unroll
-    for (int e = 0; e < 4; ++e) {
-      const __nv_bfloat16 b1 = __float2bfloat16_rn(v[e]);
-      const float r1 = v[e] - __bfloat162float(b1);
-      const __nv_bfloat16 b2 = __float2bfloat16_rn(r1);
-      const float r2 = r1 - __bfloat162float(b2);
-      const __nv_bfloat16 b3 = __float2bfloat16_rn(r2);
-      h1[e] = __bfloat16_as_ushort(b1); h2[e] = __bfloat16_as_ushort(b2); h3[e] = __bfloat16_as_ushort(b3);
-    }
-    p1[i] = make_uint2(h1[0] | (h1[1] << 16), h1[2] | (h1[3] << 16));
-    p2[i] = make_uint2(h2[0] | (h2[1] << 16), h2[2] | (h2[3] << 16));
-    p3[i] = make_uint2(h3[0] | (h3[1] << 16), h3[2] | (h3[3] << 16));
   }
 }
 

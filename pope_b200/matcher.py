@@ -7,7 +7,8 @@ state-dict keys, and the same `load_state_dict` that strips a leading 'matcher.'
 
 Steps 3-5 of the forward (coarse match, fine-window gather, fine match; matcher.py:71-79) run in
 libpope_b200.so; the backbone and the two transformers are stock PyTorch modules (feature_net.py) unless the bf16
-CUDA paths are switched on (`fine_cuda_bf16`, `coarse_cuda_bf16`).
+CUDA paths are switched on (`fine_cuda_bf16`, `coarse_cuda_bf16`) or the fp32-accuracy CUDA coarse transformer is
+(`coarse_cuda_fp32`).
 """
 from __future__ import annotations
 
@@ -21,13 +22,17 @@ from .fine_preprocess import FinePreprocess
 
 
 class Matcher(nn.Module):
-    def __init__(self, config: dict, fine_cuda_bf16: bool = False, coarse_cuda_bf16: bool = False):
+    def __init__(self, config: dict, fine_cuda_bf16: bool = False, coarse_cuda_bf16: bool = False,
+                 coarse_cuda_fp32: bool = False):
         """`fine_cuda_bf16` (not in the reference): run the fine level -- window gather, FinePreprocess Linears, fine
         transformer, fine matching -- in bfloat16 inside libpope_b200.so instead of fp32 torch modules between the CUDA
         stages.  `coarse_cuda_bf16` (not in the reference): add the position encoding, lay the coarse maps out token-major
         and run the coarse transformer in bfloat16 inside libpope_b200.so; the coarse matcher then takes the bf16
-        features, and `forward(data, only_att_fea=True)` returns them as bfloat16.  Parameters and state-dict keys are
-        unchanged either way."""
+        features, and `forward(data, only_att_fea=True)` returns them as bfloat16.  `coarse_cuda_fp32` (not in the
+        reference): run the coarse transformer at fp32 accuracy inside libpope_b200.so (bf16 tensor cores on operands
+        split into three bf16 terms); everything else, the position encoding included, stays as in the stock flow, and
+        the features keep their dtype (fp32), shape and values up to rounding.  The two coarse flags exclude each other
+        (ValueError).  Parameters and state-dict keys are unchanged either way."""
         super().__init__()
         self.config = config
         self.backbone = build_backbone(config)
@@ -38,8 +43,12 @@ class Matcher(nn.Module):
         self.fine_preprocess = FinePreprocess(config)
         self.loftr_fine = FineTransformerB200(config["fine"])
         self.fine_matching = FineMatching()
+        if coarse_cuda_bf16 and coarse_cuda_fp32:
+            raise ValueError("coarse_cuda_bf16 and coarse_cuda_fp32 exclude each other")
+        self.coarse_cuda_fp32 = False
         self.set_fine_cuda_bf16(fine_cuda_bf16)
         self.set_coarse_cuda_bf16(coarse_cuda_bf16)
+        self.set_coarse_cuda_fp32(coarse_cuda_fp32)
 
     def set_fine_cuda_bf16(self, on: bool) -> None:
         if on and not self.loftr_fine.cuda_supported():
@@ -51,8 +60,19 @@ class Matcher(nn.Module):
     def set_coarse_cuda_bf16(self, on: bool) -> None:
         if on and not self.loftr_coarse.cuda_supported():
             raise NotImplementedError("the CUDA coarse transformer covers d_model 256 / 8 heads / linear attention")
+        if on and self.coarse_cuda_fp32:
+            raise ValueError("coarse_cuda_bf16 and coarse_cuda_fp32 exclude each other")
         self.coarse_cuda_bf16 = bool(on)
-        self.loftr_coarse.inplace = bool(on)
+        self.loftr_coarse.inplace = self.coarse_cuda_bf16 or self.coarse_cuda_fp32
+
+    def set_coarse_cuda_fp32(self, on: bool) -> None:
+        if on and not self.loftr_coarse.cuda_supported():
+            raise NotImplementedError("the CUDA coarse transformer covers d_model 256 / 8 heads / linear attention")
+        if on and self.coarse_cuda_bf16:
+            raise ValueError("coarse_cuda_bf16 and coarse_cuda_fp32 exclude each other")
+        self.coarse_cuda_fp32 = bool(on)
+        self.loftr_coarse.cuda_fp32 = self.coarse_cuda_fp32
+        self.loftr_coarse.inplace = self.coarse_cuda_bf16 or self.coarse_cuda_fp32
 
     def fine_level(self, device) -> dict:
         """The packed bf16 weights of the fine level for `ops.match_pairs_device(..., fine_level=...)` (and the driver's

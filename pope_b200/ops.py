@@ -191,9 +191,24 @@ def fine_transformer(feat0: torch.Tensor, feat1: torch.Tensor, packed_layers: to
     return feat0, feat1
 
 
-def pack_coarse_layer(sd: Dict[str, torch.Tensor], device) -> torch.Tensor:
-    """One LoFTREncoderLayer state dict (d_model 256) -> the packed byte layout of include/pope_b200.h
-    (POPE_COARSE_TF_LAYER_BYTES)."""
+def split3_bf16(w: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """fp32 -> three bf16 terms w1 + w2 + w3 (8 mantissa bits each, every residual exact in fp32): the operand split of the
+    fp32-accuracy tensor-core paths (csrc/split3.cuh).  The sum is w exactly for fp32 values down to 2^-110 in
+    magnitude; below that the third term runs into the bf16 subnormal range and the sum is w to within 2^-134."""
+    w = w.to(torch.float32)
+    w1 = w.to(torch.bfloat16)
+    r1 = w - w1.float()
+    w2 = r1.to(torch.bfloat16)
+    w3 = (r1 - w2.float()).to(torch.bfloat16)
+    return w1, w2, w3
+
+
+def pack_coarse_layer(sd: Dict[str, torch.Tensor], device, dtype: torch.dtype = torch.bfloat16) -> torch.Tensor:
+    """One LoFTREncoderLayer state dict (d_model 256) -> the packed byte layout of include/pope_b200.h:
+    POPE_COARSE_TF_LAYER_BYTES for dtype=torch.bfloat16 (the bf16 transformer), POPE_COARSE_TF_F32_LAYER_BYTES for
+    dtype=torch.float32 (the fp32-accuracy transformer: every matrix as its three bf16 planes, split3_bf16)."""
+    if dtype not in (torch.bfloat16, torch.float32):
+        raise _lib.PopeError(f"the coarse transformer packs for torch.bfloat16 or torch.float32, not {dtype}")
     mats = [sd["q_proj.weight"], sd["k_proj.weight"], sd["v_proj.weight"], sd["merge.weight"], sd["mlp.0.weight"],
             sd["mlp.2.weight"]]
     shapes = [(256, 256)] * 4 + [(512, 512), (256, 512)]
@@ -203,22 +218,33 @@ def pack_coarse_layer(sd: Dict[str, torch.Tensor], device) -> torch.Tensor:
     for k in ("norm1.weight", "norm1.bias", "norm2.weight", "norm2.bias"):
         if tuple(sd[k].shape) != (256,):
             raise _lib.PopeError(f"coarse transformer {k} of shape {tuple(sd[k].shape)}, expected (256,)")
-    w = torch.cat([t.detach().to(device=device, dtype=torch.bfloat16).reshape(-1) for t in mats]).view(torch.uint8)
+    if dtype == torch.bfloat16:
+        w = torch.cat([t.detach().to(device=device, dtype=torch.bfloat16).reshape(-1) for t in mats]).view(torch.uint8)
+        size = _lib.COARSE_TF_LAYER_BYTES
+    else:
+        # q | k | v stacked as one [768, 256] matrix, then split: plane p of a matrix holds term p of every element
+        qkv = torch.cat([t.detach().to(device=device, dtype=torch.float32) for t in mats[:3]])
+        groups = [qkv] + [t.detach().to(device=device, dtype=torch.float32) for t in mats[3:]]
+        w = torch.cat([p.reshape(-1) for g in groups for p in split3_bf16(g)]).view(torch.uint8)
+        size = _lib.COARSE_TF_F32_LAYER_BYTES
     ln = torch.cat([sd[k].detach().to(device=device, dtype=torch.float32).reshape(-1)
                     for k in ("norm1.weight", "norm1.bias", "norm2.weight", "norm2.bias")]).view(torch.uint8)
     out = torch.cat([w, ln])
-    assert out.numel() == _lib.COARSE_TF_LAYER_BYTES
+    assert out.numel() == size
     return out
 
 
 def coarse_transformer(feat0: torch.Tensor, feat1: torch.Tensor, packed_layers: torch.Tensor, layer_names,
                        workspace: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
-    """LocalFeatureTransformer.forward (d_model 256, 8 heads, linear attention, no masks) on bf16 token-major features
-    feat0 [N, L, 256] and feat1 [N, S, 256], IN PLACE (returns the same tensors).  `packed_layers`: concatenation of
-    pack_coarse_layer() of every layer, `layer_names`: 'self' / 'cross'.  `workspace`: reused when large enough."""
+    """LocalFeatureTransformer.forward (d_model 256, 8 heads, linear attention, no masks) on token-major features
+    feat0 [N, L, 256] and feat1 [N, S, 256], IN PLACE (returns the same tensors).  bfloat16 features run the bf16
+    transformer, float32 features the fp32-accuracy one; `packed_layers`: concatenation of
+    pack_coarse_layer(..., dtype=<the features' dtype>) of every layer, `layer_names`: 'self' / 'cross'.
+    `workspace`: reused when large enough."""
     dev = require_cuda(feat0, feat1, packed_layers)
-    if feat0.dtype != torch.bfloat16 or feat1.dtype != torch.bfloat16:
-        raise _lib.PopeError("the CUDA coarse transformer takes bfloat16 features")
+    if feat0.dtype != feat1.dtype or feat0.dtype not in (torch.bfloat16, torch.float32):
+        raise _lib.PopeError("the CUDA coarse transformer takes bfloat16 or float32 features (both sides alike)")
+    f32 = feat0.dtype == torch.float32
     if feat0.dim() != 3 or feat1.dim() != 3 or feat0.shape[0] != feat1.shape[0] or feat0.shape[2] != 256 \
             or feat1.shape[2] != 256:
         raise _lib.PopeError("feat0 / feat1 must be [N, L, 256] / [N, S, 256]")
@@ -229,23 +255,34 @@ def coarse_transformer(feat0: torch.Tensor, feat1: torch.Tensor, packed_layers: 
         if name not in ("self", "cross"):
             raise KeyError(name)
         kinds.append(0 if name == "self" else 1)
-    if packed_layers.numel() != len(kinds) * _lib.COARSE_TF_LAYER_BYTES:
+    per_layer = _lib.COARSE_TF_F32_LAYER_BYTES if f32 else _lib.COARSE_TF_LAYER_BYTES
+    if packed_layers.numel() != len(kinds) * per_layer:
+        other = _lib.COARSE_TF_LAYER_BYTES if f32 else _lib.COARSE_TF_F32_LAYER_BYTES
+        if packed_layers.numel() == len(kinds) * other:
+            raise _lib.PopeError(f"{feat0.dtype} features need layers packed with pack_coarse_layer(..., dtype={feat0.dtype})")
         raise _lib.PopeError("packed_layers does not hold one packed layer per layer name")
     n, L, S = feat0.shape[0], feat0.shape[1], feat1.shape[1]
     if n == 0 or L == 0 or S == 0:
         return feat0, feat1
-    workspace = coarse_tf_workspace(n, L, S, dev, workspace)
+    workspace = coarse_tf_workspace(n, L, S, dev, workspace, dtype=feat0.dtype)
     arr = (_lib.C.c_int * max(len(kinds), 1))(*kinds)
+    fn, name = ((lib().pope_coarse_transformer_f32, "pope_coarse_transformer_f32") if f32 else
+                (lib().pope_coarse_transformer, "pope_coarse_transformer"))
     with torch.cuda.device(dev):
-        st = lib().pope_coarse_transformer(ptr(feat0), ptr(feat1), n, L, S, ptr(packed_layers), len(kinds), arr,
-                                           ptr(workspace), workspace.numel(), stream_ptr(dev))
-    check(st, "pope_coarse_transformer")
+        st = fn(ptr(feat0), ptr(feat1), n, L, S, ptr(packed_layers), len(kinds), arr, ptr(workspace), workspace.numel(),
+                stream_ptr(dev))
+    check(st, name)
     return feat0, feat1
 
 
-def coarse_tf_workspace(n: int, L: int, S: int, dev, workspace: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """Scratch of the CUDA coarse transformer for n pairs of L and S tokens; `workspace` is returned when large enough."""
-    need = lib().pope_coarse_tf_workspace_bytes(int(n), int(L), int(S))
+def coarse_tf_workspace(n: int, L: int, S: int, dev, workspace: Optional[torch.Tensor] = None,
+                        dtype: torch.dtype = torch.bfloat16) -> torch.Tensor:
+    """Scratch of the CUDA coarse transformer (bf16, or fp32 accuracy for dtype=torch.float32) for n pairs of L and S
+    tokens; `workspace` is returned when large enough."""
+    if dtype not in (torch.bfloat16, torch.float32):
+        raise _lib.PopeError(f"the CUDA coarse transformer runs in torch.bfloat16 or torch.float32, not {dtype}")
+    query = lib().pope_coarse_tf_f32_workspace_bytes if dtype == torch.float32 else lib().pope_coarse_tf_workspace_bytes
+    need = query(int(n), int(L), int(S))
     if need == 0:
         raise _lib.PopeError(f"coarse transformer shape n={n}, L={L}, S={S} is outside what the kernels index")
     if workspace is None or workspace.numel() < need or workspace.device != dev:

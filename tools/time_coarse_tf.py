@@ -1,6 +1,7 @@
 """Times the coarse LoFTR transformer (8 layers, d_model 256) on N pairs at 480x640 (60x80 = 4800 tokens per image;
-default N = 64): the stock PyTorch modules in fp32 and cast to bf16, and the CUDA bf16 path (csrc/coarse_tf.cu); then
-Matcher.forward from images with the default flags, with fine_cuda_bf16 and with both bf16 flags.  CUDA events, after
+default N = 64): the stock PyTorch modules in fp32 and cast to bf16, the CUDA fp32-accuracy path and the CUDA bf16 path
+(csrc/coarse_tf.cu); then Matcher.forward from images with the default flags, with fine_cuda_bf16, with both bf16 flags
+and with coarse_cuda_fp32.  CUDA events, after
 a warm-up of every timed shape; the inputs (N x 4800 x 256 per side) are larger than the 126 MB L2 at N = 64.
 Prints the card's name and power limit and one JSON line (also written to the path given with --json)."""
 import argparse
@@ -71,17 +72,27 @@ with torch.no_grad():
     ws = ops.coarse_tf_workspace(N, L, L, dev)
     a, b = f0.clone(), f1.clone()
     res["tf_cuda_bf16_ms"] = timed(lambda: ops.coarse_transformer(a, b, packed, tf.layer_names, ws), args.reps)
-    for k in ("tf_stock_fp32", "tf_stock_bf16", "tf_cuda_bf16"):
+    del a, b, ws
+    packed32 = tf._packed_weights(dev, torch.float32)
+    ws32 = ops.coarse_tf_workspace(N, L, L, dev, dtype=torch.float32)
+    a32, b32 = x0.clone(), x1.clone()
+    res["tf_cuda_fp32_ms"] = timed(lambda: ops.coarse_transformer(a32, b32, packed32, tf.layer_names, ws32), args.reps)
+    del a32, b32, ws32
+    torch.cuda.empty_cache()
+    for k in ("tf_stock_fp32", "tf_cuda_fp32", "tf_stock_bf16", "tf_cuda_bf16"):
         tflops = FLOP_PER_PAIR * N / (res[k + "_ms"] * 1e-3) / 1e12
         res[k + "_tflops"] = round(tflops, 1)
         res[k + "_share_of_sustained_bf16_peak"] = round(tflops / BF16_PEAK_TFLOPS["sustained"], 4)
     res["cuda_speedup_vs_stock_bf16"] = round(res["tf_stock_bf16_ms"] / res["tf_cuda_bf16_ms"], 3)
+    res["cuda_fp32_speedup_vs_stock_fp32"] = round(res["tf_stock_fp32_ms"] / res["tf_cuda_fp32_ms"], 3)
+    res["tf_cuda_fp32_bf16_mma_tflops"] = round(6 * res["tf_cuda_fp32_tflops"], 1)   # six bf16 products per fp32 one
 
     gen = torch.Generator(device=dev).manual_seed(2)
     img = {"image0": torch.rand(N, 1, 480, 640, device=dev, generator=gen),
            "image1": torch.rand(N, 1, 480, 640, device=dev, generator=gen)}
     for name, flags in (("matcher_default", {}), ("matcher_fine_bf16", {"fine_cuda_bf16": True}),
-                        ("matcher_fine_and_coarse_bf16", {"fine_cuda_bf16": True, "coarse_cuda_bf16": True})):
+                        ("matcher_fine_and_coarse_bf16", {"fine_cuda_bf16": True, "coarse_cuda_bf16": True}),
+                        ("matcher_coarse_fp32", {"coarse_cuda_fp32": True})):
         mm = pope_b200.Matcher(cfg, **flags).eval().to(dev)
         mm.load_state_dict(m.state_dict())
         res[name + "_ms"] = timed(lambda: mm(dict(img)), max(2, args.reps // 2))
