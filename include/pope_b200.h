@@ -364,6 +364,49 @@ int pope_fine_merge_coarse_ex(void* win0, void* win1, int64_t m_windows, const i
                               const int64_t* b_ids, const int64_t* i_ids, const int64_t* j_ids, const void* weights,
                               void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- fine-level transformer and FinePreprocess Linears at fp32 accuracy -------------------------------------------------
+ * The same layers on fp32 windows, computed on the bf16 tensor cores with every GEMM operand split into three bf16 terms
+ * w = w1 + w2 + w3 (24 mantissa bits) and the six significant products accumulated in fp32; activations, the attention,
+ * the LayerNorms, biases and residuals are fp32.  Results agree with the fp32 modules up to rounding.
+ *
+ * Packed weights: the bf16 layouts above with every matrix as three consecutive bf16 planes [plane][out][in] (w1 = bf16(w),
+ * w2 = bf16(w - w1), w3 = bf16(w - w1 - w2), each residual exact in fp32) at 3x its bf16 offset, the fp32 tail unchanged.
+ * ONE LoFTREncoderLayer, POPE_FINE_TF_F32_LAYER_BYTES bytes:
+ *   +0       q_proj | k_proj | v_proj   3 planes of [384, 128]  (planes 98304 bytes apart)
+ *   +294912  merge.weight               3 planes of [128, 128]  (32768 bytes apart)
+ *   +393216  mlp.0.weight               3 planes of [256, 256]  (131072 bytes apart)
+ *   +786432  mlp.2.weight               3 planes of [128, 256]  (65536 bytes apart)
+ *   +983040  norm1.weight, norm1.bias, norm2.weight, norm2.bias   4 x [128] fp32
+ * FinePreprocess, POPE_FINE_PRE_F32_BYTES bytes:
+ *   +0       down_proj.weight  3 planes of [128, 256] (65536 bytes apart)
+ *   +196608  merge_feat.weight 3 planes of [128, 256] (65536 bytes apart)
+ *   +393216  down_proj.bias [128] fp32            +393728 merge_feat.bias [128] fp32                                   */
+#define POPE_FINE_TF_F32_LAYER_BYTES 985088
+#define POPE_FINE_PRE_F32_BYTES 394240
+
+/* Bytes of device scratch of pope_fine_transformer_f32: 5 fp32 activation planes and 9 bf16 split planes of
+ * [m_windows * window_tokens, 128], 4 864 bytes per token (19.8 GB at 162 812 windows of 25 tokens). */
+size_t pope_fine_tf_f32_workspace_bytes(int64_t m_windows, int window_tokens);
+
+/* pope_fine_transformer on fp32 windows [m_windows, window_tokens, 128] (contiguous, updated IN PLACE) with layers packed
+ * as above.  Same arguments and error codes; pointers 16-byte aligned (POPE_ERR_ALIGNMENT), m_windows * window_tokens
+ * below 2^31 - 128 (POPE_ERR_SHAPE).  Never synchronises; m_windows == 0 is a no-op; each window's output depends on that
+ * window's inputs only, bit for bit. */
+int pope_fine_transformer_f32(void* feat0, void* feat1, int64_t m_windows, int window_tokens, const void* weights,
+                              int n_layers, const int* layer_kinds, void* workspace, size_t workspace_bytes, void* stream);
+
+/* Bytes of device scratch of pope_fine_merge_coarse_f32 (gathered and projected coarse rows with their split planes,
+ * per-window vectors; 8 704 bytes per window, for any window size). */
+size_t pope_fine_merge_f32_workspace_bytes(int64_t m_windows);
+
+/* pope_fine_merge_coarse on fp32 windows win0/win1 [m, window_tokens, 128] and fp32 feat_c0 [N, L, 256] / feat_c1
+ * [N, S, 256] with weights packed as above.  Same arguments and error codes; windows, coarse features, weights and
+ * workspace 16-byte aligned (POPE_ERR_ALIGNMENT), m * window_tokens below 2^31 - 128 (POPE_ERR_SHAPE). */
+int pope_fine_merge_coarse_f32(void* win0, void* win1, int64_t m_windows, int window_tokens, const void* feat_c0,
+                               const void* feat_c1, int L, int S, int C, const int64_t* b_ids, const int64_t* i_ids,
+                               const int64_t* j_ids, const void* weights, void* workspace, size_t workspace_bytes,
+                               void* stream);
+
 /* ---- coarse-level transformer (bf16) ----------------------------------------------------------------------------------
  * Replace src/matcher/matcher.py:57-58 (pos_encoding + rearrange to token-major) and transformer.py:34-58,95-104 +
  * linear_attention.py:21-47 for LocalFeatureTransformer(config['coarse']): d_model 256, 8 heads, 'linear' attention,

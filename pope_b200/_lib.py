@@ -21,6 +21,8 @@ FINE_TF_LAYER_BYTES = 329728      # include/pope_b200.h: packed weights of one L
 FINE_PRE_BYTES = 132096           # ... of FinePreprocess' down_proj + merge_feat
 COARSE_TF_LAYER_BYTES = 1314816   # ... of one d_model-256 LoFTREncoderLayer (the coarse transformer)
 COARSE_TF_F32_LAYER_BYTES = 3936256   # ... of the same layer for the fp32-accuracy transformer (three bf16 planes a matrix)
+FINE_TF_F32_LAYER_BYTES = 985088  # ... of one d_model-128 LoFTREncoderLayer for the fp32-accuracy fine level
+FINE_PRE_F32_BYTES = 394240       # ... of FinePreprocess' down_proj + merge_feat for the fp32-accuracy fine level
 
 _p, _i, _i64, _f, _sz = C.c_void_p, C.c_int, C.c_int64, C.c_float, C.c_size_t
 
@@ -49,6 +51,10 @@ SIGNATURES = {
     "pope_coarse_pos_encode": (_i, [_p, _p, _i64, _i, _i, _i, _i, _i, _p, _p]),
     "pope_coarse_tf_f32_workspace_bytes": (_sz, [_i64, _i, _i]),
     "pope_coarse_transformer_f32": (_i, [_p, _p, _i64, _i, _i, _p, _i, C.POINTER(_i), _p, _sz, _p]),
+    "pope_fine_tf_f32_workspace_bytes": (_sz, [_i64, _i]),
+    "pope_fine_transformer_f32": (_i, [_p, _p, _i64, _i, _p, _i, C.POINTER(_i), _p, _sz, _p]),
+    "pope_fine_merge_f32_workspace_bytes": (_sz, [_i64]),
+    "pope_fine_merge_coarse_f32": (_i, [_p, _p, _i64, _i, _p, _p, _i, _i, _i, _p, _p, _p, _p, _p, _sz, _p]),
     "pope_match_order_by_ref": (_i, [_p, _i, _i, _p, _p, _p]),
     "pope_savetxt_f32": (_i, [C.c_char_p, _p, _i64, _i]),
     "pope_savetxt_f64": (_i, [C.c_char_p, _p, _i64, _i]),

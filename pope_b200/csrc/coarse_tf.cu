@@ -492,32 +492,6 @@ coarse_pos_encode_kernel(const float* __restrict__ feat, const float* __restrict
 
 // ---- host side ---------------------------------------------------------------------------------------------------------
 struct Dst { void* ptr; int64_t pitch; };         // one 256-column output block (row pitch in elements)
-struct Planes { const void* ptr; size_t stride; }; // three bf16 planes: plane 0 and the byte distance between planes
-
-// [rows, cols] fp32 with a row pitch of `pitch` elements, box = 32 columns (128 bytes) x 32 rows, 128-byte swizzle
-bool make_map2d_f32(CUtensorMap* m, const void* base, int64_t rows, int cols, int64_t pitch) {
-  EncodeTiledFn enc = encode_fn();
-  if (!enc) return false;
-  cuuint64_t dims[2] = {cuuint64_t(cols), cuuint64_t(rows)};
-  cuuint64_t strides[1] = {cuuint64_t(pitch) * 4};
-  cuuint32_t box[2] = {32, 32};
-  cuuint32_t estr[2] = {1, 1};
-  return enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(base), dims, strides, box, estr,
-             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-// three [rows, cols] bf16 planes (row pitch = cols), box = 64 columns x box_rows rows x one plane, 128-byte swizzle
-bool make_map_planes(CUtensorMap* m, Planes p, int64_t rows, int cols, int box_rows) {
-  EncodeTiledFn enc = encode_fn();
-  if (!enc) return false;
-  cuuint64_t dims[3] = {cuuint64_t(cols), cuuint64_t(rows), 3};
-  cuuint64_t strides[2] = {cuuint64_t(cols) * 2, cuuint64_t(p.stride)};
-  cuuint32_t box[3] = {64, cuuint32_t(box_rows), 1};
-  cuuint32_t estr[3] = {1, 1, 1};
-  return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(p.ptr), dims, strides, box, estr,
-             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
 
 template <bool kSplit>
 cudaError_t gemm_launch(const CUtensorMap& ma0, const CUtensorMap& ma1, const CUtensorMap& mw, const CUtensorMap (&mo)[3],
@@ -681,15 +655,6 @@ cudaError_t encoder_layer(__nv_bfloat16* x, const __nv_bfloat16* src, int64_t n,
   P.mode[0] = EPI_LN_RES; P.gamma = ln + 2 * kC; P.beta = ln + 3 * kC;
   const Dst ox[3] = {{x, kC}, none, none};
   return gemm_run(Tx, w.hid, 2 * kC, nullptr, 0, wl + kOffMlp2, 256, ox, P, x, st);
-}
-
-// fp32 [elems] -> three bf16 planes `stride` bytes apart (split3_kernel; elems is a multiple of 256)
-cudaError_t split_planes(const float* src, __nv_bfloat16* dst, size_t stride, size_t elems, cudaStream_t st) {
-  char* d = reinterpret_cast<char*>(dst);
-  split3_kernel<<<148 * 8, 256, 0, st>>>(reinterpret_cast<const float4*>(src), reinterpret_cast<uint2*>(d),
-                                         reinterpret_cast<uint2*>(d + stride), reinterpret_cast<uint2*>(d + 2 * stride),
-                                         elems / 4);
-  return cudaGetLastError();
 }
 
 // the same layer on fp32 activations at fp32 accuracy: every GEMM operand is split into three bf16 planes first

@@ -14,9 +14,18 @@
 // between them, LayerNorm2 and the residual) is one launch of mlp_fused_kernel.  The attention itself (8 heads x 16 x 16
 // per window) is a warp-per-window kernel: mma.sync tensor cores for windows of at most 32 tokens, fp32 SIMT above.
 // Activations are bf16 in HBM, all arithmetic accumulates in fp32.
+//
+// The same level also runs at fp32 accuracy on the bf16 tensor cores (pope_fine_transformer_f32,
+// pope_fine_merge_coarse_f32): activations are fp32 in HBM, every GEMM operand is split into three bf16 planes (weights
+// once when packed, activations by split3_kernel ahead of each GEMM) and fine_gemm_split_kernel accumulates the six
+// significant products of every k-chunk in fp32 TMEM.  The MLP is two such launches (ReLU; LayerNorm2 + residual), the
+// attention is fine_attn_kernel<float> for every window size (DESIGN §4.6).
 #include <cuda.h>
 
+#include <type_traits>
+
 #include "common.cuh"
+#include "split3.cuh"
 #include "tc_ptx.cuh"
 
 namespace pope {
@@ -45,7 +54,9 @@ constexpr int kSmemW = 34 * 1024;                     // 1024-aligned, past the 
 static_assert(kSmemTmemPtr + 16 <= kSmemW, "barrier block overlaps the weights");
 constexpr int kSmemAlloc = kSmemBudget;               // > 113 KB -> one CTA per SM, so the CTA may take all 512 TMEM columns
 
-enum EpiMode : int { EPI_COPY = 0, EPI_ELU1 = 1, EPI_SCALE = 2, EPI_LN = 3, EPI_ADDVEC = 4 };
+// EPI_RELU and EPI_LN_RES (LayerNorm, then + the residual row) are modes of fine_gemm_split_kernel only: the bf16 level
+// runs the MLP as mlp_fused_kernel
+enum EpiMode : int { EPI_COPY = 0, EPI_ELU1 = 1, EPI_SCALE = 2, EPI_LN = 3, EPI_ADDVEC = 4, EPI_RELU = 5, EPI_LN_RES = 6 };
 
 struct LinParams {
   int T;                       // token rows
@@ -588,16 +599,290 @@ mlp_fused_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constant
   }
 }
 
+// ---- fp32-accuracy GEMM: every Linear of the fp32 fine level ------------------------------------------------------------
+// Y[T, N] = epilogue(cat(A0[T, K0], A1[T, K1]) . W[N, K0 + K1]^T) with A0, A1 and W as three bf16 planes each (split3):
+// each k-chunk accumulates a1w1 + a2w1 + a3w1 + a1w2 + a2w2 + a1w3 into one fp32 TMEM accumulator, the technique of
+// coarse_gemm_kernel<true> (coarse_tf.cu), except that a1w1 and the five small products go to two accumulators that the
+// epilogue adds: each tcgen05.mma rounds its fp32 accumulator, and with all six products in one accumulator that rounding
+// happened six times per k-step (measured: 8x the rms error of the stock fp32 Linear on FinePreprocess; the small-term
+// accumulator is 2^-8 of the main one, so its roundings are that much smaller).  An item is 128 token rows x one
+// 128-column output block (two slots x two accumulators of 128 TMEM columns), so the LayerNorm epilogues see whole rows
+// (d_model 128).  A stage holds the three A planes and the three W planes of one k-chunk, six
+// 16 KB boxes; two stages.  The weights stream through the ring with the activations: three planes of the q/k/v weight
+// are 288 KB, more than a CTA's shared memory (which is why linear_tc_kernel, weight-stationary, cannot take this mode).
+// Rows leave as fp32 through a 32-row x 32-column staging box and a TMA store; the residual of EPI_LN_RES comes in the
+// same way.  warp 0: TMA, warp 1: TMEM allocator + MMA, warps 2-9: epilogue (two sets of four alternate items).
+namespace sg {
+constexpr int kStageBytes = 6 * kBoxBytes;                    // A planes 1-3, W planes 1-3 of one k-chunk
+constexpr int kStages = 2;
+constexpr int kOut = 0;                                       // 8 x 4 KB staging boxes
+constexpr int kBar = kEpiWarps * kStageOutBytes;
+constexpr int kNumBars = 2 * kStages + 4 + kEpiWarps;
+constexpr int kTmemPtr = kBar + kNumBars * 8;
+constexpr int kRing = kBar + 1024;
+static_assert(kTmemPtr + 16 <= kRing, "barrier block overlaps the ring");
+constexpr int kAlloc = kRing + kStages * kStageBytes + 1024;
+static_assert(kAlloc <= 227 * 1024, "split fine GEMM shared memory");
+}  // namespace sg
+
+struct SplitParams {
+  int T;                       // token rows
+  int kchunks;                 // (K0 + K1) / 64
+  int ksplit;                  // k-chunks [0, ksplit) come from mapA0, the rest from mapA1 (torch.cat along the channels)
+  int nblk;                    // N / 128 (<= 3); output block j goes through mapO<j>
+  int mode[3];
+  float scale;                 // EPI_SCALE
+  const float* bias;           // [N] or nullptr, added before the mode is applied
+  const float* gamma;          // EPI_LN / EPI_LN_RES: [128]
+  const float* beta;
+  const float* rowvec;         // EPI_ADDVEC: row r gets rowvec[(row0 + r) / rows_per_vec]
+  int rows_per_vec;
+  int64_t row0;
+};
+
+__global__ void __launch_bounds__(kLinThreads, 1)
+fine_gemm_split_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant__ CUtensorMap mapA1,
+                       const __grid_constant__ CUtensorMap mapW, const __grid_constant__ CUtensorMap mapO0,
+                       const __grid_constant__ CUtensorMap mapO1, const __grid_constant__ CUtensorMap mapO2,
+                       const __grid_constant__ CUtensorMap mapR, const SplitParams P) {
+  using namespace sg;
+  extern __shared__ uint8_t smem_raw[];
+  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
+  const uint32_t sbase = smem_u32(smem);
+  const uint32_t bar_full = sbase + kBar, bar_empty = bar_full + 8 * kStages;
+  const uint32_t bar_acc_full = bar_empty + 8 * kStages, bar_acc_empty = bar_acc_full + 16;
+  const uint32_t bar_res = bar_acc_empty + 16;                 // one per epilogue warp
+  const uint32_t ring = sbase + kRing;
+  volatile uint32_t* tmem_ptr_smem = reinterpret_cast<volatile uint32_t*>(smem + kTmemPtr);
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int ntiles = (P.T + kTile - 1) / kTile, nitems = ntiles * P.nblk;
+
+  if (warp == 0 && lane == 0) {
+    prefetch_tmap(&mapA0); prefetch_tmap(&mapA1); prefetch_tmap(&mapW);
+    prefetch_tmap(&mapO0); prefetch_tmap(&mapO1); prefetch_tmap(&mapO2); prefetch_tmap(&mapR);
+    for (int s = 0; s < kStages; ++s) { mbar_init(bar_full + 8 * s, 1); mbar_init(bar_empty + 8 * s, 1); }
+    for (int s = 0; s < 2; ++s) { mbar_init(bar_acc_full + 8 * s, 1); mbar_init(bar_acc_empty + 8 * s, 4); }
+    for (int s = 0; s < kEpiWarps; ++s) mbar_init(bar_res + 8 * s, 1);
+    fence_barrier_init();
+  }
+  if (warp == 1) {
+    tmem_alloc(sbase + kTmemPtr, 512u);
+    tmem_relinquish();
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *tmem_ptr_smem;
+
+  if (warp == 0) {
+    // =============================== TMA producer ===============================
+    if (lane == 0) {
+      int stage = 0;
+      uint32_t phase = 0;
+      for (int it = blockIdx.x; it < nitems; it += gridDim.x) {
+        const int t = it / P.nblk, j = it - t * P.nblk;
+        for (int kc = 0; kc < P.kchunks; ++kc) {
+          const CUtensorMap* ma = kc < P.ksplit ? &mapA0 : &mapA1;
+          const int ka = (kc < P.ksplit ? kc : kc - P.ksplit) * kBoxK;
+          mbar_wait(bar_empty + 8 * stage, phase ^ 1);
+          const uint32_t dst = ring + stage * kStageBytes;
+          mbar_expect_tx(bar_full + 8 * stage, kStageBytes);
+          for (int p = 0; p < 3; ++p) tma_load_3d(dst + p * kBoxBytes, ma, bar_full + 8 * stage, ka, t * kTile, p);
+          for (int p = 0; p < 3; ++p) tma_load_3d(dst + (3 + p) * kBoxBytes, &mapW, bar_full + 8 * stage, kc * kBoxK, j * kD, p);
+          if (++stage == kStages) { stage = 0; phase ^= 1; }
+        }
+      }
+    }
+  } else if (warp == 1) {
+    // =============================== MMA issuer ===============================
+    if (lane == 0) {
+      constexpr uint32_t idesc = idesc_bf16(kTile, kD);
+      int stage = 0;
+      uint32_t phase = 0, li = 0;
+      for (int it = blockIdx.x; it < nitems; it += gridDim.x, ++li) {
+        const uint32_t slot = li & 1;
+        mbar_wait(bar_acc_empty + 8 * slot, ((li >> 1) & 1) ^ 1);      // the epilogue has drained this accumulator
+        tc_fence_after();
+        const uint32_t d = tmem_base + slot * 2 * kD;
+        for (int kc = 0; kc < P.kchunks; ++kc) {
+          mbar_wait(bar_full + 8 * stage, phase);
+          tc_fence_after();
+          const uint32_t a_addr = ring + stage * kStageBytes, b_addr = a_addr + 3 * kBoxBytes;
+          // a1w1 into the main accumulator, a2w1 + a3w1 + a1w2 + a2w2 + a1w3 into the small-term one (plane of A, of W)
+#pragma unroll
+          for (int q = 0; q < 6; ++q) {
+            const uint32_t pa = q == 1 || q == 4 ? 1u : (q == 2 ? 2u : 0u), pw = q < 3 ? 0u : (q < 5 ? 1u : 2u);
+#pragma unroll
+            for (int ks = 0; ks < kBoxK / 16; ++ks)
+              umma_bf16(q == 0 ? d : d + kD, umma_desc(a_addr + pa * kBoxBytes + ks * 32),
+                        umma_desc(b_addr + pw * kBoxBytes + ks * 32), idesc, (kc | (q > 1 ? 1 : 0) | ks) ? 1u : 0u);
+          }
+          umma_commit(bar_empty + 8 * stage);                           // ring slot free once these MMAs have read it
+          if (++stage == kStages) { stage = 0; phase ^= 1; }
+        }
+        umma_commit(bar_acc_full + 8 * slot);
+      }
+    }
+  } else {
+    // =============================== epilogue: thread = token row, 128 channels in two passes of 64 ==================
+    const int ew = warp - 2, set = ew >> 2, quad = warp & 3;
+    const uint32_t lane_addr = uint32_t(quad * 32) << 16;
+    const uint32_t stage_buf = sbase + kOut + ew * kStageOutBytes;
+    const uint32_t my_row = stage_buf + lane * 128;
+    const uint32_t sw = uint32_t(lane & 7);
+    const uint32_t bar_my_res = bar_res + 8 * ew;
+    uint32_t res_phase = 0, li = 0;
+    for (int it = blockIdx.x; it < nitems; it += gridDim.x, ++li) {
+      if ((li & 1u) != uint32_t(set)) continue;
+      const uint32_t slot = li & 1;
+      const int t = it / P.nblk, j = it - t * P.nblk;
+      const int mode = j == 0 ? P.mode[0] : (j == 1 ? P.mode[1] : P.mode[2]);   // (no dynamic index: P stays in param space)
+      const int row0 = t * kTile + quad * 32, row = row0 + lane;
+      const CUtensorMap* mo = j == 0 ? &mapO0 : (j == 1 ? &mapO1 : &mapO2);
+      const uint32_t taddr = tmem_base + lane_addr + slot * 2 * kD;
+      const float* bias = P.bias ? P.bias + j * kD : nullptr;
+      // 64 output columns from `col` on: main + small-term accumulator, plus the bias
+      auto load64 = [&](int col, float* v) {
+        tmem_ld32(taddr + col, v);
+        tmem_ld32(taddr + col + 32, v + 32);
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+          float s[32];
+          tmem_ld32(taddr + kD + col + 32 * h, s);
+#pragma unroll
+          for (int c = 0; c < 32; ++c) v[32 * h + c] += s[c];
+        }
+        if (bias) {
+          const float4* b4 = reinterpret_cast<const float4*>(bias + col);
+#pragma unroll
+          for (int c = 0; c < 64; c += 4) {
+            const float4 b = __ldg(b4 + (c >> 2));
+            v[c] += b.x; v[c + 1] += b.y; v[c + 2] += b.z; v[c + 3] += b.w;
+          }
+        }
+      };
+      mbar_wait(bar_acc_full + 8 * slot, (li >> 1) & 1);
+      tc_fence_after();
+      float mean = 0.f, rstd = 0.f;
+      if (mode == EPI_LN || mode == EPI_LN_RES) {   // nn.LayerNorm statistics: mean first, then the biased variance
+        float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
+#pragma unroll 1
+        for (int qc = 0; qc < 2; ++qc) {
+          float v[64];
+          load64(qc * 64, v);
+#pragma unroll
+          for (int c = 0; c < 64; c += 4) { s0 += v[c]; s1 += v[c + 1]; s2 += v[c + 2]; s3 += v[c + 3]; }
+        }
+        mean = ((s0 + s1) + (s2 + s3)) * (1.f / kD);
+        s0 = s1 = s2 = s3 = 0.f;
+#pragma unroll 1
+        for (int qc = 0; qc < 2; ++qc) {
+          float v[64];
+          load64(qc * 64, v);
+#pragma unroll
+          for (int c = 0; c < 64; c += 4) {
+            const float d0 = v[c] - mean, d1 = v[c + 1] - mean, d2 = v[c + 2] - mean, d3 = v[c + 3] - mean;
+            s0 = fmaf(d0, d0, s0); s1 = fmaf(d1, d1, s1); s2 = fmaf(d2, d2, s2); s3 = fmaf(d3, d3, s3);
+          }
+        }
+        rstd = rsqrtf(((s0 + s1) + (s2 + s3)) * (1.f / kD) + 1e-5f);
+      }
+#pragma unroll 1
+      for (int qc = 0; qc < 2; ++qc) {
+        const int col = qc * 64;
+        float v[64];
+        load64(col, v);
+        if (qc == 1) {                 // last read of this accumulator
+          tc_fence_before();
+          __syncwarp();
+          if (lane == 0) mbar_arrive(bar_acc_empty + 8 * slot);
+        }
+        if (mode == EPI_ELU1) {        // elu(x) + 1 as torch evaluates it (expm1, then + 1)
+#pragma unroll
+          for (int c = 0; c < 64; ++c) v[c] = v[c] > 0.f ? v[c] + 1.f : expm1f(v[c]) + 1.f;
+        } else if (mode == EPI_SCALE) {
+#pragma unroll
+          for (int c = 0; c < 64; ++c) v[c] *= P.scale;
+        } else if (mode == EPI_RELU) {
+#pragma unroll
+          for (int c = 0; c < 64; ++c) v[c] = fmaxf(v[c], 0.f);
+        } else if (mode == EPI_LN || mode == EPI_LN_RES) {
+          const float4* g4 = reinterpret_cast<const float4*>(P.gamma + col);
+          const float4* b4 = reinterpret_cast<const float4*>(P.beta + col);
+#pragma unroll
+          for (int c = 0; c < 64; c += 4) {
+            const float4 g = __ldg(g4 + (c >> 2)), b = __ldg(b4 + (c >> 2));
+            v[c] = fmaf((v[c] - mean) * rstd, g.x, b.x); v[c + 1] = fmaf((v[c + 1] - mean) * rstd, g.y, b.y);
+            v[c + 2] = fmaf((v[c + 2] - mean) * rstd, g.z, b.z); v[c + 3] = fmaf((v[c + 3] - mean) * rstd, g.w, b.w);
+          }
+        } else if (mode == EPI_ADDVEC && row < P.T) {
+          const float4* a4 = reinterpret_cast<const float4*>(P.rowvec + size_t((P.row0 + row) / P.rows_per_vec) * kD + col);
+#pragma unroll
+          for (int c = 0; c < 64; c += 4) {
+            const float4 a = __ldg(a4 + (c >> 2));
+            v[c] += a.x; v[c + 1] += a.y; v[c + 2] += a.z; v[c + 3] += a.w;
+          }
+        }
+#pragma unroll
+        for (int hh = 0; hh < 2; ++hh) {   // fp32 rows: two boxes of 32 columns through the 4 KB staging box
+          float* vh = v + hh * 32;
+          if (lane == 0) tma_store_wait_read();                 // the previous store out of this box has read it
+          __syncwarp();
+          if (mode == EPI_LN_RES) {                             // + x: the residual rows through the staging box
+            if (lane == 0) {
+              mbar_expect_tx(bar_my_res, kStageOutBytes);
+              tma_load_2d(stage_buf, &mapR, bar_my_res, col + hh * 32, row0);
+            }
+            __syncwarp();
+            mbar_wait(bar_my_res, res_phase);
+            res_phase ^= 1;
+#pragma unroll
+            for (int c8 = 0; c8 < 8; ++c8) {
+              float4 r;
+              asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w)
+                           : "r"(my_row + ((uint32_t(c8) ^ sw) << 4)));
+              vh[c8 * 4] += r.x; vh[c8 * 4 + 1] += r.y; vh[c8 * 4 + 2] += r.z; vh[c8 * 4 + 3] += r.w;
+            }
+            __syncwarp();
+          }
+#pragma unroll
+          for (int c8 = 0; c8 < 8; ++c8)
+            asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};"
+                         ::"r"(my_row + ((uint32_t(c8) ^ sw) << 4)), "f"(vh[c8 * 4]), "f"(vh[c8 * 4 + 1]),
+                           "f"(vh[c8 * 4 + 2]), "f"(vh[c8 * 4 + 3]) : "memory");
+          fence_proxy_async();
+          __syncwarp();
+          if (lane == 0) {
+            tma_store_2d(mo, stage_buf, col + hh * 32, row0);   // rows past T are clipped by the tensor map
+            tma_store_commit();
+          }
+        }
+      }
+    }
+    if (lane == 0) tma_store_wait_all();                        // global writes complete before the CTA exits
+  }
+
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 1) {
+    tc_fence_after();
+    tmem_dealloc(tmem_base, 512u);
+  }
+}
+
 // ---- linear attention, one warp per 25-token window ------------------------------------------------------------------
 // q, k already hold elu(.)+1 and v holds values / S (fused into the projection's epilogue).  Per head h (16 dims):
 //   KV[d][e] = sum_s k[s][d] v[s][e],  ksum[d] = sum_s k[s][d],  out[l][e] = S * (q[l] . KV[:, e]) / (q[l] . ksum + eps)
 // Phase 1: lane (h, r) accumulates KV rows d = 4r..4r+3 (64 values) over the window; the 256 values of a head go through
 // shared memory so that in phase 2 lane (h, r) owns output columns e = 4r..4r+3 for every token (no shuffles).
+// T: the activation type (__nv_bfloat16, or float for the fp32-accuracy layer, which runs this kernel for every window size)
 constexpr int kAttnWarps = 4;
 
+template <typename T>
 __global__ void __launch_bounds__(kAttnWarps * 32)
-fine_attn_kernel(const __nv_bfloat16* __restrict__ q, const __nv_bfloat16* __restrict__ k, const __nv_bfloat16* __restrict__ v,
-                 __nv_bfloat16* __restrict__ out, int64_t m, const int32_t* live, int S, float eps) {
+fine_attn_kernel(const T* __restrict__ q, const T* __restrict__ k, const T* __restrict__ v, T* __restrict__ out, int64_t m,
+                 const int32_t* live, int S, float eps) {
+  constexpr bool kF32 = std::is_same<T, float>::value;
   __shared__ float kv_s[kAttnWarps][kHeads][kHeadDim][kHeadDim + 1];
   __shared__ float ks_s[kAttnWarps][kHeads][kHeadDim];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -613,15 +898,26 @@ fine_attn_kernel(const __nv_bfloat16* __restrict__ q, const __nv_bfloat16* __res
     for (int e = 0; e < kHeadDim; ++e) kv[d][e] = 0.f;
   }
   for (int s = 0; s < S; ++s) {
+    float kd[4], ve[kHeadDim];
+    if constexpr (kF32) {
+      const float4 kk = *reinterpret_cast<const float4*>(k + base + size_t(s) * kD + h * kHeadDim + 4 * r);
+      const float4* vp = reinterpret_cast<const float4*>(v + base + size_t(s) * kD + h * kHeadDim);
+      kd[0] = kk.x; kd[1] = kk.y; kd[2] = kk.z; kd[3] = kk.w;
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        const float4 vv = vp[e];
+        ve[4 * e] = vv.x; ve[4 * e + 1] = vv.y; ve[4 * e + 2] = vv.z; ve[4 * e + 3] = vv.w;
+      }
+    } else {
     const uint2 kk = *reinterpret_cast<const uint2*>(k + base + size_t(s) * kD + h * kHeadDim + 4 * r);
     const uint4* vp = reinterpret_cast<const uint4*>(v + base + size_t(s) * kD + h * kHeadDim);
     const uint4 v0 = vp[0], v1 = vp[1];
-    const float kd[4] = {__uint_as_float(kk.x << 16), __uint_as_float(kk.x & 0xffff0000u), __uint_as_float(kk.y << 16),
-                         __uint_as_float(kk.y & 0xffff0000u)};
+    kd[0] = __uint_as_float(kk.x << 16); kd[1] = __uint_as_float(kk.x & 0xffff0000u); kd[2] = __uint_as_float(kk.y << 16);
+    kd[3] = __uint_as_float(kk.y & 0xffff0000u);
     const uint32_t vw[8] = {v0.x, v0.y, v0.z, v0.w, v1.x, v1.y, v1.z, v1.w};
-    float ve[kHeadDim];
 #pragma unroll
     for (int e = 0; e < 8; ++e) { ve[2 * e] = __uint_as_float(vw[e] << 16); ve[2 * e + 1] = __uint_as_float(vw[e] & 0xffff0000u); }
+    }
 #pragma unroll
     for (int d = 0; d < 4; ++d) {
       ks[d] += kd[d];
@@ -645,10 +941,27 @@ fine_attn_kernel(const __nv_bfloat16* __restrict__ q, const __nv_bfloat16* __res
   }
   const float fs = float(S);
   for (int l = 0; l < S; ++l) {
+    float z = 0.f, o[4] = {0.f, 0.f, 0.f, 0.f};
+    if constexpr (kF32) {
+      const float4* qp = reinterpret_cast<const float4*>(q + base + size_t(l) * kD + h * kHeadDim);
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        const float4 q4 = qp[e];
+        const float qe[4] = {q4.x, q4.y, q4.z, q4.w};
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+          z = fmaf(qe[i], ksum[4 * e + i], z);
+#pragma unroll
+          for (int c = 0; c < 4; ++c) o[c] = fmaf(qe[i], kvc[4 * e + i][c], o[c]);
+        }
+      }
+      const float zi = fs / (z + eps);
+      *reinterpret_cast<float4*>(out + base + size_t(l) * kD + h * kHeadDim + 4 * r) =
+          make_float4(o[0] * zi, o[1] * zi, o[2] * zi, o[3] * zi);
+    } else {
     const uint4* qp = reinterpret_cast<const uint4*>(q + base + size_t(l) * kD + h * kHeadDim);
     const uint4 q0 = qp[0], q1 = qp[1];
     const uint32_t qw[8] = {q0.x, q0.y, q0.z, q0.w, q1.x, q1.y, q1.z, q1.w};
-    float z = 0.f, o[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
     for (int e = 0; e < 8; ++e) {
       const float qa = __uint_as_float(qw[e] << 16), qb = __uint_as_float(qw[e] & 0xffff0000u);
@@ -660,6 +973,7 @@ fine_attn_kernel(const __nv_bfloat16* __restrict__ q, const __nv_bfloat16* __res
     const float zi = fs / (z + eps);
     *reinterpret_cast<uint2*>(out + base + size_t(l) * kD + h * kHeadDim + 4 * r) =
         make_uint2(pack_bf16(o[0] * zi, o[1] * zi), pack_bf16(o[2] * zi, o[3] * zi));
+    }
   }
 }
 
@@ -824,23 +1138,23 @@ fine_attn_mma_kernel(const __nv_bfloat16* __restrict__ q, const __nv_bfloat16* _
 }
 
 // rows [0, m): f0[b, i, :], rows [m, 2m): f1[b, j, :]   (fine_preprocess.py:50-51, the cat along dim 0); with a live count
-// only rows [0, live) and [m, m + live) (the ids past it are never read)
-__global__ void __launch_bounds__(256) gather_coarse_rows_kernel(const __nv_bfloat16* __restrict__ f0,
-                                                                const __nv_bfloat16* __restrict__ f1,
+// only rows [0, live) and [m, m + live) (the ids past it are never read).  T: __nv_bfloat16 or float (16 B per lane and step)
+template <typename T>
+__global__ void __launch_bounds__(256) gather_coarse_rows_kernel(const T* __restrict__ f0, const T* __restrict__ f1,
                                                                 const int64_t* __restrict__ b_ids,
                                                                 const int64_t* __restrict__ i_ids,
                                                                 const int64_t* __restrict__ j_ids, int64_t m,
                                                                 const int32_t* __restrict__ live, int L, int S, int C,
-                                                                __nv_bfloat16* __restrict__ out) {
+                                                                T* __restrict__ out) {
+  constexpr int kVec = 16 / int(sizeof(T));
   const int64_t row = int64_t(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (row >= 2 * m) return;
   const int lane = threadIdx.x & 31;
   const bool second = row >= m;
   const int64_t mm = second ? row - m : row;
   if (mm >= live_count(m, live, 1)) return;
-  const __nv_bfloat16* src = second ? f1 + (size_t(b_ids[mm]) * S + size_t(j_ids[mm])) * C
-                                    : f0 + (size_t(b_ids[mm]) * L + size_t(i_ids[mm])) * C;
-  for (int c = lane * 8; c < C; c += 256)
+  const T* src = second ? f1 + (size_t(b_ids[mm]) * S + size_t(j_ids[mm])) * C : f0 + (size_t(b_ids[mm]) * L + size_t(i_ids[mm])) * C;
+  for (int c = lane * kVec; c < C; c += 32 * kVec)
     *reinterpret_cast<uint4*>(out + size_t(row) * C + c) = *reinterpret_cast<const uint4*>(src + c);
 }
 
@@ -937,7 +1251,7 @@ TfScratch carve_tf(void* base, int64_t m, int S) {
 cudaError_t attention_run(const __nv_bfloat16* q, const __nv_bfloat16* k, const __nv_bfloat16* v, __nv_bfloat16* out, int64_t m,
                           const int32_t* live, int S, cudaStream_t st) {
   if (S > kTileRows) {
-    fine_attn_kernel<<<unsigned((m + kAttnWarps - 1) / kAttnWarps), kAttnWarps * 32, 0, st>>>(q, k, v, out, m, live, S, 1e-6f);
+    fine_attn_kernel<__nv_bfloat16><<<unsigned((m + kAttnWarps - 1) / kAttnWarps), kAttnWarps * 32, 0, st>>>(q, k, v, out, m, live, S, 1e-6f);
     return cudaGetLastError();
   }
   int dev = 0, sms = 0;
@@ -977,6 +1291,157 @@ cudaError_t encoder_layer(__nv_bfloat16* x, const __nv_bfloat16* src, int64_t m,
   const Dst om[3] = {{w.m1, kD}, {nullptr, 0}, {nullptr, 0}};
   if ((e = linear_run(T, live, S, w.msg, wl + kOffMerge, 128, kD, kD, om, P, st)) != cudaSuccess) return e;
   return mlp_fused_run(x, w.m1, T, live, S, wl + kOffMlp1, wl + kOffMlp2, ln + 256, ln + 384, st);
+}
+
+// ---- the fp32-accuracy level ---------------------------------------------------------------------------------------------
+// packed weights: the bf16 layouts with every matrix as three consecutive bf16 planes (w = w1 + w2 + w3), so a matrix
+// starts at 3x its bf16 offset and its planes lie one bf16 matrix apart; the fp32 LayerNorm / bias tail is unchanged
+constexpr size_t kF32LayerBytes = 3 * kOffLn + 4 * 128 * 4;
+static_assert(kF32LayerBytes == POPE_FINE_TF_F32_LAYER_BYTES, "include/pope_b200.h documents this layout");
+constexpr size_t kF32PreBytes = 3 * kOffPreBias + 2 * 128 * 4;
+static_assert(kF32PreBytes == POPE_FINE_PRE_F32_BYTES, "include/pope_b200.h documents this layout");
+
+struct DstF { float* ptr; int64_t pitch; };                  // one 128-column fp32 output block (row pitch in elements)
+
+// Y[T, N] = epilogue(cat(A0[T, K0], A1[T, K1]) . W[N, K0 + K1]^T) at fp32 accuracy: A0, A1 and W as three bf16 planes
+// each, W rows w_pitch elements apart; out[j] receives output columns [128 j, 128 j + 128) as fp32 rows.
+// resid (EPI_LN_RES): [T, 128] fp32 rows added after the LayerNorm.
+cudaError_t gemm_split_run(int64_t T, Planes A0, int K0, Planes A1, int K1, Planes W, int N, int64_t w_pitch,
+                           const DstF (&out)[3], SplitParams P, const float* resid, cudaStream_t st) {
+  if (T <= 0) return cudaSuccess;
+  if (T > 0x7fffffff - kTile || N % kD || N / kD > 3 || K0 % kBoxK || K1 % kBoxK || K0 + K1 > w_pitch)
+    return cudaErrorInvalidValue;
+  CUtensorMap ma0, ma1, mw, mo[3], mr;
+  if (!make_map_planes(&ma0, A0, T, K0, kTile)) return cudaErrorInvalidValue;
+  if (!make_map_planes(&ma1, K1 ? A1 : A0, T, K1 ? K1 : K0, kTile)) return cudaErrorInvalidValue;
+  if (!make_map_planes(&mw, W, N, K0 + K1, kD, w_pitch)) return cudaErrorInvalidValue;
+  for (int j = 0; j < 3; ++j) {
+    const DstF& o = out[j < N / kD ? j : 0];                  // unused maps still have to be valid descriptors
+    if (!o.ptr || !make_map2d_f32(&mo[j], o.ptr, T, kD, o.pitch)) return cudaErrorInvalidValue;
+  }
+  if (!make_map2d_f32(&mr, resid ? resid : out[0].ptr, T, kD, resid ? kD : out[0].pitch)) return cudaErrorInvalidValue;
+  P.T = int(T);
+  P.kchunks = (K0 + K1) / kBoxK;
+  P.ksplit = K0 / kBoxK;
+  P.nblk = N / kD;
+  int dev = 0, sms = 0;
+  cudaError_t e;
+  if ((e = cudaGetDevice(&dev)) != cudaSuccess) return e;
+  if ((e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
+  if ((e = cudaFuncSetAttribute(fine_gemm_split_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, sg::kAlloc)) != cudaSuccess)
+    return e;
+  const int64_t nitems = (T + kTile - 1) / kTile * P.nblk;
+  fine_gemm_split_kernel<<<unsigned(nitems < sms ? nitems : sms), kLinThreads, sg::kAlloc, st>>>(ma0, ma1, mw, mo[0], mo[1],
+                                                                                                   mo[2], mr, P);
+  return cudaGetLastError();
+}
+
+// Five fp32 planes of [m * S, 128] (q, k, v, msg, m1; the MLP's hidden [T, 256] spans the q and k planes, dead by then),
+// three bf16 planes of x (xs) and six bf16 [m * S, 128] units that hold, interleaved, the three planes of msg / LN1's
+// output (ms, even units) and of a 'cross' layer's source (ss, odd units), and later the three [T, 256] planes of the
+// hidden (two units each, from ms): the layout of the fp32 coarse scratch (coarse_tf.cu).  4 864 bytes per token.
+struct TfScratchF32 {
+  float *q, *k, *v, *msg, *m1, *hid;
+  __nv_bfloat16 *xs, *ms, *ss;
+  size_t unit2;                // bytes of one bf16 [m * S, 128] unit
+  size_t bytes;
+};
+TfScratchF32 carve_tf_f32(void* base, int64_t m, int S) {
+  TfScratchF32 w{};
+  char* p = static_cast<char*>(base);
+  const size_t unit = align_up(size_t(m) * S * kD * 4, 256);
+  w.unit2 = align_up(size_t(m) * S * kD * 2, 256);
+  size_t off = 0;
+  w.q = reinterpret_cast<float*>(p + off); off += unit;
+  w.k = reinterpret_cast<float*>(p + off); off += unit;
+  w.v = reinterpret_cast<float*>(p + off); off += unit;
+  w.msg = reinterpret_cast<float*>(p + off); off += unit;
+  w.m1 = reinterpret_cast<float*>(p + off); off += unit;
+  w.hid = w.q;
+  w.xs = reinterpret_cast<__nv_bfloat16*>(p + off); off += 3 * w.unit2;
+  w.ms = reinterpret_cast<__nv_bfloat16*>(p + off);
+  w.ss = reinterpret_cast<__nv_bfloat16*>(p + off + w.unit2); off += 6 * w.unit2;
+  w.bytes = off;
+  return w;
+}
+
+// the layer of encoder_layer above on fp32 windows at fp32 accuracy, in place on x: every GEMM operand is split first
+cudaError_t encoder_layer(float* x, const float* src, int64_t m, int S, const char* wl, const TfScratchF32& w, cudaStream_t st) {
+  const int64_t T = m * S;
+  const float* ln = reinterpret_cast<const float*>(wl + 3 * kOffLn);
+  const DstF none{nullptr, 0};
+  const Planes xs{w.xs, w.unit2}, ms{w.ms, 2 * w.unit2}, no{nullptr, 0};
+  auto weight = [wl](size_t off, size_t rows, size_t cols) { return Planes{wl + 3 * off, rows * cols * 2}; };
+  cudaError_t e;
+  if ((e = split_planes(x, w.xs, xs.stride, size_t(T) * kD, st)) != cudaSuccess) return e;
+  SplitParams P{};
+  if (x == src) {                       // self: one pass over x produces q, k, v
+    P.mode[0] = EPI_ELU1; P.mode[1] = EPI_ELU1; P.mode[2] = EPI_SCALE; P.scale = 1.f / float(S);
+    const DstF o[3] = {{w.q, kD}, {w.k, kD}, {w.v, kD}};
+    if ((e = gemm_split_run(T, xs, kD, no, 0, weight(kOffQkv, 384, 128), 384, kD, o, P, nullptr, st)) != cudaSuccess) return e;
+  } else {
+    const Planes ss{w.ss, 2 * w.unit2};
+    if ((e = split_planes(src, w.ss, ss.stride, size_t(T) * kD, st)) != cudaSuccess) return e;
+    P.mode[0] = EPI_ELU1;
+    const DstF oq[3] = {{w.q, kD}, none, none};
+    if ((e = gemm_split_run(T, xs, kD, no, 0, weight(kOffQkv, 384, 128), 128, kD, oq, P, nullptr, st)) != cudaSuccess) return e;
+    P.mode[0] = EPI_ELU1; P.mode[1] = EPI_SCALE; P.scale = 1.f / float(S);
+    const DstF okv[3] = {{w.k, kD}, {w.v, kD}, none};
+    Planes wkv = weight(kOffQkv, 384, 128);
+    wkv.ptr = static_cast<const char*>(wkv.ptr) + 128 * 128 * 2;    // k_proj and v_proj rows of every plane
+    if ((e = gemm_split_run(T, ss, kD, no, 0, wkv, 256, kD, okv, P, nullptr, st)) != cudaSuccess) return e;
+  }
+  fine_attn_kernel<float><<<unsigned((m + kAttnWarps - 1) / kAttnWarps), kAttnWarps * 32, 0, st>>>(w.q, w.k, w.v, w.msg, m,
+                                                                                                   nullptr, S, 1e-6f);
+  if ((e = cudaGetLastError()) != cudaSuccess) return e;
+  if ((e = split_planes(w.msg, w.ms, ms.stride, size_t(T) * kD, st)) != cudaSuccess) return e;
+  P = SplitParams{};
+  P.mode[0] = EPI_LN; P.gamma = ln; P.beta = ln + 128;
+  const DstF om[3] = {{w.m1, kD}, none, none};
+  if ((e = gemm_split_run(T, ms, kD, no, 0, weight(kOffMerge, 128, 128), 128, kD, om, P, nullptr, st)) != cudaSuccess) return e;
+  if ((e = split_planes(w.m1, w.ms, ms.stride, size_t(T) * kD, st)) != cudaSuccess) return e;
+  // MLP: relu(W1 . cat(x, m1)) -> hid [T, 256] fp32, then x <- x + LayerNorm2(W2 . hid)      (transformer.py:52-58)
+  P = SplitParams{};
+  P.mode[0] = EPI_RELU; P.mode[1] = EPI_RELU;
+  const DstF oh[3] = {{w.hid, 2 * kD}, {w.hid + kD, 2 * kD}, none};
+  if ((e = gemm_split_run(T, xs, kD, ms, kD, weight(kOffMlp1, 256, 256), 256, 256, oh, P, nullptr, st)) != cudaSuccess) return e;
+  if ((e = split_planes(w.hid, w.ms, ms.stride, size_t(T) * 2 * kD, st)) != cudaSuccess) return e;   // [T, 256] planes
+  P = SplitParams{};
+  P.mode[0] = EPI_LN_RES; P.gamma = ln + 256; P.beta = ln + 384;
+  const DstF ox[3] = {{x, kD}, none, none};
+  return gemm_split_run(T, ms, 2 * kD, no, 0, weight(kOffMlp2, 128, 256), 128, 256, ox, P, x, st);
+}
+
+// FinePreprocess at fp32 accuracy: gathered coarse rows cg [2m, 256] fp32 and their planes (a region of three
+// [2m, 256] bf16 planes that later holds the planes of window row chunks, 4m rows each), projected rows cd [2m, 128]
+// fp32 and their planes, per-window vectors [2m, 128] fp32.  8 704 bytes per window, whatever the window size.
+struct MergeScratchF32 {
+  float *cg, *cd, *cvec;
+  __nv_bfloat16 *cgs, *cds;
+  size_t cgs_stride, cds_stride;
+  int64_t chunk_rows;          // window rows split at a time (the cgs region: 4m rows of 128)
+  size_t bytes;
+};
+MergeScratchF32 carve_merge_f32(void* base, int64_t m) {
+  MergeScratchF32 w{};
+  char* p = static_cast<char*>(base);
+  size_t off = 0;
+  w.cg = reinterpret_cast<float*>(p + off); off += align_up(size_t(2 * m) * 256 * 4, 256);
+  w.cgs_stride = align_up(size_t(2 * m) * 256 * 2, 256);
+  w.cgs = reinterpret_cast<__nv_bfloat16*>(p + off); off += 3 * w.cgs_stride;
+  w.cd = reinterpret_cast<float*>(p + off); off += align_up(size_t(2 * m) * 128 * 4, 256);
+  w.cds_stride = align_up(size_t(2 * m) * 128 * 2, 256);
+  w.cds = reinterpret_cast<__nv_bfloat16*>(p + off); off += 3 * w.cds_stride;
+  w.cvec = reinterpret_cast<float*>(p + off); off += align_up(size_t(2 * m) * 128 * 4, 256);
+  w.chunk_rows = 4 * m;
+  w.bytes = off;
+  return w;
+}
+
+// rows the fp32 level indexes with int32 (T of a GEMM, 2m coarse rows)
+bool too_many_rows(int64_t m, int tokens) {
+  const int64_t lim = 0x7fffffff - kTile;
+  return m > lim / 2 || m > lim / tokens;
 }
 
 }  // namespace
@@ -1053,7 +1518,7 @@ extern "C" int pope_fine_merge_coarse_ex(void* win0, void* win1, int64_t m_windo
   float* cvec = reinterpret_cast<float*>(reinterpret_cast<char*>(cd) + align_up(size_t(2 * m) * 128 * 2, 256));
   const char* wp = static_cast<const char*>(weights);
   const float* bias = reinterpret_cast<const float*>(wp + kOffPreBias);
-  gather_coarse_rows_kernel<<<unsigned((2 * m + 7) / 8), 256, 0, st>>>(
+  gather_coarse_rows_kernel<__nv_bfloat16><<<unsigned((2 * m + 7) / 8), 256, 0, st>>>(
       static_cast<const __nv_bfloat16*>(feat_c0), static_cast<const __nv_bfloat16*>(feat_c1), b_ids, i_ids, j_ids, m, m_dev, L, S,
       C, cg);
   cudaError_t e = cudaGetLastError();
@@ -1093,4 +1558,104 @@ extern "C" int pope_fine_merge_coarse(void* win0, void* win1, int64_t m_windows,
                                       void* stream) {
   return pope_fine_merge_coarse_ex(win0, win1, m_windows, nullptr, window_tokens, feat_c0, feat_c1, L, S, C, b_ids, i_ids, j_ids,
                                    weights, workspace, workspace_bytes, stream);
+}
+
+extern "C" size_t pope_fine_tf_f32_workspace_bytes(int64_t m_windows, int window_tokens) {
+  if (m_windows <= 0 || window_tokens <= 0) return 0;
+  return carve_tf_f32(nullptr, m_windows, window_tokens).bytes;
+}
+
+extern "C" int pope_fine_transformer_f32(void* feat0, void* feat1, int64_t m_windows, int window_tokens, const void* weights,
+                                         int n_layers, const int* layer_kinds, void* workspace, size_t workspace_bytes,
+                                         void* stream) {
+  if (!feat0 || !feat1 || !weights || !layer_kinds || !workspace) return POPE_ERR_INVALID_ARG;
+  if (m_windows < 0 || window_tokens <= 0 || n_layers < 0) return POPE_ERR_INVALID_ARG;
+  for (int l = 0; l < n_layers; ++l)
+    if (layer_kinds[l] != 0 && layer_kinds[l] != 1) return POPE_ERR_INVALID_ARG;
+  if ((reinterpret_cast<uintptr_t>(feat0) | reinterpret_cast<uintptr_t>(feat1) | reinterpret_cast<uintptr_t>(weights) |
+       reinterpret_cast<uintptr_t>(workspace)) & 15u)
+    return POPE_ERR_ALIGNMENT;
+  if (m_windows == 0) return POPE_OK;
+  if (too_many_rows(m_windows, window_tokens)) return POPE_ERR_SHAPE;
+  const TfScratchF32 w = carve_tf_f32(workspace, m_windows, window_tokens);
+  if (workspace_bytes < w.bytes) return POPE_ERR_WORKSPACE;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  float* x0 = static_cast<float*>(feat0);
+  float* x1 = static_cast<float*>(feat1);
+  for (int l = 0; l < n_layers; ++l) {
+    const char* wl = static_cast<const char*>(weights) + size_t(l) * kF32LayerBytes;
+    cudaError_t e;
+    if (layer_kinds[l] == 0) {            // 'self'  (transformer.py:96-98)
+      if ((e = encoder_layer(x0, x0, m_windows, window_tokens, wl, w, st)) != cudaSuccess) return int(e);
+      if ((e = encoder_layer(x1, x1, m_windows, window_tokens, wl, w, st)) != cudaSuccess) return int(e);
+    } else {                              // 'cross' (:99-101): feat1 attends to the UPDATED feat0
+      if ((e = encoder_layer(x0, x1, m_windows, window_tokens, wl, w, st)) != cudaSuccess) return int(e);
+      if ((e = encoder_layer(x1, x0, m_windows, window_tokens, wl, w, st)) != cudaSuccess) return int(e);
+    }
+  }
+  return POPE_OK;
+}
+
+extern "C" size_t pope_fine_merge_f32_workspace_bytes(int64_t m_windows) {
+  return m_windows > 0 ? carve_merge_f32(nullptr, m_windows).bytes : 0;
+}
+
+extern "C" int pope_fine_merge_coarse_f32(void* win0, void* win1, int64_t m_windows, int window_tokens, const void* feat_c0,
+                                          const void* feat_c1, int L, int S, int C, const int64_t* b_ids, const int64_t* i_ids,
+                                          const int64_t* j_ids, const void* weights, void* workspace, size_t workspace_bytes,
+                                          void* stream) {
+  if (!win0 || !win1 || !feat_c0 || !feat_c1 || !b_ids || !i_ids || !j_ids || !weights || !workspace)
+    return POPE_ERR_INVALID_ARG;
+  if (m_windows < 0 || window_tokens <= 0 || L <= 0 || S <= 0) return POPE_ERR_INVALID_ARG;
+  if (C != 256) return POPE_ERR_SHAPE;
+  if ((reinterpret_cast<uintptr_t>(win0) | reinterpret_cast<uintptr_t>(win1) | reinterpret_cast<uintptr_t>(feat_c0) |
+       reinterpret_cast<uintptr_t>(feat_c1) | reinterpret_cast<uintptr_t>(weights) | reinterpret_cast<uintptr_t>(workspace)) & 15u)
+    return POPE_ERR_ALIGNMENT;
+  if (m_windows == 0) return POPE_OK;
+  if (too_many_rows(m_windows, window_tokens)) return POPE_ERR_SHAPE;
+  const MergeScratchF32 w = carve_merge_f32(workspace, m_windows);
+  if (workspace_bytes < w.bytes) return POPE_ERR_WORKSPACE;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int64_t m = m_windows;
+  const char* wp = static_cast<const char*>(weights);
+  const float* bias = reinterpret_cast<const float*>(wp + 3 * kOffPreBias);
+  auto weight = [wp](size_t off, int64_t col) { return Planes{wp + 3 * off + col * 2, 128 * 256 * 2}; };  // [128, 256] planes
+  const DstF none{nullptr, 0};
+  const Planes no{nullptr, 0};
+  gather_coarse_rows_kernel<float><<<unsigned((2 * m + 7) / 8), 256, 0, st>>>(
+      static_cast<const float*>(feat_c0), static_cast<const float*>(feat_c1), b_ids, i_ids, j_ids, m, nullptr, L, S, C, w.cg);
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return int(e);
+  // feat_c_win = down_proj(cat(c0, c1))                                                    (fine_preprocess.py:50-51)
+  if ((e = split_planes(w.cg, w.cgs, w.cgs_stride, size_t(2 * m) * 256, st)) != cudaSuccess) return int(e);
+  SplitParams P{};
+  P.mode[0] = EPI_COPY; P.bias = bias;
+  const DstF od[3] = {{w.cd, kD}, none, none};
+  if ((e = gemm_split_run(2 * m, Planes{w.cgs, w.cgs_stride}, 256, no, 0, weight(kOffDown, 0), 128, 256, od, P, nullptr, st)) !=
+      cudaSuccess)
+    return int(e);
+  // merge_feat(cat(win, repeat(c))) = win . Wa^T + (c . Wb^T + bias): the second term once per window         (:52-55)
+  if ((e = split_planes(w.cd, w.cds, w.cds_stride, size_t(2 * m) * kD, st)) != cudaSuccess) return int(e);
+  P = SplitParams{};
+  P.mode[0] = EPI_COPY; P.bias = bias + 128;
+  const DstF ov[3] = {{w.cvec, kD}, none, none};
+  if ((e = gemm_split_run(2 * m, Planes{w.cds, w.cds_stride}, 128, no, 0, weight(kOffMergeFeat, 128), 128, 256, ov, P, nullptr,
+                          st)) != cudaSuccess)
+    return int(e);
+  // the window part in place, in chunks of rows whose planes fit the (now dead) planes of the gathered rows
+  const int64_t T = m * window_tokens;
+  for (int side = 0; side < 2; ++side) {
+    float* win = static_cast<float*>(side ? win1 : win0);
+    for (int64_t r0 = 0; r0 < T; r0 += w.chunk_rows) {
+      const int64_t rows = T - r0 < w.chunk_rows ? T - r0 : w.chunk_rows;
+      if ((e = split_planes(win + r0 * kD, w.cgs, w.cgs_stride, size_t(rows) * kD, st)) != cudaSuccess) return int(e);
+      P = SplitParams{};
+      P.mode[0] = EPI_ADDVEC; P.rowvec = w.cvec + size_t(side) * m * kD; P.rows_per_vec = window_tokens; P.row0 = r0;
+      const DstF ow[3] = {{win + r0 * kD, kD}, none, none};
+      if ((e = gemm_split_run(rows, Planes{w.cgs, w.cgs_stride}, 128, no, 0, weight(kOffMergeFeat, 0), 128, 256, ow, P, nullptr,
+                              st)) != cudaSuccess)
+        return int(e);
+    }
+  }
+  return POPE_OK;
 }

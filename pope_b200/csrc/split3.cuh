@@ -31,5 +31,14 @@ __global__ void __launch_bounds__(256) split3_kernel(const float4* __restrict__ 
   }
 }
 
+// fp32 [elems] -> three bf16 planes `stride` bytes apart (elems a multiple of 4, src 16-byte aligned)
+inline cudaError_t split_planes(const float* src, __nv_bfloat16* dst, size_t stride, size_t elems, cudaStream_t st) {
+  char* d = reinterpret_cast<char*>(dst);
+  split3_kernel<<<148 * 8, 256, 0, st>>>(reinterpret_cast<const float4*>(src), reinterpret_cast<uint2*>(d),
+                                         reinterpret_cast<uint2*>(d + stride), reinterpret_cast<uint2*>(d + 2 * stride),
+                                         elems / 4);
+  return cudaGetLastError();
+}
+
 }  // namespace
 }  // namespace pope

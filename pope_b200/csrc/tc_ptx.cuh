@@ -248,4 +248,31 @@ inline bool make_map2d(CUtensorMap* m, const void* base, int64_t rows, int cols,
              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
+// [rows, cols] fp32 with a row pitch of `pitch` elements, box = 32 columns (128 bytes) x 32 rows, 128-byte swizzle
+inline bool make_map2d_f32(CUtensorMap* m, const void* base, int64_t rows, int cols, int64_t pitch) {
+  EncodeTiledFn enc = encode_fn();
+  if (!enc) return false;
+  cuuint64_t dims[2] = {cuuint64_t(cols), cuuint64_t(rows)};
+  cuuint64_t strides[1] = {cuuint64_t(pitch) * 4};
+  cuuint32_t box[2] = {32, 32};
+  cuuint32_t estr[2] = {1, 1};
+  return enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(base), dims, strides, box, estr,
+             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
+// three bf16 planes of an fp32 operand split by split3 (csrc/split3.cuh): plane 0 and the byte distance between planes
+struct Planes { const void* ptr; size_t stride; };
+// three [rows, cols] bf16 planes (row pitch `pitch` elements, 0 = cols), box = 64 columns x box_rows rows x one plane,
+// 128-byte swizzle
+inline bool make_map_planes(CUtensorMap* m, Planes p, int64_t rows, int cols, int box_rows, int64_t pitch = 0) {
+  EncodeTiledFn enc = encode_fn();
+  if (!enc) return false;
+  cuuint64_t dims[3] = {cuuint64_t(cols), cuuint64_t(rows), 3};
+  cuuint64_t strides[2] = {cuuint64_t(pitch ? pitch : cols) * 2, cuuint64_t(p.stride)};
+  cuuint32_t box[3] = {64, cuuint32_t(box_rows), 1};
+  cuuint32_t estr[3] = {1, 1, 1};
+  return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(p.ptr), dims, strides, box, estr,
+             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
 }  // namespace pope

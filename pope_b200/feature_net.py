@@ -220,30 +220,35 @@ class FineTransformerB200(LocalFeatureTransformer):
     """`loftr_fine` with the encoder layers running in libpope_b200.so (csrc/fine_tf.cu: tcgen05 Linears with fused
     epilogues + tensor-core linear attention) when it is handed CUDA bfloat16 windows; same parameters, same state-dict
     keys as LocalFeatureTransformer (transformer.py:61-106).  fp32 windows keep the stock PyTorch layers (the
-    reference's precision); masks are not supported by the CUDA path (no inference caller passes them to the fine level).
+    reference's precision) unless `cuda_fp32` is set: then CUDA fp32 windows run the fp32-accuracy fine transformer (every
+    GEMM operand split into three bf16 terms, fp32 activations) and come back fp32.  Masks are not supported by the CUDA
+    paths (no inference caller passes them to the fine level).
 
     `inplace`: update the given window tensors (the Matcher owns them) instead of working on copies."""
 
     def __init__(self, config: dict, d_model: Optional[int] = None, LAYER_NAMES: Optional[List[str]] = None):
         super().__init__(config, d_model, LAYER_NAMES)
         self.inplace = False
-        self._packed = None
-        self._packed_key = None
+        self.cuda_fp32 = False
+        self._packed = {}
+        self._packed_key = {}
         self._workspace = None
 
     def cuda_supported(self) -> bool:
         return self.d_model == 128 and self.nhead == 8 and self.config["attention"] == "linear"
 
-    def _packed_weights(self, dev):
+    def _packed_weights(self, dev, dtype: torch.dtype = torch.bfloat16):
         from . import ops
         key = (str(dev),) + tuple((p.data_ptr(), p._version) for p in self.parameters())
-        if self._packed is None or self._packed_key != key:
-            self._packed = torch.cat([ops.pack_fine_layer(layer.state_dict(), dev) for layer in self.layers])
-            self._packed_key = key
-        return self._packed
+        if dtype not in self._packed or self._packed_key[dtype] != key:
+            self._packed[dtype] = torch.cat([ops.pack_fine_layer(layer.state_dict(), dev, dtype) for layer in self.layers])
+            self._packed_key[dtype] = key
+        return self._packed[dtype]
 
     def forward(self, feat0, feat1, mask0=None, mask1=None):
-        if not (feat0.is_cuda and feat0.dtype == torch.bfloat16 and feat1.dtype == torch.bfloat16):
+        bf16 = feat0.dtype == torch.bfloat16 and feat1.dtype == torch.bfloat16
+        fp32 = self.cuda_fp32 and feat0.dtype == torch.float32 and feat1.dtype == torch.float32
+        if not (feat0.is_cuda and (bf16 or fp32)):
             return super().forward(feat0, feat1, mask0, mask1)
         if mask0 is not None or mask1 is not None or not self.cuda_supported():
             raise NotImplementedError("the CUDA fine transformer covers d_model 128 / 8 heads / linear attention without masks")
@@ -253,8 +258,9 @@ class FineTransformerB200(LocalFeatureTransformer):
             feat0, feat1 = feat0.clone(), feat1.clone()
         feat0, feat1 = feat0.contiguous(), feat1.contiguous()
         self._workspace = ops.fine_level_workspace(feat0.shape[0], feat0.shape[1], feat0.device, self._workspace,
-                                                   merge=False)
-        return ops.fine_transformer(feat0, feat1, self._packed_weights(feat0.device), self.layer_names, self._workspace)
+                                                   merge=False, dtype=feat0.dtype)
+        return ops.fine_transformer(feat0, feat1, self._packed_weights(feat0.device, feat0.dtype), self.layer_names,
+                                    self._workspace)
 
 
 class CoarseTransformerB200(LocalFeatureTransformer):

@@ -3,7 +3,9 @@
 The window extraction (F.unfold of both fine maps + gather of the matched cells, :40-47) runs in
 libpope_b200.so (`pope_fine_gather`): only the M matched 5x5 windows are read.  The two small Linears that mix
 in the coarse feature (:50-57) stay torch/cuBLAS in the reference's fp32 precision; with `cuda_bf16 = True` the windows
-are gathered in bfloat16 and the Linears run in libpope_b200.so too (`pope_fine_merge_coarse`, csrc/fine_tf.cu).
+are gathered in bfloat16 and the Linears run in libpope_b200.so too (`pope_fine_merge_coarse`, csrc/fine_tf.cu); with
+`cuda_fp32 = True` the fp32 windows go through the Linears in libpope_b200.so at fp32 accuracy
+(`pope_fine_merge_coarse_f32`).
 Parameter names (`down_proj`, `merge_feat`) are the reference's.
 """
 from __future__ import annotations
@@ -29,15 +31,16 @@ class FinePreprocess(nn.Module):
             if p.dim() > 1:
                 nn.init.kaiming_normal_(p, mode="fan_out", nonlinearity="relu")
         self.cuda_bf16 = False          # bf16 windows + CUDA Linears (set by Matcher(config, fine_cuda_bf16=True))
-        self._packed = None
-        self._packed_key = None
+        self.cuda_fp32 = False          # fp32 windows + CUDA Linears at fp32 accuracy (Matcher(config, fine_cuda_fp32=True))
+        self._packed = {}
+        self._packed_key = {}
 
-    def _packed_weights(self, dev):
+    def _packed_weights(self, dev, dtype: torch.dtype = torch.bfloat16):
         key = (str(dev),) + tuple((p.data_ptr(), p._version) for p in self.parameters())
-        if self._packed is None or self._packed_key != key:
-            self._packed = ops.pack_fine_pre(self.state_dict(), dev)
-            self._packed_key = key
-        return self._packed
+        if dtype not in self._packed or self._packed_key[dtype] != key:
+            self._packed[dtype] = ops.pack_fine_pre(self.state_dict(), dev, dtype)
+            self._packed_key[dtype] = key
+        return self._packed[dtype]
 
     def forward(self, feat_f0, feat_f1, feat_c0, feat_c1, data):
         W = self.W
@@ -60,6 +63,10 @@ class FinePreprocess(nn.Module):
             win0, win1 = ops.fine_merge_coarse(win0, win1, feat_c0.to(torch.bfloat16).contiguous(),
                                                feat_c1.to(torch.bfloat16).contiguous(), b_ids, i_ids, j_ids,
                                                self._packed_weights(win0.device))
+        elif self.cat_c_feat and self.cuda_fp32 and win0.is_cuda and win0.dtype == torch.float32 \
+                and self.d_model_f == 128 and feat_c0.shape[2] == 256:
+            win0, win1 = ops.fine_merge_coarse(win0, win1, feat_c0.float().contiguous(), feat_c1.float().contiguous(), b_ids,
+                                               i_ids, j_ids, self._packed_weights(win0.device, torch.float32))
         elif self.cat_c_feat:
             m = b_ids.shape[0]
             c_win = self.down_proj(torch.cat([feat_c0[b_ids, i_ids], feat_c1[b_ids, j_ids]], 0))      # [2M, Cf]

@@ -7,8 +7,8 @@ state-dict keys, and the same `load_state_dict` that strips a leading 'matcher.'
 
 Steps 3-5 of the forward (coarse match, fine-window gather, fine match; matcher.py:71-79) run in
 libpope_b200.so; the backbone and the two transformers are stock PyTorch modules (feature_net.py) unless the bf16
-CUDA paths are switched on (`fine_cuda_bf16`, `coarse_cuda_bf16`) or the fp32-accuracy CUDA coarse transformer is
-(`coarse_cuda_fp32`).
+CUDA paths are switched on (`fine_cuda_bf16`, `coarse_cuda_bf16`) or the fp32-accuracy CUDA paths are
+(`coarse_cuda_fp32`, `fine_cuda_fp32`).
 """
 from __future__ import annotations
 
@@ -23,7 +23,7 @@ from .fine_preprocess import FinePreprocess
 
 class Matcher(nn.Module):
     def __init__(self, config: dict, fine_cuda_bf16: bool = False, coarse_cuda_bf16: bool = False,
-                 coarse_cuda_fp32: bool = False):
+                 coarse_cuda_fp32: bool = False, fine_cuda_fp32: bool = False):
         """`fine_cuda_bf16` (not in the reference): run the fine level -- window gather, FinePreprocess Linears, fine
         transformer, fine matching -- in bfloat16 inside libpope_b200.so instead of fp32 torch modules between the CUDA
         stages.  `coarse_cuda_bf16` (not in the reference): add the position encoding, lay the coarse maps out token-major
@@ -31,8 +31,11 @@ class Matcher(nn.Module):
         features, and `forward(data, only_att_fea=True)` returns them as bfloat16.  `coarse_cuda_fp32` (not in the
         reference): run the coarse transformer at fp32 accuracy inside libpope_b200.so (bf16 tensor cores on operands
         split into three bf16 terms); everything else, the position encoding included, stays as in the stock flow, and
-        the features keep their dtype (fp32), shape and values up to rounding.  The two coarse flags exclude each other
-        (ValueError).  Parameters and state-dict keys are unchanged either way."""
+        the features keep their dtype (fp32), shape and values up to rounding.  `fine_cuda_fp32` (not in the reference):
+        run FinePreprocess' Linears and the fine transformer at fp32 accuracy inside libpope_b200.so on the fp32 windows;
+        the windows keep their dtype (fp32), so the outputs keep theirs.  The two coarse flags exclude each other, and so
+        do the two fine flags (ValueError); a coarse flag combines with either fine flag.  Parameters and state-dict keys
+        are unchanged either way."""
         super().__init__()
         self.config = config
         self.backbone = build_backbone(config)
@@ -45,17 +48,33 @@ class Matcher(nn.Module):
         self.fine_matching = FineMatching()
         if coarse_cuda_bf16 and coarse_cuda_fp32:
             raise ValueError("coarse_cuda_bf16 and coarse_cuda_fp32 exclude each other")
+        if fine_cuda_bf16 and fine_cuda_fp32:
+            raise ValueError("fine_cuda_bf16 and fine_cuda_fp32 exclude each other")
         self.coarse_cuda_fp32 = False
+        self.fine_cuda_fp32 = False
         self.set_fine_cuda_bf16(fine_cuda_bf16)
+        self.set_fine_cuda_fp32(fine_cuda_fp32)
         self.set_coarse_cuda_bf16(coarse_cuda_bf16)
         self.set_coarse_cuda_fp32(coarse_cuda_fp32)
 
     def set_fine_cuda_bf16(self, on: bool) -> None:
         if on and not self.loftr_fine.cuda_supported():
             raise NotImplementedError("the CUDA fine transformer covers d_model 128 / 8 heads / linear attention")
+        if on and self.fine_cuda_fp32:
+            raise ValueError("fine_cuda_bf16 and fine_cuda_fp32 exclude each other")
         self.fine_cuda_bf16 = bool(on)
         self.fine_preprocess.cuda_bf16 = bool(on)
-        self.loftr_fine.inplace = bool(on)
+        self.loftr_fine.inplace = self.fine_cuda_bf16 or self.fine_cuda_fp32
+
+    def set_fine_cuda_fp32(self, on: bool) -> None:
+        if on and not self.loftr_fine.cuda_supported():
+            raise NotImplementedError("the CUDA fine transformer covers d_model 128 / 8 heads / linear attention")
+        if on and self.fine_cuda_bf16:
+            raise ValueError("fine_cuda_bf16 and fine_cuda_fp32 exclude each other")
+        self.fine_cuda_fp32 = bool(on)
+        self.fine_preprocess.cuda_fp32 = self.fine_cuda_fp32
+        self.loftr_fine.cuda_fp32 = self.fine_cuda_fp32
+        self.loftr_fine.inplace = self.fine_cuda_bf16 or self.fine_cuda_fp32
 
     def set_coarse_cuda_bf16(self, on: bool) -> None:
         if on and not self.loftr_coarse.cuda_supported():

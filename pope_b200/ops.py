@@ -126,30 +126,58 @@ def fine_match(win0: torch.Tensor, win1: torch.Tensor, mkpts1_c: torch.Tensor, c
     return expec, mk1f
 
 
-def pack_fine_layer(sd: Dict[str, torch.Tensor], device) -> torch.Tensor:
-    """One LoFTREncoderLayer state dict (d_model 128) -> the packed byte layout of include/pope_b200.h."""
+def _split_packed(mats, device) -> torch.Tensor:
+    """Matrices -> their three bf16 planes each (split3_bf16), consecutive: the fp32-accuracy packed layouts."""
+    return torch.cat([p.reshape(-1) for t in mats for p in split3_bf16(t.detach().to(device=device, dtype=torch.float32))
+                      ]).view(torch.uint8)
+
+
+def _check_pack_dtype(dtype, what) -> None:
+    if dtype not in (torch.bfloat16, torch.float32):
+        raise _lib.PopeError(f"the {what} packs for torch.bfloat16 or torch.float32, not {dtype}")
+
+
+def pack_fine_layer(sd: Dict[str, torch.Tensor], device, dtype: torch.dtype = torch.bfloat16) -> torch.Tensor:
+    """One LoFTREncoderLayer state dict (d_model 128) -> the packed byte layout of include/pope_b200.h:
+    POPE_FINE_TF_LAYER_BYTES for dtype=torch.bfloat16 (the bf16 fine transformer), POPE_FINE_TF_F32_LAYER_BYTES for
+    dtype=torch.float32 (the fp32-accuracy one: every matrix as its three bf16 planes, split3_bf16, q | k | v split as one
+    stacked [384, 128] matrix)."""
+    _check_pack_dtype(dtype, "fine transformer")
     mats = [sd["q_proj.weight"], sd["k_proj.weight"], sd["v_proj.weight"], sd["merge.weight"], sd["mlp.0.weight"],
             sd["mlp.2.weight"]]
     shapes = [(128, 128)] * 4 + [(256, 256), (128, 256)]
     for t, shp in zip(mats, shapes):
         if tuple(t.shape) != shp:
             raise _lib.PopeError(f"fine transformer weight of shape {tuple(t.shape)}, expected {shp} (d_model 128, 8 heads)")
-    w = torch.cat([t.detach().to(device=device, dtype=torch.bfloat16).reshape(-1) for t in mats]).view(torch.uint8)
+    if dtype == torch.bfloat16:
+        w = torch.cat([t.detach().to(device=device, dtype=torch.bfloat16).reshape(-1) for t in mats]).view(torch.uint8)
+        size = _lib.FINE_TF_LAYER_BYTES
+    else:
+        w = _split_packed([torch.cat(mats[:3])] + mats[3:], device)
+        size = _lib.FINE_TF_F32_LAYER_BYTES
     ln = torch.cat([sd[k].detach().to(device=device, dtype=torch.float32).reshape(-1)
                     for k in ("norm1.weight", "norm1.bias", "norm2.weight", "norm2.bias")]).view(torch.uint8)
     out = torch.cat([w, ln])
-    assert out.numel() == _lib.FINE_TF_LAYER_BYTES
+    assert out.numel() == size
     return out
 
 
-def pack_fine_pre(sd: Dict[str, torch.Tensor], device) -> torch.Tensor:
-    """FinePreprocess state dict (down_proj, merge_feat) -> the packed byte layout of include/pope_b200.h."""
-    w = torch.cat([sd[k].detach().to(device=device, dtype=torch.bfloat16).reshape(-1)
-                   for k in ("down_proj.weight", "merge_feat.weight")]).view(torch.uint8)
+def pack_fine_pre(sd: Dict[str, torch.Tensor], device, dtype: torch.dtype = torch.bfloat16) -> torch.Tensor:
+    """FinePreprocess state dict (down_proj, merge_feat) -> the packed byte layout of include/pope_b200.h:
+    POPE_FINE_PRE_BYTES for dtype=torch.bfloat16, POPE_FINE_PRE_F32_BYTES for dtype=torch.float32 (each matrix as its
+    three bf16 planes)."""
+    _check_pack_dtype(dtype, "FinePreprocess")
+    mats = [sd["down_proj.weight"], sd["merge_feat.weight"]]
+    if dtype == torch.bfloat16:
+        w = torch.cat([t.detach().to(device=device, dtype=torch.bfloat16).reshape(-1) for t in mats]).view(torch.uint8)
+        size = _lib.FINE_PRE_BYTES
+    else:
+        w = _split_packed(mats, device)
+        size = _lib.FINE_PRE_F32_BYTES
     b = torch.cat([sd[k].detach().to(device=device, dtype=torch.float32).reshape(-1)
                    for k in ("down_proj.bias", "merge_feat.bias")]).view(torch.uint8)
     out = torch.cat([w, b])
-    assert out.numel() == _lib.FINE_PRE_BYTES
+    assert out.numel() == size
     return out
 
 
@@ -158,16 +186,35 @@ def _check_m_dev(m_dev: Optional[torch.Tensor], dev) -> None:
         raise _lib.PopeError("m_dev must be a device int32 tensor (the live count) on the device of the windows")
 
 
+def _fine_dtype(what: str, *tensors: torch.Tensor) -> bool:
+    """True for fp32 tensors, False for bf16 ones; anything else (or a mix) raises."""
+    dt = tensors[0].dtype
+    if dt not in (torch.bfloat16, torch.float32) or any(t.dtype != dt for t in tensors):
+        raise _lib.PopeError(f"{what} takes bfloat16 or float32 tensors (all alike)")
+    return dt == torch.float32
+
+
+def _check_packing(packed: torch.Tensor, count: int, f32: bool, bf16_bytes: int, f32_bytes: int, what: str, packer: str):
+    per, other = (f32_bytes, bf16_bytes) if f32 else (bf16_bytes, f32_bytes)
+    if packed.numel() != count * per:
+        if packed.numel() == count * other:
+            dt = torch.float32 if f32 else torch.bfloat16
+            raise _lib.PopeError(f"{dt} tensors need {what} packed with {packer}(..., dtype={dt})")
+        raise _lib.PopeError(f"{what} does not hold the packed bytes of {packer}")
+
+
 def fine_transformer(feat0: torch.Tensor, feat1: torch.Tensor, packed_layers: torch.Tensor, layer_names,
                      workspace: Optional[torch.Tensor] = None, m_dev: Optional[torch.Tensor] = None
                      ) -> Tuple[torch.Tensor, torch.Tensor]:
-    """LocalFeatureTransformer.forward on bf16 windows [M, WW, 128], IN PLACE (returns the same tensors).
-    `packed_layers`: concatenation of pack_fine_layer() of every layer, `layer_names`: 'self' / 'cross'.
-    `m_dev` (device int32): live window count; M is then the capacity and windows >= *m_dev are left untouched."""
+    """LocalFeatureTransformer.forward on windows [M, WW, 128], IN PLACE (returns the same tensors).  bfloat16 windows run
+    the bf16 fine transformer, float32 windows the fp32-accuracy one; `packed_layers`: concatenation of
+    pack_fine_layer(..., dtype=<the windows' dtype>) of every layer, `layer_names`: 'self' / 'cross'.
+    `m_dev` (device int32, bf16 only): live window count; M is then the capacity and windows >= *m_dev are left untouched."""
     dev = require_cuda(feat0, feat1, packed_layers)
     _check_m_dev(m_dev, dev)
-    if feat0.dtype != torch.bfloat16 or feat1.dtype != torch.bfloat16:
-        raise _lib.PopeError("the CUDA fine transformer takes bfloat16 windows")
+    f32 = _fine_dtype("the CUDA fine transformer", feat0, feat1)
+    if f32 and m_dev is not None:
+        raise _lib.PopeError("the fp32 fine transformer has no device-count bound (m_dev): it runs on all M windows")
     if feat0.shape != feat1.shape or feat0.dim() != 3 or feat0.shape[2] != 128:
         raise _lib.PopeError("feat0 / feat1 must both be [M, WW, 128]")
     if not (feat0.is_contiguous() and feat1.is_contiguous()):
@@ -177,17 +224,21 @@ def fine_transformer(feat0: torch.Tensor, feat1: torch.Tensor, packed_layers: to
         if name not in ("self", "cross"):
             raise KeyError(name)
         kinds.append(0 if name == "self" else 1)
-    if packed_layers.numel() != len(kinds) * _lib.FINE_TF_LAYER_BYTES:
-        raise _lib.PopeError("packed_layers does not hold one packed layer per layer name")
+    _check_packing(packed_layers, len(kinds), f32, _lib.FINE_TF_LAYER_BYTES, _lib.FINE_TF_F32_LAYER_BYTES,
+                   "packed_layers", "pack_fine_layer")
     M, WW, _ = feat0.shape
     if M == 0:
         return feat0, feat1
-    workspace = fine_level_workspace(M, WW, dev, workspace, merge=False)
+    workspace = fine_level_workspace(M, WW, dev, workspace, merge=False, dtype=feat0.dtype)
     arr = (_lib.C.c_int * max(len(kinds), 1))(*kinds)
     with torch.cuda.device(dev):
-        st = lib().pope_fine_transformer_ex(ptr(feat0), ptr(feat1), M, ptr(m_dev), WW, ptr(packed_layers), len(kinds), arr,
-                                            ptr(workspace), workspace.numel(), stream_ptr(dev))
-    check(st, "pope_fine_transformer")
+        if f32:
+            st = lib().pope_fine_transformer_f32(ptr(feat0), ptr(feat1), M, WW, ptr(packed_layers), len(kinds), arr,
+                                                 ptr(workspace), workspace.numel(), stream_ptr(dev))
+        else:
+            st = lib().pope_fine_transformer_ex(ptr(feat0), ptr(feat1), M, ptr(m_dev), WW, ptr(packed_layers), len(kinds),
+                                                arr, ptr(workspace), workspace.numel(), stream_ptr(dev))
+    check(st, "pope_fine_transformer_f32" if f32 else "pope_fine_transformer")
     return feat0, feat1
 
 
@@ -311,24 +362,34 @@ def coarse_pos_encode(feat: torch.Tensor, pe: torch.Tensor) -> torch.Tensor:
 def fine_merge_coarse(win0: torch.Tensor, win1: torch.Tensor, feat_c0: torch.Tensor, feat_c1: torch.Tensor, b_ids, i_ids,
                       j_ids, packed_pre: torch.Tensor, workspace: Optional[torch.Tensor] = None,
                       m_dev: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
-    """FinePreprocess' down_proj / merge_feat on bf16 windows [M, WW, 128], IN PLACE (returns the same tensors).
-    `m_dev` (device int32): live window count; M is then the capacity and windows / ids >= *m_dev are never touched."""
+    """FinePreprocess' down_proj / merge_feat on windows [M, WW, 128], IN PLACE (returns the same tensors): bfloat16
+    tensors in bf16, float32 tensors at fp32 accuracy (`packed_pre` from pack_fine_pre(..., dtype=<their dtype>)).
+    `m_dev` (device int32, bf16 only): live window count; M is then the capacity and windows / ids >= *m_dev are never
+    touched."""
     dev = require_cuda(win0, win1, feat_c0, feat_c1, b_ids, i_ids, j_ids, packed_pre)
     _check_m_dev(m_dev, dev)
-    for t in (win0, win1, feat_c0, feat_c1):
-        if t.dtype != torch.bfloat16 or not t.is_contiguous():
-            raise _lib.PopeError("fine_merge_coarse takes contiguous bfloat16 tensors")
+    f32 = _fine_dtype("fine_merge_coarse", win0, win1, feat_c0, feat_c1)
+    if not all(t.is_contiguous() for t in (win0, win1, feat_c0, feat_c1)):
+        raise _lib.PopeError("fine_merge_coarse takes contiguous tensors")
+    if f32 and m_dev is not None:
+        raise _lib.PopeError("the fp32 fine_merge_coarse has no device-count bound (m_dev): it runs on all M windows")
+    _check_packing(packed_pre, 1, f32, _lib.FINE_PRE_BYTES, _lib.FINE_PRE_F32_BYTES, "packed_pre", "pack_fine_pre")
     M, WW, _ = win0.shape
     if M == 0:
         return win0, win1
     n, L, C_ = feat_c0.shape
     S = feat_c1.shape[1]
-    workspace = fine_level_workspace(M, WW, dev, workspace, transformer=False)
+    workspace = fine_level_workspace(M, WW, dev, workspace, transformer=False, dtype=win0.dtype)
+    ids = (ptr(b_ids.contiguous()), ptr(i_ids.contiguous()), ptr(j_ids.contiguous()))
     with torch.cuda.device(dev):
-        st = lib().pope_fine_merge_coarse_ex(ptr(win0), ptr(win1), M, ptr(m_dev), WW, ptr(feat_c0), ptr(feat_c1), L, S, C_,
-                                             ptr(b_ids.contiguous()), ptr(i_ids.contiguous()), ptr(j_ids.contiguous()),
-                                             ptr(packed_pre), ptr(workspace), workspace.numel(), stream_ptr(dev))
-    check(st, "pope_fine_merge_coarse")
+        if f32:
+            st = lib().pope_fine_merge_coarse_f32(ptr(win0), ptr(win1), M, WW, ptr(feat_c0), ptr(feat_c1), L, S, C_, *ids,
+                                                  ptr(packed_pre), ptr(workspace), workspace.numel(), stream_ptr(dev))
+        else:
+            st = lib().pope_fine_merge_coarse_ex(ptr(win0), ptr(win1), M, ptr(m_dev), WW, ptr(feat_c0), ptr(feat_c1), L, S,
+                                                 C_, *ids, ptr(packed_pre), ptr(workspace), workspace.numel(),
+                                                 stream_ptr(dev))
+    check(st, "pope_fine_merge_coarse_f32" if f32 else "pope_fine_merge_coarse")
     return win0, win1
 
 
@@ -411,13 +472,18 @@ def running_topk(scores: torch.Tensor, k: int = 3):
 
 
 def fine_level_workspace(m: int, ww: int, dev, workspace: Optional[torch.Tensor] = None, merge: bool = True,
-                         transformer: bool = True) -> torch.Tensor:
-    """Scratch of the bf16 fine level for m windows of ww tokens, sized for the stages that will use it: the FinePreprocess
-    Linears (`merge`) and the fine transformer (`transformer`, 5 planes of [m * ww, 128] bf16).  They run one after the
-    other on one stream, so with both the scratch is shared (at 25 tokens its size is the transformer's).  A stage that
-    is handed no scratch gets one of its own size only, so a caller that does not share pays for no more than it uses."""
-    need = max(lib().pope_fine_tf_workspace_bytes(int(m), int(ww)) if transformer else 0,
-               lib().pope_fine_merge_workspace_bytes(int(m)) if merge else 0, 16)
+                         transformer: bool = True, dtype: torch.dtype = torch.bfloat16) -> torch.Tensor:
+    """Scratch of the fine level for m windows of ww tokens (bf16, or fp32 accuracy for dtype=torch.float32), sized for
+    the stages that will use it: the FinePreprocess Linears (`merge`) and the fine transformer (`transformer`, 5 planes of
+    [m * ww, 128] bf16; in fp32, 5 fp32 planes and 9 bf16 split planes).  They run one after the other on one stream, so
+    with both the scratch is shared (at 25 tokens its size is the transformer's).  A stage that is handed no scratch gets
+    one of its own size only, so a caller that does not share pays for no more than it uses."""
+    if dtype not in (torch.bfloat16, torch.float32):
+        raise _lib.PopeError(f"the CUDA fine level runs in torch.bfloat16 or torch.float32, not {dtype}")
+    h = lib()
+    tf, mg = ((h.pope_fine_tf_f32_workspace_bytes, h.pope_fine_merge_f32_workspace_bytes) if dtype == torch.float32 else
+              (h.pope_fine_tf_workspace_bytes, h.pope_fine_merge_workspace_bytes))
+    need = max(tf(int(m), int(ww)) if transformer else 0, mg(int(m)) if merge else 0, 16)
     if workspace is None or workspace.numel() < need or workspace.device != dev:
         workspace = torch.empty(need, dtype=torch.uint8, device=dev)
     return workspace
