@@ -214,9 +214,20 @@ int pope_pipeline_last_f1_mode(const pope_pipeline_t* pl);
  * pope_pipeline_destroy frees them.  At 16 pairs x 480x640 per chunk (76 800 windows) that is 0.98 GB of windows plus
  * 2.5 GB of scratch (computed from the sizes).
  * Returns POPE_ERR_INVALID_ARG (null handle; layers without layer_kinds or with n_layers < 1; a kind other than 0 / 1),
- * POPE_ERR_DTYPE (fp32 pipeline), POPE_ERR_SHAPE (C != 256), POPE_ERR_ALIGNMENT, or a cudaError_t from an allocation. */
+ * POPE_ERR_DTYPE (fp32 pipeline), POPE_ERR_SHAPE (C != 256), POPE_ERR_ALIGNMENT, or a cudaError_t from an allocation.
+ * pope_pipeline_set_fine_level(...) is pope_pipeline_set_fine_level_ex(pl, POPE_BF16, ...). */
 int pope_pipeline_set_fine_level(pope_pipeline_t* pl, const void* pre, const void* layers, int n_layers,
                                  const int* layer_kinds);
+/* pope_pipeline_set_fine_level for either packing: dtype (POPE_BF16 or POPE_F32) names the layouts pre and layers are packed
+ * in and must be the pipeline's dtype, otherwise POPE_ERR_DTYPE.  On a POPE_F32 pipeline every chunk runs the
+ * fp32-accuracy level (pope_fine_merge_coarse_f32_ex / pope_fine_transformer_f32_ex, packed layouts of
+ * pope_fine_merge_coarse_f32 / pope_fine_transformer_f32), which is what Matcher(config, fine_cuda_fp32=True) computes; the
+ * first attach then allocates fp32 windows win0 / win1 [chunk * min(L,S), 25, 128] and one fine scratch of
+ * max(pope_fine_tf_f32_workspace_bytes(chunk * min(L,S), 25), pope_fine_merge_f32_workspace_bytes(chunk * min(L,S)))
+ * bytes.  At 16 pairs x 480x640 per chunk (76 800 windows) that is 1.97 GB of windows plus 9.3 GB of scratch (computed
+ * from the sizes).  Every form of the fine maps (union, windows, bulk) works with either level. */
+int pope_pipeline_set_fine_level_ex(pope_pipeline_t* pl, int dtype, const void* pre, const void* layers, int n_layers,
+                                    const int* layer_kinds);
 
 /* One-shot convenience: create + run + destroy. */
 int pope_match_pairs_host(const void* feat_c0, const void* feat_c1, const void* feat_f0, const void* feat_f1,
@@ -395,6 +406,17 @@ size_t pope_fine_tf_f32_workspace_bytes(int64_t m_windows, int window_tokens);
 int pope_fine_transformer_f32(void* feat0, void* feat1, int64_t m_windows, int window_tokens, const void* weights,
                               int n_layers, const int* layer_kinds, void* workspace, size_t workspace_bytes, void* stream);
 
+/* pope_fine_transformer_f32 bounded by a live count kept on the device (the convention of pope_fine_transformer_ex), so
+ * that the fp32-accuracy level can follow pope_coarse_match / pope_fine_gather without a host sync (and be captured in a
+ * CUDA graph).  m_windows is the launch capacity: tensor maps, grids and the workspace are sized by it.  m_dev (may be
+ * NULL = all m_windows windows): device int32 live window count; windows, ids and scratch rows at or past
+ * min(*m_dev, m_windows) are never read or written, and their contents never reach a live window.  A live count of 0
+ * is a no-op.  Same results as pope_fine_transformer_f32 on the live windows, bit for bit, and the same error codes.
+ * pope_fine_transformer_f32(...) is pope_fine_transformer_f32_ex(..., m_dev = NULL, ...). */
+int pope_fine_transformer_f32_ex(void* feat0, void* feat1, int64_t m_windows, const int32_t* m_dev, int window_tokens,
+                                 const void* weights, int n_layers, const int* layer_kinds,
+                                 void* workspace, size_t workspace_bytes, void* stream);
+
 /* Bytes of device scratch of pope_fine_merge_coarse_f32 (gathered and projected coarse rows with their split planes,
  * per-window vectors; 8 704 bytes per window, for any window size). */
 size_t pope_fine_merge_f32_workspace_bytes(int64_t m_windows);
@@ -406,6 +428,16 @@ int pope_fine_merge_coarse_f32(void* win0, void* win1, int64_t m_windows, int wi
                                const void* feat_c1, int L, int S, int C, const int64_t* b_ids, const int64_t* i_ids,
                                const int64_t* j_ids, const void* weights, void* workspace, size_t workspace_bytes,
                                void* stream);
+
+/* pope_fine_merge_coarse_f32 bounded by a live count kept on the device (the convention of pope_fine_transformer_ex):
+ * m_windows is the capacity (length of the id arrays and of the windows, workspace sized by it), m_dev (may be NULL)
+ * the device int32 live count; ids, windows and scratch rows at or past min(*m_dev, m_windows) are never read or written
+ * (scratch: rows of either side).  Same results as pope_fine_merge_coarse_f32 on the live windows, bit for bit, and the
+ * same error codes.  pope_fine_merge_coarse_f32(...) is pope_fine_merge_coarse_f32_ex(..., m_dev = NULL, ...). */
+int pope_fine_merge_coarse_f32_ex(void* win0, void* win1, int64_t m_windows, const int32_t* m_dev, int window_tokens,
+                                  const void* feat_c0, const void* feat_c1, int L, int S, int C,
+                                  const int64_t* b_ids, const int64_t* i_ids, const int64_t* j_ids, const void* weights,
+                                  void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- coarse-level transformer (bf16) ----------------------------------------------------------------------------------
  * Replace src/matcher/matcher.py:57-58 (pos_encoding + rearrange to token-major) and transformer.py:34-58,95-104 +

@@ -55,6 +55,8 @@ SIGNATURES = {
     "pope_fine_transformer_f32": (_i, [_p, _p, _i64, _i, _p, _i, C.POINTER(_i), _p, _sz, _p]),
     "pope_fine_merge_f32_workspace_bytes": (_sz, [_i64]),
     "pope_fine_merge_coarse_f32": (_i, [_p, _p, _i64, _i, _p, _p, _i, _i, _i, _p, _p, _p, _p, _p, _sz, _p]),
+    "pope_fine_transformer_f32_ex": (_i, [_p, _p, _i64, _p, _i, _p, _i, C.POINTER(_i), _p, _sz, _p]),
+    "pope_fine_merge_coarse_f32_ex": (_i, [_p, _p, _i64, _p, _i, _p, _p, _i, _i, _i, _p, _p, _p, _p, _p, _sz, _p]),
     "pope_match_order_by_ref": (_i, [_p, _i, _i, _p, _p, _p]),
     "pope_savetxt_f32": (_i, [C.c_char_p, _p, _i64, _i]),
     "pope_savetxt_f64": (_i, [C.c_char_p, _p, _i64, _i]),
@@ -77,6 +79,7 @@ SIGNATURES = {
     "pope_pipeline_last_h2d_bytes": (_i64, [_p]),
     "pope_pipeline_last_f1_mode": (_i, [_p]),
     "pope_pipeline_set_fine_level": (_i, [_p, _p, _p, _i, C.POINTER(_i)]),
+    "pope_pipeline_set_fine_level_ex": (_i, [_p, _i, _p, _p, _i, C.POINTER(_i)]),
     "pope_match_pairs_host": (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _f, _f, _f, _f, _i, _i,
                                    _i, _i, _p, _p, _p, _p, _p, _p, _p]),
 }

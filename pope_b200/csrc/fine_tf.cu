@@ -20,6 +20,8 @@
 // once when packed, activations by split3_kernel ahead of each GEMM) and fine_gemm_split_kernel accumulates the six
 // significant products of every k-chunk in fp32 TMEM.  The MLP is two such launches (ReLU; LayerNorm2 + residual), the
 // attention is fine_attn_kernel<float> for every window size (DESIGN §4.6).
+// Both levels have forms bounded by a live window count kept on the device (the _ex entry points: capacity-sized launches
+// whose kernels read the count), so that they can follow pope_coarse_match without a host sync.
 #include <cuda.h>
 
 #include <type_traits>
@@ -85,8 +87,9 @@ __device__ __forceinline__ int64_t live_count(int64_t cap, const int32_t* live, 
 }
 
 // A 32-row output box that straddles the live bound is not TMA-stored (the store would write the rows past the bound):
-// each lane below the bound copies its own 64-column half row out of the 128B-swizzled staging box instead.
-__device__ __forceinline__ void store_staged_half_row(uint32_t my_row, uint32_t sw, __nv_bfloat16* dst) {
+// each lane below the bound copies its own 128-byte row (64 bf16 or 32 fp32 columns) out of the 128B-swizzled staging box
+// instead.
+__device__ __forceinline__ void store_staged_half_row(uint32_t my_row, uint32_t sw, void* dst) {
 #pragma unroll
   for (int c8 = 0; c8 < 8; ++c8) {
     uint4 r;
@@ -94,6 +97,12 @@ __device__ __forceinline__ void store_staged_half_row(uint32_t my_row, uint32_t 
                  : "r"(my_row + ((uint32_t(c8) ^ sw) << 4)));
     reinterpret_cast<uint4*>(dst)[c8] = r;
   }
+}
+
+__device__ __forceinline__ int grid_ctas() {
+  int n;
+  asm volatile("mov.u32 %0, %%nctaid.x;" : "=r"(n));
+  return n;
 }
 
 // mapX: activations [T, K]; mapO[j]: output block j as a [T, 128] bf16 tensor (box 64 x 32 rows).
@@ -637,14 +646,27 @@ struct SplitParams {
   const float* beta;
   const float* rowvec;         // EPI_ADDVEC: row r gets rowvec[(row0 + r) / rows_per_vec]
   int rows_per_vec;
-  int64_t row0;
+  int64_t row0;                // also the launch's first row in an array of live items (SplitBound)
 };
 
+// the parameters of a launch bounded by a device count (its own type, so that the unbounded launches keep their
+// parameter layout, code and registers)
+struct SplitBound : SplitParams {
+  const int32_t* live;         // device count of live items; rows >= *live * rows_per_item - row0 are not written and
+  int rows_per_item;           // tiles past them not run (T is the capacity the tensor maps and the grid are sized for)
+  int out_pitch;               // output block j as a plain pointer, out + j * out_block with rows out_pitch elements
+  float* out;                  // apart, for the one 32-row box that straddles the live bound (a TMA store of it would
+  int64_t out_block;           // write rows past the bound); 32 bytes, as a larger struct made ptxas spill
+};
+
+// kBounded: P is a SplitBound (a separate instantiation, so that the unbounded launches keep their code and registers)
+template <bool kBounded>
 __global__ void __launch_bounds__(kLinThreads, 1)
 fine_gemm_split_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant__ CUtensorMap mapA1,
                        const __grid_constant__ CUtensorMap mapW, const __grid_constant__ CUtensorMap mapO0,
                        const __grid_constant__ CUtensorMap mapO1, const __grid_constant__ CUtensorMap mapO2,
-                       const __grid_constant__ CUtensorMap mapR, const SplitParams P) {
+                       const __grid_constant__ CUtensorMap mapR,
+                       const std::conditional_t<kBounded, SplitBound, SplitParams> P) {
   using namespace sg;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -654,8 +676,16 @@ fine_gemm_split_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_c
   const uint32_t bar_res = bar_acc_empty + 16;                 // one per epilogue warp
   const uint32_t ring = sbase + kRing;
   volatile uint32_t* tmem_ptr_smem = reinterpret_cast<volatile uint32_t*>(smem + kTmemPtr);
+  volatile int* live_rows_smem = reinterpret_cast<volatile int*>(smem + kTmemPtr + 8);   // as in linear_tc_kernel
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int ntiles = (P.T + kTile - 1) / kTile, nitems = ntiles * P.nblk;
+  int T_run = P.T;
+  if constexpr (kBounded)              // live rows of this launch: [row0, row0 + T) of the item array, clamped to the live items
+    T_run = int(max(live_count(P.row0 + P.T, P.live, P.rows_per_item) - P.row0, int64_t(0)));
+  const int ntiles = (T_run + kTile - 1) / kTile, nitems = ntiles * P.nblk;
+  if (kBounded) {
+    if (int(blockIdx.x) >= nitems) return;           // capacity-sized grid, fewer live items: no load issued, no TMEM held
+    if (threadIdx.x == 0) *live_rows_smem = T_run;   // (every thread read the same count; published by the sync below)
+  }
 
   if (warp == 0 && lane == 0) {
     prefetch_tmap(&mapA0); prefetch_tmap(&mapA1); prefetch_tmap(&mapW);
@@ -732,7 +762,8 @@ fine_gemm_split_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_c
     const uint32_t sw = uint32_t(lane & 7);
     const uint32_t bar_my_res = bar_res + 8 * ew;
     uint32_t res_phase = 0, li = 0;
-    for (int it = blockIdx.x; it < nitems; it += gridDim.x, ++li) {
+    // (kBounded: %nctaid.x re-read per item, which ptxas otherwise keeps in a register and spills at the 168-register cap)
+    for (int it = blockIdx.x; it < nitems; it += kBounded ? grid_ctas() : int(gridDim.x), ++li) {
       if ((li & 1u) != uint32_t(set)) continue;
       const uint32_t slot = li & 1;
       const int t = it / P.nblk, j = it - t * P.nblk;
@@ -815,7 +846,7 @@ fine_gemm_split_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_c
             v[c] = fmaf((v[c] - mean) * rstd, g.x, b.x); v[c + 1] = fmaf((v[c + 1] - mean) * rstd, g.y, b.y);
             v[c + 2] = fmaf((v[c + 2] - mean) * rstd, g.z, b.z); v[c + 3] = fmaf((v[c + 3] - mean) * rstd, g.w, b.w);
           }
-        } else if (mode == EPI_ADDVEC && row < P.T) {
+        } else if (mode == EPI_ADDVEC && row < (kBounded ? *live_rows_smem : P.T)) {
           const float4* a4 = reinterpret_cast<const float4*>(P.rowvec + size_t((P.row0 + row) / P.rows_per_vec) * kD + col);
 #pragma unroll
           for (int c = 0; c < 64; c += 4) {
@@ -852,9 +883,20 @@ fine_gemm_split_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_c
                            "f"(vh[c8 * 4 + 2]), "f"(vh[c8 * 4 + 3]) : "memory");
           fence_proxy_async();
           __syncwarp();
-          if (lane == 0) {
-            tma_store_2d(mo, stage_buf, col + hh * 32, row0);   // rows past T are clipped by the tensor map
-            tma_store_commit();
+          if constexpr (!kBounded) {
+            if (lane == 0) {
+              tma_store_2d(mo, stage_buf, col + hh * 32, row0);   // rows past T are clipped by the tensor map
+              tma_store_commit();
+            }
+          } else if (const int T = *live_rows_smem; row0 + 32 <= T || T == P.T) {
+            if (lane == 0) {
+              tma_store_2d(mo, stage_buf, col + hh * 32, row0);
+              tma_store_commit();
+            }
+          } else {                                                 // the box straddles the live bound (32 fp32 per lane)
+            if (row < T)
+              store_staged_half_row(my_row, sw, P.out + j * P.out_block + int64_t(row) * P.out_pitch + col + hh * 32);
+            __syncwarp();                                          // every lane has read its row before the box is refilled
           }
         }
       }
@@ -1301,13 +1343,38 @@ static_assert(kF32LayerBytes == POPE_FINE_TF_F32_LAYER_BYTES, "include/pope_b200
 constexpr size_t kF32PreBytes = 3 * kOffPreBias + 2 * 128 * 4;
 static_assert(kF32PreBytes == POPE_FINE_PRE_F32_BYTES, "include/pope_b200.h documents this layout");
 
+// split3_kernel on the live part of a capacity-sized array: element e of `in` is element elem0 + e of an array of items of
+// per_item elements, *live of them live; elements at or past the live ones are neither read nor written
+__global__ void __launch_bounds__(256) split3_live_kernel(const float4* __restrict__ in, uint2* __restrict__ p1,
+                                                         uint2* __restrict__ p2, uint2* __restrict__ p3, size_t n4,
+                                                         const int32_t* __restrict__ live, size_t per_item, size_t elem0) {
+  const size_t end = size_t(max(*live, 0)) * per_item;
+  const size_t n = end > elem0 ? (end - elem0) / 4 : 0;
+  split3_range(in, p1, p2, p3, n < n4 ? n : n4);
+}
+
+// split_planes bounded by a device count: `live` (may be null = all elems) items of per_item elements, src starting at
+// element elem0 of the item array (per_item and elem0 multiples of 4)
+inline cudaError_t split_planes(const float* src, __nv_bfloat16* dst, size_t stride, size_t elems, const int32_t* live,
+                                size_t per_item, size_t elem0, cudaStream_t st) {
+  if (!live) return split_planes(src, dst, stride, elems, st);
+  char* d = reinterpret_cast<char*>(dst);
+  split3_live_kernel<<<148 * 8, 256, 0, st>>>(reinterpret_cast<const float4*>(src), reinterpret_cast<uint2*>(d),
+                                              reinterpret_cast<uint2*>(d + stride), reinterpret_cast<uint2*>(d + 2 * stride),
+                                              elems / 4, live, per_item, elem0);
+  return cudaGetLastError();
+}
+
 struct DstF { float* ptr; int64_t pitch; };                  // one 128-column fp32 output block (row pitch in elements)
 
 // Y[T, N] = epilogue(cat(A0[T, K0], A1[T, K1]) . W[N, K0 + K1]^T) at fp32 accuracy: A0, A1 and W as three bf16 planes
 // each, W rows w_pitch elements apart; out[j] receives output columns [128 j, 128 j + 128) as fp32 rows.
 // resid (EPI_LN_RES): [T, 128] fp32 rows added after the LayerNorm.
+// live (may be null): device count of live items of rows_per_item rows each, the launch covering rows [P.row0, P.row0 + T)
+// of them; T is then the capacity.
 cudaError_t gemm_split_run(int64_t T, Planes A0, int K0, Planes A1, int K1, Planes W, int N, int64_t w_pitch,
-                           const DstF (&out)[3], SplitParams P, const float* resid, cudaStream_t st) {
+                           const DstF (&out)[3], SplitParams P, const float* resid, cudaStream_t st,
+                           const int32_t* live = nullptr, int rows_per_item = 1) {
   if (T <= 0) return cudaSuccess;
   if (T > 0x7fffffff - kTile || N % kD || N / kD > 3 || K0 % kBoxK || K1 % kBoxK || K0 + K1 > w_pitch)
     return cudaErrorInvalidValue;
@@ -1328,11 +1395,28 @@ cudaError_t gemm_split_run(int64_t T, Planes A0, int K0, Planes A1, int K1, Plan
   cudaError_t e;
   if ((e = cudaGetDevice(&dev)) != cudaSuccess) return e;
   if ((e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
-  if ((e = cudaFuncSetAttribute(fine_gemm_split_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, sg::kAlloc)) != cudaSuccess)
-    return e;
   const int64_t nitems = (T + kTile - 1) / kTile * P.nblk;
-  fine_gemm_split_kernel<<<unsigned(nitems < sms ? nitems : sms), kLinThreads, sg::kAlloc, st>>>(ma0, ma1, mw, mo[0], mo[1],
-                                                                                                   mo[2], mr, P);
+  const unsigned grid = unsigned(nitems < sms ? nitems : sms);
+  if (live) {
+    SplitBound B{};
+    static_cast<SplitParams&>(B) = P;
+    B.live = live;
+    B.rows_per_item = rows_per_item;
+    B.out = out[0].ptr;
+    B.out_pitch = int(out[0].pitch);
+    B.out_block = P.nblk > 1 ? out[1].ptr - out[0].ptr : 0;
+    for (int j = 1; j < P.nblk; ++j)                          // the bounded launches' output blocks are evenly spaced
+      if (out[j].ptr != out[0].ptr + j * B.out_block || out[j].pitch != out[0].pitch) return cudaErrorInvalidValue;
+    if ((e = cudaFuncSetAttribute(fine_gemm_split_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, sg::kAlloc)) !=
+        cudaSuccess)
+      return e;
+    fine_gemm_split_kernel<true><<<grid, kLinThreads, sg::kAlloc, st>>>(ma0, ma1, mw, mo[0], mo[1], mo[2], mr, B);
+  } else {
+    if ((e = cudaFuncSetAttribute(fine_gemm_split_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, sg::kAlloc)) !=
+        cudaSuccess)
+      return e;
+    fine_gemm_split_kernel<false><<<grid, kLinThreads, sg::kAlloc, st>>>(ma0, ma1, mw, mo[0], mo[1], mo[2], mr, P);
+  }
   return cudaGetLastError();
 }
 
@@ -1365,51 +1449,59 @@ TfScratchF32 carve_tf_f32(void* base, int64_t m, int S) {
   return w;
 }
 
-// the layer of encoder_layer above on fp32 windows at fp32 accuracy, in place on x: every GEMM operand is split first
-cudaError_t encoder_layer(float* x, const float* src, int64_t m, int S, const char* wl, const TfScratchF32& w, cudaStream_t st) {
+// the layer of encoder_layer above on fp32 windows at fp32 accuracy, in place on x: every GEMM operand is split first.
+// live (may be null): device count of live windows, as in the bf16 layer; every launch is bounded by it.
+cudaError_t encoder_layer(float* x, const float* src, int64_t m, const int32_t* live, int S, const char* wl,
+                          const TfScratchF32& w, cudaStream_t st) {
   const int64_t T = m * S;
+  const size_t row = size_t(S) * kD;    // elements of one window
   const float* ln = reinterpret_cast<const float*>(wl + 3 * kOffLn);
   const DstF none{nullptr, 0};
   const Planes xs{w.xs, w.unit2}, ms{w.ms, 2 * w.unit2}, no{nullptr, 0};
   auto weight = [wl](size_t off, size_t rows, size_t cols) { return Planes{wl + 3 * off, rows * cols * 2}; };
   cudaError_t e;
-  if ((e = split_planes(x, w.xs, xs.stride, size_t(T) * kD, st)) != cudaSuccess) return e;
+  if ((e = split_planes(x, w.xs, xs.stride, size_t(T) * kD, live, row, 0, st)) != cudaSuccess) return e;
   SplitParams P{};
   if (x == src) {                       // self: one pass over x produces q, k, v
     P.mode[0] = EPI_ELU1; P.mode[1] = EPI_ELU1; P.mode[2] = EPI_SCALE; P.scale = 1.f / float(S);
     const DstF o[3] = {{w.q, kD}, {w.k, kD}, {w.v, kD}};
-    if ((e = gemm_split_run(T, xs, kD, no, 0, weight(kOffQkv, 384, 128), 384, kD, o, P, nullptr, st)) != cudaSuccess) return e;
+    if ((e = gemm_split_run(T, xs, kD, no, 0, weight(kOffQkv, 384, 128), 384, kD, o, P, nullptr, st, live, S)) != cudaSuccess)
+      return e;
   } else {
     const Planes ss{w.ss, 2 * w.unit2};
-    if ((e = split_planes(src, w.ss, ss.stride, size_t(T) * kD, st)) != cudaSuccess) return e;
+    if ((e = split_planes(src, w.ss, ss.stride, size_t(T) * kD, live, row, 0, st)) != cudaSuccess) return e;
     P.mode[0] = EPI_ELU1;
     const DstF oq[3] = {{w.q, kD}, none, none};
-    if ((e = gemm_split_run(T, xs, kD, no, 0, weight(kOffQkv, 384, 128), 128, kD, oq, P, nullptr, st)) != cudaSuccess) return e;
+    if ((e = gemm_split_run(T, xs, kD, no, 0, weight(kOffQkv, 384, 128), 128, kD, oq, P, nullptr, st, live, S)) != cudaSuccess)
+      return e;
     P.mode[0] = EPI_ELU1; P.mode[1] = EPI_SCALE; P.scale = 1.f / float(S);
     const DstF okv[3] = {{w.k, kD}, {w.v, kD}, none};
     Planes wkv = weight(kOffQkv, 384, 128);
     wkv.ptr = static_cast<const char*>(wkv.ptr) + 128 * 128 * 2;    // k_proj and v_proj rows of every plane
-    if ((e = gemm_split_run(T, ss, kD, no, 0, wkv, 256, kD, okv, P, nullptr, st)) != cudaSuccess) return e;
+    if ((e = gemm_split_run(T, ss, kD, no, 0, wkv, 256, kD, okv, P, nullptr, st, live, S)) != cudaSuccess) return e;
   }
   fine_attn_kernel<float><<<unsigned((m + kAttnWarps - 1) / kAttnWarps), kAttnWarps * 32, 0, st>>>(w.q, w.k, w.v, w.msg, m,
-                                                                                                   nullptr, S, 1e-6f);
+                                                                                                   live, S, 1e-6f);
   if ((e = cudaGetLastError()) != cudaSuccess) return e;
-  if ((e = split_planes(w.msg, w.ms, ms.stride, size_t(T) * kD, st)) != cudaSuccess) return e;
+  if ((e = split_planes(w.msg, w.ms, ms.stride, size_t(T) * kD, live, row, 0, st)) != cudaSuccess) return e;
   P = SplitParams{};
   P.mode[0] = EPI_LN; P.gamma = ln; P.beta = ln + 128;
   const DstF om[3] = {{w.m1, kD}, none, none};
-  if ((e = gemm_split_run(T, ms, kD, no, 0, weight(kOffMerge, 128, 128), 128, kD, om, P, nullptr, st)) != cudaSuccess) return e;
-  if ((e = split_planes(w.m1, w.ms, ms.stride, size_t(T) * kD, st)) != cudaSuccess) return e;
+  if ((e = gemm_split_run(T, ms, kD, no, 0, weight(kOffMerge, 128, 128), 128, kD, om, P, nullptr, st, live, S)) != cudaSuccess)
+    return e;
+  if ((e = split_planes(w.m1, w.ms, ms.stride, size_t(T) * kD, live, row, 0, st)) != cudaSuccess) return e;
   // MLP: relu(W1 . cat(x, m1)) -> hid [T, 256] fp32, then x <- x + LayerNorm2(W2 . hid)      (transformer.py:52-58)
   P = SplitParams{};
   P.mode[0] = EPI_RELU; P.mode[1] = EPI_RELU;
   const DstF oh[3] = {{w.hid, 2 * kD}, {w.hid + kD, 2 * kD}, none};
-  if ((e = gemm_split_run(T, xs, kD, ms, kD, weight(kOffMlp1, 256, 256), 256, 256, oh, P, nullptr, st)) != cudaSuccess) return e;
-  if ((e = split_planes(w.hid, w.ms, ms.stride, size_t(T) * 2 * kD, st)) != cudaSuccess) return e;   // [T, 256] planes
+  if ((e = gemm_split_run(T, xs, kD, ms, kD, weight(kOffMlp1, 256, 256), 256, 256, oh, P, nullptr, st, live, S)) != cudaSuccess)
+    return e;
+  if ((e = split_planes(w.hid, w.ms, ms.stride, size_t(T) * 2 * kD, live, 2 * row, 0, st)) != cudaSuccess)   // [T, 256] planes
+    return e;
   P = SplitParams{};
   P.mode[0] = EPI_LN_RES; P.gamma = ln + 256; P.beta = ln + 384;
   const DstF ox[3] = {{x, kD}, none, none};
-  return gemm_split_run(T, ms, 2 * kD, no, 0, weight(kOffMlp2, 128, 256), 128, 256, ox, P, x, st);
+  return gemm_split_run(T, ms, 2 * kD, no, 0, weight(kOffMlp2, 128, 256), 128, 256, ox, P, x, st, live, S);
 }
 
 // FinePreprocess at fp32 accuracy: gathered coarse rows cg [2m, 256] fp32 and their planes (a region of three
@@ -1565,9 +1657,9 @@ extern "C" size_t pope_fine_tf_f32_workspace_bytes(int64_t m_windows, int window
   return carve_tf_f32(nullptr, m_windows, window_tokens).bytes;
 }
 
-extern "C" int pope_fine_transformer_f32(void* feat0, void* feat1, int64_t m_windows, int window_tokens, const void* weights,
-                                         int n_layers, const int* layer_kinds, void* workspace, size_t workspace_bytes,
-                                         void* stream) {
+extern "C" int pope_fine_transformer_f32_ex(void* feat0, void* feat1, int64_t m_windows, const int32_t* m_dev,
+                                            int window_tokens, const void* weights, int n_layers, const int* layer_kinds,
+                                            void* workspace, size_t workspace_bytes, void* stream) {
   if (!feat0 || !feat1 || !weights || !layer_kinds || !workspace) return POPE_ERR_INVALID_ARG;
   if (m_windows < 0 || window_tokens <= 0 || n_layers < 0) return POPE_ERR_INVALID_ARG;
   for (int l = 0; l < n_layers; ++l)
@@ -1586,24 +1678,31 @@ extern "C" int pope_fine_transformer_f32(void* feat0, void* feat1, int64_t m_win
     const char* wl = static_cast<const char*>(weights) + size_t(l) * kF32LayerBytes;
     cudaError_t e;
     if (layer_kinds[l] == 0) {            // 'self'  (transformer.py:96-98)
-      if ((e = encoder_layer(x0, x0, m_windows, window_tokens, wl, w, st)) != cudaSuccess) return int(e);
-      if ((e = encoder_layer(x1, x1, m_windows, window_tokens, wl, w, st)) != cudaSuccess) return int(e);
+      if ((e = encoder_layer(x0, x0, m_windows, m_dev, window_tokens, wl, w, st)) != cudaSuccess) return int(e);
+      if ((e = encoder_layer(x1, x1, m_windows, m_dev, window_tokens, wl, w, st)) != cudaSuccess) return int(e);
     } else {                              // 'cross' (:99-101): feat1 attends to the UPDATED feat0
-      if ((e = encoder_layer(x0, x1, m_windows, window_tokens, wl, w, st)) != cudaSuccess) return int(e);
-      if ((e = encoder_layer(x1, x0, m_windows, window_tokens, wl, w, st)) != cudaSuccess) return int(e);
+      if ((e = encoder_layer(x0, x1, m_windows, m_dev, window_tokens, wl, w, st)) != cudaSuccess) return int(e);
+      if ((e = encoder_layer(x1, x0, m_windows, m_dev, window_tokens, wl, w, st)) != cudaSuccess) return int(e);
     }
   }
   return POPE_OK;
+}
+
+extern "C" int pope_fine_transformer_f32(void* feat0, void* feat1, int64_t m_windows, int window_tokens, const void* weights,
+                                         int n_layers, const int* layer_kinds, void* workspace, size_t workspace_bytes,
+                                         void* stream) {
+  return pope_fine_transformer_f32_ex(feat0, feat1, m_windows, nullptr, window_tokens, weights, n_layers, layer_kinds,
+                                      workspace, workspace_bytes, stream);
 }
 
 extern "C" size_t pope_fine_merge_f32_workspace_bytes(int64_t m_windows) {
   return m_windows > 0 ? carve_merge_f32(nullptr, m_windows).bytes : 0;
 }
 
-extern "C" int pope_fine_merge_coarse_f32(void* win0, void* win1, int64_t m_windows, int window_tokens, const void* feat_c0,
-                                          const void* feat_c1, int L, int S, int C, const int64_t* b_ids, const int64_t* i_ids,
-                                          const int64_t* j_ids, const void* weights, void* workspace, size_t workspace_bytes,
-                                          void* stream) {
+extern "C" int pope_fine_merge_coarse_f32_ex(void* win0, void* win1, int64_t m_windows, const int32_t* m_dev, int window_tokens,
+                                             const void* feat_c0, const void* feat_c1, int L, int S, int C,
+                                             const int64_t* b_ids, const int64_t* i_ids, const int64_t* j_ids,
+                                             const void* weights, void* workspace, size_t workspace_bytes, void* stream) {
   if (!win0 || !win1 || !feat_c0 || !feat_c1 || !b_ids || !i_ids || !j_ids || !weights || !workspace)
     return POPE_ERR_INVALID_ARG;
   if (m_windows < 0 || window_tokens <= 0 || L <= 0 || S <= 0) return POPE_ERR_INVALID_ARG;
@@ -1623,39 +1722,61 @@ extern "C" int pope_fine_merge_coarse_f32(void* win0, void* win1, int64_t m_wind
   const DstF none{nullptr, 0};
   const Planes no{nullptr, 0};
   gather_coarse_rows_kernel<float><<<unsigned((2 * m + 7) / 8), 256, 0, st>>>(
-      static_cast<const float*>(feat_c0), static_cast<const float*>(feat_c1), b_ids, i_ids, j_ids, m, nullptr, L, S, C, w.cg);
+      static_cast<const float*>(feat_c0), static_cast<const float*>(feat_c1), b_ids, i_ids, j_ids, m, m_dev, L, S, C, w.cg);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return int(e);
-  // feat_c_win = down_proj(cat(c0, c1))                                                    (fine_preprocess.py:50-51)
-  if ((e = split_planes(w.cg, w.cgs, w.cgs_stride, size_t(2 * m) * 256, st)) != cudaSuccess) return int(e);
+  // The [2m, .] arrays hold side 1 from row m (the capacity) on, so with a live count their live rows are [0, live) and
+  // [m, m + live): each side is then its own launch, bounded by the count.  Without one, both sides are a single launch.
+  const int nseg = m_dev ? 2 : 1;
+  const int64_t seg = 2 * m / nseg;
   SplitParams P{};
-  P.mode[0] = EPI_COPY; P.bias = bias;
-  const DstF od[3] = {{w.cd, kD}, none, none};
-  if ((e = gemm_split_run(2 * m, Planes{w.cgs, w.cgs_stride}, 256, no, 0, weight(kOffDown, 0), 128, 256, od, P, nullptr, st)) !=
-      cudaSuccess)
-    return int(e);
-  // merge_feat(cat(win, repeat(c))) = win . Wa^T + (c . Wb^T + bias): the second term once per window         (:52-55)
-  if ((e = split_planes(w.cd, w.cds, w.cds_stride, size_t(2 * m) * kD, st)) != cudaSuccess) return int(e);
-  P = SplitParams{};
-  P.mode[0] = EPI_COPY; P.bias = bias + 128;
-  const DstF ov[3] = {{w.cvec, kD}, none, none};
-  if ((e = gemm_split_run(2 * m, Planes{w.cds, w.cds_stride}, 128, no, 0, weight(kOffMergeFeat, 128), 128, 256, ov, P, nullptr,
-                          st)) != cudaSuccess)
-    return int(e);
-  // the window part in place, in chunks of rows whose planes fit the (now dead) planes of the gathered rows
+  for (int s = 0; s < nseg; ++s) {
+    // feat_c_win = down_proj(cat(c0, c1))                                                  (fine_preprocess.py:50-51)
+    const Planes cgs{w.cgs + s * seg * 256, w.cgs_stride}, cds{w.cds + s * seg * kD, w.cds_stride};
+    if ((e = split_planes(w.cg + s * seg * 256, w.cgs + s * seg * 256, w.cgs_stride, size_t(seg) * 256, m_dev, 256, 0, st)) !=
+        cudaSuccess)
+      return int(e);
+    P = SplitParams{};
+    P.mode[0] = EPI_COPY; P.bias = bias;
+    const DstF od[3] = {{w.cd + s * seg * kD, kD}, none, none};
+    if ((e = gemm_split_run(seg, cgs, 256, no, 0, weight(kOffDown, 0), 128, 256, od, P, nullptr, st, m_dev)) != cudaSuccess)
+      return int(e);
+    // merge_feat(cat(win, repeat(c))) = win . Wa^T + (c . Wb^T + bias): the second term once per window       (:52-55)
+    if ((e = split_planes(w.cd + s * seg * kD, w.cds + s * seg * kD, w.cds_stride, size_t(seg) * kD, m_dev, kD, 0, st)) !=
+        cudaSuccess)
+      return int(e);
+    P = SplitParams{};
+    P.mode[0] = EPI_COPY; P.bias = bias + 128;
+    const DstF ov[3] = {{w.cvec + s * seg * kD, kD}, none, none};
+    if ((e = gemm_split_run(seg, cds, 128, no, 0, weight(kOffMergeFeat, 128), 128, 256, ov, P, nullptr, st, m_dev)) != cudaSuccess)
+      return int(e);
+  }
+  // the window part in place, in chunks of rows whose planes fit the (now dead) planes of the gathered rows; with a live
+  // count each chunk is clamped to the live rows it covers (row0 on), and a chunk past them launches nothing that works
   const int64_t T = m * window_tokens;
+  const size_t row = size_t(window_tokens) * kD;            // elements of one window
   for (int side = 0; side < 2; ++side) {
     float* win = static_cast<float*>(side ? win1 : win0);
     for (int64_t r0 = 0; r0 < T; r0 += w.chunk_rows) {
       const int64_t rows = T - r0 < w.chunk_rows ? T - r0 : w.chunk_rows;
-      if ((e = split_planes(win + r0 * kD, w.cgs, w.cgs_stride, size_t(rows) * kD, st)) != cudaSuccess) return int(e);
+      if ((e = split_planes(win + r0 * kD, w.cgs, w.cgs_stride, size_t(rows) * kD, m_dev, row, size_t(r0) * kD, st)) !=
+          cudaSuccess)
+        return int(e);
       P = SplitParams{};
       P.mode[0] = EPI_ADDVEC; P.rowvec = w.cvec + size_t(side) * m * kD; P.rows_per_vec = window_tokens; P.row0 = r0;
       const DstF ow[3] = {{win + r0 * kD, kD}, none, none};
       if ((e = gemm_split_run(rows, Planes{w.cgs, w.cgs_stride}, 128, no, 0, weight(kOffMergeFeat, 0), 128, 256, ow, P, nullptr,
-                              st)) != cudaSuccess)
+                              st, m_dev, window_tokens)) != cudaSuccess)
         return int(e);
     }
   }
   return POPE_OK;
+}
+
+extern "C" int pope_fine_merge_coarse_f32(void* win0, void* win1, int64_t m_windows, int window_tokens, const void* feat_c0,
+                                          const void* feat_c1, int L, int S, int C, const int64_t* b_ids, const int64_t* i_ids,
+                                          const int64_t* j_ids, const void* weights, void* workspace, size_t workspace_bytes,
+                                          void* stream) {
+  return pope_fine_merge_coarse_f32_ex(win0, win1, m_windows, nullptr, window_tokens, feat_c0, feat_c1, L, S, C, b_ids, i_ids,
+                                       j_ids, weights, workspace, workspace_bytes, stream);
 }

@@ -157,7 +157,7 @@ struct pope_pipeline {
   unsigned long long* fetched = nullptr;     // device: pixels of the fine maps the union fetch has copied in this run
   unsigned long long* h_fetched = nullptr;   // pinned staging for it
   Slot slot[2];
-  // the bf16 fine level (pope_pipeline_set_fine_level): caller-owned packed weights; windows, image 0's cell mask and
+  // the fine level (pope_pipeline_set_fine_level_ex, in the pipeline's dtype): caller-owned packed weights; windows, image 0's cell mask and
   // scratch are allocated on the first attach and shared by both slots (all of it is touched on s_comp only)
   const void* fine_pre = nullptr;
   const void* fine_layers = nullptr;
@@ -254,8 +254,8 @@ fail:
   return rc;
 }
 
-extern "C" int pope_pipeline_set_fine_level(pope_pipeline_t* pl, const void* pre, const void* layers, int n_layers,
-                                            const int* layer_kinds) {
+extern "C" int pope_pipeline_set_fine_level_ex(pope_pipeline_t* pl, int dtype, const void* pre, const void* layers,
+                                               int n_layers, const int* layer_kinds) {
   if (!pl) return POPE_ERR_INVALID_ARG;
   if (!layers) {                 // detach; the windows and scratch stay allocated until pope_pipeline_destroy
     pl->fine_pre = pl->fine_layers = nullptr;
@@ -265,7 +265,7 @@ extern "C" int pope_pipeline_set_fine_level(pope_pipeline_t* pl, const void* pre
   if (n_layers < 1 || !layer_kinds) return POPE_ERR_INVALID_ARG;
   for (int l = 0; l < n_layers; ++l)
     if (layer_kinds[l] != 0 && layer_kinds[l] != 1) return POPE_ERR_INVALID_ARG;
-  if (pl->dtype != POPE_BF16) return POPE_ERR_DTYPE;
+  if (dtype != pl->dtype) return POPE_ERR_DTYPE;
   if (pl->C != 256) return POPE_ERR_SHAPE;
   if ((reinterpret_cast<uintptr_t>(pre) | reinterpret_cast<uintptr_t>(layers)) & 15u) return POPE_ERR_ALIGNMENT;
   int rc = POPE_OK;
@@ -273,10 +273,14 @@ extern "C" int pope_pipeline_set_fine_level(pope_pipeline_t* pl, const void* pre
   if (!kinds) return int(cudaErrorMemoryAllocation);
   for (int l = 0; l < n_layers; ++l) kinds[l] = layer_kinds[l];
   if (!pl->win0) {
-    // sized by the chunk's capacity, like every other slot buffer: the launches are bounded by the device count
+    // sized by the chunk's capacity, like every other slot buffer: the launches are bounded by the device count; the
+    // windows have the pipeline's element type
     const int64_t m = int64_t(pl->chunk) * pl->cap;
-    const size_t win_bytes = size_t(m) * pl->W * pl->W * pl->Cf * 2;
-    const size_t tf = pope_fine_tf_workspace_bytes(m, pl->W * pl->W), mg = pope_fine_merge_workspace_bytes(m);
+    const int ww = pl->W * pl->W;
+    const size_t win_bytes = size_t(m) * ww * pl->Cf * pl->esize;
+    const bool f32 = pl->dtype == POPE_F32;
+    const size_t tf = f32 ? pope_fine_tf_f32_workspace_bytes(m, ww) : pope_fine_tf_workspace_bytes(m, ww);
+    const size_t mg = f32 ? pope_fine_merge_f32_workspace_bytes(m) : pope_fine_merge_workspace_bytes(m);
     PL_CUDA(cudaSetDevice(pl->device));
     PL_CUDA(cudaMalloc(&pl->win0, win_bytes));
     PL_CUDA(cudaMalloc(&pl->win1, win_bytes));
@@ -296,6 +300,11 @@ fail:
   pl->win0 = pl->win1 = pl->fine_ws = nullptr;
   pl->cellmask0 = nullptr;
   return rc;
+}
+
+extern "C" int pope_pipeline_set_fine_level(pope_pipeline_t* pl, const void* pre, const void* layers, int n_layers,
+                                            const int* layer_kinds) {
+  return pope_pipeline_set_fine_level_ex(pl, POPE_BF16, pre, layers, n_layers, layer_kinds);
 }
 
 extern "C" int pope_pipeline_run(pope_pipeline_t* pl, const void* feat_c0, const void* feat_c1, const void* feat_f0,
@@ -402,13 +411,16 @@ extern "C" int pope_pipeline_run(pope_pipeline_t* pl, const void* feat_c0, const
                             pl->dtype, n, pl->Cf, Hf0, Wf0, st0, Hf1, Wf1, st1, pl->w0c, pl->w1c, pl->fstride, pl->W, s.b_ids,
                             s.i_ids, s.j_ids, m, m_dev, pl->win0, pl->win1, pl->s_comp);
       if (rc) goto fail;
+      const bool f32 = pl->dtype == POPE_F32;
       if (pl->fine_pre) {
-        rc = pope_fine_merge_coarse_ex(pl->win0, pl->win1, m, m_dev, ww, s.fc0, s.fc1, pl->L, pl->S, pl->C, s.b_ids, s.i_ids,
-                                       s.j_ids, pl->fine_pre, pl->fine_ws, pl->fine_ws_bytes, pl->s_comp);
+        rc = (f32 ? pope_fine_merge_coarse_f32_ex : pope_fine_merge_coarse_ex)(
+            pl->win0, pl->win1, m, m_dev, ww, s.fc0, s.fc1, pl->L, pl->S, pl->C, s.b_ids, s.i_ids, s.j_ids, pl->fine_pre,
+            pl->fine_ws, pl->fine_ws_bytes, pl->s_comp);
         if (rc) goto fail;
       }
-      rc = pope_fine_transformer_ex(pl->win0, pl->win1, m, m_dev, ww, pl->fine_layers, pl->fine_n_layers, pl->fine_kinds,
-                                    pl->fine_ws, pl->fine_ws_bytes, pl->s_comp);
+      rc = (f32 ? pope_fine_transformer_f32_ex : pope_fine_transformer_ex)(pl->win0, pl->win1, m, m_dev, ww, pl->fine_layers,
+                                                                           pl->fine_n_layers, pl->fine_kinds, pl->fine_ws,
+                                                                           pl->fine_ws_bytes, pl->s_comp);
       if (rc) goto fail;
       rc = pope_fine_match(pl->win0, pl->win1, pl->dtype, m, m_dev, ww, pl->Cf, s.mk1, coord_scale, s.expec, s.mk1f,
                            pl->s_comp);

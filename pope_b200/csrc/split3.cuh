@@ -10,8 +10,8 @@
 namespace pope {
 namespace {   // (a kernel defined in a header: one private copy per translation unit)
 
-__global__ void __launch_bounds__(256) split3_kernel(const float4* __restrict__ in, uint2* __restrict__ p1, uint2* __restrict__ p2,
-                                                    uint2* __restrict__ p3, size_t n4) {
+__device__ __forceinline__ void split3_range(const float4* __restrict__ in, uint2* __restrict__ p1, uint2* __restrict__ p2,
+                                             uint2* __restrict__ p3, size_t n4) {
   for (size_t i = size_t(blockIdx.x) * blockDim.x + threadIdx.x; i < n4; i += size_t(gridDim.x) * blockDim.x) {
     const float4 a = __ldcs(in + i);
     const float v[4] = {a.x, a.y, a.z, a.w};
@@ -29,6 +29,11 @@ __global__ void __launch_bounds__(256) split3_kernel(const float4* __restrict__ 
     p2[i] = make_uint2(h2[0] | (h2[1] << 16), h2[2] | (h2[3] << 16));
     p3[i] = make_uint2(h3[0] | (h3[1] << 16), h3[2] | (h3[3] << 16));
   }
+}
+
+__global__ void __launch_bounds__(256) split3_kernel(const float4* __restrict__ in, uint2* __restrict__ p1, uint2* __restrict__ p2,
+                                                    uint2* __restrict__ p3, size_t n4) {
+  split3_range(in, p1, p2, p3, n4);
 }
 
 // fp32 [elems] -> three bf16 planes `stride` bytes apart (elems a multiple of 4, src 16-byte aligned)

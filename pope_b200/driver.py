@@ -31,14 +31,22 @@ def _fine_to_nhwc(ff: torch.Tensor) -> torch.Tensor:
 
 
 def _check_fine_level(fine_level: dict, dtype: torch.dtype, C_coarse: int, device: int):
-    """What `pope_pipeline_set_fine_level` needs, checked before any GPU call; returns its (pre, layers, kinds) arguments."""
-    if dtype != torch.bfloat16 or C_coarse != 256:
-        raise _lib.PopeError("the bf16 fine level needs a bfloat16 pipeline with C_coarse = 256")
+    """What `pope_pipeline_set_fine_level_ex` needs, checked before any GPU call; returns its (pre, layers, kinds)
+    arguments.  The bundle's packing (its "dtype", bf16 when absent) must be the pipeline's dtype."""
+    from .ops import _fine_level_dtype
+    level = _fine_level_dtype(fine_level)
+    if level != dtype:
+        raise _lib.PopeError(f"the fine level is packed for {level}, the pipeline runs {dtype}: they must agree "
+                             f"(Matcher.fine_level(device, dtype={dtype}))")
+    if C_coarse != 256:
+        raise _lib.PopeError("the fine level needs a pipeline with C_coarse = 256")
+    f32 = dtype == torch.float32
+    layer_bytes = _lib.FINE_TF_F32_LAYER_BYTES if f32 else _lib.FINE_TF_LAYER_BYTES
+    pre_bytes = _lib.FINE_PRE_F32_BYTES if f32 else _lib.FINE_PRE_BYTES
     names, layers, pre = list(fine_level["layer_names"]), fine_level["layers"], fine_level["pre"]
-    if not names or any(nm not in ("self", "cross") for nm in names) \
-            or layers.numel() != len(names) * _lib.FINE_TF_LAYER_BYTES:
+    if not names or any(nm not in ("self", "cross") for nm in names) or layers.numel() != len(names) * layer_bytes:
         raise _lib.PopeError("the fine level's layer names and packed layers do not agree")
-    if pre is not None and pre.numel() != _lib.FINE_PRE_BYTES:
+    if pre is not None and pre.numel() != pre_bytes:
         raise _lib.PopeError("the fine level's packed FinePreprocess weights have the wrong size")
     dev = torch.device("cuda", device)
     for t in (layers, pre):
@@ -55,7 +63,10 @@ class Pipeline:
     window gather and fine matching -- FinePreprocess' two Linears and the fine transformer, in bf16 -- so that the results
     equal `ops.match_pairs_device(..., fine_level=...)` and thereby `Matcher(config, fine_cuda_bf16=True)`, bit for bit.
     Needs a bf16 pipeline with C_coarse = 256.  The pipeline keeps a reference to the dict, so the packed weights outlive
-    the handle; it allocates windows and fine scratch for one chunk (0.98 GB + 2.5 GB at 16 pairs of 480x640)."""
+    the handle; it allocates windows and fine scratch for one chunk (0.98 GB + 2.5 GB at 16 pairs of 480x640).
+    An fp32 pipeline takes `Matcher.fine_level(device, dtype=torch.float32)`, the fp32-accuracy level: the results then
+    equal the fp32 device step and `Matcher(config, fine_cuda_fp32=True)`; one chunk's fp32 windows and fine scratch are
+    1.97 GB + 9.3 GB at 16 pairs of 480x640 (computed from the sizes).  The bundle's packing must be the pipeline's dtype."""
 
     def __init__(self, dtype: torch.dtype, chunk_pairs: int, hw0_i: Sequence[int], hw0_c: Sequence[int],
                  hw1_c: Sequence[int], C_coarse: int = 256, C_fine: int = 128, fine_stride: int = 4, W: int = 5,
@@ -97,8 +108,9 @@ class Pipeline:
         pre, layers, kinds = _check_fine_level(fine_level, self.dtype, self.C, self.device)
         # the weights may have been packed just now on torch's stream, which the pipeline's own streams do not wait for
         torch.cuda.current_stream(layers.device).synchronize()
-        check(lib().pope_pipeline_set_fine_level(self._h, None if pre is None else pre.data_ptr(), layers.data_ptr(),
-                                                 len(kinds), kinds), "pope_pipeline_set_fine_level")
+        code = _lib.POPE_F32 if self.dtype == torch.float32 else _lib.POPE_BF16
+        check(lib().pope_pipeline_set_fine_level_ex(self._h, code, None if pre is None else pre.data_ptr(),
+                                                    layers.data_ptr(), len(kinds), kinds), "pope_pipeline_set_fine_level")
         self.fine_level = fine_level          # keeps the packed tensors alive while the handle may read them
 
     def alloc_outputs(self, n: int, pinned: bool = True) -> Dict[str, torch.Tensor]:
@@ -146,7 +158,9 @@ def match_pairs_host(feat_c0, feat_c1, feat_f0, feat_f1, hw0_i, hw0_c, hw1_c, ch
                      fine_level: Optional[dict] = None, **kw) -> Dict[str, torch.Tensor]:
     """One-shot host-buffer entry: feat_f* are logical [N, Cf, Hf, Wf] CPU tensors (channels-last is free).  With
     `fine_level` (`Matcher.fine_level(torch.device("cuda", device))`) the results equal what
-    `Matcher(config, fine_cuda_bf16=True)` computes from these features (see `Pipeline`)."""
+    `Matcher(config, fine_cuda_bf16=True)` computes from these features; with fp32 features and
+    `Matcher.fine_level(torch.device("cuda", device), dtype=torch.float32)`, what `Matcher(config, fine_cuda_fp32=True)`
+    computes (see `Pipeline`)."""
     n = feat_c0.shape[0]
     pl = Pipeline(feat_c0.dtype, min(chunk_pairs, n), hw0_i, hw0_c, hw1_c, feat_c0.shape[2], feat_f0.shape[1],
                   feat_f0.shape[2] // hw0_c[0], device=device, fine_level=fine_level, **kw)
@@ -175,7 +189,10 @@ class DeviceBatchRunner:
     the next batch's sweep (B200, 64 pairs at 480x640: 0.97 -> 0.91 ms per batch).  No host synchronisation anywhere:
     results are capacity-sized `CoarseResult`s whose match count stays on the device; call `join()` before reading them
     on another stream.  With `submit(..., fine_level=Matcher.fine_level(device))` each batch also runs the bf16
-    FinePreprocess Linears and fine transformer (see `ops.match_pairs_device`), in a fine scratch kept per stream."""
+    FinePreprocess Linears and fine transformer (see `ops.match_pairs_device`), in a fine scratch kept per stream; with
+    `Matcher.fine_level(device, dtype=torch.float32)` and fp32 features, the fp32-accuracy level.  One fine scratch per
+    stream is sized by the batch's capacity: at 64 pairs x 480x640 the fp32 level holds 37.4 GB of scratch per stream, so
+    two streams hold about 75 GB (computed from the workspace formulas)."""
 
     def __init__(self, device, n_streams: int = 2):
         self.device = torch.device(device)

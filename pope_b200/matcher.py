@@ -93,16 +93,21 @@ class Matcher(nn.Module):
         self.loftr_coarse.cuda_fp32 = self.coarse_cuda_fp32
         self.loftr_coarse.inplace = self.coarse_cuda_bf16 or self.coarse_cuda_fp32
 
-    def fine_level(self, device) -> dict:
-        """The packed bf16 weights of the fine level for `ops.match_pairs_device(..., fine_level=...)` (and the driver's
+    def fine_level(self, device, dtype: torch.dtype = torch.bfloat16) -> dict:
+        """The packed weights of the fine level for `ops.match_pairs_device(..., fine_level=...)` (and the driver's
         batched steps built on it): {"pre": FinePreprocess' down_proj + merge_feat (None when fine_concat_coarse_feat is
-        off), "layers": the fine transformer's layers, "layer_names": their 'self' / 'cross' schedule}.  The packed
+        off), "layers": the fine transformer's layers, "layer_names": their 'self' / 'cross' schedule, "dtype": the
+        packing}.  dtype=torch.bfloat16 packs the bf16 level (what `fine_cuda_bf16=True` runs), dtype=torch.float32 the
+        fp32-accuracy one (what `fine_cuda_fp32=True` runs); a bundle without "dtype" is read as bf16.  The packed
         tensors are the modules' own caches, repacked only when a parameter changes."""
         if not self.loftr_fine.cuda_supported():
             raise NotImplementedError("the CUDA fine transformer covers d_model 128 / 8 heads / linear attention")
+        from . import ops
+        ops._check_pack_dtype(dtype, "fine level")
         dev = torch.device(device)
-        pre = self.fine_preprocess._packed_weights(dev) if self.fine_preprocess.cat_c_feat else None
-        return {"pre": pre, "layers": self.loftr_fine._packed_weights(dev), "layer_names": list(self.loftr_fine.layer_names)}
+        pre = self.fine_preprocess._packed_weights(dev, dtype) if self.fine_preprocess.cat_c_feat else None
+        return {"pre": pre, "layers": self.loftr_fine._packed_weights(dev, dtype),
+                "layer_names": list(self.loftr_fine.layer_names), "dtype": dtype}
 
     def forward(self, data: dict, only_att_fea: bool = False):
         img0, img1 = data["image0"], data["image1"]

@@ -210,11 +210,17 @@ def fine_transformer(feat0: torch.Tensor, feat1: torch.Tensor, packed_layers: to
     the bf16 fine transformer, float32 windows the fp32-accuracy one; `packed_layers`: concatenation of
     pack_fine_layer(..., dtype=<the windows' dtype>) of every layer, `layer_names`: 'self' / 'cross'.
     `m_dev` (device int32, bf16 only): live window count; M is then the capacity and windows >= *m_dev are left untouched."""
+    if m_dev is not None and (feat0.dtype == torch.float32 or feat1.dtype == torch.float32):
+        raise _lib.PopeError("the fp32 fine transformer has no device-count bound (m_dev): it runs on all M windows")
+    return _fine_transformer(feat0, feat1, packed_layers, layer_names, workspace, m_dev)
+
+
+def _fine_transformer(feat0, feat1, packed_layers, layer_names, workspace, m_dev):
+    """fine_transformer with a device-count bound for either dtype (the fp32 one through pope_fine_transformer_f32_ex,
+    which ops.match_pairs_device uses)."""
     dev = require_cuda(feat0, feat1, packed_layers)
     _check_m_dev(m_dev, dev)
     f32 = _fine_dtype("the CUDA fine transformer", feat0, feat1)
-    if f32 and m_dev is not None:
-        raise _lib.PopeError("the fp32 fine transformer has no device-count bound (m_dev): it runs on all M windows")
     if feat0.shape != feat1.shape or feat0.dim() != 3 or feat0.shape[2] != 128:
         raise _lib.PopeError("feat0 / feat1 must both be [M, WW, 128]")
     if not (feat0.is_contiguous() and feat1.is_contiguous()):
@@ -231,13 +237,10 @@ def fine_transformer(feat0: torch.Tensor, feat1: torch.Tensor, packed_layers: to
         return feat0, feat1
     workspace = fine_level_workspace(M, WW, dev, workspace, merge=False, dtype=feat0.dtype)
     arr = (_lib.C.c_int * max(len(kinds), 1))(*kinds)
+    fn = lib().pope_fine_transformer_f32_ex if f32 else lib().pope_fine_transformer_ex
     with torch.cuda.device(dev):
-        if f32:
-            st = lib().pope_fine_transformer_f32(ptr(feat0), ptr(feat1), M, WW, ptr(packed_layers), len(kinds), arr,
-                                                 ptr(workspace), workspace.numel(), stream_ptr(dev))
-        else:
-            st = lib().pope_fine_transformer_ex(ptr(feat0), ptr(feat1), M, ptr(m_dev), WW, ptr(packed_layers), len(kinds),
-                                                arr, ptr(workspace), workspace.numel(), stream_ptr(dev))
+        st = fn(ptr(feat0), ptr(feat1), M, ptr(m_dev), WW, ptr(packed_layers), len(kinds), arr, ptr(workspace),
+                workspace.numel(), stream_ptr(dev))
     check(st, "pope_fine_transformer_f32" if f32 else "pope_fine_transformer")
     return feat0, feat1
 
@@ -366,13 +369,19 @@ def fine_merge_coarse(win0: torch.Tensor, win1: torch.Tensor, feat_c0: torch.Ten
     tensors in bf16, float32 tensors at fp32 accuracy (`packed_pre` from pack_fine_pre(..., dtype=<their dtype>)).
     `m_dev` (device int32, bf16 only): live window count; M is then the capacity and windows / ids >= *m_dev are never
     touched."""
+    if m_dev is not None and any(t.dtype == torch.float32 for t in (win0, win1, feat_c0, feat_c1)):
+        raise _lib.PopeError("the fp32 fine_merge_coarse has no device-count bound (m_dev): it runs on all M windows")
+    return _fine_merge_coarse(win0, win1, feat_c0, feat_c1, b_ids, i_ids, j_ids, packed_pre, workspace, m_dev)
+
+
+def _fine_merge_coarse(win0, win1, feat_c0, feat_c1, b_ids, i_ids, j_ids, packed_pre, workspace, m_dev):
+    """fine_merge_coarse with a device-count bound for either dtype (the fp32 one through pope_fine_merge_coarse_f32_ex,
+    which ops.match_pairs_device uses)."""
     dev = require_cuda(win0, win1, feat_c0, feat_c1, b_ids, i_ids, j_ids, packed_pre)
     _check_m_dev(m_dev, dev)
     f32 = _fine_dtype("fine_merge_coarse", win0, win1, feat_c0, feat_c1)
     if not all(t.is_contiguous() for t in (win0, win1, feat_c0, feat_c1)):
         raise _lib.PopeError("fine_merge_coarse takes contiguous tensors")
-    if f32 and m_dev is not None:
-        raise _lib.PopeError("the fp32 fine_merge_coarse has no device-count bound (m_dev): it runs on all M windows")
     _check_packing(packed_pre, 1, f32, _lib.FINE_PRE_BYTES, _lib.FINE_PRE_F32_BYTES, "packed_pre", "pack_fine_pre")
     M, WW, _ = win0.shape
     if M == 0:
@@ -381,14 +390,10 @@ def fine_merge_coarse(win0: torch.Tensor, win1: torch.Tensor, feat_c0: torch.Ten
     S = feat_c1.shape[1]
     workspace = fine_level_workspace(M, WW, dev, workspace, transformer=False, dtype=win0.dtype)
     ids = (ptr(b_ids.contiguous()), ptr(i_ids.contiguous()), ptr(j_ids.contiguous()))
+    fn = lib().pope_fine_merge_coarse_f32_ex if f32 else lib().pope_fine_merge_coarse_ex
     with torch.cuda.device(dev):
-        if f32:
-            st = lib().pope_fine_merge_coarse_f32(ptr(win0), ptr(win1), M, WW, ptr(feat_c0), ptr(feat_c1), L, S, C_, *ids,
-                                                  ptr(packed_pre), ptr(workspace), workspace.numel(), stream_ptr(dev))
-        else:
-            st = lib().pope_fine_merge_coarse_ex(ptr(win0), ptr(win1), M, ptr(m_dev), WW, ptr(feat_c0), ptr(feat_c1), L, S,
-                                                 C_, *ids, ptr(packed_pre), ptr(workspace), workspace.numel(),
-                                                 stream_ptr(dev))
+        st = fn(ptr(win0), ptr(win1), M, ptr(m_dev), WW, ptr(feat_c0), ptr(feat_c1), L, S, C_, *ids, ptr(packed_pre),
+                ptr(workspace), workspace.numel(), stream_ptr(dev))
     check(st, "pope_fine_merge_coarse_f32" if f32 else "pope_fine_merge_coarse")
     return win0, win1
 
@@ -489,15 +494,23 @@ def fine_level_workspace(m: int, ww: int, dev, workspace: Optional[torch.Tensor]
     return workspace
 
 
-def _check_fine_level_inputs(feat_c0, feat_c1, feat_f0, feat_f1, W) -> None:
+def _fine_level_dtype(fine_level: dict) -> torch.dtype:
+    """The packing of a fine-level bundle (`Matcher.fine_level`): its "dtype" entry; a bundle without one is bf16."""
+    dt = fine_level.get("dtype", torch.bfloat16)
+    if dt not in (torch.bfloat16, torch.float32):
+        raise _lib.PopeError(f"a fine level is packed for torch.bfloat16 or torch.float32, not {dt}")
+    return dt
+
+
+def _check_fine_level_inputs(feat_c0, feat_c1, feat_f0, feat_f1, W, dtype) -> None:
     require_cuda(feat_c0, feat_c1, feat_f0, feat_f1)
-    if feat_c0.dtype != torch.bfloat16 or feat_c1.dtype != torch.bfloat16 or feat_c0.shape[-1] != 256:
-        raise _lib.PopeError("the bf16 fine level takes bfloat16 coarse features with C = 256")
-    if feat_f0.dtype != torch.bfloat16 or feat_f1.dtype != torch.bfloat16 or feat_f0.shape[1] != 128 \
-            or feat_f1.shape[1] != 128:
-        raise _lib.PopeError("the bf16 fine level takes bfloat16 fine maps with Cf = 128")
+    name = "bf16" if dtype == torch.bfloat16 else "fp32"
+    if feat_c0.dtype != dtype or feat_c1.dtype != dtype or feat_c0.shape[-1] != 256:
+        raise _lib.PopeError(f"the {name} fine level takes {dtype} coarse features with C = 256")
+    if feat_f0.dtype != dtype or feat_f1.dtype != dtype or feat_f0.shape[1] != 128 or feat_f1.shape[1] != 128:
+        raise _lib.PopeError(f"the {name} fine level takes {dtype} fine maps with Cf = 128")
     if W != 5:
-        raise _lib.PopeError("the bf16 fine level takes 5 x 5 windows")
+        raise _lib.PopeError(f"the {name} fine level takes 5 x 5 windows")
 
 
 def match_pairs_device(feat_c0, feat_c1, feat_f0, feat_f1, hw0_i, hw0_c, hw1_c, thr=0.2, border_rm=2,
@@ -514,9 +527,16 @@ def match_pairs_device(feat_c0, feat_c1, feat_f0, feat_f1, hw0_i, hw0_c, hw1_c, 
     takes the unfused route.  The result then also holds `fine_workspace` (pass it back in to reuse it).  Memory is sized
     by the capacity n * L, not by the match count: at 64 pairs x 480x640 (307 200 windows) that is 3.9 GB of windows plus
     9.8 GB of fine scratch per call, about 13.8 GB; the Matcher flow, sized by the count, needs about half of that at the
-    synthetic inputs' match rate."""
+    synthetic inputs' match rate.
+
+    `fine_level=Matcher.fine_level(device, dtype=torch.float32)`: the fp32-accuracy level instead (gather -> FinePreprocess
+    Linears -> fine transformer -> fine match, every launch bounded by the device count, no host sync), which computes what
+    `Matcher(config, fine_cuda_fp32=True)` computes, bit for bit on the live rows.  The bundle's dtype selects the level;
+    coarse features and fine maps must then both be float32 (any mix raises).  Its cost, from the workspace formulas (not
+    measured): at 64 pairs x 480x640 (307 200 windows) 7.9 GB of fp32 windows plus 37.4 GB of fine scratch per call."""
     if fine_level is not None:
-        _check_fine_level_inputs(feat_c0, feat_c1, feat_f0, feat_f1, W)
+        level_dtype = _fine_level_dtype(fine_level)
+        _check_fine_level_inputs(feat_c0, feat_c1, feat_f0, feat_f1, W, level_dtype)
         if fused_fine:
             raise _lib.PopeError("fine_level runs between window gather and fine matching: it takes the unfused route")
         fused_fine = False
@@ -531,11 +551,11 @@ def match_pairs_device(feat_c0, feat_c1, feat_f0, feat_f1, hw0_i, hw0_c, hw1_c, 
         win0, win1 = fine_gather(feat_f0, feat_f1, res["b_ids"], res["i_ids"], res["j_ids"], hw0_c[1], hw1_c[1],
                                  stride, W, m_dev)
         cap = win0.shape[0]
-        fine_workspace = fine_level_workspace(cap, W * W, win0.device, fine_workspace)
+        fine_workspace = fine_level_workspace(cap, W * W, win0.device, fine_workspace, dtype=level_dtype)
         if fine_level["pre"] is not None:
-            fine_merge_coarse(win0, win1, feat_c0.contiguous(), feat_c1.contiguous(), res["b_ids"], res["i_ids"],
-                              res["j_ids"], fine_level["pre"], fine_workspace, m_dev)
-        fine_transformer(win0, win1, fine_level["layers"], fine_level["layer_names"], fine_workspace, m_dev)
+            _fine_merge_coarse(win0, win1, feat_c0.contiguous(), feat_c1.contiguous(), res["b_ids"], res["i_ids"],
+                               res["j_ids"], fine_level["pre"], fine_workspace, m_dev)
+        _fine_transformer(win0, win1, fine_level["layers"], fine_level["layer_names"], fine_workspace, m_dev)
         expec, mk1f = fine_match(win0, win1, res["mkpts1_c"], coord_scale, m_dev)
         res.update(win0=win0, win1=win1, fine_workspace=fine_workspace)
     elif fused_fine:

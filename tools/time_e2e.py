@@ -4,7 +4,8 @@ after every copy has landed).  usage: python tools/time_e2e.py [pairs] [--chunks
 
 --fine-level: the same pipeline with and without the bf16 fine level of a random-init Matcher(fine_cuda_bf16=True)
 attached (pope_pipeline_set_fine_level), the two forms alternated run by run on the same handle and pinned buffers; also
-prints the GPU's name and power limit."""
+prints the GPU's name and power limit.  --dtype float32: fp32 features on an fp32 pipeline (with --fine-level, the
+fp32-accuracy level of Matcher(fine_cuda_fp32=True), pope_pipeline_set_fine_level_ex)."""
 import argparse
 import json
 import os
@@ -25,21 +26,23 @@ def main():
     ap.add_argument("--modes", default="union")
     ap.add_argument("--reps", type=int, default=4)
     ap.add_argument("--fine-level", action="store_true",
-                    help="time each chunk / mode with and without the bf16 fine level, alternating")
+                    help="time each chunk / mode with and without the fine level (of --dtype), alternating")
+    ap.add_argument("--dtype", choices=("bfloat16", "float32"), default="bfloat16")
     a = ap.parse_args()
+    a.dtype = getattr(torch, a.dtype)
     n, hc, wc = a.pairs, 60, 80
     L = hc * wc
-    f0, f1 = synth.coarse_features(1234, n, L, L, 256, dtype=torch.bfloat16)
+    f0, f1 = synth.coarse_features(1234, n, L, L, 256, dtype=a.dtype)
     g = torch.Generator().manual_seed(4321)
     driver.bind_host_to_gpu(0)
     h_f0, h_f1 = f0.pin_memory(), f1.pin_memory()
-    h_ff0 = torch.randn(n, hc * 4, wc * 4, 128, generator=g).to(torch.bfloat16).pin_memory()
-    h_ff1 = torch.randn(n, hc * 4, wc * 4, 128, generator=g).to(torch.bfloat16).pin_memory()
+    h_ff0 = torch.randn(n, hc * 4, wc * 4, 128, generator=g).to(a.dtype).pin_memory()
+    h_ff1 = torch.randn(n, hc * 4, wc * 4, 128, generator=g).to(a.dtype).pin_memory()
     if a.fine_level:
         return fine_level_rows(a, n, hc, wc, (h_f0, h_f1, h_ff0, h_ff1))
     rows = []
     for chunk in [int(c) for c in a.chunks.split(",")]:
-        pl = driver.Pipeline(torch.bfloat16, chunk, (480, 640), (hc, wc), (hc, wc), device=0)
+        pl = driver.Pipeline(a.dtype, chunk, (480, 640), (hc, wc), (hc, wc), device=0)
         out = pl.alloc_outputs(n)
         for mode in a.modes.split(","):
             os.environ["POPE_PIPELINE_F1"] = mode
@@ -61,10 +64,11 @@ def fine_level_rows(a, n, hc, wc, host):
                        capture_output=True, text=True)
     print(json.dumps({"gpu": q.stdout.strip() or q.stderr.strip()}), flush=True)
     torch.manual_seed(0)
-    matcher = pope_b200.Matcher(pope_b200.make_default_cfg(), fine_cuda_bf16=True).eval().to("cuda:0")
-    fl = matcher.fine_level(torch.device("cuda", 0))
+    f32 = a.dtype == torch.float32
+    matcher = pope_b200.Matcher(pope_b200.make_default_cfg(), fine_cuda_bf16=not f32, fine_cuda_fp32=f32).eval().to("cuda:0")
+    fl = matcher.fine_level(torch.device("cuda", 0), dtype=a.dtype)
     for chunk in [int(c) for c in a.chunks.split(",")]:
-        pl = driver.Pipeline(torch.bfloat16, chunk, (480, 640), (hc, wc), (hc, wc), device=0)
+        pl = driver.Pipeline(a.dtype, chunk, (480, 640), (hc, wc), (hc, wc), device=0)
         out = pl.alloc_outputs(n)
         for mode in a.modes.split(","):
             os.environ["POPE_PIPELINE_F1"] = mode
@@ -79,7 +83,8 @@ def fine_level_rows(a, n, hc, wc, host):
                     h2d[fine], matches[fine] = pl.last_h2d_bytes, int(out["counts"].sum())
             for fine in (False, True):
                 dt = sum(times[fine]) / len(times[fine])
-                print(json.dumps({"chunk": chunk, "mode": pl.last_f1_mode, "fine_level": fine, "ms": round(1e3 * dt, 3),
+                print(json.dumps({"dtype": str(a.dtype)[6:], "chunk": chunk, "mode": pl.last_f1_mode, "fine_level": fine,
+                                  "ms": round(1e3 * dt, 3),
                                   "ms_min_max": [round(1e3 * min(times[fine]), 3), round(1e3 * max(times[fine]), 3)],
                                   "pairs_per_s": round(n / dt, 1), "h2d_gb": round(h2d[fine] / 1e9, 4),
                                   "h2d_gbs": round(h2d[fine] / dt / 1e9, 2), "matches": matches[fine]}), flush=True)

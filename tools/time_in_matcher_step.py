@@ -1,13 +1,15 @@
 """Steps 3-5 of Matcher.forward (coarse match -> window gather -> FinePreprocess Linears -> fine transformer -> fine match)
-in bf16 on 64 pairs at 480x640, with the synthetic inputs of bench.py's `in_matcher_figure`, four ways (CUDA events after
-warm-up, one line of JSON):
-  (a) module      the Matcher(config, fine_cuda_bf16=True) modules: one host sync per step (the match count)
-  (b) device      ops.match_pairs_device(fine_level=Matcher.fine_level(dev)) on one stream, no host sync
+in bf16 (or, with `float32`, at fp32 accuracy) on 64 pairs at 480x640, with the synthetic inputs of bench.py's
+`in_matcher_figure`, four ways (CUDA events after warm-up, one line of JSON with each arm's peak
+torch.cuda.max_memory_allocated):
+  (a) module      the Matcher(config, fine_cuda_bf16=True) modules (fine_cuda_fp32=True for float32): one host sync per step
+                  (the match count)
+  (b) device      ops.match_pairs_device(fine_level=Matcher.fine_level(dev, dtype)) on one stream, no host sync
   (c) runner      driver.DeviceBatchRunner with two streams over the timed steps
   (d) graph       a CUDA graph of (b), replayed
 (b) is checked against (a) on the live rows, bit for bit.  All four run the same kernels, (b)-(d) in their forms bounded by
 the device match count on capacity-sized launches; (a) has the host sync instead.
-    python tools/time_in_matcher_step.py [pairs] [steps]"""
+    python tools/time_in_matcher_step.py [pairs] [steps] [bfloat16|float32]"""
 import json
 import os
 import subprocess
@@ -21,6 +23,9 @@ from pope_b200 import _lib, driver, ops, synth
 
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 64
 K = int(sys.argv[2]) if len(sys.argv) > 2 else 20
+DT = getattr(torch, sys.argv[3]) if len(sys.argv) > 3 else torch.bfloat16
+assert DT in (torch.bfloat16, torch.float32), DT
+F32 = DT == torch.float32
 dev = torch.device("cuda:0")
 H, W_IMG, HC, WC = 480, 640, 60, 80
 L = HC * WC
@@ -29,13 +34,13 @@ shapes = {"hw0_i": torch.Size([H, W_IMG]), "hw1_i": torch.Size([H, W_IMG]), "hw0
           "hw1_c": torch.Size([HC, WC]), "hw0_f": torch.Size([hf, wf]), "hw1_f": torch.Size([hf, wf]), "bs": n}
 
 torch.manual_seed(0)
-m = pope_b200.Matcher(pope_b200.make_default_cfg(), fine_cuda_bf16=True).eval().to(dev)
-f0, f1 = synth.coarse_features(99, n, L, L, 256, dtype=torch.bfloat16)
+m = pope_b200.Matcher(pope_b200.make_default_cfg(), fine_cuda_bf16=not F32, fine_cuda_fp32=F32).eval().to(dev)
+f0, f1 = synth.coarse_features(99, n, L, L, 256, dtype=DT)
 g = torch.Generator(device=dev).manual_seed(98)
-ff0 = torch.randn(n, hf, wf, 128, device=dev, generator=g).to(torch.bfloat16).permute(0, 3, 1, 2)
-ff1 = torch.randn(n, hf, wf, 128, device=dev, generator=g).to(torch.bfloat16).permute(0, 3, 1, 2)
+ff0 = torch.randn(n, hf, wf, 128, device=dev, generator=g).to(DT).permute(0, 3, 1, 2)
+ff1 = torch.randn(n, hf, wf, 128, device=dev, generator=g).to(DT).permute(0, 3, 1, 2)
 f0, f1 = f0.to(dev), f1.to(dev)
-fl = m.fine_level(dev)
+fl = m.fine_level(dev, dtype=DT)
 args = (f0, f1, ff0, ff1, (H, W_IMG), (HC, WC), (HC, WC))
 
 
@@ -50,8 +55,9 @@ def module_step():
     return data
 
 
-ws = torch.empty(_lib.lib().pope_coarse_workspace_bytes_ex(n, L, L, 256, _lib.POPE_BF16), dtype=torch.uint8, device=dev)
-fws = ops.fine_level_workspace(n * L, 25, dev)
+ws = torch.empty(_lib.lib().pope_coarse_workspace_bytes_ex(n, L, L, 256, _lib.dtype_code(f0)), dtype=torch.uint8,
+                 device=dev)
+fws = ops.fine_level_workspace(n * L, 25, dev, dtype=DT)
 
 
 def device_step():
@@ -59,6 +65,7 @@ def device_step():
 
 
 def timed(fn, warm=3):
+    torch.cuda.reset_peak_memory_stats(dev)
     for _ in range(warm):
         fn()
     torch.cuda.synchronize()
@@ -79,7 +86,10 @@ same = k == data["b_ids"].numel() and all(torch.equal(res[key][:k], data[key]) f
 same = same and all(torch.equal(res[key][:k].view(torch.int32), data[key].view(torch.int32)) for key in ("expec_f", "mkpts1_f"))
 del res, data
 
-out = {"module_ms": timed(module_step), "device_ms": timed(device_step)}
+out, peak = {}, {}
+for key, fn in (("module", module_step), ("device", device_step)):
+    out[key + "_ms"] = timed(fn)
+    peak[key] = torch.cuda.max_memory_allocated(dev)
 
 runner = driver.DeviceBatchRunner(dev, 2)
 
@@ -91,6 +101,7 @@ def runner_steps():
     runner.join()
 
 
+torch.cuda.reset_peak_memory_stats(dev)
 runner_steps()
 torch.cuda.synchronize()
 e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -99,6 +110,7 @@ runner_steps()
 e1.record()
 torch.cuda.synchronize()
 out["runner_ms"] = e0.elapsed_time(e1) / K
+peak["runner"] = torch.cuda.max_memory_allocated(dev)
 del runner
 torch.cuda.empty_cache()
 
@@ -112,6 +124,7 @@ graph = torch.cuda.CUDAGraph()
 with torch.cuda.graph(graph, stream=side):
     gres = device_step()
 out["graph_ms"] = timed(graph.replay)
+peak["graph"] = torch.cuda.max_memory_allocated(dev)
 graph_same = gres.total() == k
 
 try:
@@ -119,10 +132,12 @@ try:
                                  capture_output=True, text=True, check=True).stdout.strip().split(", ")
 except Exception:
     name, power = torch.cuda.get_device_name(dev), "unknown"
-line = {"workload": f"{n} pairs at 480x640, bf16, steps 3-5 of Matcher.forward incl. the fine level", "pairs": n,
+prec = "fp32 accuracy" if F32 else "bf16"
+line = {"workload": f"{n} pairs at 480x640, {prec}, steps 3-5 of Matcher.forward incl. the fine level", "pairs": n,
         "matches": k, "steps_timed": K, "card": name, "power_limit": power, "device_equals_module": bool(same),
         "graph_count_equal": bool(graph_same)}
 for key in ("module", "device", "runner", "graph"):
-    line[key] = {"ms_per_step": round(out[key + "_ms"], 4), "pairs_per_s": round(n / out[key + "_ms"] * 1e3)}
+    line[key] = {"ms_per_step": round(out[key + "_ms"], 4), "pairs_per_s": round(n / out[key + "_ms"] * 1e3),
+                 "peak_gb": round(peak[key] / 1e9, 2)}
 print(json.dumps(line))
 sys.exit(0 if same and graph_same else 1)
