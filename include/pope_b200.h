@@ -174,7 +174,9 @@ int pope_running_topk(const float* scores, int R, int k, float* slot_scores, int
  *             union | windows | bulk in the environment selects the form for image 1, see pope_pipeline_last_f1_mode;
  *             POPE_PIPELINE_WINDOWS_IN_PLACE=0 is the older spelling of bulk).  With a fine level attached
  *             (pope_pipeline_set_fine_level) the fine transformer needs all 25 pixels of image 0's windows, so image 0's
- *             map reaches the device in the same form as image 1's (a pageable image-0 buffer is copied whole).
+ *             map reaches the device in the same form as image 1's (a pageable image-0 buffer is copied whole).  With a
+ *             coarse level attached (pope_pipeline_set_coarse_level) feat_c0 / feat_c1 are the backbone's fp32 maps
+ *             [n,C,h0c,w0c] / [n,C,h1c,w1c] instead, whatever the pipeline's dtype.
  *   Outputs : per-pair slots of cap = min(L,S) entries: i_ids, j_ids int64[n][cap]; mconf float[n][cap];
  *             mkpts0_f, mkpts1_f float[n][cap][2]; counts int32[n]; flags (optional, may be NULL) int32[1] = OR of the
  *             POPE_FLAG_* bits of all chunks.  pope_pipeline_run returns after every copy has landed. */
@@ -228,6 +230,27 @@ int pope_pipeline_set_fine_level(pope_pipeline_t* pl, const void* pre, const voi
  * from the sizes).  Every form of the fine maps (union, windows, bulk) works with either level. */
 int pope_pipeline_set_fine_level_ex(pope_pipeline_t* pl, int dtype, const void* pre, const void* layers, int n_layers,
                                     const int* layer_kinds);
+/* Attach the coarse level (position encoding + coarse LoFTR transformer) to a pipeline, so that it starts where the
+ * backbone stops: from now on pope_pipeline_run's feat_c0 / feat_c1 are the backbone's coarse maps, host fp32
+ * [n, C, h0c, w0c] / [n, C, h1c, w1c] (contiguous) whatever the pipeline's dtype, and every chunk runs
+ *   copy the maps (fp32) -> pope_coarse_pos_encode_ex (to the pipeline's dtype) -> pope_coarse_transformer[_f32] -> coarse
+ *   match -> ... as before
+ * which is what Matcher(config, coarse_cuda_bf16=True) (POPE_BF16) or coarse_cuda_fp32=True (POPE_F32) computes after
+ * its backbone; the fine level, when attached, reads the transformed features.  The maps cross the link in fp32 (the
+ * encoding is added in fp32 before any rounding), 4 bytes per element in pope_pipeline_last_h2d_bytes.
+ * dtype names the packing of `layers` (pope_coarse_transformer / pope_coarse_transformer_f32 layouts) and must be the
+ * pipeline's dtype (POPE_ERR_DTYPE); pe: the encoding's [C, pe_h, pe_w] fp32 buffer (4-byte aligned), layers (16-byte
+ * aligned): device pointers on the pipeline's device, caller-owned and alive while the pipeline runs; layer_kinds[l] in
+ * {0 self, 1 cross}, copied.  Requires C == 256 and both coarse grids within pe_h x pe_w (POPE_ERR_SHAPE).
+ * layers == NULL detaches the level again: the pipeline then runs exactly as one that never had it.
+ * The first attach allocates, per slot, an fp32 staging buffer for one chunk's maps (chunk * (L + S) * C * 4 bytes) and,
+ * shared by both slots (it is touched on the compute stream only), one transformer scratch of
+ * pope_coarse_tf_workspace_bytes(chunk, L, S) (bf16) or pope_coarse_tf_f32_workspace_bytes(chunk, L, S) (fp32) bytes;
+ * pope_pipeline_destroy frees them.  Returns POPE_ERR_INVALID_ARG (null handle; layers without pe or layer_kinds, n_layers
+ * < 1, a non-positive pe_h / pe_w, a kind other than 0 / 1), POPE_ERR_DTYPE, POPE_ERR_SHAPE, POPE_ERR_ALIGNMENT, or a
+ * cudaError_t from an allocation. */
+int pope_pipeline_set_coarse_level(pope_pipeline_t* pl, int dtype, const void* pe, int pe_h, int pe_w, const void* layers,
+                                   int n_layers, const int* layer_kinds);
 
 /* One-shot convenience: create + run + destroy. */
 int pope_match_pairs_host(const void* feat_c0, const void* feat_c1, const void* feat_f0, const void* feat_f1,
@@ -495,6 +518,15 @@ int pope_coarse_transformer_f32(void* feat0, void* feat1, int64_t n_pairs, int L
  * bf16 (16-byte aligned).  C must be 256 and H <= pe_h, W <= pe_w (POPE_ERR_SHAPE); n == 0 is a no-op. */
 int pope_coarse_pos_encode(const void* feat, const void* pe, int64_t n, int C, int H, int W, int pe_h, int pe_w, void* out,
                            void* stream);
+
+/* pope_coarse_pos_encode with the output's element type: out_dtype = POPE_BF16 is pope_coarse_pos_encode itself;
+ * out_dtype = POPE_F32 writes out [n, H * W, C] fp32 (16-byte aligned),
+ *   out[b, y * W + x, c] = feat[b, c, y, x] + pe[c, y, x]      (one fp32 add, nothing rounded after it)
+ * which is bit for bit `(feat + pe[..., :H, :W]).flatten(2).transpose(1, 2)` in torch: the token-major input of
+ * pope_coarse_transformer_f32.  Any other out_dtype returns POPE_ERR_DTYPE; the other checks are those of
+ * pope_coarse_pos_encode.  pope_coarse_pos_encode(...) is pope_coarse_pos_encode_ex(..., POPE_BF16, stream). */
+int pope_coarse_pos_encode_ex(const void* feat, const void* pe, int64_t n, int C, int H, int W, int pe_h, int pe_w,
+                              void* out, int out_dtype, void* stream);
 
 #ifdef __cplusplus
 }

@@ -49,6 +49,7 @@ SIGNATURES = {
     "pope_coarse_tf_workspace_bytes": (_sz, [_i64, _i, _i]),
     "pope_coarse_transformer": (_i, [_p, _p, _i64, _i, _i, _p, _i, C.POINTER(_i), _p, _sz, _p]),
     "pope_coarse_pos_encode": (_i, [_p, _p, _i64, _i, _i, _i, _i, _i, _p, _p]),
+    "pope_coarse_pos_encode_ex": (_i, [_p, _p, _i64, _i, _i, _i, _i, _i, _p, _i, _p]),
     "pope_coarse_tf_f32_workspace_bytes": (_sz, [_i64, _i, _i]),
     "pope_coarse_transformer_f32": (_i, [_p, _p, _i64, _i, _i, _p, _i, C.POINTER(_i), _p, _sz, _p]),
     "pope_fine_tf_f32_workspace_bytes": (_sz, [_i64, _i]),
@@ -80,6 +81,7 @@ SIGNATURES = {
     "pope_pipeline_last_f1_mode": (_i, [_p]),
     "pope_pipeline_set_fine_level": (_i, [_p, _p, _p, _i, C.POINTER(_i)]),
     "pope_pipeline_set_fine_level_ex": (_i, [_p, _i, _p, _p, _i, C.POINTER(_i)]),
+    "pope_pipeline_set_coarse_level": (_i, [_p, _i, _p, _i, _i, _p, _i, C.POINTER(_i)]),
     "pope_match_pairs_host": (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _f, _f, _f, _f, _i, _i,
                                    _i, _i, _p, _p, _p, _p, _p, _p, _p]),
 }

@@ -467,12 +467,14 @@ coarse_attn_apply_kernel(const T* __restrict__ q, const float* __restrict__ kv, 
   }
 }
 
-// ---- position encoding + layout: out[b, y W + x, c] = bf16(feat[b, c, y, x] + pe[c, y, x]) ---------------------------
+// ---- position encoding + layout: out[b, y W + x, c] = T(feat[b, c, y, x] + pe[c, y, x]) ------------------------------
+// T = __nv_bfloat16 (one round to nearest even) or float (the fp32 sum itself)
 constexpr int kPePix = 32;
 
+template <typename T>
 __global__ void __launch_bounds__(256)
 coarse_pos_encode_kernel(const float* __restrict__ feat, const float* __restrict__ pe, int H, int W, int pe_h, int pe_w,
-                         __nv_bfloat16* __restrict__ out) {
+                         T* __restrict__ out) {
   __shared__ float tile[kPePix][kC + 1];
   const int b = blockIdx.y, p0 = blockIdx.x * kPePix, HW = H * W;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -483,10 +485,19 @@ coarse_pos_encode_kernel(const float* __restrict__ feat, const float* __restrict
       tile[lane][c] = feat[(size_t(b) * kC + c) * HW + p] + pe[(size_t(c) * pe_h + y) * pe_w + x];
   }
   __syncthreads();
-  for (int pp = warp; pp < kPePix && p0 + pp < HW; pp += 8) {   // write: lane = 8 channels of one token row
-    const float* r = &tile[pp][lane * 8];
-    *reinterpret_cast<uint4*>(out + (size_t(b) * HW + p0 + pp) * kC + lane * 8) =
-        make_uint4(pack_bf16(r[0], r[1]), pack_bf16(r[2], r[3]), pack_bf16(r[4], r[5]), pack_bf16(r[6], r[7]));
+  for (int pp = warp; pp < kPePix && p0 + pp < HW; pp += 8) {   // write one token row per warp
+    T* o = out + (size_t(b) * HW + p0 + pp) * kC;
+    if constexpr (sizeof(T) == 2) {                  // lane = 8 channels
+      const float* r = &tile[pp][lane * 8];
+      *reinterpret_cast<uint4*>(o + lane * 8) =
+          make_uint4(pack_bf16(r[0], r[1]), pack_bf16(r[2], r[3]), pack_bf16(r[4], r[5]), pack_bf16(r[6], r[7]));
+    } else {                                         // lane = 4 channels in each half of the row
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+        const float* r = &tile[pp][h * (kC / 2) + lane * 4];
+        *reinterpret_cast<float4*>(o + h * (kC / 2) + lane * 4) = make_float4(r[0], r[1], r[2], r[3]);
+      }
+    }
   }
 }
 
@@ -767,17 +778,30 @@ extern "C" int pope_coarse_transformer_f32(void* feat0, void* feat1, int64_t n_p
                                    stream);
 }
 
-extern "C" int pope_coarse_pos_encode(const void* feat, const void* pe, int64_t n, int C, int H, int W, int pe_h, int pe_w,
-                                      void* out, void* stream) {
+extern "C" int pope_coarse_pos_encode_ex(const void* feat, const void* pe, int64_t n, int C, int H, int W, int pe_h,
+                                         int pe_w, void* out, int out_dtype, void* stream) {
   if (!feat || !pe || !out) return POPE_ERR_INVALID_ARG;
   if (n < 0 || H <= 0 || W <= 0 || pe_h <= 0 || pe_w <= 0) return POPE_ERR_INVALID_ARG;
+  if (out_dtype != POPE_BF16 && out_dtype != POPE_F32) return POPE_ERR_DTYPE;
   if (C != kC || H > pe_h || W > pe_w) return POPE_ERR_SHAPE;
   if (((reinterpret_cast<uintptr_t>(feat) | reinterpret_cast<uintptr_t>(pe)) & 3u) || (reinterpret_cast<uintptr_t>(out) & 15u))
     return POPE_ERR_ALIGNMENT;
   if (int64_t(H) * W > 0x7fffffff - kPePix || n > 65535) return POPE_ERR_SHAPE;
   if (n == 0) return POPE_OK;
   const int hw = H * W;
-  coarse_pos_encode_kernel<<<dim3((hw + kPePix - 1) / kPePix, unsigned(n)), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-      static_cast<const float*>(feat), static_cast<const float*>(pe), H, W, pe_h, pe_w, static_cast<__nv_bfloat16*>(out));
+  const dim3 grid((hw + kPePix - 1) / kPePix, unsigned(n));
+  const float* f = static_cast<const float*>(feat);
+  const float* p = static_cast<const float*>(pe);
+  if (out_dtype == POPE_BF16)
+    coarse_pos_encode_kernel<__nv_bfloat16><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(
+        f, p, H, W, pe_h, pe_w, static_cast<__nv_bfloat16*>(out));
+  else
+    coarse_pos_encode_kernel<float><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(f, p, H, W, pe_h, pe_w,
+                                                                                          static_cast<float*>(out));
   return int(cudaGetLastError());
+}
+
+extern "C" int pope_coarse_pos_encode(const void* feat, const void* pe, int64_t n, int C, int H, int W, int pe_h, int pe_w,
+                                      void* out, void* stream) {
+  return pope_coarse_pos_encode_ex(feat, pe, n, C, H, W, pe_h, pe_w, out, POPE_BF16, stream);
 }

@@ -3,7 +3,8 @@
 // Replaces the batch-1 loop of the eval drivers (eval_linemod_json.py:103-122: three sequential matcher(batch)
 // calls per test pair, each followed by three .cpu() syncs) by a chunked, double-buffered stream pipeline:
 //   copy stream   : host -> device copies of chunk k+1
-//   compute stream: coarse match -> fused window gather + fine match -> per-pair slotting of chunk k (no host sync:
+//   compute stream: [with a coarse level attached (pope_pipeline_set_coarse_level): position encoding of the chunk's
+//                   backbone maps -> coarse transformer ->] coarse match -> fused window gather + fine match -> per-pair slotting of chunk k (no host sync:
 //                   the match count stays on the device and gates the fine kernels); with a fine level attached
 //                   (pope_pipeline_set_fine_level) coarse match -> window gather -> FinePreprocess Linears -> fine
 //                   transformer -> fine match -> slotting, every launch bounded by the same device count
@@ -139,6 +140,7 @@ struct Slot {
   int32_t* counts = nullptr;
   int32_t* h_counts = nullptr;   // pinned staging for the flag word
   uint8_t* cellmask = nullptr;   // [chunk, S] matched image-1 cells of the chunk (union fetch)
+  char* maps = nullptr;          // with a coarse level: the chunk's fp32 backbone maps [chunk, C, L] | [chunk, C, S]
   cudaEvent_t uploaded = nullptr, computed = nullptr, drained = nullptr;
 };
 
@@ -166,6 +168,16 @@ struct pope_pipeline {
   char *win0 = nullptr, *win1 = nullptr, *fine_ws = nullptr;
   size_t fine_ws_bytes = 0;
   uint8_t* cellmask0 = nullptr;              // [chunk, L] matched image-0 cells of the chunk (union fetch of image 0)
+  // the coarse level (pope_pipeline_set_coarse_level, in the pipeline's dtype): caller-owned encoding and packed layers;
+  // each slot's map staging buffer (Slot::maps) and one transformer scratch shared by both slots (touched on s_comp only)
+  // are allocated on the first attach
+  const void* coarse_pe = nullptr;
+  int pe_h = 0, pe_w = 0;
+  const void* coarse_layers = nullptr;
+  int coarse_n_layers = 0;
+  int* coarse_kinds = nullptr;               // host copy of layer_kinds
+  char* coarse_ws = nullptr;
+  size_t coarse_ws_bytes = 0;
 };
 
 #define PL_CUDA(x)                                   \
@@ -179,7 +191,7 @@ extern "C" int pope_pipeline_destroy(pope_pipeline_t* pl) {
   cudaSetDevice(pl->device);
   for (Slot& s : pl->slot) {
     void* bufs[] = {s.fc0, s.fc1, s.ff0, s.ff1, s.ws, s.b_ids, s.i_ids, s.j_ids, s.o_i, s.o_j, s.mconf,
-                    s.mk0, s.mk1, s.expec, s.mk1f, s.o_conf, s.o_mk0, s.o_mk1, s.counts, s.cellmask};
+                    s.mk0, s.mk1, s.expec, s.mk1f, s.o_conf, s.o_mk0, s.o_mk1, s.counts, s.cellmask, s.maps};
     for (void* b : bufs) if (b) cudaFree(b);
     if (s.h_counts) cudaFreeHost(s.h_counts);
     if (s.uploaded) cudaEventDestroy(s.uploaded);
@@ -188,9 +200,10 @@ extern "C" int pope_pipeline_destroy(pope_pipeline_t* pl) {
   }
   if (pl->fetched) cudaFree(pl->fetched);
   if (pl->h_fetched) cudaFreeHost(pl->h_fetched);
-  void* fine_bufs[] = {pl->win0, pl->win1, pl->fine_ws, pl->cellmask0};
+  void* fine_bufs[] = {pl->win0, pl->win1, pl->fine_ws, pl->cellmask0, pl->coarse_ws};
   for (void* b : fine_bufs) if (b) cudaFree(b);
   free(pl->fine_kinds);
+  free(pl->coarse_kinds);
   if (pl->s_copy) cudaStreamDestroy(pl->s_copy);
   if (pl->s_comp) cudaStreamDestroy(pl->s_comp);
   if (pl->s_drain) cudaStreamDestroy(pl->s_drain);
@@ -307,6 +320,52 @@ extern "C" int pope_pipeline_set_fine_level(pope_pipeline_t* pl, const void* pre
   return pope_pipeline_set_fine_level_ex(pl, POPE_BF16, pre, layers, n_layers, layer_kinds);
 }
 
+extern "C" int pope_pipeline_set_coarse_level(pope_pipeline_t* pl, int dtype, const void* pe, int pe_h, int pe_w,
+                                              const void* layers, int n_layers, const int* layer_kinds) {
+  if (!pl) return POPE_ERR_INVALID_ARG;
+  if (!layers) {                 // detach; the staging buffers and scratch stay allocated until pope_pipeline_destroy
+    pl->coarse_pe = pl->coarse_layers = nullptr;
+    pl->coarse_n_layers = 0;
+    return POPE_OK;
+  }
+  if (!pe || pe_h <= 0 || pe_w <= 0 || n_layers < 1 || !layer_kinds) return POPE_ERR_INVALID_ARG;
+  for (int l = 0; l < n_layers; ++l)
+    if (layer_kinds[l] != 0 && layer_kinds[l] != 1) return POPE_ERR_INVALID_ARG;
+  if (dtype != pl->dtype) return POPE_ERR_DTYPE;
+  if (pl->C != 256 || pl->h0c > pe_h || pl->w0c > pe_w || pl->h1c > pe_h || pl->w1c > pe_w) return POPE_ERR_SHAPE;
+  if ((reinterpret_cast<uintptr_t>(pe) & 3u) || (reinterpret_cast<uintptr_t>(layers) & 15u)) return POPE_ERR_ALIGNMENT;
+  const bool f32 = pl->dtype == POPE_F32;
+  const size_t tf = f32 ? pope_coarse_tf_f32_workspace_bytes(pl->chunk, pl->L, pl->S)
+                        : pope_coarse_tf_workspace_bytes(pl->chunk, pl->L, pl->S);
+  if (tf == 0) return POPE_ERR_SHAPE;
+  int rc = POPE_OK;
+  int* kinds = static_cast<int*>(malloc(sizeof(int) * size_t(n_layers)));
+  if (!kinds) return int(cudaErrorMemoryAllocation);
+  for (int l = 0; l < n_layers; ++l) kinds[l] = layer_kinds[l];
+  if (!pl->coarse_ws) {
+    // the maps cross the link in fp32 whatever the pipeline's dtype: the encoding is added in fp32 before any rounding
+    const size_t map_bytes = size_t(pl->chunk) * (pl->L + pl->S) * pl->C * sizeof(float);
+    PL_CUDA(cudaSetDevice(pl->device));
+    for (Slot& s : pl->slot) PL_CUDA(cudaMalloc(&s.maps, map_bytes));
+    PL_CUDA(cudaMalloc(&pl->coarse_ws, tf));
+    pl->coarse_ws_bytes = tf;
+  }
+  free(pl->coarse_kinds);
+  pl->coarse_kinds = kinds;
+  pl->coarse_pe = pe;
+  pl->pe_h = pe_h;
+  pl->pe_w = pe_w;
+  pl->coarse_layers = layers;
+  pl->coarse_n_layers = n_layers;
+  return POPE_OK;
+fail:
+  free(kinds);
+  for (Slot& s : pl->slot) { cudaFree(s.maps); s.maps = nullptr; }     // (cudaFree(NULL) is a no-op)
+  cudaFree(pl->coarse_ws);
+  pl->coarse_ws = nullptr;
+  return rc;
+}
+
 extern "C" int pope_pipeline_run(pope_pipeline_t* pl, const void* feat_c0, const void* feat_c1, const void* feat_f0,
                                  const void* feat_f1, int n_pairs, int64_t* i_ids, int64_t* j_ids, float* mconf,
                                  float* mkpts0_f, float* mkpts1_f, int32_t* counts, int32_t* flags) {
@@ -359,6 +418,10 @@ extern "C" int pope_pipeline_run(pope_pipeline_t* pl, const void* feat_c0, const
   // place, or (image 1 copied whole, or a pageable image-0 buffer) the whole map is copied.  (f0_union implies f1_union.)
   const bool fine = pl->fine_layers != nullptr;
   if (fine && !f1_dev_view) f0_dev_view = nullptr;
+  // With a coarse level, feat_c0 / feat_c1 are the backbone's fp32 maps [n, C, h, w]: they are staged in the slot and turned
+  // into the token-major transformed features s.fc0 / s.fc1 on the compute stream.
+  const bool coarse = pl->coarse_layers != nullptr;
+  const size_t in_c0_pair = coarse ? L * C * sizeof(float) : fc0_pair, in_c1_pair = coarse ? S * C * sizeof(float) : fc1_pair;
   const bool f0_union = fine && f1_union && f0_dev_view;
   int64_t h2d = 0;
   int32_t flag_acc = 0;
@@ -376,15 +439,29 @@ extern "C" int pope_pipeline_run(pope_pipeline_t* pl, const void* feat_c0, const
       PL_CUDA(cudaEventSynchronize(s.drained));
       flag_acc |= s.h_counts[pl->chunk + 1];
     }
-    PL_CUDA(cudaMemcpyAsync(s.fc0, static_cast<const char*>(feat_c0) + p0 * fc0_pair, n * fc0_pair, cudaMemcpyHostToDevice, pl->s_copy));
-    PL_CUDA(cudaMemcpyAsync(s.fc1, static_cast<const char*>(feat_c1) + p0 * fc1_pair, n * fc1_pair, cudaMemcpyHostToDevice, pl->s_copy));
+    char* dc0 = coarse ? s.maps : s.fc0;
+    char* dc1 = coarse ? s.maps + size_t(pl->chunk) * in_c0_pair : s.fc1;
+    PL_CUDA(cudaMemcpyAsync(dc0, static_cast<const char*>(feat_c0) + p0 * in_c0_pair, n * in_c0_pair, cudaMemcpyHostToDevice, pl->s_copy));
+    PL_CUDA(cudaMemcpyAsync(dc1, static_cast<const char*>(feat_c1) + p0 * in_c1_pair, n * in_c1_pair, cudaMemcpyHostToDevice, pl->s_copy));
     if (!f0_dev_view)
       PL_CUDA(cudaMemcpyAsync(s.ff0, static_cast<const char*>(feat_f0) + p0 * ff0_pair, n * ff0_pair, cudaMemcpyHostToDevice, pl->s_copy));
-    h2d += int64_t(n) * int64_t(fc0_pair + fc1_pair + (f1_dev_view ? 0 : ff1_pair) + (f0_dev_view ? 0 : ff0_pair));
+    h2d += int64_t(n) * int64_t(in_c0_pair + in_c1_pair + (f1_dev_view ? 0 : ff1_pair) + (f0_dev_view ? 0 : ff0_pair));
     if (!f1_dev_view)
       PL_CUDA(cudaMemcpyAsync(s.ff1, static_cast<const char*>(feat_f1) + p0 * ff1_pair, n * ff1_pair, cudaMemcpyHostToDevice, pl->s_copy));
     PL_CUDA(cudaEventRecord(s.uploaded, pl->s_copy));
     PL_CUDA(cudaStreamWaitEvent(pl->s_comp, s.uploaded, 0));
+    if (coarse) {
+      rc = pope_coarse_pos_encode_ex(dc0, pl->coarse_pe, n, int(C), pl->h0c, pl->w0c, pl->pe_h, pl->pe_w, s.fc0, pl->dtype,
+                                     pl->s_comp);
+      if (rc) goto fail;
+      rc = pope_coarse_pos_encode_ex(dc1, pl->coarse_pe, n, int(C), pl->h1c, pl->w1c, pl->pe_h, pl->pe_w, s.fc1, pl->dtype,
+                                     pl->s_comp);
+      if (rc) goto fail;
+      rc = (pl->dtype == POPE_F32 ? pope_coarse_transformer_f32 : pope_coarse_transformer)(
+          s.fc0, s.fc1, n, pl->L, pl->S, pl->coarse_layers, pl->coarse_n_layers, pl->coarse_kinds, pl->coarse_ws,
+          pl->coarse_ws_bytes, pl->s_comp);
+      if (rc) goto fail;
+    }
     rc = pope_coarse_match(s.fc0, s.fc1, pl->dtype, n, pl->L, pl->S, pl->C, pl->h0c, pl->w0c, pl->h1c, pl->w1c,
                            pl->pixel_scale, pl->temperature, pl->thr, pl->border, pl->impl, s.ws, pl->ws_bytes, s.b_ids,
                            s.i_ids, s.j_ids, s.mconf, s.mk0, s.mk1, s.counts, int64_t(capt), pl->s_comp);

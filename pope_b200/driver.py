@@ -56,6 +56,31 @@ def _check_fine_level(fine_level: dict, dtype: torch.dtype, C_coarse: int, devic
     return pre, layers, (C.c_int * len(names))(*[0 if nm == "self" else 1 for nm in names])
 
 
+def _check_coarse_level(coarse_level: dict, dtype: torch.dtype, C_coarse: int, device: int, hw0_c, hw1_c):
+    """What `pope_pipeline_set_coarse_level` needs, checked before any GPU call; returns its (pe, layers, kinds) arguments.
+    The bundle's packing (its "dtype") must be the pipeline's dtype."""
+    level = coarse_level.get("dtype")
+    if level != dtype:
+        raise _lib.PopeError(f"the coarse level is packed for {level}, the pipeline runs {dtype}: they must agree "
+                             f"(Matcher.coarse_level(device, dtype={dtype}))")
+    if C_coarse != 256:
+        raise _lib.PopeError("the coarse level needs a pipeline with C_coarse = 256")
+    per_layer = _lib.COARSE_TF_F32_LAYER_BYTES if dtype == torch.float32 else _lib.COARSE_TF_LAYER_BYTES
+    names, layers, pe = list(coarse_level["layer_names"]), coarse_level["layers"], coarse_level["pe"]
+    if not names or any(nm not in ("self", "cross") for nm in names) or layers.numel() != len(names) * per_layer:
+        raise _lib.PopeError("the coarse level's layer names and packed layers do not agree")
+    if pe.dtype != torch.float32 or pe.dim() != 4 or tuple(pe.shape[:2]) != (1, 256):
+        raise _lib.PopeError("the coarse level's position encoding must be the fp32 [1, 256, Hmax, Wmax] buffer")
+    for h, w in (hw0_c, hw1_c):
+        if h > pe.shape[2] or w > pe.shape[3]:
+            raise _lib.PopeError(f"a coarse grid of {(h, w)} is larger than the position encoding {tuple(pe.shape[2:])}")
+    dev = torch.device("cuda", device)
+    if layers.device != dev or layers.dtype != torch.uint8 or not layers.is_contiguous() or pe.device != dev \
+            or not pe.is_contiguous():
+        raise _lib.PopeError(f"the coarse level's tensors must be contiguous and on {dev} (Matcher.coarse_level({dev}))")
+    return pe, layers, (C.c_int * len(names))(*[0 if nm == "self" else 1 for nm in names])
+
+
 class Pipeline:
     """Owns one `pope_pipeline_t` (device slots + streams for one geometry).
 
@@ -66,12 +91,20 @@ class Pipeline:
     the handle; it allocates windows and fine scratch for one chunk (0.98 GB + 2.5 GB at 16 pairs of 480x640).
     An fp32 pipeline takes `Matcher.fine_level(device, dtype=torch.float32)`, the fp32-accuracy level: the results then
     equal the fp32 device step and `Matcher(config, fine_cuda_fp32=True)`; one chunk's fp32 windows and fine scratch are
-    1.97 GB + 9.3 GB at 16 pairs of 480x640 (computed from the sizes).  The bundle's packing must be the pipeline's dtype."""
+    1.97 GB + 9.3 GB at 16 pairs of 480x640 (computed from the sizes).  The bundle's packing must be the pipeline's dtype.
+
+    `coarse_level` (`Matcher.coarse_level(torch.device("cuda", device), dtype=<the pipeline's dtype>)`): the pipeline starts
+    where the backbone stops.  `run`'s feat_c0 / feat_c1 are then the backbone's coarse maps, CPU fp32 [n, 256, Hc, Wc]
+    whatever the pipeline's dtype (the encoding is added in fp32 before any rounding, so the maps cross the link in fp32,
+    counted at 4 bytes per element in `last_h2d_bytes`); every chunk adds the position encoding and runs the coarse
+    transformer before the coarse match.  With both levels the results equal the device step with both levels and thereby
+    `Matcher(config, coarse_cuda_X=True, fine_cuda_X=True)`.  The first attach allocates an fp32 staging buffer for one
+    chunk's maps per slot and one transformer scratch."""
 
     def __init__(self, dtype: torch.dtype, chunk_pairs: int, hw0_i: Sequence[int], hw0_c: Sequence[int],
                  hw1_c: Sequence[int], C_coarse: int = 256, C_fine: int = 128, fine_stride: int = 4, W: int = 5,
                  thr: float = 0.2, border_rm: int = 2, temperature: float = 0.1, impl: int = _lib.COARSE_AUTO,
-                 device: int = 0, fine_level: Optional[dict] = None):
+                 device: int = 0, fine_level: Optional[dict] = None, coarse_level: Optional[dict] = None):
         self.dtype, self.chunk, self.device = dtype, chunk_pairs, device
         self.hw0_c, self.hw1_c = tuple(hw0_c), tuple(hw1_c)
         self.L, self.S = hw0_c[0] * hw0_c[1], hw1_c[0] * hw1_c[1]
@@ -83,6 +116,8 @@ class Pipeline:
             raise _lib.PopeError(f"unsupported dtype {dtype}")
         if fine_level is not None:
             _check_fine_level(fine_level, dtype, C_coarse, device)
+        if coarse_level is not None:
+            _check_coarse_level(coarse_level, dtype, C_coarse, device, self.hw0_c, self.hw1_c)
         pixel_scale = hw0_i[0] / hw0_c[0]
         fine_scale = hw0_i[0] / (hw0_c[0] * fine_stride)
         st = lib().pope_pipeline_create(C.byref(self._h), device, code, chunk_pairs, C_coarse, C_fine,
@@ -90,13 +125,30 @@ class Pipeline:
                                         float(pixel_scale), float(fine_scale), float(temperature), float(thr),
                                         int(border_rm), int(impl))
         check(st, "pope_pipeline_create")
-        self.fine_level = None
-        if fine_level is not None:
-            try:
+        self.fine_level = self.coarse_level = None
+        try:
+            if fine_level is not None:
                 self.set_fine_level(fine_level)
-            except BaseException:
-                self.close()
-                raise
+            if coarse_level is not None:
+                self.set_coarse_level(coarse_level)
+        except BaseException:
+            self.close()
+            raise
+
+    def set_coarse_level(self, coarse_level: Optional[dict]) -> None:
+        """Attach a coarse level (see the class docstring) or, with None, detach it: the pipeline then takes token-major
+        coarse features again and returns what a pipeline created without one returns."""
+        if coarse_level is None:
+            check(lib().pope_pipeline_set_coarse_level(self._h, 0, None, 0, 0, None, 0, None), "pope_pipeline_set_coarse_level")
+            self.coarse_level = None
+            return
+        pe, layers, kinds = _check_coarse_level(coarse_level, self.dtype, self.C, self.device, self.hw0_c, self.hw1_c)
+        # the weights may have been packed just now on torch's stream, which the pipeline's own streams do not wait for
+        torch.cuda.current_stream(layers.device).synchronize()
+        code = _lib.POPE_F32 if self.dtype == torch.float32 else _lib.POPE_BF16
+        check(lib().pope_pipeline_set_coarse_level(self._h, code, pe.data_ptr(), pe.shape[2], pe.shape[3], layers.data_ptr(),
+                                                   len(kinds), kinds), "pope_pipeline_set_coarse_level")
+        self.coarse_level = coarse_level      # keeps the encoding and the packed tensors alive while the handle may read them
 
     def set_fine_level(self, fine_level: Optional[dict]) -> None:
         """Attach a fine level (see the class docstring) or, with None, detach it: the pipeline then returns what a pipeline
@@ -124,13 +176,20 @@ class Pipeline:
                 "flags": torch.zeros(1, dtype=torch.int32, **kw)}
 
     def run(self, feat_c0, feat_c1, feat_f0_nhwc, feat_f1_nhwc, out: Optional[Dict[str, torch.Tensor]] = None):
-        """Inputs: CPU tensors feat_c* [n,L|S,C], feat_f*_nhwc [n,Hf,Wf,Cf] (memory order), same dtype.  Outputs: per-pair
-        slots (`flatten_slots` packs them) holding what `ops.match_pairs_device` returns on the same inputs -- with the fine
-        level attached, what it returns with `fine_level=`."""
+        """Inputs: CPU tensors feat_c* [n,L|S,C], feat_f*_nhwc [n,Hf,Wf,Cf] (memory order), same dtype; with a coarse level
+        attached, feat_c* are fp32 maps [n,C,Hc,Wc] instead.  Outputs: per-pair slots (`flatten_slots` packs them) holding
+        what `ops.match_pairs_device` returns on the same inputs -- with the fine / coarse level attached, what it returns
+        with `fine_level=` / `coarse_level=`."""
         n = feat_c0.shape[0]
-        for t in (feat_c0, feat_c1, feat_f0_nhwc, feat_f1_nhwc):
+        for t in (feat_f0_nhwc, feat_f1_nhwc) + (() if self.coarse_level is not None else (feat_c0, feat_c1)):
             if t.dtype != self.dtype or not t.is_contiguous() or t.device.type != "cpu":
                 raise _lib.PopeError("pipeline inputs must be contiguous CPU tensors of the pipeline dtype")
+        if self.coarse_level is not None:
+            for t, hw in ((feat_c0, self.hw0_c), (feat_c1, self.hw1_c)):
+                if t.dtype != torch.float32 or not t.is_contiguous() or t.device.type != "cpu" \
+                        or tuple(t.shape) != (n, self.C) + hw:
+                    raise _lib.PopeError(f"with a coarse level the pipeline takes contiguous CPU fp32 coarse maps "
+                                         f"[{n}, {self.C}, {hw[0]}, {hw[1]}]")
         if out is None:
             out = self.alloc_outputs(n)
         st = lib().pope_pipeline_run(self._h, feat_c0.data_ptr(), feat_c1.data_ptr(), feat_f0_nhwc.data_ptr(),
@@ -155,15 +214,19 @@ class Pipeline:
 
 
 def match_pairs_host(feat_c0, feat_c1, feat_f0, feat_f1, hw0_i, hw0_c, hw1_c, chunk_pairs: int = 16, device: int = 0,
-                     fine_level: Optional[dict] = None, **kw) -> Dict[str, torch.Tensor]:
+                     fine_level: Optional[dict] = None, coarse_level: Optional[dict] = None, **kw) -> Dict[str, torch.Tensor]:
     """One-shot host-buffer entry: feat_f* are logical [N, Cf, Hf, Wf] CPU tensors (channels-last is free).  With
     `fine_level` (`Matcher.fine_level(torch.device("cuda", device))`) the results equal what
     `Matcher(config, fine_cuda_bf16=True)` computes from these features; with fp32 features and
     `Matcher.fine_level(torch.device("cuda", device), dtype=torch.float32)`, what `Matcher(config, fine_cuda_fp32=True)`
-    computes (see `Pipeline`)."""
+    computes (see `Pipeline`).  With `coarse_level` (`Matcher.coarse_level(torch.device("cuda", device), dtype)`) feat_c* are
+    the backbone's fp32 coarse maps [N, 256, Hc, Wc], the pipeline runs in the bundle's dtype (the fine maps must have it),
+    and with a fine level of that dtype the results equal `Matcher(config, coarse_cuda_X=True, fine_cuda_X=True)`."""
     n = feat_c0.shape[0]
-    pl = Pipeline(feat_c0.dtype, min(chunk_pairs, n), hw0_i, hw0_c, hw1_c, feat_c0.shape[2], feat_f0.shape[1],
-                  feat_f0.shape[2] // hw0_c[0], device=device, fine_level=fine_level, **kw)
+    dtype, C_coarse = ((coarse_level.get("dtype"), feat_c0.shape[1]) if coarse_level is not None
+                       else (feat_c0.dtype, feat_c0.shape[2]))
+    pl = Pipeline(dtype, min(chunk_pairs, n), hw0_i, hw0_c, hw1_c, C_coarse, feat_f0.shape[1],
+                  feat_f0.shape[2] // hw0_c[0], device=device, fine_level=fine_level, coarse_level=coarse_level, **kw)
     try:
         return pl.run(_pin(feat_c0), _pin(feat_c1), _fine_to_nhwc(feat_f0), _fine_to_nhwc(feat_f1))
     finally:
@@ -200,6 +263,7 @@ class DeviceBatchRunner:
                         else [torch.cuda.current_stream(self.device)])
         self.workspaces = [None] * len(self.streams)
         self.fine_workspaces = [None] * len(self.streams)
+        self.coarse_workspaces = [None] * len(self.streams)
         self._k = 0
         self._pending = []          # weak references to the results submitted since the last join()
 
@@ -222,24 +286,33 @@ class DeviceBatchRunner:
             res = ref()
             if res is not None and st != cur:
                 for key, v in res.items():
-                    if key not in ("workspace", "fine_workspace") and isinstance(v, torch.Tensor) and v.is_cuda:   # (the scratch stays with its stream)
+                    if key not in ("workspace", "fine_workspace", "coarse_workspace") and isinstance(v, torch.Tensor) \
+                            and v.is_cuda:   # (the scratch stays with its stream)
                         v.record_stream(cur)
         self._pending.clear()
 
-    def submit(self, feat_c0, feat_c1, feat_f0, feat_f1, hw0_i, hw0_c, hw1_c, after=None, fine_level=None, **kw):
+    def submit(self, feat_c0, feat_c1, feat_f0, feat_f1, hw0_i, hw0_c, hw1_c, after=None, fine_level=None,
+               coarse_level=None, **kw):
         """Queues one batch; returns (result, stream it was queued on).  `after(result)` runs inside the batch's stream
-        context (e.g. to append the batch's records to a job buffer)."""
+        context (e.g. to append the batch's records to a job buffer).  `coarse_level` (`Matcher.coarse_level(device,
+        dtype)`): feat_c0 / feat_c1 are the backbone's fp32 coarse maps and the batch also runs the position encoding and
+        the coarse transformer (see `ops.match_pairs_device`), in a coarse-transformer scratch kept per stream (from the
+        workspace formulas about 0.8 GB in bf16 and 3.0 GB in fp32 per stream at 64 pairs x 480x640)."""
         from . import ops
         k = self._k % len(self.streams)
         self._k += 1
         with torch.cuda.stream(self.streams[k]):
             if fine_level is not None:
                 kw.update(fine_level=fine_level, fine_workspace=self.fine_workspaces[k])
+            if coarse_level is not None:
+                kw.update(coarse_level=coarse_level, coarse_workspace=self.coarse_workspaces[k])
             res = ops.match_pairs_device(feat_c0, feat_c1, feat_f0, feat_f1, hw0_i, hw0_c, hw1_c,
                                          workspace=self.workspaces[k], **kw)
             self.workspaces[k] = res["workspace"]
             if fine_level is not None:
                 self.fine_workspaces[k] = res["fine_workspace"]
+            if coarse_level is not None:
+                self.coarse_workspaces[k] = res["coarse_workspace"]
             if after is not None:
                 after(res)
         if len(self._pending) >= 64:         # callers that never join(): forget the results that are gone

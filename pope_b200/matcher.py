@@ -109,6 +109,21 @@ class Matcher(nn.Module):
         return {"pre": pre, "layers": self.loftr_fine._packed_weights(dev, dtype),
                 "layer_names": list(self.loftr_fine.layer_names), "dtype": dtype}
 
+    def coarse_level(self, device, dtype: torch.dtype = torch.bfloat16) -> dict:
+        """The coarse level for `ops.match_pairs_device(..., coarse_level=...)` (and the driver's batched steps built on
+        it), which then starts from the backbone's fp32 coarse maps: {"pe": the position encoding's buffer on `device`,
+        "layers": the coarse transformer's packed layers, "layer_names": their 'self' / 'cross' schedule, "dtype": the
+        packing}.  dtype=torch.bfloat16 is what `coarse_cuda_bf16=True` runs, dtype=torch.float32 what `coarse_cuda_fp32=True`
+        runs.  The tensors are the modules' own caches (the buffer itself when it already lives on `device`; the packed
+        layers repacked only when a parameter changes)."""
+        if not self.loftr_coarse.cuda_supported():
+            raise NotImplementedError("the CUDA coarse transformer covers d_model 256 / 8 heads / linear attention")
+        from . import ops
+        ops._check_pack_dtype(dtype, "coarse level")
+        dev = torch.device(device)
+        return {"pe": self.pos_encoding.pe.to(dev), "layers": self.loftr_coarse._packed_weights(dev, dtype),
+                "layer_names": list(self.loftr_coarse.layer_names), "dtype": dtype}
+
     def forward(self, data: dict, only_att_fea: bool = False):
         img0, img1 = data["image0"], data["image1"]
         data.update({"bs": img0.size(0), "hw0_i": img0.shape[2:], "hw1_i": img1.shape[2:]})

@@ -344,10 +344,13 @@ def coarse_tf_workspace(n: int, L: int, S: int, dev, workspace: Optional[torch.T
     return workspace
 
 
-def coarse_pos_encode(feat: torch.Tensor, pe: torch.Tensor) -> torch.Tensor:
-    """PositionEncodingSine + flatten(2).transpose(1, 2) + .to(torch.bfloat16) in one kernel: feat [N, 256, H, W] fp32 ->
-    [N, H*W, 256] bf16, bit-identical to `(feat + pe[..., :H, :W]).flatten(2).transpose(1, 2).to(torch.bfloat16)`.
-    `pe`: the encoding's `pe` buffer [1, 256, Hmax, Wmax] fp32."""
+def coarse_pos_encode(feat: torch.Tensor, pe: torch.Tensor, dtype: torch.dtype = torch.bfloat16) -> torch.Tensor:
+    """PositionEncodingSine + flatten(2).transpose(1, 2) + .to(dtype) in one kernel: feat [N, 256, H, W] fp32 ->
+    [N, H*W, 256] contiguous, bit-identical to `(feat + pe[..., :H, :W]).flatten(2).transpose(1, 2).to(dtype)`.
+    dtype=torch.bfloat16 (the input of the bf16 coarse transformer) or torch.float32 (the fp32 sum itself, the input of the
+    fp32-accuracy one).  `pe`: the encoding's `pe` buffer [1, 256, Hmax, Wmax] fp32."""
+    if dtype not in (torch.bfloat16, torch.float32):
+        raise _lib.PopeError(f"coarse_pos_encode writes torch.bfloat16 or torch.float32, not {dtype}")
     dev = require_cuda(feat, pe)
     if feat.dtype != torch.float32 or pe.dtype != torch.float32 or feat.dim() != 4 or pe.dim() != 4 or pe.shape[0] != 1:
         raise _lib.PopeError("coarse_pos_encode takes an fp32 [N, C, H, W] map and the fp32 [1, C, Hmax, Wmax] encoding")
@@ -355,9 +358,10 @@ def coarse_pos_encode(feat: torch.Tensor, pe: torch.Tensor) -> torch.Tensor:
         raise _lib.PopeError("the encoding and the map differ in channels")
     feat, pe = feat.contiguous(), pe.contiguous()
     n, c, h, w = feat.shape
-    out = torch.empty(n, h * w, c, dtype=torch.bfloat16, device=dev)
+    out = torch.empty(n, h * w, c, dtype=dtype, device=dev)
     with torch.cuda.device(dev):
-        st = lib().pope_coarse_pos_encode(ptr(feat), ptr(pe), n, c, h, w, pe.shape[2], pe.shape[3], ptr(out), stream_ptr(dev))
+        st = lib().pope_coarse_pos_encode_ex(ptr(feat), ptr(pe), n, c, h, w, pe.shape[2], pe.shape[3], ptr(out),
+                                             dtype_code(out), stream_ptr(dev))
     check(st, "pope_coarse_pos_encode")
     return out
 
@@ -502,10 +506,11 @@ def _fine_level_dtype(fine_level: dict) -> torch.dtype:
     return dt
 
 
-def _check_fine_level_inputs(feat_c0, feat_c1, feat_f0, feat_f1, W, dtype) -> None:
+def _check_fine_level_inputs(feat_c0, feat_c1, feat_f0, feat_f1, W, dtype, coarse_features: bool = True) -> None:
+    """`coarse_features=False`: feat_c0 / feat_c1 are backbone maps that a coarse level turns into the features."""
     require_cuda(feat_c0, feat_c1, feat_f0, feat_f1)
     name = "bf16" if dtype == torch.bfloat16 else "fp32"
-    if feat_c0.dtype != dtype or feat_c1.dtype != dtype or feat_c0.shape[-1] != 256:
+    if coarse_features and (feat_c0.dtype != dtype or feat_c1.dtype != dtype or feat_c0.shape[-1] != 256):
         raise _lib.PopeError(f"the {name} fine level takes {dtype} coarse features with C = 256")
     if feat_f0.dtype != dtype or feat_f1.dtype != dtype or feat_f0.shape[1] != 128 or feat_f1.shape[1] != 128:
         raise _lib.PopeError(f"the {name} fine level takes {dtype} fine maps with Cf = 128")
@@ -513,9 +518,38 @@ def _check_fine_level_inputs(feat_c0, feat_c1, feat_f0, feat_f1, W, dtype) -> No
         raise _lib.PopeError(f"the {name} fine level takes 5 x 5 windows")
 
 
+def _check_coarse_level(coarse_level: dict, fine_level: Optional[dict], feat_c0, feat_c1, hw0_c, hw1_c) -> torch.dtype:
+    """What the coarse level of the step needs, checked before any launch; returns the bundle's dtype."""
+    dt = coarse_level.get("dtype")
+    if dt not in (torch.bfloat16, torch.float32):
+        raise _lib.PopeError(f"a coarse level is packed for torch.bfloat16 or torch.float32, not {dt}")
+    if fine_level is not None and _fine_level_dtype(fine_level) != dt:
+        raise _lib.PopeError(f"a coarse level of {dt} with a fine level of {_fine_level_dtype(fine_level)}: the step runs "
+                             "both levels in one dtype")
+    pe, layers, names = coarse_level["pe"], coarse_level["layers"], list(coarse_level["layer_names"])
+    for t in (feat_c0, feat_c1):
+        if t.dtype != torch.float32 or t.dim() != 4:
+            raise _lib.PopeError("with a coarse level, feat_c0 / feat_c1 are the backbone's fp32 maps [N, 256, Hc, Wc]")
+        if t.shape[1] != 256:
+            raise _lib.PopeError(f"the coarse level takes maps with C = 256, not {t.shape[1]}")
+    if feat_c0.shape[0] != feat_c1.shape[0]:
+        raise _lib.PopeError("feat_c0 and feat_c1 hold different numbers of pairs")
+    for t, hw in ((feat_c0, hw0_c), (feat_c1, hw1_c)):
+        if tuple(t.shape[2:]) != (int(hw[0]), int(hw[1])):
+            raise _lib.PopeError(f"a coarse map of grid {tuple(t.shape[2:])} with hw_c = {tuple(hw)}")
+        if pe.dim() != 4 or pe.shape[1] != 256 or t.shape[2] > pe.shape[2] or t.shape[3] > pe.shape[3]:
+            raise _lib.PopeError(f"a coarse grid of {tuple(t.shape[2:])} is larger than the position encoding "
+                                 f"{tuple(pe.shape[2:])}")
+    per_layer = _lib.COARSE_TF_F32_LAYER_BYTES if dt == torch.float32 else _lib.COARSE_TF_LAYER_BYTES
+    if not names or any(nm not in ("self", "cross") for nm in names) or layers.numel() != len(names) * per_layer:
+        raise _lib.PopeError("the coarse level's layer names and packed layers do not agree")
+    require_cuda(feat_c0, feat_c1, pe, layers)
+    return dt
+
+
 def match_pairs_device(feat_c0, feat_c1, feat_f0, feat_f1, hw0_i, hw0_c, hw1_c, thr=0.2, border_rm=2,
                        temperature=0.1, W=5, impl=_lib.COARSE_AUTO, workspace=None, fused_fine=None, fine_level=None,
-                       fine_workspace=None) -> CoarseResult:
+                       fine_workspace=None, coarse_level=None, coarse_workspace=None) -> CoarseResult:
     """The hot path on device-resident inputs with NO host synchronisation: coarse match -> window gather ->
     fine match, the match count staying on the device (`m_dev`).  Returns the capacity-sized CoarseResult
     extended with `expec_f`, `mkpts0_f`, `mkpts1_f` (and `win0`, `win1` on the unfused route).
@@ -533,14 +567,36 @@ def match_pairs_device(feat_c0, feat_c1, feat_f0, feat_f1, hw0_i, hw0_c, hw1_c, 
     Linears -> fine transformer -> fine match, every launch bounded by the device count, no host sync), which computes what
     `Matcher(config, fine_cuda_fp32=True)` computes, bit for bit on the live rows.  The bundle's dtype selects the level;
     coarse features and fine maps must then both be float32 (any mix raises).  Its cost, from the workspace formulas (not
-    measured): at 64 pairs x 480x640 (307 200 windows) 7.9 GB of fp32 windows plus 37.4 GB of fine scratch per call."""
+    measured): at 64 pairs x 480x640 (307 200 windows) 7.9 GB of fp32 windows plus 37.4 GB of fine scratch per call.
+
+    `coarse_level` (`Matcher.coarse_level(device, dtype)`): start where the backbone stops.  feat_c0 / feat_c1 are then the
+    backbone's fp32 coarse maps [N, 256, Hc, Wc] with (Hc, Wc) = hw0_c / hw1_c; the step adds the position encoding and lays
+    them out token-major in the bundle's dtype (`coarse_pos_encode`), runs the coarse transformer on them in place
+    (`coarse_transformer`), and continues as above on the transformed features -- what
+    `Matcher(config, coarse_cuda_bf16=True)` (bf16 bundle) or `coarse_cuda_fp32=True` (fp32 bundle) computes after its
+    backbone, bit for bit, still without a host sync.  The result also holds `feat_c0` / `feat_c1` (the transformed
+    features, what `Matcher.forward(data, only_att_fea=True)` returns) and `coarse_workspace` (pass it back in to reuse
+    it; from the workspace formulas about 0.8 GB in bf16 and 3.0 GB in fp32 at 64 pairs x 480x640, not measured).  A
+    coarse level goes alone or with a fine level of the same dtype; any other mix, maps that are not fp32 4-D, C != 256,
+    a grid other than hw_c or larger than the encoding raise `PopeError` before any launch."""
+    coarse_dtype = None
+    if coarse_level is not None:
+        coarse_dtype = _check_coarse_level(coarse_level, fine_level, feat_c0, feat_c1, hw0_c, hw1_c)
     if fine_level is not None:
         level_dtype = _fine_level_dtype(fine_level)
-        _check_fine_level_inputs(feat_c0, feat_c1, feat_f0, feat_f1, W, level_dtype)
+        _check_fine_level_inputs(feat_c0, feat_c1, feat_f0, feat_f1, W, level_dtype, coarse_features=coarse_dtype is None)
         if fused_fine:
             raise _lib.PopeError("fine_level runs between window gather and fine matching: it takes the unfused route")
         fused_fine = False
+    if coarse_level is not None:
+        feat_c0 = coarse_pos_encode(feat_c0, coarse_level["pe"], coarse_dtype)
+        feat_c1 = coarse_pos_encode(feat_c1, coarse_level["pe"], coarse_dtype)
+        coarse_workspace = coarse_tf_workspace(feat_c0.shape[0], feat_c0.shape[1], feat_c1.shape[1], feat_c0.device,
+                                               coarse_workspace, dtype=coarse_dtype)
+        coarse_transformer(feat_c0, feat_c1, coarse_level["layers"], coarse_level["layer_names"], coarse_workspace)
     res = coarse_match(feat_c0, feat_c1, hw0_c, hw1_c, hw0_i[0] / hw0_c[0], thr, border_rm, temperature, impl, workspace)
+    if coarse_level is not None:
+        res.update(feat_c0=feat_c0, feat_c1=feat_c1, coarse_workspace=coarse_workspace)
     n = res["n_pairs"]
     m_dev = res["counts"][n:n + 1]
     stride = feat_f0.shape[2] // hw0_c[0]
